@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our CUDA path
     python bench.py --impl reference --gpus N ...             # the reference algorithm on the host CPUs
+    python bench.py ... --dump-outputs DIR                    # also save a sample of the last step's records
 
 Workload (config.workload): a UniProt-like synthetic proteome (SURVEY.md section 8(d), config 4:
 100M proteins / ~35G residues over 8 GPUs), 12.5M proteins per GPU, generated ON DEVICE with
@@ -36,6 +37,8 @@ B_FIXED_PER_PROT = 168.0  # 160 B record + 8 B offset per protein; + 1 B per res
 SEED = 1004          # config 4
 LN_MEDIAN, SIGMA, MIN_LEN, MAX_LEN = math.log(290.0), 0.62, 16, 40000
 PRD_RATE, X_RATE = 0.05, 1e-4
+# 27 record fields + the protein index in float64, 13 non-finite classes in float32: 55.2 MB at most
+DUMP_PROTEINS, DUMP_SEED = 200_000, 0
 
 BG_SCER = [0, 0.0550, 0.0126, 0.0586, 0.0655, 0.0441, 0.0498, 0.0217, 0.0655, 0.0735, 0.0950, 0.0207,
            0.0615, 0.0438, 0.0396, 0.0444, 0.0899, 0.0592, 0.0556, 0.0104, 0.0337, 0]
@@ -43,10 +46,17 @@ PRD_28 = [0, 0.04865, 0.00219, 0.01638, 0.00783, 0.02537, 0.07603, 0.0181, 0.020
           0.02975, 0.25885, 0.05126, 0.15178, 0.025, 0.10988, 0.03841, 0.01972, 0.00157, 0.05624, 0]
 
 
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError(f"must be at least 1, got {v}")
+    return v
+
+
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=positive_int, default=5, help="timed steps")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--proteins-per-gpu", type=int, default=12_500_000)
@@ -58,6 +68,10 @@ def parse():
     ap.add_argument("--no-per-residue", action="store_true", help="skip the config-2 (per-residue mode) side measurement")
     ap.add_argument("--no-extras", action="store_true",
                     help="skip the config-5 (long sequences) and ranking side measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the records of the last timed step (rank 0's shard, a fixed sample of at most "
+                         f"{DUMP_PROTEINS} proteins) as DIR/<field>.npy in float64, with DIR/protein_index.npy; "
+                         "NaN and infinities are written as 0 and marked in DIR/<field>_nonfinite.npy")
     return ap.parse_args()
 
 
@@ -258,7 +272,6 @@ def main():
         return
 
     # (NCCL_DEBUG is left as the launcher set it: whatever NCCL prints on fd 1 goes to stderr, see claim_stdout)
-    import numpy as np
     import torch
     import torch.distributed as dist
 
@@ -275,20 +288,7 @@ def main():
     nprot = args.proteins_per_gpu
     first = rank * nprot
 
-    # ---- synthetic shard, generated on device -------------------------------------------------
-    lens = torch.empty(nprot, dtype=torch.int64, device=dev)
-    rc = L.plaac_bench_synth_lengths(None, SEED, first, nprot, LN_MEDIAN, SIGMA, MIN_LEN, MAX_LEN, lens.data_ptr())
-    assert rc == 0
-    offsets = torch.zeros(nprot + 1, dtype=torch.int64, device=dev)
-    torch.cumsum(lens, 0, out=offsets[1:])
-    ntotal = int(offsets[-1].item())
-    del lens
-    codes = torch.empty(ntotal + 64, dtype=torch.uint8, device=dev)
-    bg = np.array(BG_SCER, dtype=np.float64)
-    prd = np.array(PRD_28, dtype=np.float64)
-    rc = L.plaac_bench_synth_residues(None, SEED, first, nprot, offsets.data_ptr(), bg.ctypes.data, prd.ctypes.data,
-                                      PRD_RATE, X_RATE, codes.data_ptr())
-    assert rc == 0
+    codes, offsets, ntotal = synth_shard(L, dev, first, nprot)
     summaries = torch.empty(nprot * 160, dtype=torch.uint8, device=dev)
     torch.cuda.synchronize()
 
@@ -335,6 +335,8 @@ def main():
     else:
         t_max, res_total = float(t_rank[0]), float(ntotal)
     value = res_total * args.steps / t_max
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, summaries, first, nprot)
 
     # ---- roofline of the dominant kernel (rank-local) ---------------------------------------------
     kern_ms = sum(score_ms) / len(score_ms)
@@ -444,6 +446,55 @@ def main():
     scorer.close()
     if world > 1:
         dist.destroy_process_group()
+
+
+def synth_shard(L, dev, first, nprot):
+    """Proteins first .. first+nprot-1 of the synthetic proteome, generated on device: (codes, offsets, residues).
+    codes carries 64 bytes of padding after the last residue."""
+    import numpy as np
+    import torch
+
+    lens = torch.empty(nprot, dtype=torch.int64, device=dev)
+    rc = L.plaac_bench_synth_lengths(None, SEED, first, nprot, LN_MEDIAN, SIGMA, MIN_LEN, MAX_LEN, lens.data_ptr())
+    assert rc == 0
+    offsets = torch.zeros(nprot + 1, dtype=torch.int64, device=dev)
+    torch.cumsum(lens, 0, out=offsets[1:])
+    ntotal = int(offsets[-1].item())
+    del lens
+    codes = torch.empty(ntotal + 64, dtype=torch.uint8, device=dev)
+    bg = np.array(BG_SCER, dtype=np.float64)
+    prd = np.array(PRD_28, dtype=np.float64)
+    rc = L.plaac_bench_synth_residues(None, SEED, first, nprot, offsets.data_ptr(), bg.ctypes.data, prd.ctypes.data,
+                                      PRD_RATE, X_RATE, codes.data_ptr())
+    assert rc == 0
+    return codes, offsets, ntotal
+
+
+def dump_outputs(out_dir, summaries, first, nprot):
+    """The 160-byte records in `summaries` (device) of a fixed, seeded sample of the shard's proteins, one float64 array
+    per record field, and the global index of each sampled protein; the same arguments give the same sample.
+    Every array written is finite: a record holds NaN where a score is undefined (core_score without a CORE, for one)
+    and -Inf as the LLR of a protein shorter than the core, so each double field is written with those entries as 0
+    and, beside it,
+    <field>_nonfinite (0 finite, 1 NaN, 2 +Inf, 3 -Inf)."""
+    import numpy as np
+    import torch
+
+    import plaac_b200
+
+    n = min(nprot, DUMP_PROTEINS)
+    pick = np.sort(np.random.default_rng(DUMP_SEED).choice(nprot, size=n, replace=False))
+    rows = summaries.view(nprot, 160)[torch.from_numpy(pick).to(summaries.device)]
+    rec = rows.cpu().numpy().reshape(-1).view(plaac_b200.SUMMARY_DTYPE)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "protein_index.npy"), (first + pick).astype(np.float64))
+    for name in plaac_b200.SUMMARY_DTYPE.names:
+        v = rec[name].astype(np.float64)
+        if rec.dtype[name].kind == "f":
+            cls = np.select([np.isnan(v), v == np.inf, v == -np.inf], [1, 2, 3], 0).astype(np.float32)
+            np.save(os.path.join(out_dir, name + "_nonfinite.npy"), cls)
+            v[cls != 0] = 0.0
+        np.save(os.path.join(out_dir, name + ".npy"), v)
 
 
 def measure_e2e(args, scorer, dev, world, barrier, codes, offsets, summaries, nprot, ntotal, res_total):

@@ -28,6 +28,38 @@ def proteome(nprot, seed, median=407.0, sigma=0.66, min_len=16, max_len=40000, p
     return codes, offsets
 
 
+def repeat_proteome(nprot, seed):
+    """Yeast-like proteins whose Q/N-rich parts repeat, as real prion domains do, so that several windows of the
+    60-residue LLR and CORE searches have the same composition: in turn a block and a copy of it, a block and a
+    permutation of it, and an oligopeptide repeat.  Which of such windows the reference picks is decided by the
+    rounding of its running sums (over the -1e6 mask outside the PrD for the CORE)."""
+    rng = np.random.default_rng(seed)
+    bg, prd = BG_SCER / BG_SCER.sum(), PRD_28 / PRD_28.sum()
+    seqs = []
+    for i in range(nprot):
+        n = int(np.clip(np.rint(rng.lognormal(np.log(407.0), 0.66)), 200, 4000))
+        s = rng.choice(22, size=n, p=bg).astype(np.uint8)
+        if i % 3 == 0:
+            w = rng.choice(22, size=int(rng.integers(60, 81)), p=prd).astype(np.uint8)
+            a, b = np.sort(rng.choice(n - len(w), size=2, replace=False))
+            s[a:a + len(w)] = w
+            s[b:b + len(w)] = w
+        elif i % 3 == 1:
+            w = rng.choice(22, size=60, p=prd).astype(np.uint8)
+            a, b = np.sort(rng.choice(n - 60, size=2, replace=False))
+            s[a:a + 60] = w
+            s[b:b + 60] = rng.permutation(w)
+        else:
+            m = rng.choice(22, size=int(rng.integers(4, 12)), p=prd).astype(np.uint8)
+            a = int(rng.integers(0, n - 80))
+            s[a:a + 80] = np.resize(m, 80)
+        seqs.append(s)
+    lens = np.array([len(x) for x in seqs], dtype=np.int64)
+    offsets = np.zeros(nprot + 1, dtype=np.int64)
+    np.cumsum(lens, out=offsets[1:])
+    return np.concatenate(seqs), offsets
+
+
 def edge_cases(seed=7):
     """Ragged / degenerate inputs: n = 1..3, around the window (20/21/40/41/42) and core
     (59/60/61) and MW (79/80/81) sizes, all-X, poly-Q, poly-P (PAPA proline rule), stop codons inside."""

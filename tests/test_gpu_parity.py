@@ -228,27 +228,37 @@ def test_other_parameters(kw):
     _check(got, ref, str(kw), P, codes, offs, max_ties=6)
 
 
-def test_real_yeast_proteome_if_staged(scorer):
-    """cli/example/Scer.fasta of the reference (staged into oracle/_ref by build(); not in git)."""
-    path = os.path.join(ROOT, "oracle", "_ref", "Scer.fasta")
-    if not os.path.exists(path):
-        pytest.skip("oracle/_ref/Scer.fasta not staged")
-    seqs, cur = [], None
-    for line in open(path):
-        line = line.rstrip("\r\n")
-        if line.startswith(">"):
-            cur = []
-            seqs.append(cur)
-        elif not line:
-            cur = None
-        elif cur is not None:
-            cur.append(line)
-    seqs = [plaac_b200.encode("".join(s)) for s in seqs]
-    codes, offs = plaac_b200.pack(seqs)
+def _composition_ties(codes, offs, starts, width=60):
+    """(proteins whose chosen window has a composition-identical twin, those where the choice is not the earliest twin)"""
+    tied = later = 0
+    for i in range(len(offs) - 1):
+        s, st = codes[offs[i]:offs[i + 1]], int(starts[i])
+        if st < 0:
+            continue
+        cum = np.zeros((len(s) + 1, 22), np.int32)
+        cum[np.arange(1, len(s) + 1), s] = 1
+        cum = cum.cumsum(0)
+        comp = cum[width:] - cum[:-width]
+        twins = np.nonzero((comp == comp[st]).all(1))[0]
+        tied += len(twins) > 1
+        later += bool(twins[0] < st)
+    return tied, later
+
+
+def test_composition_identical_best_windows(scorer):
+    """Proteins with repeated Q/N-rich blocks (tests/synth.py repeat_proteome): many have several best LLR and CORE
+    windows of identical composition, and the reference picks the one its running sums round highest -- often not the
+    earliest, and for the CORE over sums polluted by the -1e6 mask.  LLR and CORE positions and scores must match the
+    oracle exactly.  A copied block can also put two PAPA centres on a plateau equal to the last bit: the PAPA fields
+    are held to the documented tie-class rule, for at most two proteins."""
+    codes, offs = synth.repeat_proteome(1500, seed=2024)
     got = scorer.score(codes, offs)
-    ref = orc.score_batch(orc.make_params(), codes, offs, nthreads=NT)
-    _check(got, ref, "Scer.fasta")
-    assert len(seqs) > 5000
+    P = orc.make_params()
+    ref = orc.score_batch(P, codes, offs, nthreads=NT)
+    _check(got, ref, "composition-identical best windows", P, codes, offs, max_ties=2)
+    for f in ("llr_start", "core_start"):
+        tied, later = _composition_ties(codes, offs, ref[f])
+        assert tied > 300 and later > 100, (f, tied, later)
 
 
 def test_chunked_host_path_and_permutation_invariance(scorer):

@@ -1,6 +1,5 @@
 """GPU FASTA ingest (N2) and background counts (N3) against a Python restatement of the jar's reader
 (fastareader plaac.java:4302-4375, string2aa :1764, '*' strip :758, computeaafreq/isvalidprotein :1655-1739)."""
-import os
 import re
 import subprocess
 
@@ -146,14 +145,3 @@ def test_ingest_matches_host_cli_background_counts(scorer, tmp_path):
     got = scorer.ingest_fasta(data, bg_counts=True)
     assert got["bg_counts"].tolist() == cli_counts
 
-
-def test_ingest_real_yeast_proteome_if_staged(scorer):
-    path = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "Scer.fasta")
-    if not os.path.exists(path):
-        pytest.skip("oracle/_ref/Scer.fasta not staged")
-    data = open(path, "rb").read()
-    got = scorer.ingest_fasta(data, bg_counts=True)
-    names, codes, offs, counts = expected(data)
-    assert len(names) > 5000 and got["names"] == names
-    assert got["offsets"].tolist() == offs.tolist() and (got["codes"] == codes).all()
-    assert got["bg_counts"].tolist() == counts.tolist()
