@@ -288,22 +288,24 @@ void plaac_encode_host(const char *chars, int64_t n, uint8_t *codes);
 /* Tuning/testing knob for plaac_score(): upper bounds of one device chunk (0 = keep default). */
 int plaac_set_chunk(plaac_ctx *ctx, int64_t max_residues, int64_t max_proteins);
 
-/* Long-sequence path (BASELINE config 5).  Summary mode: proteins of at least min_len residues are scored by one CTA
- * each, cut into <= 384 chunks (csrc/long_kernel.cuh): a warp-shuffle scan of 2x2 max-plus chunk matrices and
- * warm-started LUT forward chunks fix the absolute magnitudes, then both recurrences are re-run chunk-parallel in the
- * jar's own binade, where every rounding commutes with the chunk's shift, so the combined HMMall / HMMvit / Viterbi
- * path have the jar's bits.  The path is a latency device (a CTA per protein is less efficient per residue than the
- * bucketed kernel).  min_len > 0: fixed threshold (default 8192, where a lane's sequential walk of the protein,
- * ~1.4 ms, exceeds what a whole typical batch takes; raised to 1024 / four times the longest window if smaller).
- * min_len = -1: automatic threshold per batch -- the smallest length, at least 1024 residues and at least
+/* Long-sequence path (BASELINE config 5).  Summary mode: the record of a protein of at least min_len residues is
+ * computed chunk-parallel.  Its HMM columns (forward score, Viterbi parse and score) come from the thread-block cluster
+ * of the per-residue mode below, in records-only form (csrc/long_residue.cuh).  Beside it, two CTAs per protein cut it
+ * into <= 384 chunks (csrc/long_kernel.cuh): one computes the plain fp64 sums and the MW and LLR searches, the other the
+ * window columns.  Every chunk of a recurrence or sum is re-run in the jar's own binade, where every rounding commutes
+ * with the chunk's shift, so the combined values have the jar's bits.  Two small kernels then compute longestrun, the
+ * CORE search and the two HMM scores.  The path is a latency device (whole CTAs per protein are less efficient per
+ * residue than the bucketed kernel).  min_len > 0: fixed threshold (default 8192, where a lane's sequential walk of
+ * the protein, ~1.4 ms, exceeds what a whole typical batch takes; raised to 1024 / four times the longest window if
+ * smaller).  min_len = -1: automatic threshold per batch -- the smallest length, at least 1024 residues and at least
  * ntotal/81600 + 220 (the walk must be a visible part of the batch's time), that leaves no more long proteins than the
  * GPU has SMs; best latency for small proteomes (a yeast-sized set: 0.9 instead of 1.4 ms) at the price of one more
- * host synchronisation per device-resident call.  min_len = 0: path off.  warm: forward warm-up length, 0 keeps the
- * current value (default 256); a negative value redoes every forward chunk sequentially (testing).  Both paths give the
- * same bytes in every column (the recurrences by the binade-frame argument, the window columns because their sums are
- * exact on a 2^-41 grid), so records do not depend on the setting, the batching or the sharding.
- * Since round 2 the HMM columns of such a record (forward score, Viterbi parse and score) come from the cluster kernel
- * below, run beside the CTA that computes the other columns; the bytes are the same.
+ * host synchronisation per device-resident call.  min_len = 0: path off.  warm: warm-up length in residues of the
+ * cluster kernel's forward (and backward) chunks, rounded up to whole chunks; 0 keeps the current value (default 256),
+ * a negative value is taken by its magnitude.  A short warm-up only costs time: -1 gives the shortest, with which
+ * nearly every chunk is redone sequentially (testing).  Both paths give the same bytes in every column (the
+ * recurrences by the binade-frame argument, the window columns because their sums are exact on a 2^-41 grid), so
+ * records do not depend on the setting, the batching or the sharding.
  * Per-residue mode (plotsomefastas :610-647 on long proteins): the same threshold sends a protein to one thread-block
  * cluster (csrc/long_residue.cuh: 1 CTA below 32768 residues, 8 above; forward, backward and Viterbi recurrences
  * chunk-parallel in the jar's binade with an exact carry over the chunk boundaries, relayed between the CTAs through
@@ -327,7 +329,8 @@ typedef struct plaac_stats {
     float last_score_ms;       /* dominant kernel of the last device call */
     int64_t last_padded_slots; /* 16-byte lane slots in the bucketed stream of the last call */
     int64_t long_proteins;     /* proteins scored by the long-sequence path so far */
-    int64_t long_redone_chunks; /* forward chunks of that path redone sequentially (warm-up had not coalesced) */
+    int64_t long_redone_chunks; /* chunks of that path's cluster kernel redone sequentially although they had frames
+                                   (their warm-up had not coalesced) */
 } plaac_stats;
 int plaac_get_stats(plaac_ctx *ctx, plaac_stats *out);
 

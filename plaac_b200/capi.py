@@ -450,8 +450,9 @@ class Scorer:
         self._check(lib().plaac_set_chunk(self._h, max_residues, max_proteins))
 
     def set_long_path(self, min_len: int, warm: int = 0):
-        """plaac_set_long_path: length threshold of the chunked long-sequence path (0 = off); warm < 0 forces its
-        sequential forward fallback."""
+        """plaac_set_long_path: length threshold of the chunked long-sequence path (0 = off, -1 = automatic); warm:
+        warm-up residues of its chunks (0 keeps the current value, a negative value is taken by its magnitude; -1 gives
+        the shortest warm-up, with which nearly every chunk is redone sequentially)."""
         self._check(lib().plaac_set_long_path(self._h, min_len, warm))
 
     def set_kernel_variant(self, variant: int):

@@ -1,33 +1,35 @@
-// Long-sequence path (BASELINE config 5: titin-length and 100k-residue proteins; summary mode).
+// Long-sequence path, summary mode (BASELINE config 5: titin-length and 100k-residue proteins).
 //
 // In the bucketed kernel one lane walks one protein, so a lone long protein costs its full dependent chain
-// (~150 ns per residue: 15 ms for 100k residues).  Here ONE CTA owns one long protein and cuts it into <= 384
-// chunks, one lane per chunk, 32 consecutive chunks per warp:
+// (~150 ns per residue: 15 ms for 100k residues).  Here a long protein's record is computed by four kernels:
 //
-//   Viterbi   (viterbidecodel :3077-3121) pass 1: every chunk runs the max-plus recurrence from both unit start
-//             vectors, which gives its 2x2 max-plus transfer matrix; the chunk matrices are combined by a warp-shuffle
-//             Kogge-Stone SCAN of 2x2 max-plus matrices with a carry across groups of 32 chunks.
-//   forward   (posteriorl :3349-3375 with the LUT log-sum-exp :1024-1047) the LUT recurrence is not associative,
-//             but d = a1 - a0 forgets its start (SURVEY H1): pass 1 re-runs the recurrence from `warm` residues
-//             before each chunk and prefix-sums the chunk increments of a0 (warp-shuffle scan).
-//   Pass 1 is exact mathematics but NOT the jar's rounding: at |s| ~ 3e5 every addition of the jar rounds to
-//   ulp = 5.8e-11 and the dropped low bits of lt/le are the same at every step, so the jar's HMMall/HMMvit carry a
-//   systematic drift (3e-7 at n = 100k, measured) that a chunk-local frame does not have.  Pass 2 therefore re-runs
-//   both recurrences in the jar's own binade, started from pass 1's absolute values: every addition has an operand of
-//   the running magnitude, rounding is monotone and commutes with shifts by multiples of the ulp, hence a chunk
-//   reproduces the jar's sequential values up to an EXACT shift.  Viterbi transfer entries and forward increments are
-//   then exact multiples of the ulp and their ordered combination is the jar's number BIT FOR BIT.  The forward chunk
-//   runs in two frames one ulp apart and the frame is accepted that enters the chunk an EVEN number of ulps from the
-//   exact a0 and with exactly the bits of d the previous chunk left with (round-half-even ties look at the parity of
-//   the sum; the quantised recurrence coalesces during the warm-up); chunks in which the magnitude crosses a power of
-//   two (about one per binade) or lies in a binade where a table constant is an exact tie, and forward chunks without
-//   an acceptable frame, are redone sequentially from the exact values.
-//   windows   (disorderreport :4866-5068) the running window sums restart 2w residues before the chunk; FoldIndex
-//             runs and the PAPA first-strict-maximum are reduced per chunk and merged in chunk order.
-//   sums      the plain sequential fp64 sums of plaac.java -- psum[] of the LLR window search (hss2 :1206-1257), hmm0's
-//             log-emission sum, the hydropathy mean -- go through the same two passes (no state besides the sum), the
-//             window maxima are merged in chunk order; the Q/N window is integer work.  The -1e6-masked CORE search
-//             runs last on the Viterbi bits with the exact binade jumps of k_core_search_jump.
+//   k_long_post   (long_residue.cuh) one thread-block cluster per protein: the forward score, the Viterbi parse and
+//                 the Viterbi score, bit for bit the jar's
+//   k_long_score  TWO CTAs per protein (blockIdx.y), each with an ext copy of its own and one lane per chunk (<= 384
+//                 chunks, 32 consecutive chunks per warp).  CTA 0, the sums and the searches:
+//     sums        the plain sequential fp64 sums of plaac.java -- psum[] of the LLR window search (hss2 :1206-1257),
+//                 hmm0's log-emission sum, the hydropathy mean.  Pass 1 sums every chunk in a chunk-local frame and a
+//                 prefix over the chunk sums gives approximate absolute values.  That is exact mathematics but NOT the
+//                 jar's rounding: at |s| ~ 3e5 every addition of the jar rounds to ulp = 5.8e-11 and the dropped low
+//                 bits of the addends are the same at every step, so the jar's sums carry a systematic drift that a
+//                 chunk-local frame does not have.  Pass 2 therefore re-runs every chunk in the jar's own binade,
+//                 started from pass 1's absolute value: every addition has an operand of the running magnitude,
+//                 rounding is monotone and commutes with shifts by multiples of the ulp, hence a chunk reproduces the
+//                 jar's sequential values up to an EXACT shift.  Chunk increments and window differences are then
+//                 exact multiples of the ulp and their ordered combination is the jar's number BIT FOR BIT.  The
+//                 exception is an exact tie: round-half-even decides it by the parity of the sum, which a shift by an
+//                 odd number of ulps changes.  The host lists the binades in which a table constant is such a tie
+//                 (LongArgs::tie_mask); chunks there, and chunks in which the magnitude crosses a power of two (about
+//                 one per binade), are redone sequentially from the exact values.  (k_long_post's recurrences get the
+//                 same treatment; its forward recurrence has data-dependent addends and handles parity with two
+//                 frames one ulp apart.)
+//     searches    the LLR window maxima are merged in chunk order; the Q/N window and the charge sum are integer work.
+//                 CTA 1, the windows (disorderreport :4866-5068): the running window sums restart 2w residues before
+//                 the chunk; FoldIndex runs and the PAPA first-strict-maximum are reduced per chunk and merged in chunk
+//                 order.
+//   k_long_final  from k_long_post's parse: longestrun and the -1e6-masked CORE search with the exact binade jumps of
+//                 k_core_search_jump, PrD expansion and PRDscore
+//   k_long_fix    the two HMM scores, once k_long_post's scores and k_long_score's hmm0 sum are there
 //
 // Result: every column has the bits of the bucketed kernel, which has the bits of the jar.
 #pragma once
@@ -41,30 +43,21 @@ constexpr int kLongChunkWarps = 12;
 constexpr int kLongMaxChunks = kLongChunkWarps * 32;
 constexpr int kLongMinChunk = 256;
 constexpr int kLongPadTail = 128;  // ext bytes past the end are pad codes
-constexpr int kLongChunkMajorMin = 49152;  // from here on the chunk lanes read a chunk-major copy (LongArgs::extT)
 
 // Chunk geometry of one long protein: C residues per chunk (a multiple of 32 that holds a whole CORE / MW window), K
-// chunks (<= kLongMaxChunks), Kp = row pitch of the chunk-major copies (room for the chunk after the last one).
-__host__ __device__ inline void long_geometry(int64_t n, int c, int mw, int* C, int* K, int* Kp)
+// chunks (<= kLongMaxChunks).
+__host__ __device__ inline void long_geometry(int64_t n, int c, int mw, int* C, int* K)
 {
     int64_t cc = (n + kLongMaxChunks - 1) / kLongMaxChunks;
     cc = (cc + 31) & ~(int64_t)31;
     if (cc < kLongMinChunk) cc = kLongMinChunk;
     const int64_t wmin = (((c > mw ? c : mw) + 32) + 31) & ~(int64_t)31;
     if (cc < wmin) cc = wmin;
-    const int64_t kk = (n + cc - 1) / cc;
     *C = (int)cc;
-    *K = (int)kk;
-    *Kp = (int)(((kk + 1) + 31) & ~(int64_t)31);
+    *K = (int)((n + cc - 1) / cc);
 }
-// Scratch bytes per array (ext, chunk-major ext, chunk-major traceback) of one long protein.
-__host__ __device__ inline int64_t long_scratch_need(int64_t n, int c, int mw)
-{
-    int C, K, Kp;
-    long_geometry(n, c, mw, &C, &K, &Kp);
-    const int64_t a = n + kLongPadTail, b = (int64_t)C * Kp;
-    return ((a > b ? a : b) + 127) & ~(int64_t)127;
-}
+// Scratch bytes per array (one byte per residue and the pad tail) of one long protein; a multiple of 128.
+__host__ __device__ inline int64_t long_scratch_need(int64_t n) { return (n + kLongPadTail + 127) & ~(int64_t)127; }
 
 struct LongArgs {
     const uint8_t* codes;
@@ -75,68 +68,41 @@ struct LongArgs {
     KScalars ks;
     const DeviceTables* tabs;
     plaac_summary* out;
-    // hmm_ext = 1: the Viterbi parse and both HMM scores come from k_long_post (long_residue.cuh: one thread-block cluster
-    // per protein); this kernel then computes only the plain sums, the window columns and the MW / LLR searches, leaves
-    // sum0 (hmm0's log-emission sum) in sum0_out[i] and k_long_final completes the record
-    int hmm_ext;
-    double* sum0_out;
-    // split = 1 (with hmm_ext): two CTAs per protein, blockIdx.y = 0: sums, MW and LLR searches; 1: the window columns
-    // (FoldIndex runs, PAPA centre and its values) from an ext copy of its own (extT's space, protein-major)
-    int split;
-    uint8_t* ext;   // ext code per residue (same byte layout as the bucketed stream)
-    uint8_t* extT;  // the same, chunk-major: [position in chunk][chunk], so the 32 chunk lanes of a warp read 32
-                    // consecutive bytes per step (one sector) instead of 32 different lines.  Used from cm_min
-                    // residues on: with few chunk lanes the L1 hits of the protein-major copy are the faster choice
-                    // (measured: 100 k residues 1.72 -> 1.46 ms chunk-major, 35 k residues 0.93 -> 0.99 ms)
-    uint8_t* tb;    // 4 traceback bits per residue, same layout as the copy the lanes read: variant A (P0, P1), variant B (P0, P1)
-    int cm_min;     // proteins of at least this many residues use the chunk-major layout
-    long long* dbg_clocks;       // optional: phase time stamps of the CTA with blockIdx 0 (16 slots)
-    unsigned long long* redone;  // statistics: forward chunks redone sequentially because d had not coalesced
-    uint32_t* vit;  // Viterbi bits, one word per 32 residues
+    double* sum0_out;     // per listed protein: hmm0's log-emission sum, for k_long_fix
+    uint8_t* ext;         // ext code per residue (same byte layout as the bucketed stream): CTA 0's copy
+    uint8_t* ext_win;     // the same, CTA 1's copy
+    uint32_t* vit;        // Viterbi bits, one word per 32 residues (k_long_final)
     int* errflag;
     // Round-half-even breaks the shift argument exactly at ties (an addend whose bits below the binade's ulp are
-    // 1000...0): the rounding then depends on the parity of the sum.  For the recurrences whose addends are table
-    // constants only, the host lists the binades (bit b: values in [2^b, 2^(b+1))) in which some constant is such a
-    // tie; chunks there are redone sequentially.  [0] Viterbi (lt, le), [1] LLR psum (llr), [2] hmm0 sum (le0),
-    // [3] hydropathy sum.  The forward recurrence has data-dependent addends and handles parity explicitly.
-    unsigned long long tie_mask[4];
-    int warm;       // forward warm-up length
-    int force_seq_forward;  // testing: always take the sequential forward fallback
+    // 1000...0): the rounding then depends on the parity of the sum.  The host lists the binades (bit b: values in
+    // [2^b, 2^(b+1))) in which some table constant of a sum is such a tie; chunks there are redone sequentially.
+    // [0] LLR psum (llr), [1] hmm0 sum (le0), [2] hydropathy sum.
+    unsigned long long tie_mask[3];
 };
 
 struct LongShared {
-    double2 lut2[PLAAC_LUT_LEN + 1];
-    double2 le[32];
+    double le0[32];
     double llr[kTabN], hyd[kTabN], pap[kTabN], hydw[kTabN];
-    // per chunk
-    double M[4][kLongMaxChunks];       // Viterbi transfer matrix: [0] 0->0, [1] 0->1, [2] 1->0, [3] 1->1
-    double Sa[2][kLongMaxChunks];      // pass 1: approximate Viterbi scores at the chunk's last residue
-    double f_inc[kLongMaxChunks], f_mid[kLongMaxChunks], f_dexit[kLongMaxChunks];   // pass 1 (f_dexit[0]: true)
-    // pass 2, two frames of opposite parity: increment of a0 over the chunk, a0 and d at entry, d at exit
-    double g_inc[2][kLongMaxChunks], g_ea0[2][kLongMaxChunks], g_den[2][kLongMaxChunks], g_dex[2][kLongMaxChunks];
-    double A_cs[kLongMaxChunks], A_ts[kLongMaxChunks], A_end;  // pass 1: forward a0 before the chunk / at its warm-up start
+    // per chunk: windows (CTA 1)
     double p_tb[kLongMaxChunks], p_wb[kLongMaxChunks], p_vfi[kLongMaxChunks];
     int p_cen[kLongMaxChunks];
     int fi_pre[kLongMaxChunks], fi_suf[kLongMaxChunks], fi_sum[kLongMaxChunks], fi_max[kLongMaxChunks];
-    int v_pre[kLongMaxChunks], v_suf[kLongMaxChunks], v_max[kLongMaxChunks];
-    unsigned char fi_all[kLongMaxChunks], v_all[kLongMaxChunks], choice[kLongMaxChunks], endstate[kLongMaxChunks],
-        variant[kLongMaxChunks], cross_v[kLongMaxChunks], cross_f[kLongMaxChunks];
-    // sequential sums (psum[] of the LLR search, hmm0's emission sum, hydropathy sum): [0] LLR, [1] hmm0, [2] hydropathy
+    unsigned char fi_all[kLongMaxChunks];
+    // per chunk: sequential sums (psum[] of the LLR search, hmm0's emission sum, hydropathy sum): [0] LLR, [1] hmm0,
+    // [2] hydropathy (CTA 0)
     double q_sum[3][kLongMaxChunks], q_min[3][kLongMaxChunks], q_max[3][kLongMaxChunks];  // pass 1, chunk-local
     double q_abs[3][kLongMaxChunks];                                                      // pass 1: value before the chunk
     double q_inc[3][kLongMaxChunks], q_mid[kLongMaxChunks], q_best[kLongMaxChunks];       // pass 2, exact
     int q_stop[kLongMaxChunks], m_best[kLongMaxChunks], m_stop[kLongMaxChunks], c_sum[kLongMaxChunks];
     unsigned char cross_q[3][kLongMaxChunks];
     // results of the combines
-    double llr_best, sum0, sh, lvit, lmarg;
-    int llr_stop, csum, mw_best, mw_stop, vlast, fwd_redone;
-    int fi_numaa, fi_maxrun, pcen;
-    double pTb, pWb, pVfi;
+    double llr_best, sum0, sh;
+    int llr_stop, csum, mw_best, mw_stop;
 };
 
-// Proteins of at least long_min residues are scored by k_long_score; the bucketed path sees them as empty.
+// Proteins of at least long_min residues are scored by the long-sequence path; the bucketed path sees them as empty.
 __global__ void __launch_bounds__(256)
-k_long_select(const int64_t* __restrict__ offsets, int64_t nprot, int64_t long_min, int c, int mw,
+k_long_select(const int64_t* __restrict__ offsets, int64_t nprot, int64_t long_min,
               int32_t* __restrict__ list, int64_t* __restrict__ scratch_off,
               unsigned long long* __restrict__ counters /* [0] count, [1] scratch cursor, [2] count of >= big_min residues */,
               int64_t big_min)
@@ -146,41 +112,19 @@ k_long_select(const int64_t* __restrict__ offsets, int64_t nprot, int64_t long_m
     const int64_t len = offsets[i + 1] - offsets[i];
     if (len < long_min) return;
     const unsigned long long slot = atomicAdd(&counters[0], 1ull);
-    const unsigned long long need = (unsigned long long)long_scratch_need(len, c, mw);
+    const unsigned long long need = (unsigned long long)long_scratch_need(len);
     list[slot] = (int32_t)i;
     scratch_off[slot] = (int64_t)atomicAdd(&counters[1], need);
     if (len >= big_min) atomicAdd(&counters[2], 1ull);
 }
 
-// barrier of the chunk warps only: the single-lane walks on the other warps take longer and join at the end
+// barrier of the chunk warps only (the other warps leave after phase 0)
 __device__ __forceinline__ void long_chunk_bar()
 {
     // (barrier.sync without .aligned: the compiler may place the statement on both sides of a branch a warp has diverged
     // on -- compute-sanitizer's synccheck found warps arriving divergent at the aligned form; __syncwarp first)
     __syncwarp();
     asm volatile("barrier.sync 1, %0;" ::"n"(kLongChunkWarps * 32) : "memory");
-}
-
-// The exact forward combine (the longest single-lane walk: it redoes the binade-crossing chunks sequentially, ~300 cycles per
-// residue) runs on warp kLongChunkWarps beside everything that does not need its result (the other combines, the
-// traceback, the CORE search).  Barrier 2: pass 2 is complete (chunk warps + that warp).  Barrier 3: the other combines
-// are complete (the chunk warps only arrive; the forward warp waits for hmm0's emission sum there).
-constexpr int kLongFwdWarp = kLongChunkWarps;
-__device__ __forceinline__ void long_pass2_bar()
-{
-    __syncwarp();
-    asm volatile("barrier.sync 2, %0;" ::"n"((kLongChunkWarps + 1) * 32) : "memory");
-}
-__device__ __forceinline__ void long_combined_arrive()
-{
-    __threadfence_block();
-    __syncwarp();
-    asm volatile("barrier.arrive 3, %0;" ::"n"((kLongChunkWarps + 1) * 32) : "memory");
-}
-__device__ __forceinline__ void long_combined_wait()
-{
-    __syncwarp();
-    asm volatile("barrier.sync 3, %0;" ::"n"((kLongChunkWarps + 1) * 32) : "memory");
 }
 
 // Automatic threshold: length bins from 1024 up (256-residue steps to 16384, then powers of two); the host picks the
@@ -199,7 +143,7 @@ inline int64_t long_edge(int b) { return b < 60 ? 1024 + 256 * (int64_t)b : (int
 
 // per bin: [b] proteins, [kLongBins + b] scratch bytes, [2 * kLongBins + b] longest member
 __global__ void __launch_bounds__(256)
-k_long_levels(const int64_t* __restrict__ offsets, int64_t nprot, int c, int mw, unsigned long long* __restrict__ bins)
+k_long_levels(const int64_t* __restrict__ offsets, int64_t nprot, unsigned long long* __restrict__ bins)
 {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= nprot) return;
@@ -207,44 +151,13 @@ k_long_levels(const int64_t* __restrict__ offsets, int64_t nprot, int c, int mw,
     const int b = long_bin(len);
     if (b < 0) return;
     atomicAdd(&bins[b], 1ull);
-    atomicAdd(&bins[kLongBins + b], (unsigned long long)long_scratch_need(len, c, mw));
+    atomicAdd(&bins[kLongBins + b], (unsigned long long)long_scratch_need(len));
     atomicMax(&bins[2 * kLongBins + b], (unsigned long long)len);
 }
 
-struct MP2 {  // 2x2 max-plus matrix
-    double m00, m01, m10, m11;
-};
-__device__ __forceinline__ MP2 mp_mul(const MP2& a, const MP2& b)
-{
-    MP2 r;  // (a (x) b)[i][e] = max_m a[i][m] + b[m][e]
-    r.m00 = fmax(a.m00 + b.m00, a.m01 + b.m10);
-    r.m01 = fmax(a.m00 + b.m01, a.m01 + b.m11);
-    r.m10 = fmax(a.m10 + b.m00, a.m11 + b.m10);
-    r.m11 = fmax(a.m10 + b.m01, a.m11 + b.m11);
-    return r;
-}
-__device__ __forceinline__ MP2 mp_shfl_up(const MP2& a, int d)
-{
-    MP2 r;
-    r.m00 = __shfl_up_sync(0xffffffffu, a.m00, d);
-    r.m01 = __shfl_up_sync(0xffffffffu, a.m01, d);
-    r.m10 = __shfl_up_sync(0xffffffffu, a.m10, d);
-    r.m11 = __shfl_up_sync(0xffffffffu, a.m11, d);
-    return r;
-}
-
-#define LONG_STAMP(i)                                                              \
-    do {                                                                           \
-        if (g.dbg_clocks && tid == 0 && blockIdx.x == 0) g.dbg_clocks[i] = clock64(); \
-    } while (0)
-// the same from whichever single lane runs a walk (slots 9..14: ends of the single-lane combines)
-#define LONG_STAMP_LANE(i)                                                    \
-    do {                                                                      \
-        if (g.dbg_clocks && blockIdx.x == 0) g.dbg_clocks[i] = clock64();     \
-    } while (0)
-
-template <bool CM>
-__device__ __forceinline__ void long_score_body(const LongArgs& g)
+// Grid (long proteins, 2): blockIdx.y = 0 computes the sums, the MW and LLR searches and the means; 1 the window
+// columns (FoldIndex runs, PAPA centre and its values).
+__global__ void __launch_bounds__(kLongThreads, 1) k_long_score(LongArgs g)
 {
     extern __shared__ __align__(16) unsigned char long_smem[];
     LongShared& sm = *reinterpret_cast<LongShared*>(long_smem);
@@ -254,30 +167,16 @@ __device__ __forceinline__ void long_score_body(const LongArgs& g)
     const int64_t so = g.scratch_off[blockIdx.x];
     const int n = (int)(g.offsets[prot + 1] - g.offsets[prot]);
     const uint8_t* src = g.codes + (g.offsets[prot] - g.off_base);
-    // part 0 / 1 of a split protein (see LongArgs::split); do_main: everything but the window columns, do_win: those
-    const int part = g.split ? (int)blockIdx.y : 0;
-    const bool do_main = !g.split || part == 0, do_win = !g.split || part == 1;
-    uint8_t* __restrict__ ext = (g.split && part == 1 ? g.extT : g.ext) + so;
-    uint8_t* __restrict__ extT = g.extT + so;
-    uint8_t* __restrict__ tbT = g.tb + so;
-    uint32_t* __restrict__ vit = g.vit + (so >> 5);
+    const bool win = blockIdx.y == 1;
+    uint8_t* __restrict__ ext = (win ? g.ext_win : g.ext) + so;
     const int c = ks.core_len, w = ks.w, mw = ks.mw_window;
-    int C, K, Kp;
-    long_geometry(n, c, mw, &C, &K, &Kp);
-    // layout the chunk lanes walk (CM: chunk-major copies, else the protein-major ones): byte of residue rel of chunk kk
-    // at rel * sR + kk * sK
-    constexpr bool cm = CM;
-    const size_t sR = cm ? (size_t)Kp : 1, sK = cm ? 1 : (size_t)C;
+    int C, K;
+    long_geometry(n, c, mw, &C, &K);
 
     // ---- tables
     {
         const DeviceTables* T = g.tabs;
-        for (int i = tid; i <= PLAAC_LUT_LEN; i += kLongThreads) {
-            const double l0 = i < PLAAC_LUT_LEN ? T->lut[i] : 0.0;
-            const double l1 = i + 1 < PLAAC_LUT_LEN ? T->lut[i + 1] : 0.0;
-            sm.lut2[i] = make_double2(l0, l1);
-        }
-        if (tid < 32) sm.le[tid] = make_double2(T->le0[tid], T->le1[tid]);
+        if (tid < 32) sm.le0[tid] = T->le0[tid];
         if (tid < kTabN) {
             sm.llr[tid] = T->llr[tid];
             sm.hyd[tid] = T->hyd[tid];
@@ -288,10 +187,6 @@ __device__ __forceinline__ void long_score_body(const LongArgs& g)
     // ---- phase 0: ext codes (k_pack's byte layout: code | PAPA proline mask << 5 | charge class << 6)
     {
         int bad = 0;
-        if (cm) {
-            for (int i = tid; i < C * Kp; i += kLongThreads) extT[i] = (uint8_t)kPad;
-            __syncthreads();
-        }
         // eight residues per thread and trip, all loads issued before the first use (a single byte load per trip left
         // the CTA waiting on DRAM latency: 0.1 ms of the 1.4 ms at 100 k residues)
         constexpr int kU = 8;
@@ -320,739 +215,171 @@ __device__ __forceinline__ void long_score_body(const LongArgs& g)
                 else if ((ks.charge_minus >> c0) & 1u)
                     e |= 0xc0u;
                 ext[i] = (uint8_t)e;
-                if (cm) extT[(size_t)(i % C) * Kp + i / C] = (uint8_t)e;
             }
         }
         for (int i = n + tid; i < n + kLongPadTail; i += kLongThreads) ext[i] = (uint8_t)kPad;
         if (bad) atomicOr(g.errflag, 1);
     }
     __syncthreads();
+    if (wid >= kLongChunkWarps) return;
 
-    LONG_STAMP(0);
-    const uint32_t lut_addr = smem_u32(&sm.lut2[0]);
-
-    const int warm = max(1, min(g.warm, C));
-    if (wid < kLongChunkWarps) {
-        const int k = tid;
-        const bool live = k < K;
-        const int cs = k * C, ce = min(n, cs + C);
-        // residue t through the strided copy: t lies in this lane's chunk or in a neighbour (halos, lags <= C)
-        auto xt = [&](int t) -> uint32_t {
-            if constexpr (!CM) return ext[t];
-            int rel = t - cs, kk = k;
-            if (rel < 0) {
-                rel += C;
-                kk--;
-            } else if (rel >= C) {
-                rel -= C;
-                kk++;
+    const int k = tid;
+    const bool live = k < K;
+    const int cs = k * C, ce = min(n, cs + C);
+    // ================= pass 1: chunk-local frame =================
+    if (live && !win) {
+        // the chunk-local sums of the three sequential-sum columns (running extremes for the binade test), the charge
+        // sum and the Q/N window: independent dependency chains in one loop
+        double q0 = 0, q1 = 0, q2 = 0, mn0 = 0, mn1 = 0, mn2 = 0, mx0 = 0, mx1 = 0, mx2 = 0;
+        int cq = 0;
+        int qn = 0, mbest = -1, mstop = -1;
+        for (int t = max(0, cs - mw); t < cs; t++) qn += (int)((ks.qn_mask >> (ext[t] & 31)) & 1u);
+        auto stats = [&](int t, uint32_t e) {
+            q0 = q0 + sm.llr[e & 31];
+            q1 = q1 + sm.le0[e & 31];
+            q2 = q2 + sm.hyd[e & 63];
+            mn0 = fmin(mn0, q0), mx0 = fmax(mx0, q0);
+            mn1 = fmin(mn1, q1), mx1 = fmax(mx1, q1);
+            mn2 = fmin(mn2, q2), mx2 = fmax(mx2, q2);
+            cq += (int)(int8_t)e >> 6;
+            // Q/N window :764-771: first strict maximum of the count in [t-mw+1, t] (n >= mw here)
+            qn += (int)((ks.qn_mask >> (e & 31)) & 1u);
+            if (t >= mw) qn -= (int)((ks.qn_mask >> (ext[t - mw] & 31)) & 1u);
+            if (t >= mw - 1 && qn > mbest) {
+                mbest = qn;
+                mstop = t;
             }
-            return extT[(size_t)rel * Kp + kk];
         };
-        uint8_t* const tbk = tbT + (size_t)k * sK;  // traceback byte of residue t of this chunk: tbk[(t - cs) * sR]
-        // ================= pass 1: chunk-local frame =================
-        if (live) {
-            // ---- Viterbi: the chunk's 2x2 max-plus transfer matrix (first chunk: the true chain, with its traceback)
-            if (do_main) {
-                double a0, a1, b0 = -INFINITY, b1 = 0.0;
-                int t0 = cs;
-                if (k == 0) {
-                    const double2 le = sm.le[xt(0) & 31];
-                    a0 = ks.li0 + le.x;
-                    a1 = ks.li1 + le.y;
-                    b1 = -INFINITY;
-                    if (!g.hmm_ext) tbk[0] = 0;
-                    t0 = 1;
-                } else {
-                    a0 = 0.0;
-                    a1 = -INFINITY;
-                }
-                // fused with the chunk-local sums of the three sequential-sum columns (running extremes for the binade
-                // test), the charge sum and the Q/N window: independent dependency chains in one loop
-                double q0 = 0, q1 = 0, q2 = 0, mn0 = 0, mn1 = 0, mn2 = 0, mx0 = 0, mx1 = 0, mx2 = 0;
-                int cq = 0;
-                int qn = 0, mbest = -1, mstop = -1;
-                for (int t = max(0, cs - mw); t < cs; t++) qn += (int)((ks.qn_mask >> (xt(t) & 31)) & 1u);
-                auto stats = [&](int t, uint32_t e) {
-                    q0 = q0 + sm.llr[e & 31];
-                    q1 = q1 + sm.le[e & 31].x;
-                    q2 = q2 + sm.hyd[e & 63];
-                    mn0 = fmin(mn0, q0), mx0 = fmax(mx0, q0);
-                    mn1 = fmin(mn1, q1), mx1 = fmax(mx1, q1);
-                    mn2 = fmin(mn2, q2), mx2 = fmax(mx2, q2);
-                    cq += (int)(int8_t)e >> 6;
-                    // Q/N window :764-771: first strict maximum of the count in [t-mw+1, t] (n >= mw here)
-                    qn += (int)((ks.qn_mask >> (e & 31)) & 1u);
-                    if (t >= mw) qn -= (int)((ks.qn_mask >> (xt(t - mw) & 31)) & 1u);
-                    if (t >= mw - 1 && qn > mbest) {
-                        mbest = qn;
-                        mstop = t;
-                    }
-                };
-                if (k == 0) stats(0, xt(0));
-                if (g.hmm_ext) {
+        int t0 = cs;
+        if (k == 0) {
+            stats(0, ext[0]);
+            t0 = 1;
+        }
 #pragma unroll 4
-                    for (int t = t0; t < ce; t++) stats(t, xt(t));
-                } else {
-#pragma unroll 4
-                for (int t = t0; t < ce; t++) {
-                    const uint32_t e = xt(t);
-                    const double2 le = sm.le[e & 31];
-                    const double vA00 = ks.lt00 + a0, vA10 = ks.lt10 + a1, vA01 = ks.lt01 + a0, vA11 = ks.lt11 + a1;
-                    const double vB00 = ks.lt00 + b0, vB10 = ks.lt10 + b1, vB01 = ks.lt01 + b0, vB11 = ks.lt11 + b1;
-                    const bool pA0 = vA10 > vA00, pA1 = vA11 > vA01;
-                    a0 = (pA0 ? vA10 : vA00) + le.x;
-                    a1 = (pA1 ? vA11 : vA01) + le.y;
-                    b0 = fmax(vB00, vB10) + le.x;
-                    b1 = fmax(vB01, vB11) + le.y;
-                    if (k == 0) tbk[(size_t)(t - cs) * sR] = (uint8_t)((int)pA0 | ((int)pA1 << 1));
-                    stats(t, e);
-                }
-                }
-                sm.M[0][k] = a0;
-                sm.M[1][k] = a1;
-                sm.M[2][k] = b0;
-                sm.M[3][k] = b1;
-                sm.q_sum[0][k] = q0, sm.q_min[0][k] = mn0, sm.q_max[0][k] = mx0;
-                sm.q_sum[1][k] = q1, sm.q_min[1][k] = mn1, sm.q_max[1][k] = mx1;
-                sm.q_sum[2][k] = q2, sm.q_min[2][k] = mn2, sm.q_max[2][k] = mx2;
-                sm.c_sum[k] = cq;
-                sm.m_best[k] = mbest;
-                sm.m_stop[k] = mstop;
-            }
-            // ---- forward LUT recurrence from `warm` residues before the chunk (first chunk: the true chain)
-            if (!g.hmm_ext) {
-                const int ts = (k == 0) ? 0 : max(0, cs - warm);
-                const int tmid = ce - warm;  // where the next chunk's warm-up starts
-                const double2 le0 = sm.le[xt(ts) & 31];
-                double a0 = ks.li0 + le0.x, a1 = ks.li1 + le0.y;
-                double e_a0 = 0.0, m_a0 = a0;
+        for (int t = t0; t < ce; t++) stats(t, ext[t]);
+        sm.q_sum[0][k] = q0, sm.q_min[0][k] = mn0, sm.q_max[0][k] = mx0;
+        sm.q_sum[1][k] = q1, sm.q_min[1][k] = mn1, sm.q_max[1][k] = mx1;
+        sm.q_sum[2][k] = q2, sm.q_min[2][k] = mn2, sm.q_max[2][k] = mx2;
+        sm.c_sum[k] = cq;
+        sm.m_best[k] = mbest;
+        sm.m_stop[k] = mstop;
+    }
+    if (live && win) {
+        // ---- sliding windows: FoldIndex runs and the PAPA centre over the positions this chunk owns
+        const int off1 = 2 * w + 1, off2 = 4 * w + 2;
+        const int full = 2 * w + 1, Wfull = full * full;
+        const int t_start = max(0, cs - 2 * w);
+        const int t_last = min(ce + 2 * w, n + w) - 1;
+        int halfw = ks.h_fi;
+        if (halfw > n / 2) halfw = n / 2;
+        const int fi_hi = n - halfw, edge_hi = n - 1 - w;
+        double SLh = 0, SGh = 0, Th = 0, Dp = 0, Tp = 0;
+        int SLc = 0, SGc = 0, Tac = 0;
+        double Tb = 0, Wb = 1, vfib = 0;
+        int pcen = -1;
+        int cur = 0, pre = 0, insum = 0, inmax = 0;
+        bool all = true;
 #pragma unroll 8
-                for (int t = ts + 1; t < ce; t++) {
-                    if (t == cs) e_a0 = a0;
-                    const double2 le = sm.le[xt(t) & 31];
-                    const double f0 = lse_lut2<false>(ks.lt00 + a0, ks.lt10 + a1, lut_addr) + le.x;
-                    const double f1 = lse_lut2<false>(ks.lt01 + a0, ks.lt11 + a1, lut_addr) + le.y;
-                    a0 = f0;
-                    a1 = f1;
-                    if (t == tmid) m_a0 = a0;
-                }
-                sm.f_inc[k] = a0 - e_a0;   // first chunk: e_a0 = 0, absolute values
-                sm.f_mid[k] = m_a0 - e_a0;
-                if (k == 0) sm.f_dexit[0] = a1 - a0;
-            }
-            // ---- sliding windows: FoldIndex runs and the PAPA centre over the positions this chunk owns
-            if (do_win) {
-                const int off1 = 2 * w + 1, off2 = 4 * w + 2;
-                const int full = 2 * w + 1, Wfull = full * full;
-                const int t_start = max(0, cs - 2 * w);
-                const int t_last = min(ce + 2 * w, n + w) - 1;
-                int halfw = ks.h_fi;
-                if (halfw > n / 2) halfw = n / 2;
-                const int fi_hi = n - halfw, edge_hi = n - 1 - w;
-                double SLh = 0, SGh = 0, Th = 0, Dp = 0, Tp = 0;
-                int SLc = 0, SGc = 0, Tac = 0;
-                double Tb = 0, Wb = 1, vfib = 0;
-                int pcen = -1;
-                int cur = 0, pre = 0, insum = 0, inmax = 0;
-                bool all = true;
-#pragma unroll 8
-                for (int t = t_start; t <= t_last; t++) {
-                    const uint32_t e0 = (t < n) ? xt(t) : (uint32_t)kPad;
-                    const uint32_t e1 = (t - off1 >= t_start) ? xt(t - off1) : (uint32_t)kPad;
-                    const uint32_t e2 = (t - off2 >= t_start) ? xt(t - off2) : (uint32_t)kPad;
-                    const double hy0 = sm.hydw[e0 & 63], hy1 = sm.hydw[e1 & 63], hy2 = sm.hydw[e2 & 63];
-                    const double pa0 = sm.pap[e0 & 63], pa1 = sm.pap[e1 & 63], pa2 = sm.pap[e2 & 63];
-                    const int ch0 = (int)(int8_t)e0 >> 6, ch1 = (int)(int8_t)e1 >> 6, ch2 = (int)(int8_t)e2 >> 6;
-                    SLh = (SLh + hy0) - hy1;
-                    SGh = (SGh + hy1) - hy2;
-                    Th = (Th + SLh) - SGh;
-                    Dp = Dp + ((pa0 + pa2) - (pa1 + pa1));
-                    Tp = Tp + Dp;
-                    SLc += ch0 - ch1;
-                    SGc += ch1 - ch2;
-                    const int aSL = abs(SLc);
-                    Tac += aSL - abs(SGc);
-                    const int p = t - w;
-                    if (p >= cs && p < ce && p >= halfw && p < fi_hi) {
-                        const double c2 = ks.cc2 * (double)(full - max(0, w - p) - max(0, p - edge_hi));
-                        const double fis = (ks.cc0 * SLh + ks.cc1 * (double)aSL) + c2;
-                        if (fis < 0) {
-                            cur += 1;
-                            if (p == halfw) cur += halfw;           // a run from the first scanned position snaps to 0
-                            if (p == fi_hi - 1) cur += n - 1 - p;   // one reaching the last scanned position snaps to n-1
-                        } else {
-                            if (all) {
-                                pre = cur;
-                                all = false;
-                            } else if (cur >= 5) {
-                                insum += cur;
-                                inmax = max(inmax, cur);
-                            }
-                            cur = 0;
-                        }
-                    }
-                    const int kk = p - w;
-                    if (kk >= cs && kk < ce && kk >= w && kk <= edge_hi) {
-                        const int ml = 2 * w - kk, mr = kk - (edge_hi - w);
-                        const double Wd =
-                            (double)(Wfull - (ml > 0 ? (ml * (ml + 1)) >> 1 : 0) - (mr > 0 ? (mr * (mr + 1)) >> 1 : 0));
-                        const double vfi = (ks.cc0 * Th + ks.cc1 * (double)Tac) + ks.cc2 * Wd;
-                        if ((pcen < 0 || Tp * Wb > Tb * Wd) && vfi < 0) {
-                            Tb = Tp;
-                            Wb = Wd;
-                            vfib = vfi;
-                            pcen = kk;
-                        }
-                    }
-                }
-                sm.fi_all[k] = all ? 1 : 0;
-                sm.fi_pre[k] = all ? cur : pre;
-                sm.fi_suf[k] = cur;
-                sm.fi_sum[k] = insum;
-                sm.fi_max[k] = inmax;
-                sm.p_cen[k] = pcen;
-                sm.p_tb[k] = Tb;
-                sm.p_wb[k] = Wb;
-                sm.p_vfi[k] = vfib;
-            }
-        }
-        long_chunk_bar();
-        LONG_STAMP(1);
-        // ================= combine 1: approximate absolute values (they only fix the binade of pass 2) =================
-        if (wid == 0 && !g.hmm_ext) {
-            // Scan of the 2x2 max-plus chunk matrices: S_k = S_0 (x) M_1 (x) ... (x) M_k, 32 chunks per round with the
-            // running product of all earlier rounds as carry (Kogge-Stone over warp shuffles).
-            double c0 = sm.M[0][0], c1 = sm.M[1][0];
-            if (lane == 0) {
-                sm.Sa[0][0] = c0;
-                sm.Sa[1][0] = c1;
-            }
-            for (int base = 1; base < K; base += 32) {
-                const int kk = base + lane;
-                MP2 m;
-                if (kk < K) {
-                    m.m00 = sm.M[0][kk];
-                    m.m01 = sm.M[1][kk];
-                    m.m10 = sm.M[2][kk];
-                    m.m11 = sm.M[3][kk];
+        for (int t = t_start; t <= t_last; t++) {
+            const uint32_t e0 = (t < n) ? ext[t] : (uint32_t)kPad;
+            const uint32_t e1 = (t - off1 >= t_start) ? ext[t - off1] : (uint32_t)kPad;
+            const uint32_t e2 = (t - off2 >= t_start) ? ext[t - off2] : (uint32_t)kPad;
+            const double hy0 = sm.hydw[e0 & 63], hy1 = sm.hydw[e1 & 63], hy2 = sm.hydw[e2 & 63];
+            const double pa0 = sm.pap[e0 & 63], pa1 = sm.pap[e1 & 63], pa2 = sm.pap[e2 & 63];
+            const int ch0 = (int)(int8_t)e0 >> 6, ch1 = (int)(int8_t)e1 >> 6, ch2 = (int)(int8_t)e2 >> 6;
+            SLh = (SLh + hy0) - hy1;
+            SGh = (SGh + hy1) - hy2;
+            Th = (Th + SLh) - SGh;
+            Dp = Dp + ((pa0 + pa2) - (pa1 + pa1));
+            Tp = Tp + Dp;
+            SLc += ch0 - ch1;
+            SGc += ch1 - ch2;
+            const int aSL = abs(SLc);
+            Tac += aSL - abs(SGc);
+            const int p = t - w;
+            if (p >= cs && p < ce && p >= halfw && p < fi_hi) {
+                const double c2 = ks.cc2 * (double)(full - max(0, w - p) - max(0, p - edge_hi));
+                const double fis = (ks.cc0 * SLh + ks.cc1 * (double)aSL) + c2;
+                if (fis < 0) {
+                    cur += 1;
+                    if (p == halfw) cur += halfw;           // a run from the first scanned position snaps to 0
+                    if (p == fi_hi - 1) cur += n - 1 - p;   // one reaching the last scanned position snaps to n-1
                 } else {
-                    m.m00 = 0.0;
-                    m.m01 = -INFINITY;
-                    m.m10 = -INFINITY;
-                    m.m11 = 0.0;
-                }
-                MP2 p = m;
-#pragma unroll
-                for (int d = 1; d < 32; d <<= 1) {
-                    const MP2 o = mp_shfl_up(p, d);
-                    if (lane >= d) p = mp_mul(o, p);
-                }
-                const double s0 = fmax(c0 + p.m00, c1 + p.m10), s1 = fmax(c0 + p.m01, c1 + p.m11);
-                if (kk < K) {
-                    sm.Sa[0][kk] = s0;
-                    sm.Sa[1][kk] = s1;
-                }
-                c0 = __shfl_sync(0xffffffffu, s0, 31);
-                c1 = __shfl_sync(0xffffffffu, s1, 31);
-            }
-        } else if (wid == 1 && !g.hmm_ext) {
-            // prefix sums of the forward increments (warp-shuffle scan with carry): a0 at cs-1 and at the warm-up start
-            double carry = 0.0;
-            for (int base = 0; base < K; base += 32) {
-                const int kk = base + lane;
-                const double v = kk < K ? sm.f_inc[kk] : 0.0;
-                double inc = v;
-#pragma unroll
-                for (int d = 1; d < 32; d <<= 1) {
-                    const double o = __shfl_up_sync(0xffffffffu, inc, d);
-                    if (lane >= d) inc += o;
-                }
-                if (kk < K) {
-                    const double before = carry + (inc - v);      // a0 at cs-1 (0 for the first chunk)
-                    sm.A_cs[kk] = before;
-                    if (kk + 1 < K) sm.A_ts[kk + 1] = before + sm.f_mid[kk];
-                }
-                carry += __shfl_sync(0xffffffffu, inc, 31);
-            }
-            if (lane == 0) sm.A_end = carry;
-        } else if (wid == 2 && lane < 3) {
-            double run = 0.0;
-            for (int kk = 0; kk < K; kk++) {
-                sm.q_abs[lane][kk] = run;
-                run += sm.q_sum[lane][kk];
-            }
-        }
-        long_chunk_bar();
-        LONG_STAMP(2);
-        // ================= pass 2: the jar's own binade =================
-        // Every fp64 addition of the two recurrences has one operand of the running magnitude |s| ~ 3t, so it rounds
-        // to a multiple of ulp(|s|); rounding is monotone and commutes with shifts by multiples of that ulp as long as
-        // no operand changes its binade.  Re-run from an approximate absolute value, a chunk therefore reproduces the
-        // jar's sequential values up to an EXACT shift: Viterbi transfer entries and forward increments become exact
-        // multiples of the ulp and their ordered combination is the jar's number bit for bit.  Chunks in which the
-        // magnitude crosses a power of two (about one per binade) are redone sequentially from the exact values.
-        if (live && k >= 1 && g.hmm_ext && do_main) {
-            // (the HMM columns come from k_long_post: only the psum[] LLR search and the two plain sums, in their own frames)
-            double lagsum = 0;
-            for (int t = cs - c; t < cs; t++) lagsum += sm.llr[xt(t) & 31];
-            double lag = sm.q_abs[0][k] - lagsum;
-            double lead = lag;
-            for (int t = cs - c; t < cs; t++) lead = lead + sm.llr[xt(t) & 31];
-            const double lead0 = lead;
-            double best = -INFINITY, mid = lead;
-            int stop = -1;
-            const double x10 = sm.q_abs[1][k], x20 = sm.q_abs[2][k];
-            double x1 = x10, x2 = x20;
-#pragma unroll 4
-            for (int t = cs; t < ce; t++) {
-                const uint32_t e = xt(t);
-                lead = lead + sm.llr[e & 31];
-                lag = lag + sm.llr[xt(t - c) & 31];
-                const double d = lead - lag;  // exact, and the jar's number
-                if (d > best) {
-                    best = d;
-                    stop = t;
-                }
-                if (t == ce - c - 1) mid = lead;
-                x1 = x1 + sm.le[e & 31].x;
-                x2 = x2 + sm.hyd[e & 63];
-            }
-            sm.q_inc[0][k] = lead - lead0;
-            sm.q_mid[k] = mid - lead0;
-            sm.q_best[k] = best;
-            sm.q_stop[k] = stop;
-            sm.q_inc[1][k] = x1 - x10;
-            sm.q_inc[2][k] = x2 - x20;
-        }
-        if (live && k >= 1 && !g.hmm_ext) {
-            {
-                const double lo = fmin(fabs(sm.Sa[0][k - 1]), fabs(sm.Sa[1][k - 1])) - 64.0;
-                const double hi = fmax(fabs(sm.Sa[0][k]), fabs(sm.Sa[1][k])) + 64.0;
-                const bool cross = !(lo >= 1024.0) || (__double2hiint(lo) >> 20) != (__double2hiint(hi) >> 20) ||
-                                   ((g.tie_mask[0] >> (((__double2hiint(lo) >> 20) & 0x7ff) - 1023)) & 1ull);
-                sm.cross_v[k] = cross ? 1 : 0;
-                // One loop over the chunk for the Viterbi frames, the psum[] LLR search and the two plain sums, each in its
-                // own binade frame: independent dependency chains that hide each other's latency.  Everything is
-                // computed whether or not its crossing flag is set (the combine step ignores flagged results); only the
-                // traceback bytes of a flagged chunk are left to the sequential redo.
-                const double R = sm.Sa[0][k - 1];
-                double a0 = R, a1 = -INFINITY, b0 = -INFINITY, b1 = R;
-                double lagsum = 0;
-                for (int t = cs - c; t < cs; t++) lagsum += sm.llr[xt(t) & 31];
-                double lag = sm.q_abs[0][k] - lagsum;  // approximate psum before residue cs-c: fixes the frame
-                double lead = lag;
-                for (int t = cs - c; t < cs; t++) lead = lead + sm.llr[xt(t) & 31];
-                const double lead0 = lead;
-                double best = -INFINITY, mid = lead;
-                int stop = -1;
-                const double x10 = sm.q_abs[1][k], x20 = sm.q_abs[2][k];
-                double x1 = x10, x2 = x20;
-#pragma unroll 4
-                for (int t = cs; t < ce; t++) {
-                    const uint32_t e = xt(t);
-                    const double2 le = sm.le[e & 31];
-                    const double vA00 = ks.lt00 + a0, vA10 = ks.lt10 + a1, vA01 = ks.lt01 + a0, vA11 = ks.lt11 + a1;
-                    const double vB00 = ks.lt00 + b0, vB10 = ks.lt10 + b1, vB01 = ks.lt01 + b0, vB11 = ks.lt11 + b1;
-                    const bool pA0 = vA10 > vA00, pA1 = vA11 > vA01, pB0 = vB10 > vB00, pB1 = vB11 > vB01;
-                    a0 = (pA0 ? vA10 : vA00) + le.x;
-                    a1 = (pA1 ? vA11 : vA01) + le.y;
-                    b0 = (pB0 ? vB10 : vB00) + le.x;
-                    b1 = (pB1 ? vB11 : vB01) + le.y;
-                    if (!cross) tbk[(size_t)(t - cs) * sR] = (uint8_t)((int)pA0 | ((int)pA1 << 1) | ((int)pB0 << 2) | ((int)pB1 << 3));
-                    lead = lead + sm.llr[e & 31];
-                    lag = lag + sm.llr[xt(t - c) & 31];
-                    const double d = lead - lag;  // exact, and the jar's number
-                    if (d > best) {
-                        best = d;
-                        stop = t;
+                    if (all) {
+                        pre = cur;
+                        all = false;
+                    } else if (cur >= 5) {
+                        insum += cur;
+                        inmax = max(inmax, cur);
                     }
-                    if (t == ce - c - 1) mid = lead;
-                    x1 = x1 + le.x;
-                    x2 = x2 + sm.hyd[e & 63];
+                    cur = 0;
                 }
-                sm.M[0][k] = a0;  // values at the chunk's last residue had the chunk been entered in state 0 with score R
-                sm.M[1][k] = a1;
-                sm.M[2][k] = b0;  // ... in state 1 with score R
-                sm.M[3][k] = b1;
-                sm.q_inc[0][k] = lead - lead0;
-                sm.q_mid[k] = mid - lead0;
-                sm.q_best[k] = best;
-                sm.q_stop[k] = stop;
-                sm.q_inc[1][k] = x1 - x10;
-                sm.q_inc[2][k] = x2 - x20;
             }
-            {
-                const double lo = fabs(sm.A_cs[k]) - 64.0;
-                const double hi = fabs(k + 1 < K ? sm.A_cs[k + 1] : sm.A_end) + 64.0;
-                const bool cross = !(lo >= 1024.0) || (__double2hiint(lo) >> 20) != (__double2hiint(hi) >> 20);
-                sm.cross_f[k] = cross ? 1 : 0;
-                if (!cross) {
-                    // Two frames one ulp apart: the shift argument needs the frame to differ from the jar's values by
-                    // an EVEN number of ulps (round-half-even at exact ties looks at the parity of the sum, and the
-                    // interpolation term is a tie about once per 2^15 additions at these magnitudes).  The combine
-                    // step takes the frame of the right parity.
-                    const int ts = max(0, cs - warm);
-                    const double2 le0 = sm.le[xt(ts) & 31];
-                    double a0 = ks.li0 + le0.x, a1 = ks.li1 + le0.y;
-                    double c0 = a0, c1 = a1;
-                    if (ts > 0) {
-                        const double u = __hiloint2double((((__double2hiint(fabs(sm.A_cs[k])) >> 20) & 0x7ff) - 52) << 20, 0);
-                        const double dd = a1 - a0;
-                        a0 = sm.A_ts[k];
-                        a1 = a0 + dd;
-                        c0 = a0 + u;
-                        c1 = c0 + dd;
-                    }
-                    double ea = 0.0, ed = 0.0, ec = 0.0, ee = 0.0;
-#pragma unroll 4
-                    for (int t = ts + 1; t < ce; t++) {
-                        if (t == cs) {
-                            ea = a0;
-                            ed = a1 - a0;
-                            ec = c0;
-                            ee = c1 - c0;
-                        }
-                        const double2 le = sm.le[xt(t) & 31];
-                        const double f0 = lse_lut2<false>(ks.lt00 + a0, ks.lt10 + a1, lut_addr) + le.x;
-                        const double f1 = lse_lut2<false>(ks.lt01 + a0, ks.lt11 + a1, lut_addr) + le.y;
-                        const double h0 = lse_lut2<false>(ks.lt00 + c0, ks.lt10 + c1, lut_addr) + le.x;
-                        const double h1 = lse_lut2<false>(ks.lt01 + c0, ks.lt11 + c1, lut_addr) + le.y;
-                        a0 = f0;
-                        a1 = f1;
-                        c0 = h0;
-                        c1 = h1;
-                    }
-                    sm.g_inc[0][k] = a0 - ea;  // exact: both are multiples of the same ulp
-                    sm.g_ea0[0][k] = ea;
-                    sm.g_den[0][k] = ed;
-                    sm.g_dex[0][k] = a1 - a0;
-                    sm.g_inc[1][k] = c0 - ec;
-                    sm.g_ea0[1][k] = ec;
-                    sm.g_den[1][k] = ee;
-                    sm.g_dex[1][k] = c1 - c0;
+            const int kk = p - w;
+            if (kk >= cs && kk < ce && kk >= w && kk <= edge_hi) {
+                const int ml = 2 * w - kk, mr = kk - (edge_hi - w);
+                const double Wd =
+                    (double)(Wfull - (ml > 0 ? (ml * (ml + 1)) >> 1 : 0) - (mr > 0 ? (mr * (mr + 1)) >> 1 : 0));
+                const double vfi = (ks.cc0 * Th + ks.cc1 * (double)Tac) + ks.cc2 * Wd;
+                if ((pcen < 0 || Tp * Wb > Tb * Wd) && vfi < 0) {
+                    Tb = Tp;
+                    Wb = Wd;
+                    vfib = vfi;
+                    pcen = kk;
                 }
             }
         }
-        if (live && do_main) {
-            // ---- the three sequential sums in their own binade (same argument, no state besides the sum itself)
-            // crossing test over every value the running sum takes in the region (for the LLR search the lagged sum
-            // starts c residues before the chunk, i.e. inside the previous chunk)
-            bool cross[3];
-#pragma unroll
-            for (int q = 0; q < 3; q++) {
-                double mn = sm.q_abs[q][k] + sm.q_min[q][k], mx = sm.q_abs[q][k] + sm.q_max[q][k];
-                if (q == 0 && k >= 1) {
-                    mn = fmin(mn, sm.q_abs[0][k - 1] + sm.q_min[0][k - 1]);
-                    mx = fmax(mx, sm.q_abs[0][k - 1] + sm.q_max[0][k - 1]);
-                }
-                const double lo = fmin(fabs(mn), fabs(mx)) * (1.0 - 1e-6), hi = fmax(fabs(mn), fabs(mx)) * (1.0 + 1e-6);
-                cross[q] = k == 0 || !(mn > 0.0 || mx < 0.0) || !(lo >= 1.0) ||
-                           (__double2hiint(lo) >> 20) != (__double2hiint(hi) >> 20) ||
-                           ((g.tie_mask[1 + q] >> (((__double2hiint(lo) >> 20) & 0x7ff) - 1023)) & 1ull);
-                sm.cross_q[q][k] = cross[q] ? 1 : 0;
-            }
-            if (k == 0) {
-                // first chunk: the true chains from residue 0 (hss2 :1206-1257, mean() :1584, hmm0's emission sum)
-                double ps = 0, psl = 0, best = 0, mid = 0;
-                int stop = -2;
-                double s0 = 0, shy = 0;
-#pragma unroll 8
-                for (int t = 0; t < ce; t++) {
-                    const uint32_t e = xt(t);
-                    ps = ps + sm.llr[e & 31];
-                    if (t >= c) psl = psl + sm.llr[xt(t - c) & 31];
-                    if (t >= c - 1) {
-                        const double d = ps - psl;
-                        if (t == c - 1 || d > best) {
-                            best = d;
-                            stop = t;
-                        }
-                    }
-                    if (t == ce - c - 1) mid = ps;
-                    s0 = (t == 0) ? sm.le[e & 31].x : s0 + sm.le[e & 31].x;
-                    shy = shy + sm.hyd[e & 63];
-                }
-                sm.q_inc[0][0] = ps, sm.q_mid[0] = mid, sm.q_best[0] = best, sm.q_stop[0] = stop;
-                sm.q_inc[1][0] = s0;
-                sm.q_inc[2][0] = shy;
-            }
-        }
-        long_pass2_bar();
-        LONG_STAMP(3);
-        // ================= combine 2: exact, in chunk order =================
-        if (wid == 0 && lane == 0 && !g.hmm_ext) {
-            double S0 = sm.M[0][0], S1 = sm.M[1][0];
-            sm.choice[0] = 0;
-            for (int kk = 1; kk < K; kk++) {
-                const int s = kk * C, e = min(n, s + C);
-                if (sm.cross_v[kk]) {
-                    // redone from the exact values; f0/f1 = state at the last residue of the previous chunk if the
-                    // state at t is 0/1 (the composition of the traceback maps, so the walk back below needs no
-                    // second pass over the chunk: its dependent loads of the just-written bytes cost more than the redo)
-                    int f0 = 0, f1 = 1;
-#pragma unroll 8
-                    for (int t = s; t < e; t++) {
-                        const double2 le = sm.le[ext[t] & 31];
-                        const double v00 = ks.lt00 + S0, v10 = ks.lt10 + S1, v01 = ks.lt01 + S0, v11 = ks.lt11 + S1;
-                        const bool p0 = v10 > v00, p1 = v11 > v01;
-                        S0 = (p0 ? v10 : v00) + le.x;
-                        S1 = (p1 ? v11 : v01) + le.y;
-                        tbT[(size_t)(t - s) * sR + (size_t)kk * sK] = (uint8_t)((int)p0 | ((int)p1 << 1));
-                        const int n0 = p0 ? f1 : f0, n1 = p1 ? f1 : f0;
-                        f0 = n0;
-                        f1 = n1;
-                    }
-                    sm.choice[kk] = (unsigned char)(f0 | (f1 << 1));
-                } else {
-                    const double R = sm.Sa[0][kk - 1];
-                    const double d0 = S0 - R, d1 = S1 - R;  // exact shifts
-                    const double x00 = d0 + sm.M[0][kk], x10 = d1 + sm.M[2][kk];
-                    const double x01 = d0 + sm.M[1][kk], x11 = d1 + sm.M[3][kk];
-                    const int ch0 = x10 > x00 ? 1 : 0, ch1 = x11 > x01 ? 1 : 0;
-                    S0 = ch0 ? x10 : x00;
-                    S1 = ch1 ? x11 : x01;
-                    sm.choice[kk] = (unsigned char)(ch0 | (ch1 << 1));
-                }
-            }
-            const double e0v = S0 + ks.lf0, e1v = S1 + ks.lf1;
-            const int vlast = e1v > e0v ? 1 : 0;
-            sm.vlast = vlast;
-            sm.lvit = vlast ? e1v : e0v;
-            int e = vlast;
-            for (int kk = K - 1; kk >= 1; kk--) {
-                sm.endstate[kk] = (unsigned char)e;
-                const int v = (sm.choice[kk] >> e) & 1;
-                sm.variant[kk] = sm.cross_v[kk] ? 0 : (unsigned char)v;  // redone chunks hold the exact bits as variant A
-                e = v;  // state at the last residue of the previous chunk
-            }
-            sm.endstate[0] = (unsigned char)e;
-            sm.variant[0] = 0;
-            LONG_STAMP_LANE(9);
-        } else if (wid == 3 && lane == 0 && do_main) {
-            // LLR window search: chunk maxima in order (first strict maximum), crossing chunks redone from exact values
-            double P = sm.q_inc[0][0], Pl = sm.q_mid[0];
-            double best = sm.q_best[0];
-            int stop = sm.q_stop[0];
-            for (int kk = 1; kk < K; kk++) {
-                const int s = kk * C, e = min(n, s + C);
-                double cand, Pl_next = P;
-                int cstop;
-                if (!sm.cross_q[0][kk]) {
-                    cand = sm.q_best[kk];
-                    cstop = sm.q_stop[kk];
-                    Pl_next = P + sm.q_mid[kk];
-                    P = P + sm.q_inc[0][kk];
-                } else {
-                    double lead = P, lag = Pl;
-                    cand = -INFINITY;
-                    cstop = -1;
-#pragma unroll 8
-                    for (int t = s; t < e; t++) {
-                        lead = lead + sm.llr[ext[t] & 31];
-                        lag = lag + sm.llr[ext[t - c] & 31];
-                        const double d = lead - lag;
-                        if (d > cand) {
-                            cand = d;
-                            cstop = t;
-                        }
-                        if (t == e - c - 1) Pl_next = lead;
-                    }
-                    P = lead;
-                }
-                if (cand > best) {
-                    best = cand;
-                    stop = cstop;
-                }
-                Pl = Pl_next;
-            }
-            sm.llr_best = best;
-            sm.llr_stop = stop;
-            LONG_STAMP_LANE(10);
-        } else if (wid == 4 && lane < 2 && do_main) {
-            // hmm0's emission sum (lane 0) and the hydropathy sum (lane 1)
-            const int q = 1 + lane;
-            double x = sm.q_inc[q][0];
-            for (int kk = 1; kk < K; kk++) {
-                if (!sm.cross_q[q][kk])
-                    x = x + sm.q_inc[q][kk];
-                else {
-                    const int s = kk * C, e = min(n, s + C);
-                    if (q == 1)
-                        for (int t = s; t < e; t++) x = x + sm.le[ext[t] & 31].x;
-                    else
-                        for (int t = s; t < e; t++) x = x + sm.hyd[ext[t] & 63];
-                }
-            }
-            if (q == 1)
-                sm.sum0 = x;
-            else
-                sm.sh = x;
-            LONG_STAMP_LANE(12 + lane);
-        } else if (wid == 5 && lane == 0 && do_main) {
-            int best = sm.m_best[0], stop = sm.m_stop[0], cq = sm.c_sum[0];
-            for (int kk = 1; kk < K; kk++) {
-                if (sm.m_best[kk] > best) {
-                    best = sm.m_best[kk];
-                    stop = sm.m_stop[kk];
-                }
-                cq += sm.c_sum[kk];
-            }
-            sm.mw_best = best;
-            sm.mw_stop = stop;
-            sm.csum = cq;
-        } else if (wid == 2 && lane == 0 && do_win) {
+        sm.fi_all[k] = all ? 1 : 0;
+        sm.fi_pre[k] = all ? cur : pre;
+        sm.fi_suf[k] = cur;
+        sm.fi_sum[k] = insum;
+        sm.fi_max[k] = inmax;
+        sm.p_cen[k] = pcen;
+        sm.p_tb[k] = Tb;
+        sm.p_wb[k] = Wb;
+        sm.p_vfi[k] = vfib;
+    }
+    long_chunk_bar();
+
+    if (win) {
+        if (tid != 0) return;
         // FoldIndex runs (:5010-5059) and PAPA centre (:4941-4948) merged in chunk order
         int open = 0, num = 0, mx = 0;
         int pcen = -1;
         double Tb = 0, Wb = 1, vfib = 0;
-        for (int k = 0; k < K; k++) {
-            if (sm.fi_all[k])
-                open += sm.fi_pre[k];
+        for (int kk = 0; kk < K; kk++) {
+            if (sm.fi_all[kk])
+                open += sm.fi_pre[kk];
             else {
-                const int r = open + sm.fi_pre[k];
+                const int r = open + sm.fi_pre[kk];
                 if (r >= 5) {
                     num += r;
                     mx = max(mx, r);
                 }
-                num += sm.fi_sum[k];
-                mx = max(mx, sm.fi_max[k]);
-                open = sm.fi_suf[k];
+                num += sm.fi_sum[kk];
+                mx = max(mx, sm.fi_max[kk]);
+                open = sm.fi_suf[kk];
             }
-            if (sm.p_cen[k] >= 0 && (pcen < 0 || sm.p_tb[k] * Wb > Tb * sm.p_wb[k])) {
-                Tb = sm.p_tb[k];
-                Wb = sm.p_wb[k];
-                vfib = sm.p_vfi[k];
-                pcen = sm.p_cen[k];
+            if (sm.p_cen[kk] >= 0 && (pcen < 0 || sm.p_tb[kk] * Wb > Tb * sm.p_wb[kk])) {
+                Tb = sm.p_tb[kk];
+                Wb = sm.p_wb[kk];
+                vfib = sm.p_vfi[kk];
+                pcen = sm.p_cen[kk];
             }
         }
         if (open >= 5) {
             num += open;
             mx = max(mx, open);
         }
-        sm.fi_numaa = num;
-        sm.fi_maxrun = mx;
-        sm.pcen = pcen;
-        sm.pTb = Tb;
-        sm.pWb = Wb;
-        sm.pVfi = vfib;
-        }
-        long_chunk_bar();
-        long_combined_arrive();
-        LONG_STAMP(4);
-        // ---- traceback of every chunk in parallel (:3110-3113) + run statistics for longestrun (:1787-1804)
-        if (live && !g.hmm_ext) {
-            int v = sm.endstate[k];
-            const int sh = 2 * sm.variant[k];
-            int cur = 0, suf = 0, inmax = 0;
-            bool closed = false;
-            uint32_t word = 0;
-#pragma unroll 8
-            for (int t = ce - 1; t >= cs; t--) {
-                word |= (uint32_t)v << (t & 31);
-                if (v)
-                    cur++;
-                else {
-                    if (!closed) {
-                        suf = cur;
-                        closed = true;
-                    } else
-                        inmax = max(inmax, cur);
-                    cur = 0;
-                }
-                if ((t & 31) == 0) {
-                    vit[t >> 5] = word;
-                    word = 0;
-                }
-                v = (tbk[(size_t)(t - cs) * sR] >> (sh + v)) & 1;
-            }
-            sm.v_all[k] = closed ? 0 : 1;
-            sm.v_pre[k] = cur;
-            sm.v_suf[k] = closed ? suf : cur;
-            sm.v_max[k] = inmax;
-        }
-        long_chunk_bar();
-    } else if (wid == kLongFwdWarp) {
-        long_pass2_bar();
-        if (lane == 0 && !g.hmm_ext) {
-            // forward: the chunk's trajectory is the jar's iff it enters the chunk with the bits of d the previous
-            // chunk left with; then its increment is added exactly.  Otherwise the chunk is redone from the exact values.
-            double A0 = sm.f_inc[0], dex = sm.f_dexit[0];
-            double A1 = A0 + dex;
-            int nfb = 0;
-            for (int kk = 1; kk < K; kk++) {
-                // a frame is the jar's trajectory iff it enters the chunk an EVEN number of ulps away from the true a0
-                // and with exactly the bits of d the previous chunk left with
-                int fr = -1;
-                if (!g.force_seq_forward && !sm.cross_f[kk]) {
-                    const double u = __hiloint2double((((__double2hiint(fabs(A0)) >> 20) & 0x7ff) - 52) << 20, 0);
-#pragma unroll
-                    for (int f = 0; f < 2; f++) {
-                        const double q = (sm.g_ea0[f][kk] - A0) / u;  // exact: a small integer
-                        if (fr < 0 && q == 2.0 * rint(0.5 * q) &&
-                            __double_as_longlong(sm.g_den[f][kk]) == __double_as_longlong(dex))
-                            fr = f;
-                    }
-                }
-                if (fr >= 0) {
-                    A0 = A0 + sm.g_inc[fr][kk];
-                    dex = sm.g_dex[fr][kk];
-                    A1 = A0 + dex;
-                } else {
-                    const int s = kk * C, e = min(n, s + C);
-#pragma unroll 8
-                    for (int t = s; t < e; t++) {
-                        const double2 le = sm.le[ext[t] & 31];
-                        const double f0 = lse_lut2<false>(ks.lt00 + A0, ks.lt10 + A1, lut_addr) + le.x;
-                        const double f1 = lse_lut2<false>(ks.lt01 + A0, ks.lt11 + A1, lut_addr) + le.y;
-                        A0 = f0;
-                        A1 = f1;
-                    }
-                    dex = A1 - A0;
-                    nfb += sm.cross_f[kk] ? 0 : 1;
-                }
-            }
-            sm.fwd_redone = nfb;
-            sm.lmarg = lse_lut2<false>(A0 + ks.lf0, A1 + ks.lf1, lut_addr);
-            LONG_STAMP_LANE(11);
-        }
-        long_combined_wait();
-        if (lane == 0 && !g.hmm_ext) {
-            g.out[prot].hmm_all = sm.lmarg - sm.sum0;
-            if (g.redone && sm.fwd_redone) atomicAdd(g.redone, (unsigned long long)sm.fwd_redone);
-        }
-        return;
-    } else
-        return;
-    LONG_STAMP(6);
-
-    if (tid != 0) return;
-    plaac_summary* r = g.out + prot;
-    if (do_main) {
-        r->prot_len = n;
-        r->mw_score = sm.mw_best;
-        r->mw_start = sm.mw_stop - mw + 1;
-        r->mw_end = sm.mw_stop;
-        r->llr = sm.llr_best;
-        r->llr_start = sm.llr_stop - c + 1;
-        r->llr_end = sm.llr_stop;
-        if (!g.hmm_ext) r->hmm_vit = sm.lvit - sm.sum0;
-        const double mh = (1.0 * sm.sh) / (double)n;
-        const double mc = (1.0 * (double)sm.csum) / (double)n;
-        r->fi_meanhydro = mh;
-        r->fi_meancharge = mc;
-        r->fi_meancombo = (ks.cc2 + ks.cc1 * fabs(mc)) + ks.cc0 * mh;
-    }
-    if (do_win) {
-        r->fi_numaa = sm.fi_numaa;
-        r->fi_maxrun = sm.fi_maxrun;
-        const int pcen = sm.pcen;
+        plaac_summary* r = g.out + prot;
+        r->fi_numaa = num;
+        r->fi_maxrun = mx;
         r->papa_center = pcen;
         if (pcen >= 0) {
-            const double prop = sm.pTb / sm.pWb;
+            const double prop = Tb / Wb;
             r->papa_combo = prop;
             r->papa_prop = prop;
-            r->papa_fi = sm.pVfi / sm.pWb;
+            r->papa_fi = vfib / Wb;
             const int full = 2 * w + 1;
             const int q0 = max(pcen - 2 * w, 0), q1 = min(pcen + 2 * w, n - 1);
             double sc = 0.0, den = 0.0, t2 = 0.0;
@@ -1066,123 +393,201 @@ __device__ __forceinline__ void long_score_body(const LongArgs& g)
                 t2 = t2 + x * (double)(full - dist);
             }
             r->papa_llr = sc / den;
-            r->papa_llr2 = t2 / sm.pWb;
+            r->papa_llr2 = t2 / Wb;
         } else {
             r->papa_combo = -INFINITY;
             r->papa_prop = r->papa_fi = r->papa_llr = r->papa_llr2 = nan("");
         }
-    }
-    if (g.hmm_ext) {
-        // Viterbi run statistics, CORE search and the two HMM scores: k_long_final, from k_long_post's parse
-        if (do_main) g.sum0_out[blockIdx.x] = sm.sum0;
         return;
     }
-    // longestrun
-    int open = 0, mx = 0;
-    for (int k = 0; k < K; k++) {
-        if (sm.v_all[k])
-            open += sm.v_pre[k];
-        else {
-            mx = max(mx, max(open + sm.v_pre[k], sm.v_max[k]));
-            open = sm.v_suf[k];
+
+    // ================= combine 1: approximate absolute values (they only fix the binade of pass 2) =================
+    if (wid == 0 && lane < 3) {
+        double run = 0.0;
+        for (int kk = 0; kk < K; kk++) {
+            sm.q_abs[lane][kk] = run;
+            run += sm.q_sum[lane][kk];
         }
     }
-    mx = max(mx, open);
-    r->vit_maxrun = mx;
-    r->core_start = -1;
-    r->core_end = -2;
-    r->prd_start = -1;
-    r->prd_end = -2;
-    r->core_score = nan("");
-    r->prd_score = 0.0;
-    LONG_STAMP(7);
-    if (mx < c) return;
-    // ---- CORE search on the masked sequence (:816-833), PrD expansion and PRDscore (:851-873), in reference order;
-    // masked stretches are applied as exact binade jumps when the masking constant is a negative integer.
-    const double big_neg = ks.big_neg;
-    const bool can_jump = big_neg < 0 && big_neg == floor(big_neg) && big_neg >= -4194304.0;
-    double ps = 0.0, lag = 0.0, best = -INFINITY, runsum = 0.0, prd_sc = 0.0;
-    int bstop = -1, run = 0, last = 0, run_start = 0, prd_s = -1, prd_e = -2;
-    bool hit = false;
-    const int nwords = (n + 31) >> 5, wpc = C >> 5;
-    for (int j = 0; j < nwords; j++) {
-        if (j % wpc == 0) {
-            // chunks without a Viterbi-1 residue are one masked stretch: skip their words
-            const int kk = j / wpc;
-            if (!sm.v_all[kk] && sm.v_pre[kk] == 0 && sm.v_suf[kk] == 0 && sm.v_max[kk] == 0) {
-                j += wpc - 1;
-                continue;
+    long_chunk_bar();
+    // ================= pass 2: the jar's own binade =================
+    // Every fp64 addition of a sum has one operand of the running magnitude, so it rounds to a multiple of that
+    // magnitude's ulp; rounding is monotone and commutes with shifts by multiples of the ulp as long as no operand changes
+    // its binade.  Re-run from an approximate absolute value, a chunk therefore reproduces the jar's sequential values up
+    // to an EXACT shift: increments and window differences are exact multiples of the ulp and their ordered combination
+    // is the jar's number bit for bit.  Chunks in which the magnitude crosses a power of two (about one per binade) are
+    // redone sequentially from the exact values.
+    if (live && k >= 1) {
+        double lagsum = 0;
+        for (int t = cs - c; t < cs; t++) lagsum += sm.llr[ext[t] & 31];
+        double lag = sm.q_abs[0][k] - lagsum;  // approximate psum before residue cs-c: fixes the frame
+        double lead = lag;
+        for (int t = cs - c; t < cs; t++) lead = lead + sm.llr[ext[t] & 31];
+        const double lead0 = lead;
+        double best = -INFINITY, mid = lead;
+        int stop = -1;
+        const double x10 = sm.q_abs[1][k], x20 = sm.q_abs[2][k];
+        double x1 = x10, x2 = x20;
+#pragma unroll 4
+        for (int t = cs; t < ce; t++) {
+            const uint32_t e = ext[t];
+            lead = lead + sm.llr[e & 31];
+            lag = lag + sm.llr[ext[t - c] & 31];
+            const double d = lead - lag;  // exact, and the jar's number
+            if (d > best) {
+                best = d;
+                stop = t;
             }
+            if (t == ce - c - 1) mid = lead;
+            x1 = x1 + sm.le0[e & 31];
+            x2 = x2 + sm.hyd[e & 63];
         }
-        uint32_t bits = vit[j];
-        while (bits) {
-            const int i = __ffs((int)bits) - 1;
-            bits &= bits - 1;
-            const int p = 32 * j + i;
-            if (p != last) {
-                if (hit) {
-                    prd_s = run_start;
-                    prd_e = last - 1;
-                    prd_sc = runsum;
-                    hit = false;
+        sm.q_inc[0][k] = lead - lead0;
+        sm.q_mid[k] = mid - lead0;
+        sm.q_best[k] = best;
+        sm.q_stop[k] = stop;
+        sm.q_inc[1][k] = x1 - x10;
+        sm.q_inc[2][k] = x2 - x20;
+    }
+    if (live) {
+        // crossing test over every value the running sum takes in the region (for the LLR search the lagged sum
+        // starts c residues before the chunk, i.e. inside the previous chunk)
+#pragma unroll
+        for (int q = 0; q < 3; q++) {
+            double mn = sm.q_abs[q][k] + sm.q_min[q][k], mx = sm.q_abs[q][k] + sm.q_max[q][k];
+            if (q == 0 && k >= 1) {
+                mn = fmin(mn, sm.q_abs[0][k - 1] + sm.q_min[0][k - 1]);
+                mx = fmax(mx, sm.q_abs[0][k - 1] + sm.q_max[0][k - 1]);
+            }
+            const double lo = fmin(fabs(mn), fabs(mx)) * (1.0 - 1e-6), hi = fmax(fabs(mn), fabs(mx)) * (1.0 + 1e-6);
+            const bool cross = k == 0 || !(mn > 0.0 || mx < 0.0) || !(lo >= 1.0) ||
+                               (__double2hiint(lo) >> 20) != (__double2hiint(hi) >> 20) ||
+                               ((g.tie_mask[q] >> (((__double2hiint(lo) >> 20) & 0x7ff) - 1023)) & 1ull);
+            sm.cross_q[q][k] = cross ? 1 : 0;
+        }
+        if (k == 0) {
+            // first chunk: the true chains from residue 0 (hss2 :1206-1257, mean() :1584, hmm0's emission sum)
+            double ps = 0, psl = 0, best = 0, mid = 0;
+            int stop = -2;
+            double s0 = 0, shy = 0;
+#pragma unroll 8
+            for (int t = 0; t < ce; t++) {
+                const uint32_t e = ext[t];
+                ps = ps + sm.llr[e & 31];
+                if (t >= c) psl = psl + sm.llr[ext[t - c] & 31];
+                if (t >= c - 1) {
+                    const double d = ps - psl;
+                    if (t == c - 1 || d > best) {
+                        best = d;
+                        stop = t;
+                    }
                 }
-                if (can_jump)
-                    ps = masked_jump(ps, p - last, big_neg);
+                if (t == ce - c - 1) mid = ps;
+                s0 = (t == 0) ? sm.le0[e & 31] : s0 + sm.le0[e & 31];
+                shy = shy + sm.hyd[e & 63];
+            }
+            sm.q_inc[0][0] = ps, sm.q_mid[0] = mid, sm.q_best[0] = best, sm.q_stop[0] = stop;
+            sm.q_inc[1][0] = s0;
+            sm.q_inc[2][0] = shy;
+        }
+    }
+    long_chunk_bar();
+    // ================= combine 2: exact, in chunk order =================
+    if (wid == 0 && lane == 0) {
+        // LLR window search: chunk maxima in order (first strict maximum), crossing chunks redone from exact values
+        double P = sm.q_inc[0][0], Pl = sm.q_mid[0];
+        double best = sm.q_best[0];
+        int stop = sm.q_stop[0];
+        for (int kk = 1; kk < K; kk++) {
+            const int s = kk * C, e = min(n, s + C);
+            double cand, Pl_next = P;
+            int cstop;
+            if (!sm.cross_q[0][kk]) {
+                cand = sm.q_best[kk];
+                cstop = sm.q_stop[kk];
+                Pl_next = P + sm.q_mid[kk];
+                P = P + sm.q_inc[0][kk];
+            } else {
+                double lead = P, lag = Pl;
+                cand = -INFINITY;
+                cstop = -1;
+#pragma unroll 8
+                for (int t = s; t < e; t++) {
+                    lead = lead + sm.llr[ext[t] & 31];
+                    lag = lag + sm.llr[ext[t - c] & 31];
+                    const double d = lead - lag;
+                    if (d > cand) {
+                        cand = d;
+                        cstop = t;
+                    }
+                    if (t == e - c - 1) Pl_next = lead;
+                }
+                P = lead;
+            }
+            if (cand > best) {
+                best = cand;
+                stop = cstop;
+            }
+            Pl = Pl_next;
+        }
+        sm.llr_best = best;
+        sm.llr_stop = stop;
+    } else if (wid == 1 && lane < 2) {
+        // hmm0's emission sum (lane 0) and the hydropathy sum (lane 1)
+        const int q = 1 + lane;
+        double x = sm.q_inc[q][0];
+        for (int kk = 1; kk < K; kk++) {
+            if (!sm.cross_q[q][kk])
+                x = x + sm.q_inc[q][kk];
+            else {
+                const int s = kk * C, e = min(n, s + C);
+                if (q == 1)
+                    for (int t = s; t < e; t++) x = x + sm.le0[ext[t] & 31];
                 else
-                    for (int q = last; q < p; q++) ps = ps + big_neg;
-                run = 0;
+                    for (int t = s; t < e; t++) x = x + sm.hyd[ext[t] & 63];
             }
-            if (run == 0) {
-                lag = ps;
-                run_start = p;
-                runsum = 0.0;
-            }
-            const double x = sm.llr[ext[p] & 31];
-            ps = ps + x;
-            runsum = runsum + x;
-            if (run >= c - 1) {
-                const double d = ps - lag;
-                if (d > best) {
-                    best = d;
-                    bstop = p;
-                    hit = true;
-                }
-                lag = lag + sm.llr[ext[p - c + 1] & 31];
-            }
-            run++;
-            last = p + 1;
         }
+        if (q == 1)
+            sm.sum0 = x;
+        else
+            sm.sh = x;
+    } else if (wid == 2 && lane == 0) {
+        int best = sm.m_best[0], stop = sm.m_stop[0], cq = sm.c_sum[0];
+        for (int kk = 1; kk < K; kk++) {
+            if (sm.m_best[kk] > best) {
+                best = sm.m_best[kk];
+                stop = sm.m_stop[kk];
+            }
+            cq += sm.c_sum[kk];
+        }
+        sm.mw_best = best;
+        sm.mw_stop = stop;
+        sm.csum = cq;
     }
-    if (hit) {
-        prd_s = run_start;
-        prd_e = last - 1;
-        prd_sc = runsum;
-    }
-    LONG_STAMP(8);
-    if (best > big_neg / 2) {
-        r->core_start = bstop - c + 1;
-        r->core_end = bstop;
-        r->core_score = best;
-        r->prd_start = prd_s;
-        r->prd_end = prd_e;
-        r->prd_score = prd_sc;
-    }
+    long_chunk_bar();
+
+    if (tid != 0) return;
+    plaac_summary* r = g.out + prot;
+    r->prot_len = n;
+    r->mw_score = sm.mw_best;
+    r->mw_start = sm.mw_stop - mw + 1;
+    r->mw_end = sm.mw_stop;
+    r->llr = sm.llr_best;
+    r->llr_start = sm.llr_stop - c + 1;
+    r->llr_end = sm.llr_stop;
+    const double mh = (1.0 * sm.sh) / (double)n;
+    const double mc = (1.0 * (double)sm.csum) / (double)n;
+    r->fi_meanhydro = mh;
+    r->fi_meancharge = mc;
+    r->fi_meancombo = (ks.cc2 + ks.cc1 * fabs(mc)) + ks.cc0 * mh;
+    g.sum0_out[blockIdx.x] = sm.sum0;
 }
 
-__global__ void __launch_bounds__(kLongThreads, 1) k_long_score(LongArgs g)
-{
-    // one instantiation per layout: the choice is per protein (per CTA), the strides are compile-time constants
-    const int32_t prot = g.list[blockIdx.x];
-    if (g.offsets[prot + 1] - g.offsets[prot] >= g.cm_min)
-        long_score_body<true>(g);
-    else
-        long_score_body<false>(g);
-}
-
-// The Viterbi-dependent columns of a long protein whose HMM columns come from k_long_post (LongArgs::hmm_ext): Viterbi
-// bytes -> bit words, longestrun (:1787-1804), the -1e6-masked CORE search with PrD expansion and PRDscore (:816-873)
-// exactly as at the end of k_long_score.  It needs nothing from k_long_score (residue codes straight from the input), so
-// it runs behind k_long_post while k_long_score is still at work; k_long_fix then writes the two HMM scores.
+// The Viterbi-dependent columns of a long protein, from k_long_post's parse: Viterbi bytes -> bit words, longestrun
+// (:1787-1804), the -1e6-masked CORE search with PrD expansion and PRDscore (:816-873), in reference order; masked
+// stretches are applied as exact binade jumps when the masking constant is a negative integer.  It needs nothing from
+// k_long_score (residue codes straight from the input), so it runs behind k_long_post while k_long_score is still at
+// work; k_long_fix then writes the two HMM scores.
 constexpr int kLongFinalThreads = 256;
 __global__ void __launch_bounds__(kLongFinalThreads)
 k_long_final(LongArgs g, const uint8_t* __restrict__ vbytes_all, const uint8_t* __restrict__ vit_out, int64_t res_base)

@@ -63,8 +63,8 @@ struct LongPostArgs {
     int cluster;                 // CTAs per protein of this launch; the launch handles proteins of its size class only
     int64_t big_min;             // class boundary: n >= big_min belongs to the kLpBigCluster launch
     unsigned long long* redone;  // statistics: chunks redone sequentially although they had frames
-    // Viterbi parse (viterbidecodel :3077-3121) for calls without records, where k_long_score does not run: chunk
-    // transfer matrices, a max-plus scan for the binades, two exact frames per chunk, exact combine, parallel traceback
+    // Viterbi parse (viterbidecodel :3077-3121), for records and for out.vit: chunk transfer matrices, a max-plus scan
+    // for the binades, two exact frames per chunk, exact combine, parallel traceback
     int want_vit;
     int want_post;               // 0: records only (summary mode): forward + Viterbi, no backward pass, no per-residue arrays
     double* hmm_out;             // per listed protein {lmarginalprob, lviterbiprob} (:3369-3375, :3102-3108) for k_long_final
@@ -810,19 +810,6 @@ __global__ void __launch_bounds__(kLpThreads, 1) k_long_post(LongPostArgs g)
         if (bad && g.errflag) atomicOr(g.errflag, 1);
     }
     LP_STAMP(7);
-}
-
-// Viterbi bits of the long proteins (k_long_score's bit words) -> one byte per residue of out.vit
-__global__ void __launch_bounds__(256)
-k_long_vit_bytes(const int64_t* __restrict__ offsets, int64_t res_base, const int32_t* __restrict__ list,
-                 const int64_t* __restrict__ scratch_off, const uint32_t* __restrict__ vit, uint8_t* __restrict__ out)
-{
-    const int32_t prot = list[blockIdx.y];
-    const int64_t o = offsets[prot];
-    const int n = (int)(offsets[prot + 1] - o);
-    const uint32_t* w = vit + (scratch_off[blockIdx.y] >> 5);
-    uint8_t* dst = out + (o - res_base);
-    for (int t = blockIdx.x * blockDim.x + threadIdx.x; t < n; t += gridDim.x * blockDim.x) dst[t] = (uint8_t)((w[t >> 5] >> (t & 31)) & 1u);
 }
 
 }  // namespace plaac

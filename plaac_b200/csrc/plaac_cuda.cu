@@ -51,7 +51,7 @@ struct Slot {
     DevBuf ing_agg, ing_cnt, ing_base, ing_misc;                 // FASTA ingest scratch
     DevBuf ing_text, ing_codes, ing_offsets, ing_npos, ing_nlen, ing_flags, ing_hist;  // staging for the host-buffer ingest
     DevBuf rk_keys[2], rk_vals[2], rk_hist, rk_offs, rk_order;                         // ranking scratch
-    DevBuf lg_list, lg_off, lg_cnt, lg_ext, lg_extT, lg_tb, lg_vit;                             // long-sequence path
+    DevBuf lg_list, lg_off, lg_cnt, lg_ext, lg_ext_win, lg_tb, lg_vit;                          // long-sequence path
     DevBuf lp_s0, lp_s1, lp_bnd, lp_lpseq;          // ... in per-residue mode (long_residue.cuh)
     DevBuf lg_hmm, lg_sum0, lg_vb;                  // ... records with the HMM columns from k_long_post (k_long_final)
     unsigned long long* h_long = nullptr;  // pinned: [0] long proteins, [1] scratch residues, or 3 x kLongBins bins
@@ -399,7 +399,7 @@ void slot_free(Slot& s)
                       &s.res_b1, &s.res_a0, &s.res_a1, &s.res_mapw, &s.res_lpseq, &s.ing_agg, &s.ing_cnt, &s.ing_base,
                       &s.ing_misc, &s.ing_text, &s.ing_codes, &s.ing_offsets, &s.ing_npos, &s.ing_nlen, &s.ing_flags,
                       &s.ing_hist, &s.rk_keys[0], &s.rk_keys[1], &s.rk_vals[0], &s.rk_vals[1], &s.rk_hist, &s.rk_offs,
-                      &s.rk_order, &s.lg_list, &s.lg_off, &s.lg_cnt, &s.lg_ext, &s.lg_extT, &s.lg_tb, &s.lg_vit, &s.lg_bins, &s.lp_s0, &s.lp_s1, &s.lp_bnd, &s.lp_lpseq, &s.lg_hmm, &s.lg_sum0, &s.lg_vb})
+                      &s.rk_order, &s.lg_list, &s.lg_off, &s.lg_cnt, &s.lg_ext, &s.lg_ext_win, &s.lg_tb, &s.lg_vit, &s.lg_bins, &s.lp_s0, &s.lp_s1, &s.lp_bnd, &s.lp_lpseq, &s.lg_hmm, &s.lg_sum0, &s.lg_vb})
         release(*b);
     if (s.h_long) cudaFreeHost(s.h_long);
     if (s.h_stage_codes) cudaFreeHost(s.h_stage_codes);
@@ -449,7 +449,7 @@ bool long_res_ok(const plaac_ctx* ctx)
     return ctx->res_plan.ok && ctx->v2_nwr > 0 && ctx->variant != 1 && !getenv("PLAAC_NO_LONG_RES");
 }
 
-// Automatic threshold (long_min == -1).  The long-sequence path is a LATENCY device: one CTA per protein is far less
+// Automatic threshold (long_min == -1).  The long-sequence path is a LATENCY device: whole CTAs per protein are far less
 // efficient per residue than the bucketed kernel, so a protein goes there only if its sequential walk (~170 ns per
 // residue in a lane of the bucketed kernel) would be a visible part of the batch's time, and only as many proteins
 // as fit one wave of CTAs.  bins: k_long_levels' layout (or the host walk's).  Returns the threshold (0 = none) and
@@ -468,7 +468,8 @@ LongChoice choose_long_threshold(const plaac_ctx* ctx, const unsigned long long*
     for (int b = kLongBins - 1; b >= 0; b--) {  // suffix sums: proteins with len >= long_edge(b)
         if (long_edge(b) < lb) break;
         // (per-residue mode: k_long_post takes a whole SM per protein (190 KB of shared memory) and the bucketed kernels need
-        // SMs beside it -- with records k_long_score runs too; measured on a yeast-sized set: 46 long proteins 0.75 ms, 146: 0.78)
+        // SMs beside it -- with records k_long_score's two CTAs per protein run too; measured on a yeast-sized set: 46 long
+        // proteins 0.75 ms, 146: 0.78)
         if (cnt + (int64_t)bins[b] > (two_ctas ? ctx->sm_count / 2 : ctx->sm_count)) break;
         cnt += (int64_t)bins[b];
         if (long_edge(b) >= kLpBigMin) c.nbig += (int64_t)bins[b];
@@ -531,8 +532,7 @@ int run_batch(plaac_ctx* ctx, Slot& s, const uint8_t* d_codes, const int64_t* d_
         // automatic threshold with device-resident offsets: bin the lengths, let the host choose
         if ((rc = ensure(ctx, s.lg_bins, 3 * kLongBins * sizeof(unsigned long long)))) return rc;
         CU(ctx, cudaMemsetAsync(s.lg_bins.p, 0, 3 * kLongBins * sizeof(unsigned long long), st));
-        k_long_levels<<<(unsigned)((nprot + 255) / 256), 256, 0, st>>>(d_offsets, nprot, ctx->ks.core_len, ctx->ks.mw_window,
-                                                                      (unsigned long long*)s.lg_bins.p);
+        k_long_levels<<<(unsigned)((nprot + 255) / 256), 256, 0, st>>>(d_offsets, nprot, (unsigned long long*)s.lg_bins.p);
         ctx->stats.kernel_launches += 1;
         CU(ctx, cudaMemcpyAsync(s.h_long, s.lg_bins.p, 3 * kLongBins * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
         CU(ctx, cudaStreamSynchronize(st));
@@ -552,8 +552,7 @@ int run_batch(plaac_ctx* ctx, Slot& s, const uint8_t* d_codes, const int64_t* d_
         // [0] count, [1] scratch cursor, [2] count of >= kLpBigMin residues, [3] redone chunks (cumulative)
         if ((rc = ensure(ctx, s.lg_cnt, 32 + 16 * 8))) return rc;
         CU(ctx, cudaMemsetAsync(s.lg_cnt.p, 0, 24, st));
-        k_long_select<<<(unsigned)((nprot + 255) / 256), 256, 0, st>>>(d_offsets, nprot, long_min, ctx->ks.core_len,
-                                                                      ctx->ks.mw_window, (int32_t*)s.lg_list.p,
+        k_long_select<<<(unsigned)((nprot + 255) / 256), 256, 0, st>>>(d_offsets, nprot, long_min, (int32_t*)s.lg_list.p,
                                                                       (int64_t*)s.lg_off.p, (unsigned long long*)s.lg_cnt.p,
                                                                       (int64_t)kLpBigMin);
         ctx->stats.kernel_launches += 1;
@@ -642,15 +641,21 @@ int run_batch(plaac_ctx* ctx, Slot& s, const uint8_t* d_codes, const int64_t* d_
     }
     CU(ctx, cudaEventRecord(s.ev_b, st));
     bool long_launched = false;
-    // k_long_score on its own stream, launched first: its CTAs (one per long protein) take SMs while the persistent CTAs
-    // of the bucketed kernel start on the others and pick up the rest of the queue as SMs free up.  In per-residue mode it
-    // also supplies the Viterbi bits of the long proteins, and the posterior kernel runs beside it on a stream of its own.
+    // The long-sequence path on streams of its own, launched first: its CTAs take SMs while the persistent CTAs of the
+    // bucketed kernel start on the others and pick up the rest of the queue as SMs free up.  k_long_post (one thread-block
+    // cluster per long protein) computes the per-residue arrays, or for records the forward score and the Viterbi parse;
+    // with records, k_long_score computes the other columns beside it (two CTAs per protein), k_long_final the
+    // Viterbi-dependent columns right behind the cluster kernel, and k_long_fix the two HMM scores when both are done.
     cudaStream_t long_st = d_res ? s.aux4 : s.aux1;
     if (use_long && nlong > 0) {
         if ((rc = ensure(ctx, s.lg_ext, (size_t)long_scratch + 256))) return rc;
-        if ((rc = ensure(ctx, s.lg_extT, (size_t)long_scratch + 256))) return rc;
+        if ((rc = ensure(ctx, s.lg_ext_win, (size_t)long_scratch + 256))) return rc;
         if ((rc = ensure(ctx, s.lg_tb, (size_t)long_scratch + 256))) return rc;
         if ((rc = ensure(ctx, s.lg_vit, (size_t)long_scratch / 8 + 256))) return rc;
+        // PLAAC_LONG_TIES (testing): "1" treats every binade as a tie binade (everything redone sequentially), "0"
+        // ignores the masks (shows what they are for)
+        const char* ties_env = getenv("PLAAC_LONG_TIES");
+        auto tie_mask = [&](int i) { return !ties_env ? ctx->long_tie[i] : (ties_env[0] == '0' ? 0ull : ~0ull >> 1); };
         LongArgs la;
         la.codes = d_codes;
         la.offsets = d_offsets;
@@ -661,127 +666,89 @@ int run_batch(plaac_ctx* ctx, Slot& s, const uint8_t* d_codes, const int64_t* d_
         la.tabs = ctx->d_tabs;
         la.out = d_summaries;
         la.ext = (uint8_t*)s.lg_ext.p;
-        la.extT = (uint8_t*)s.lg_extT.p;
-        la.cm_min = getenv("PLAAC_LONG_CM_MIN") ? atoi(getenv("PLAAC_LONG_CM_MIN")) : kLongChunkMajorMin;
-        la.tb = (uint8_t*)s.lg_tb.p;
+        la.ext_win = (uint8_t*)s.lg_ext_win.p;
         la.vit = (uint32_t*)s.lg_vit.p;
         la.errflag = (int*)s.errflag.p;
-        la.redone = (unsigned long long*)((char*)s.lg_cnt.p + 24);
-        la.dbg_clocks = getenv("PLAAC_LONG_CLOCKS") ? (long long*)((char*)s.lg_cnt.p + 32) : nullptr;
-        // PLAAC_LONG_TIES (testing): "1" treats every binade as a tie binade (everything redone sequentially), "0"
-        // ignores the masks (shows what they are for)
-        const char* ties_env = getenv("PLAAC_LONG_TIES");
-        for (int i = 0; i < 4; i++)
-            la.tie_mask[i] = !ties_env ? ctx->long_tie[i] : (ties_env[0] == '0' ? 0ull : ~0ull >> 1);
-        la.warm = std::max(1, std::abs(ctx->long_warm));
-        la.force_seq_forward = ctx->long_warm < 0 ? 1 : 0;
+        for (int i = 0; i < 3; i++) la.tie_mask[i] = tie_mask(1 + i);
         CU(ctx, cudaEventRecord(s.ev_fork, st));
         CU(ctx, cudaStreamWaitEvent(long_st, s.ev_fork, 0));
-        // (a per-residue call without records gets its Viterbi parse from k_long_post instead)
         const bool run_score = d_summaries != nullptr;
-        // Records: the HMM columns (Viterbi parse, lviterbiprob, lmarginalprob) come from
-        // k_long_post's thread-block cluster, k_long_score computes the rest beside it on its own SM and k_long_final
-        // completes the record.  PLAAC_LONG_HYBRID=0: k_long_score alone (one CTA per protein, the round-1 path).
-        const bool hybrid = run_score && !(getenv("PLAAC_LONG_HYBRID") && getenv("PLAAC_LONG_HYBRID")[0] == '0');
-        if (hybrid) {
+        if (run_score) {
             if ((rc = ensure(ctx, s.lg_hmm, sizeof(double) * 2 * (size_t)nlong))) return rc;
             if ((rc = ensure(ctx, s.lg_sum0, sizeof(double) * (size_t)nlong))) return rc;
             if ((rc = ensure(ctx, s.lg_vb, (size_t)long_scratch + 256))) return rc;
-            la.hmm_ext = 1;
             la.sum0_out = (double*)s.lg_sum0.p;
-            // (without the Viterbi and forward loops the protein-major copy is the faster one at every length: 100 k residues
-            // 0.785 -> 0.755 ms)
-            if (!getenv("PLAAC_LONG_CM_MIN")) la.cm_min = 0x7fffffff;
-            // the window columns on a second CTA (it needs the protein-major layout: its ext copy lives in extT's space)
-            la.split = (la.cm_min == 0x7fffffff && !(getenv("PLAAC_LONG_SPLIT") && getenv("PLAAC_LONG_SPLIT")[0] == '0')) ? 1 : 0;
-        } else {
-            la.hmm_ext = 0;
-            la.sum0_out = nullptr;
-            la.split = 0;
-        }
-        if (run_score) {
-            k_long_score<<<dim3((unsigned)nlong, la.split ? 2u : 1u), kLongThreads, sizeof(LongShared), long_st>>>(la);
+            k_long_score<<<dim3((unsigned)nlong, 2), kLongThreads, sizeof(LongShared), long_st>>>(la);
             ctx->stats.kernel_launches += 1;
         }
         long_launched = true;
         ctx->stats.long_proteins += nlong;
-        if (d_res || hybrid) {
-            if (d_res && d_res->vit && run_score && !hybrid) {
-                for (int64_t off = 0; off < nlong; off += 65535) {
-                    k_long_vit_bytes<<<dim3(8, (unsigned)std::min<int64_t>(65535, nlong - off)), 256, 0, long_st>>>(
-                        d_offsets, res_base, la.list + off, la.scratch_off + off, la.vit, d_res->vit);
-                    ctx->stats.kernel_launches += 1;
-                }
-            }
-            // one cluster per long protein, two size classes: posteriors + MAP parse (+ Viterbi parse), or, for records,
-            // the forward score and the Viterbi parse
-            if (d_res) {
-                if ((rc = ensure(ctx, s.lp_s0, sizeof(double) * ((size_t)long_scratch + 256)))) return rc;
-                if ((rc = ensure(ctx, s.lp_s1, sizeof(double) * ((size_t)long_scratch + 256)))) return rc;
-                if ((rc = ensure(ctx, s.lp_lpseq, sizeof(double) * (size_t)nlong))) return rc;
-            }
-            const int64_t bnd_plane = long_scratch / 32 + 64;
-            if ((rc = ensure(ctx, s.lp_bnd, sizeof(double) * (size_t)kLpBndPlanes * (size_t)bnd_plane))) return rc;
-            LongPostArgs pa;
-            pa.codes = d_codes;
-            pa.offsets = d_offsets;
-            pa.off_base = off_base;
-            pa.res_base = res_base;
-            pa.list = la.list;
-            pa.scratch_off = la.scratch_off;
-            pa.ks = ctx->ks;
-            pa.tabs = ctx->d_tabs;
-            if (d_res)
-                pa.out = *d_res;
-            else
-                memset(&pa.out, 0, sizeof(pa.out));
-            pa.S0 = d_res ? (double*)s.lp_s0.p : nullptr;
-            pa.S1 = d_res ? (double*)s.lp_s1.p : nullptr;
-            pa.bnd = (double*)s.lp_bnd.p;
-            pa.bnd_plane = bnd_plane;
-            pa.lpseq = d_res ? (double*)s.lp_lpseq.p : nullptr;
-            pa.warm = std::max(1, std::abs(ctx->long_warm));
-            pa.warm2 = getenv("PLAAC_LP_WARM2") ? atoi(getenv("PLAAC_LP_WARM2")) : 64;
-            pa.big_min = getenv("PLAAC_LP_BIG_MIN") ? atoll(getenv("PLAAC_LP_BIG_MIN")) : (int64_t)kLpBigMin;
-            pa.redone = la.redone;
-            pa.want_post = d_res ? 1 : 0;
-            pa.want_vit = hybrid ? 1 : ((!run_score && d_res->vit) ? 1 : 0);
-            pa.hmm_out = hybrid ? (double*)s.lg_hmm.p : nullptr;
-            pa.vbytes = (hybrid && !(d_res && d_res->vit)) ? (uint8_t*)s.lg_vb.p : nullptr;
-            pa.tb = la.tb;
-            pa.vit_tie_mask = la.tie_mask[0];
-            pa.errflag = la.errflag;
-            pa.dbg_clocks = (getenv("PLAAC_LONG_CLOCKS") && !run_score) ? (long long*)((char*)s.lg_cnt.p + 32) : nullptr;
-            CU(ctx, cudaStreamWaitEvent(s.aux5, s.ev_fork, 0));
-            if (pa.big_min != kLpBigMin) nbig = -1;  // (testing: the class counts are those of the default boundary)
-            for (int cls = 0; cls < 2; cls++) {
-                const int64_t ncls = nbig < 0 ? nlong : (cls ? nbig : nlong - nbig);
-                if (ncls == 0) continue;
-                pa.cluster = cls ? kLpBigCluster : 1;
-                cudaLaunchConfig_t cfg = {};
-                cfg.gridDim = dim3((unsigned)(nlong * pa.cluster));
-                cfg.blockDim = dim3(kLpThreads);
-                cfg.dynamicSmemBytes = sizeof(LpShared);
-                cfg.stream = s.aux5;
-                cudaLaunchAttribute at[1];
-                at[0].id = cudaLaunchAttributeClusterDimension;
-                at[0].val.clusterDim.x = (unsigned)pa.cluster;
-                at[0].val.clusterDim.y = 1;
-                at[0].val.clusterDim.z = 1;
-                cfg.attrs = at;
-                cfg.numAttrs = 1;
-                CU(ctx, cudaLaunchKernelEx(&cfg, k_long_post, pa));
-                ctx->stats.kernel_launches += 1;
-            }
-            if (hybrid) {
-                // the Viterbi-dependent columns right behind the cluster kernel, beside k_long_score; the two HMM scores
-                // when both are done
-                k_long_final<<<(unsigned)nlong, kLongFinalThreads, 0, s.aux5>>>(la, (const uint8_t*)s.lg_vb.p, (d_res && d_res->vit) ? d_res->vit : nullptr, res_base);
-                CU(ctx, cudaEventRecord(s.ev_j5, s.aux5));
-                CU(ctx, cudaStreamWaitEvent(long_st, s.ev_j5, 0));
-                k_long_fix<<<(unsigned)((nlong + 127) / 128), 128, 0, long_st>>>(la, (const double*)s.lg_hmm.p, (int)nlong);
-                ctx->stats.kernel_launches += 2;
-            }
+        // one cluster per long protein, two size classes: posteriors + MAP parse (+ Viterbi parse), or, for records,
+        // the forward score and the Viterbi parse
+        if (d_res) {
+            if ((rc = ensure(ctx, s.lp_s0, sizeof(double) * ((size_t)long_scratch + 256)))) return rc;
+            if ((rc = ensure(ctx, s.lp_s1, sizeof(double) * ((size_t)long_scratch + 256)))) return rc;
+            if ((rc = ensure(ctx, s.lp_lpseq, sizeof(double) * (size_t)nlong))) return rc;
+        }
+        const int64_t bnd_plane = long_scratch / 32 + 64;
+        if ((rc = ensure(ctx, s.lp_bnd, sizeof(double) * (size_t)kLpBndPlanes * (size_t)bnd_plane))) return rc;
+        LongPostArgs pa;
+        pa.codes = d_codes;
+        pa.offsets = d_offsets;
+        pa.off_base = off_base;
+        pa.res_base = res_base;
+        pa.list = la.list;
+        pa.scratch_off = la.scratch_off;
+        pa.ks = ctx->ks;
+        pa.tabs = ctx->d_tabs;
+        if (d_res)
+            pa.out = *d_res;
+        else
+            memset(&pa.out, 0, sizeof(pa.out));
+        pa.S0 = d_res ? (double*)s.lp_s0.p : nullptr;
+        pa.S1 = d_res ? (double*)s.lp_s1.p : nullptr;
+        pa.bnd = (double*)s.lp_bnd.p;
+        pa.bnd_plane = bnd_plane;
+        pa.lpseq = d_res ? (double*)s.lp_lpseq.p : nullptr;
+        pa.warm = std::max(1, std::abs(ctx->long_warm));
+        pa.warm2 = getenv("PLAAC_LP_WARM2") ? atoi(getenv("PLAAC_LP_WARM2")) : 64;
+        pa.big_min = getenv("PLAAC_LP_BIG_MIN") ? atoll(getenv("PLAAC_LP_BIG_MIN")) : (int64_t)kLpBigMin;
+        pa.redone = (unsigned long long*)((char*)s.lg_cnt.p + 24);
+        pa.want_post = d_res ? 1 : 0;
+        pa.want_vit = (run_score || d_res->vit) ? 1 : 0;
+        pa.hmm_out = run_score ? (double*)s.lg_hmm.p : nullptr;
+        pa.vbytes = (run_score && !(d_res && d_res->vit)) ? (uint8_t*)s.lg_vb.p : nullptr;
+        pa.tb = (uint8_t*)s.lg_tb.p;
+        pa.vit_tie_mask = tie_mask(0);
+        pa.errflag = la.errflag;
+        pa.dbg_clocks = (getenv("PLAAC_LONG_CLOCKS") && !run_score) ? (long long*)((char*)s.lg_cnt.p + 32) : nullptr;
+        CU(ctx, cudaStreamWaitEvent(s.aux5, s.ev_fork, 0));
+        if (pa.big_min != kLpBigMin) nbig = -1;  // (testing: the class counts are those of the default boundary)
+        for (int cls = 0; cls < 2; cls++) {
+            const int64_t ncls = nbig < 0 ? nlong : (cls ? nbig : nlong - nbig);
+            if (ncls == 0) continue;
+            pa.cluster = cls ? kLpBigCluster : 1;
+            cudaLaunchConfig_t cfg = {};
+            cfg.gridDim = dim3((unsigned)(nlong * pa.cluster));
+            cfg.blockDim = dim3(kLpThreads);
+            cfg.dynamicSmemBytes = sizeof(LpShared);
+            cfg.stream = s.aux5;
+            cudaLaunchAttribute at[1];
+            at[0].id = cudaLaunchAttributeClusterDimension;
+            at[0].val.clusterDim.x = (unsigned)pa.cluster;
+            at[0].val.clusterDim.y = 1;
+            at[0].val.clusterDim.z = 1;
+            cfg.attrs = at;
+            cfg.numAttrs = 1;
+            CU(ctx, cudaLaunchKernelEx(&cfg, k_long_post, pa));
+            ctx->stats.kernel_launches += 1;
+        }
+        if (run_score) {
+            k_long_final<<<(unsigned)nlong, kLongFinalThreads, 0, s.aux5>>>(la, (const uint8_t*)s.lg_vb.p, (d_res && d_res->vit) ? d_res->vit : nullptr, res_base);
+            CU(ctx, cudaEventRecord(s.ev_j5, s.aux5));
+            CU(ctx, cudaStreamWaitEvent(long_st, s.ev_j5, 0));
+            k_long_fix<<<(unsigned)((nlong + 127) / 128), 128, 0, long_st>>>(la, (const double*)s.lg_hmm.p, (int)nlong);
+            ctx->stats.kernel_launches += 2;
         }
     }
     if (d_summaries && use_v2) {
@@ -1695,13 +1662,13 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
                 // decided after the walk (choose_long_threshold)
                 const int b = long_bin(len);
                 bins[b]++;
-                bins[kLongBins + b] += (unsigned long long)long_scratch_need(len, ctx->ks.core_len, ctx->ks.mw_window);
+                bins[kLongBins + b] += (unsigned long long)long_scratch_need(len);
                 bins[2 * kLongBins + b] = std::max<unsigned long long>(bins[2 * kLongBins + b], (unsigned long long)len);
             } else if (long_min > 0 && len >= long_min) {
                 // scored by the long-sequence path; the bucketed stream sees an empty protein
                 nlp++;
                 nbigp += len >= kLpBigMin;
-                lp_scratch += long_scratch_need(len, ctx->ks.core_len, ctx->ks.mw_window);
+                lp_scratch += long_scratch_need(len);
             } else {
                 lmax = std::max(lmax, len);
                 nlong += len >= kHistBins;

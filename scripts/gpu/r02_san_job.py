@@ -11,13 +11,10 @@ codes = np.concatenate([sc_, lc]); lens = np.concatenate([np.diff(so), np.diff(l
 offs = np.zeros(len(lens) + 1, np.int64); np.cumsum(lens, out=offs[1:])
 sc = plaac_b200.Scorer(); sc.set_long_path(1024)
 ref_s = orc.score_batch(orc.make_params(), codes, offs)
-for hyb in ("1", "0"):
-    os.environ["PLAAC_LONG_HYBRID"] = hyb
-    got_s = sc.score(codes, offs)   # records only: k_long_post (forward + Viterbi) beside k_long_score, k_long_final, k_long_fix
-    for f in ("core_start", "core_end", "vit_maxrun", "llr_start", "mw_score", "fi_numaa"):
-        assert (got_s[f] == ref_s[f]).all(), f
-    assert np.abs(got_s["hmm_all"] - ref_s["hmm_all"]).max() < 1e-9 and np.abs(got_s["hmm_vit"] - ref_s["hmm_vit"]).max() < 1e-9
-os.environ["PLAAC_LONG_HYBRID"] = "1"
+got_s = sc.score(codes, offs)   # records only: k_long_post (forward + Viterbi) beside k_long_score, k_long_final, k_long_fix
+for f in ("core_start", "core_end", "vit_maxrun", "llr_start", "mw_score", "fi_numaa"):
+    assert (got_s[f] == ref_s[f]).all(), f
+assert np.abs(got_s["hmm_all"] - ref_s["hmm_all"]).max() < 1e-9 and np.abs(got_s["hmm_vit"] - ref_s["hmm_vit"]).max() < 1e-9
 for big in (None, "1024"):
     if big: os.environ["PLAAC_LP_BIG_MIN"] = big
     summ, res = sc.score(codes, offs, per_residue=True)

@@ -181,9 +181,11 @@ def test_long_path_mixed_batch_thresholds_and_fallback():
     sc.close()
 
 
-def test_long_path_both_scratch_layouts(monkeypatch):
-    """k_long_score walks a protein-major copy of the residues below 49 152 residues and a chunk-major one above
-    (LongArgs::extT): force each layout on proteins of both sizes; records must be the same bytes, and right."""
+def test_long_path_around_the_chunk_geometry():
+    """Long proteins of 8 192 to 60 001 residues on the default path (two CTAs of k_long_score per protein beside the
+    cluster kernel), some ending exactly on a chunk boundary (8 192 and 49 152: 32 and 192 chunks of 256 residues) and
+    others one residue off it or between, with Q/N-rich segments at a seventh, the middle and the end: records must be
+    right."""
     rng = np.random.default_rng(4242)
     bg = synth.BG_SCER / synth.BG_SCER.sum()
     prd = synth.PRD_28 / synth.PRD_28.sum()
@@ -195,16 +197,11 @@ def test_long_path_both_scratch_layouts(monkeypatch):
         seqs.append(s)
     codes, offs = plaac_b200.pack(seqs)
     ref = orc.score_batch(orc.make_params(), codes, offs, nthreads=NT)
-    recs = {}
-    for cm_min in ("0", "49152", "1000000"):
-        monkeypatch.setenv("PLAAC_LONG_CM_MIN", cm_min)
-        sc = plaac_b200.Scorer(device=0)
-        got = sc.score(codes, offs)
-        assert sc.stats().long_proteins == len(seqs)
-        sc.close()
-        _check(got, ref, f"long path, chunk-major from {cm_min}")
-        recs[cm_min] = got.tobytes()
-    assert recs["0"] == recs["49152"] == recs["1000000"]
+    sc = plaac_b200.Scorer(device=0)
+    got = sc.score(codes, offs)
+    assert sc.stats().long_proteins == len(seqs)
+    sc.close()
+    _check(got, ref, "long path around the chunk geometry")
 
 
 @pytest.mark.parametrize("kw", [dict(core_len=30), dict(core_len=100, ww1=21, ww2=21), dict(ww1=40, ww2=40),
