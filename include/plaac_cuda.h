@@ -198,6 +198,32 @@ int plaac_score_packed(plaac_ctx *ctx, const uint32_t *words, const int32_t *len
 /* The same compact output for the one-byte codes of plaac_score(). */
 int plaac_score_hits(plaac_ctx *ctx, const uint8_t *codes, const int64_t *offsets, int64_t nprot, plaac_hits *hits);
 
+/* ---- sequence variants (DESIGN.md section 11): substitution lists expanded on the device --------------------------
+ * Variants of the proteins of a reference batch: variant v is protein protein[v] with the residues at
+ * pos[first_sub[v] .. first_sub[v+1]) replaced by code[...] (0-based positions, strictly increasing within a variant;
+ * a variant with no substitution is the wild type). */
+typedef struct plaac_variants {
+    int64_t nvar;
+    const int32_t *protein;    /* nvar indices into the reference batch */
+    const int64_t *first_sub;  /* nvar + 1, first_sub[0] == 0, non-decreasing */
+    const int32_t *pos;        /* first_sub[nvar] positions, each < the protein's length */
+    const uint8_t *code;       /* first_sub[nvar] new residue codes, 0..21 */
+} plaac_variants;
+
+/* codes/offsets/nprot: the reference batch, exactly as plaac_score takes it (HOST buffers).  summaries: nvar records in
+ * variant order, each byte-identical to plaac_score's record for the mutated protein.  Blocks until done.  Summary mode
+ * only.  The reference is uploaded once; per chunk of the variant list only its slice of the four arrays crosses the
+ * link, and the variant residues are built on the device.
+ * PLAAC_E_INVALID, with the variant's index in plaac_last_error: a protein index outside [0, nprot), a position outside
+ * the protein, positions of a variant that do not strictly increase, a code > 21, a bad first_sub array, or a NULL array
+ * with nvar > 0.  The substitutions are validated during the chunk walk, so the records of earlier chunks may already
+ * have been written when such an error is returned.  nvar == 0: PLAAC_OK, nothing written.  Reference bytes > 21 are
+ * scored as X and reported as PLAAC_E_INVALID after the batch, as in plaac_score.  The call's chunks use the automatic
+ * long-path threshold (plaac_set_long_path(ctx, -1, .)) whatever the ctx's setting, which it leaves unchanged: records do
+ * not depend on the threshold, and equal-length variants are scored most efficiently by the bucketed kernel. */
+int plaac_score_variants(plaac_ctx *ctx, const uint8_t *codes, const int64_t *offsets, int64_t nprot,
+                         const plaac_variants *variants, plaac_summary *summaries);
+
 /* ---- multi-GPU (SURVEY.md section 8e): proteins are independent, so the batch is cut into contiguous,
  * residue-balanced shards, one per ctx (each ctx on its own GPU), scored concurrently by one host thread per
  * ctx, each writing its records / per-residue rows straight into the caller's arrays at the input position.

@@ -77,6 +77,13 @@ class Hits(C.Structure):
                 ("index", C.c_void_p), ("count", C.c_int64), ("n_core", C.c_int64)]
 
 
+class Variants(C.Structure):
+    _fields_ = [("nvar", C.c_int64), ("protein", C.c_void_p), ("first_sub", C.c_void_p), ("pos", C.c_void_p),
+                ("code", C.c_void_p)]
+
+
+assert C.sizeof(Variants) == 40
+
 _lib = None
 
 
@@ -150,6 +157,8 @@ def lib():
         L.plaac_score_multi_packed.restype = C.c_int
         L.plaac_score_multi_packed.argtypes = [C.POINTER(vp), C.c_int, vp, vp, i64, i64, vp, C.POINTER(ResidueOut), C.POINTER(Hits)]
         L.plaac_score_hits.restype = C.c_int
+        L.plaac_score_variants.restype = C.c_int
+        L.plaac_score_variants.argtypes = [vp, vp, vp, i64, C.POINTER(Variants), vp]
         L.plaac_score_hits.argtypes = [vp, vp, vp, i64, C.POINTER(Hits)]
         L.plaac_bench_synth_lengths.restype = C.c_int
         L.plaac_bench_synth_lengths.argtypes = [vp, C.c_uint64, i64, i64, dbl, dbl, i32, i32, vp]
@@ -383,6 +392,30 @@ class Scorer:
         self._check(lib().plaac_score_hits(self._h, codes.ctypes.data, offsets.ctypes.data, nprot, C.byref(h)))
         return {"records": rec[:h.count], "index": idx[:h.count], "n_core": int(h.n_core)}
 
+    def score_variants(self, codes: np.ndarray, offsets: np.ndarray, protein: np.ndarray, first_sub: np.ndarray,
+                       pos: np.ndarray, code: np.ndarray, out: np.ndarray | None = None) -> np.ndarray:
+        """plaac_score_variants: variant v is reference protein protein[v] with the residues at
+        pos[first_sub[v]:first_sub[v+1]] replaced by code[...]; returns one record per variant, each the record score()
+        gives for the mutated protein.  The variant residues are built on the GPU (see saturation()).  out: optional
+        record array (e.g. a PinnedBuffer's) of len(protein) rows."""
+        codes = np.ascontiguousarray(codes, dtype=np.uint8)
+        offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+        protein = np.ascontiguousarray(protein, dtype=np.int32)
+        first_sub = np.ascontiguousarray(first_sub, dtype=np.int64)
+        pos = np.ascontiguousarray(pos, dtype=np.int32)
+        code = np.ascontiguousarray(code, dtype=np.uint8)
+        nvar = len(protein)
+        if len(first_sub) != nvar + 1:
+            raise ValueError(f"first_sub has {len(first_sub)} entries, expected nvar + 1 = {nvar + 1}")
+        if out is None:
+            out = np.zeros(nvar, dtype=SUMMARY_DTYPE)
+        assert out.dtype == SUMMARY_DTYPE and out.flags.c_contiguous and len(out) == nvar
+        v = Variants(nvar=nvar, protein=protein.ctypes.data, first_sub=first_sub.ctypes.data, pos=pos.ctypes.data,
+                     code=code.ctypes.data)
+        self._check(lib().plaac_score_variants(self._h, codes.ctypes.data, offsets.ctypes.data, len(offsets) - 1,
+                                               C.byref(v), out.ctypes.data))
+        return out
+
     def score_ptr(self, codes_ptr: int, offsets_ptr: int, nprot: int, summaries_ptr: int):
         """Raw host pointers (e.g. pinned torch tensors)."""
         self._check(lib().plaac_score(self._h, codes_ptr, offsets_ptr, nprot, summaries_ptr, None))
@@ -469,6 +502,40 @@ class Scorer:
         s = Stats()
         self._check(lib().plaac_get_stats(self._h, C.byref(s)))
         return s
+
+
+SATURATION_CODES = np.arange(1, 21, dtype=np.uint8)  # A C D E F G H I K L M N P Q R S T V W Y
+
+
+def saturation(codes: np.ndarray, offsets: np.ndarray, proteins=None):
+    """Every single substitution of the given reference proteins (default: all), as the four arrays of
+    Scorer.score_variants: (protein, first_sub, pos, code).  Per protein: the wild type first, then the positions in
+    ascending order, at each one every code 1..20 (A C D E F G H I K L M N P Q R S T V W Y) other than the residue
+    there (all 20 if that residue is X or '*')."""
+    codes = np.asarray(codes, dtype=np.uint8)
+    offsets = np.asarray(offsets, dtype=np.int64)
+    if proteins is None:
+        proteins = np.arange(len(offsets) - 1)
+    proteins = np.asarray(proteins, dtype=np.int64)
+    parts_prot, parts_pos, parts_code = [], [], []
+    for p in proteins:
+        ref = codes[offsets[p]:offsets[p + 1]]
+        alt = np.broadcast_to(SATURATION_CODES, (len(ref), 20))
+        keep = alt != ref[:, None]  # (a residue outside 1..20 keeps all 20)
+        pos = np.broadcast_to(np.arange(len(ref), dtype=np.int32)[:, None], (len(ref), 20))[keep]
+        parts_pos.append(pos)
+        parts_code.append(alt[keep])
+        parts_prot.append(np.full(len(pos) + 1, p, dtype=np.int32))
+    if not parts_prot:
+        return np.zeros(0, np.int32), np.zeros(1, np.int64), np.zeros(0, np.int32), np.zeros(0, np.uint8)
+    protein = np.concatenate(parts_prot)
+    pos = np.concatenate(parts_pos)
+    code = np.concatenate(parts_code)
+    # the wild type of each protein has no substitution, every other variant one
+    nsub = np.concatenate([np.r_[0, np.ones(len(x), np.int64)] for x in parts_pos])
+    first_sub = np.zeros(len(protein) + 1, dtype=np.int64)
+    np.cumsum(nsub, out=first_sub[1:])
+    return protein, first_sub, np.ascontiguousarray(pos, dtype=np.int32), np.ascontiguousarray(code, dtype=np.uint8)
 
 
 def shard_plan(offsets: np.ndarray, nshards: int) -> np.ndarray:

@@ -27,6 +27,7 @@
 #include "long_residue.cuh"
 #include "lean.cuh"
 #include "generic_windows.cuh"
+#include "variants.cuh"
 
 using namespace plaac;
 
@@ -45,6 +46,7 @@ struct Slot {
     DevBuf hist, cursor, order, nchunks, chunk_base, stream_buf, tbw, slot_bucket, errflag, core_list, core_count, scan_tmp, gen_f64;
     DevBuf codes, offsets, summaries;  // staging for the host-buffer API
     DevBuf words, lengths;             // ... of its packed form (plaac_score_packed)
+    DevBuf v_prot, v_first, v_pos, v_code;  // the chunk's slice of a variant list (plaac_score_variants)
     DevBuf hit_flag, hit_pos;          // compact ranked output (plaac_hits)
     DevBuf res_u8, res_f64;            // per-residue staging for the host-buffer API
     DevBuf res_b0, res_b1, res_a0, res_a1, res_mapw, res_lpseq;  // per-residue scratch (bucketed layout)
@@ -86,6 +88,7 @@ struct plaac_ctx {
     Slot slot[kSlots];
     DevBuf all_summaries;      // records of a whole host-buffer call, kept on the device for the compact ranked output
     DevBuf union_rec, union_idx, union_order, union_out_idx;  // plaac_score_multi_packed: the shards' hit rows merged on this GPU
+    DevBuf var_ref, var_ref_off;  // reference batch of plaac_score_variants, uploaded once per call
     // pageable <-> device copies of the FASTA calls: two pinned staging buffers, filled / emptied by a multi-threaded memcpy
     void* stage_buf[2] = {nullptr, nullptr};
     cudaEvent_t stage_ev[2] = {nullptr, nullptr};
@@ -395,7 +398,7 @@ int slot_init(plaac_ctx* ctx, Slot& s)
 void slot_free(Slot& s)
 {
     for (DevBuf* b : {&s.gen_f64, &s.scan_tmp, &s.hist, &s.cursor, &s.order, &s.nchunks, &s.chunk_base, &s.stream_buf, &s.tbw, &s.slot_bucket, &s.errflag,
-                      &s.core_list, &s.core_count, &s.codes, &s.offsets, &s.summaries, &s.words, &s.lengths, &s.hit_flag, &s.hit_pos, &s.res_u8, &s.res_f64, &s.res_b0,
+                      &s.core_list, &s.core_count, &s.codes, &s.offsets, &s.summaries, &s.words, &s.lengths, &s.v_prot, &s.v_first, &s.v_pos, &s.v_code, &s.hit_flag, &s.hit_pos, &s.res_u8, &s.res_f64, &s.res_b0,
                       &s.res_b1, &s.res_a0, &s.res_a1, &s.res_mapw, &s.res_lpseq, &s.ing_agg, &s.ing_cnt, &s.ing_base,
                       &s.ing_misc, &s.ing_text, &s.ing_codes, &s.ing_offsets, &s.ing_npos, &s.ing_nlen, &s.ing_flags,
                       &s.ing_hist, &s.rk_keys[0], &s.rk_keys[1], &s.rk_vals[0], &s.rk_vals[1], &s.rk_hist, &s.rk_offs,
@@ -1242,7 +1245,7 @@ void plaac_destroy(plaac_ctx* ctx)
     cudaSetDevice(ctx->device);
     for (int i = 0; i < kSlots; i++) slot_free(ctx->slot[i]);
     release(ctx->all_summaries);
-    for (DevBuf* b : {&ctx->union_rec, &ctx->union_idx, &ctx->union_order, &ctx->union_out_idx}) release(*b);
+    for (DevBuf* b : {&ctx->union_rec, &ctx->union_idx, &ctx->union_order, &ctx->union_out_idx, &ctx->var_ref, &ctx->var_ref_off}) release(*b);
     for (int b = 0; b < 2; b++) {
         if (ctx->stage_buf[b]) cudaFreeHost(ctx->stage_buf[b]);
         if (ctx->stage_ev[b]) cudaEventDestroy(ctx->stage_ev[b]);
@@ -1491,8 +1494,8 @@ try {
 
 namespace {
 
-// What the host-buffer calls are given: one-byte codes + int64 offsets (plaac_score), or radix-22 words + int32
-// lengths (plaac_score_packed).
+// What the host-buffer calls are given: one-byte codes + int64 offsets (plaac_score), radix-22 words + int32
+// lengths (plaac_score_packed), or a variant list over a reference batch of one-byte codes (plaac_score_variants).
 struct HostInput {
     const uint8_t* codes = nullptr;
     const int64_t* offsets = nullptr;
@@ -1501,8 +1504,64 @@ struct HostInput {
     int64_t nres = 0;  // packed input: the caller's total (checked against the lengths)
     int64_t pos0 = 0;  // packed input: residue index, counted from digit 0 of words[0], of the first protein (a shard of a
                        // larger batch starts in the middle of a word)
+    const plaac_variants* var = nullptr;  // variant input: codes / offsets hold the nref proteins of the reference
+    int64_t nref = 0;
     bool packed() const { return words != nullptr || lengths != nullptr; }
 };
+
+// Variant input: checks the reference, uploads it into the ctx buffers (once per call) and returns the total residue
+// count of the variants.  Protein indices and first_sub are checked here, the substitutions during the chunk walk.
+int variants_prepare(plaac_ctx* ctx, const HostInput& in, int64_t& total)
+{
+    const plaac_variants& V = *in.var;
+    if (in.nref < 0) return fail(ctx, PLAAC_E_INVALID, "negative reference protein count");
+    if (!V.protein || !V.first_sub || !V.pos || !V.code) return fail(ctx, PLAAC_E_INVALID, "NULL variant array with nvar = %lld", (long long)V.nvar);
+    if (!in.offsets) return fail(ctx, PLAAC_E_INVALID, "NULL reference offsets");
+    for (int64_t i = 0; i < in.nref; i++)
+        if (in.offsets[i + 1] < in.offsets[i]) return fail(ctx, PLAAC_E_INVALID, "reference offsets not monotone at protein %lld", (long long)i);
+    const int64_t ref_base = in.offsets[0], ref_n = in.offsets[in.nref] - ref_base;
+    if (ref_n > 0 && !in.codes) return fail(ctx, PLAAC_E_INVALID, "NULL reference codes");
+    if (V.first_sub[0] != 0) return fail(ctx, PLAAC_E_INVALID, "variant 0: first_sub[0] is %lld, not 0", (long long)V.first_sub[0]);
+    total = 0;
+    for (int64_t v = 0; v < V.nvar; v++) {
+        const int32_t p = V.protein[v];
+        if (p < 0 || p >= in.nref)
+            return fail(ctx, PLAAC_E_INVALID, "variant %lld: protein index %d outside [0, %lld)", (long long)v, p, (long long)in.nref);
+        if (V.first_sub[v + 1] < V.first_sub[v])
+            return fail(ctx, PLAAC_E_INVALID, "variant %lld: first_sub decreases (%lld after %lld)", (long long)v,
+                        (long long)V.first_sub[v + 1], (long long)V.first_sub[v]);
+        total += in.offsets[p + 1] - in.offsets[p];
+    }
+    int rc;
+    if ((rc = ensure(ctx, ctx->var_ref, (size_t)ref_n + 64))) return rc;
+    if ((rc = ensure(ctx, ctx->var_ref_off, sizeof(int64_t) * (size_t)(in.nref + 1)))) return rc;
+    // (every call blocks until done, so no earlier chunk still reads these buffers; the slots' streams start after this
+    // synchronisation)
+    cudaStream_t st = ctx->slot[0].stream;
+    if ((rc = h2d_any(ctx, ctx->var_ref.p, in.codes + ref_base, (size_t)ref_n, st))) return rc;
+    if ((rc = h2d_any(ctx, ctx->var_ref_off.p, in.offsets, sizeof(int64_t) * (size_t)(in.nref + 1), st))) return rc;
+    CU(ctx, cudaStreamSynchronize(st));
+    return PLAAC_OK;
+}
+
+// Substitutions [fs, fe) of variant v on a protein of len residues.
+int check_subs(plaac_ctx* ctx, const plaac_variants& V, int64_t v, int64_t len)
+{
+    int64_t prev = -1;
+    for (int64_t j = V.first_sub[v]; j < V.first_sub[v + 1]; j++) {
+        const int64_t q = V.pos[j];
+        if (q < 0 || q >= len)
+            return fail(ctx, PLAAC_E_INVALID, "variant %lld: position %lld outside the protein (length %lld)", (long long)v,
+                        (long long)q, (long long)len);
+        if (q <= prev)
+            return fail(ctx, PLAAC_E_INVALID, "variant %lld: positions do not strictly increase (%lld after %lld)",
+                        (long long)v, (long long)q, (long long)prev);
+        if (V.code[j] > 21)
+            return fail(ctx, PLAAC_E_INVALID, "variant %lld: substitution code %d > 21", (long long)v, (int)V.code[j]);
+        prev = q;
+    }
+    return PLAAC_OK;
+}
 
 // Compact ranked output of a whole host-buffer call: the records of every chunk were kept in ctx->all_summaries.
 // on_device: the rows stay on the GPU (slot 0: `summaries` holds the hits->count ranked records, `rk_order` their indices
@@ -1589,7 +1648,10 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
         return PLAAC_OK;
     }
     const bool packed = in.packed();
-    if (packed) {
+    const plaac_variants* var = in.var;
+    if (var) {
+        if (per_res || hits) return fail(ctx, PLAAC_E_INVALID, "variants are scored in summary mode only");
+    } else if (packed) {
         if (!in.lengths) return fail(ctx, PLAAC_E_INVALID, "NULL lengths");
         if (in.nres < 0 || (in.nres > 0 && !in.words)) return fail(ctx, PLAAC_E_INVALID, "NULL words / negative nres");
     } else {
@@ -1601,6 +1663,8 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
     const bool want_rec = summaries || hits;  // the device computes records
     int rc = PLAAC_OK;
     if (hits && (rc = ensure(ctx, ctx->all_summaries, sizeof(plaac_summary) * (size_t)nprot))) return rc;
+    int64_t var_total = 0;
+    if (var && (rc = variants_prepare(ctx, in, var_total))) return rc;
 
     // Chunking: bounded device footprint; kSlots sets of buffers so the next chunks' H2D overlap this chunk's kernels and
     // D2H.  Chunk sizes ramp up from max/8 and down again towards the end: the first chunk's copy and the last chunk's
@@ -1608,8 +1672,8 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
     // (different half-widths of the windows: 64 bytes of track scratch per residue, so summary mode chunks like per-residue mode)
     const int64_t max_res_full = (per_res || ctx->generic_windows) ? std::min(ctx->chunk_res_pr, ctx->chunk_res) : ctx->chunk_res;
     const int64_t min_res = std::max<int64_t>(max_res_full / 8, 1 << 20);
-    const int64_t first_off = packed ? 0 : in.offsets[0];
-    const int64_t total_res = packed ? in.nres : in.offsets[nprot] - first_off;
+    const int64_t first_off = packed || var ? 0 : in.offsets[0];
+    const int64_t total_res = var ? var_total : packed ? in.nres : in.offsets[nprot] - first_off;
     int64_t ramp = min_res;
     const int64_t max_prot = ctx->chunk_prot;
     int64_t start = 0;
@@ -1622,7 +1686,7 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
     // through pinned staging buffers of the slot, filled / emptied by a multi-threaded memcpy that overlaps the copies
     // and kernels of the other slots.
     const void* in_main = packed ? (const void*)in.words : (const void*)(in.codes + first_off);
-    const bool stage_in = total_res > 0 && !host_is_pinned(in_main);
+    const bool stage_in = !var && total_res > 0 && !host_is_pinned(in_main);
     const bool stage_sum = summaries && !host_is_pinned(summaries);
     auto drain = [&](int i) -> int {
         if (!pending[i]) return PLAAC_OK;
@@ -1643,11 +1707,14 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
         int64_t lmax = 0, nlong = 0, nlp = 0, lp_scratch = 0, nres = 0, nbigp = 0;
         const bool long_allowed = !per_res || long_res_ok(ctx);
         int64_t long_min = long_allowed ? effective_long_min(ctx) : 0;
-        const bool long_auto = long_allowed && ctx->long_min < 0 && ctx->v2_nwr > 0 && ctx->variant != 1;
+        // (variants: always the automatic threshold -- at a fixed one, a saturation scan of a 10 000-residue protein would
+        // send 190 000 equal-length variants to the latency path instead of the bucketed kernel)
+        const bool long_auto = long_allowed && (ctx->long_min < 0 || var) && ctx->v2_nwr > 0 && ctx->variant != 1;
         unsigned long long bins[3 * kLongBins];
         if (long_auto) memset(bins, 0, sizeof(bins));
         while (end < nprot && end - start < max_prot) {
-            const int64_t len = packed ? (int64_t)in.lengths[end] : in.offsets[end + 1] - in.offsets[end];
+            const int64_t len = var ? in.offsets[var->protein[end] + 1] - in.offsets[var->protein[end]]
+                                    : packed ? (int64_t)in.lengths[end] : in.offsets[end + 1] - in.offsets[end];
             if (len < 0) {
                 rc = fail(ctx, PLAAC_E_INVALID, packed ? "negative length at protein %lld" : "offsets not monotone at protein %lld",
                           (long long)end);
@@ -1658,6 +1725,7 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
                 break;
             }
             if (end != start && nres + len > max_res) break;
+            if (var && (rc = check_subs(ctx, *var, end, len))) break;
             if (long_auto && len >= 1024) {
                 // decided after the walk (choose_long_threshold)
                 const int b = long_bin(len);
@@ -1715,9 +1783,14 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
             if (s.codes.cap != cap0) CUB(cudaMemsetAsync(s.codes.p, 0, s.codes.cap, s.stream));
         }
         if ((rc = ensure(ctx, s.offsets, sizeof(int64_t) * (np + 1)))) break;
-        if (packed) {
-            if ((rc = ensure(ctx, s.words, sizeof(uint32_t) * (size_t)(nwords + 4)))) break;
-            if ((rc = ensure(ctx, s.lengths, sizeof(int32_t) * (size_t)np))) break;
+        if (packed && (rc = ensure(ctx, s.words, sizeof(uint32_t) * (size_t)(nwords + 4)))) break;
+        if ((packed || var) && (rc = ensure(ctx, s.lengths, sizeof(int32_t) * (size_t)np))) break;
+        const int64_t fs0 = var ? var->first_sub[start] : 0, nsub = var ? var->first_sub[end] - fs0 : 0;
+        if (var) {
+            if ((rc = ensure(ctx, s.v_prot, sizeof(int32_t) * (size_t)np))) break;
+            if ((rc = ensure(ctx, s.v_first, sizeof(int64_t) * (size_t)(np + 1)))) break;
+            if ((rc = ensure(ctx, s.v_pos, sizeof(int32_t) * (size_t)nsub))) break;
+            if ((rc = ensure(ctx, s.v_code, (size_t)nsub))) break;
         }
         plaac_summary* d_sum = nullptr;
         if (hits)
@@ -1758,7 +1831,32 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
         if (stage_sum && (rc = ensure_host(ctx, s.h_stage_sum, s.h_stage_sum_cap, sizeof(plaac_summary) * (size_t)np))) break;
         const uint8_t* d_codes = (const uint8_t*)s.codes.p;
         int64_t off_base = first_off + pos;  // offsets[] of the chunk are relative to this residue index
-        if (packed) {
+        if (var) {
+            // only the chunk's slice of the variant list crosses the link; its residues are built from the reference
+            CUB(cudaMemcpyAsync(s.v_prot.p, var->protein + start, sizeof(int32_t) * (size_t)np, cudaMemcpyHostToDevice, s.stream));
+            CUB(cudaMemcpyAsync(s.v_first.p, var->first_sub + start, sizeof(int64_t) * (size_t)(np + 1), cudaMemcpyHostToDevice, s.stream));
+            if (nsub > 0) {
+                CUB(cudaMemcpyAsync(s.v_pos.p, var->pos + fs0, sizeof(int32_t) * (size_t)nsub, cudaMemcpyHostToDevice, s.stream));
+                CUB(cudaMemcpyAsync(s.v_code.p, var->code + fs0, (size_t)nsub, cudaMemcpyHostToDevice, s.stream));
+            }
+            k_variant_lengths<<<(unsigned)((np + 255) / 256), 256, 0, s.stream>>>((const int32_t*)s.v_prot.p, np,
+                                                                                  (const int64_t*)ctx->var_ref_off.p, (int32_t*)s.lengths.p);
+            ctx->stats.kernel_launches += 1;
+            if ((rc = launch_scan(ctx, s, (const int32_t*)s.lengths.p, (int64_t*)s.offsets.p, np, s.stream))) break;
+            if (nres > 0) {
+                k_variant_expand<<<(unsigned)((nres + kExpandTile - 1) / kExpandTile), kExpandThreads, 0, s.stream>>>(
+                    (const uint8_t*)ctx->var_ref.p, (const int64_t*)ctx->var_ref_off.p, in.offsets[0], (const int32_t*)s.v_prot.p,
+                    (const int64_t*)s.offsets.p, np, nres, (uint8_t*)s.codes.p);
+                ctx->stats.kernel_launches += 1;
+            }
+            if (nsub > 0) {
+                k_variant_apply<<<(unsigned)((nsub + 255) / 256), 256, 0, s.stream>>>((const int64_t*)s.v_first.p, fs0, np,
+                                                                                     (const int32_t*)s.v_pos.p, (const uint8_t*)s.v_code.p,
+                                                                                     nsub, (const int64_t*)s.offsets.p, (uint8_t*)s.codes.p);
+                ctx->stats.kernel_launches += 1;
+            }
+            off_base = 0;
+        } else if (packed) {
             if (main_bytes > 0) CUB(cudaMemcpyAsync(s.words.p, src_main, main_bytes, cudaMemcpyHostToDevice, s.stream));
             CUB(cudaMemcpyAsync(s.lengths.p, in.lengths + start, sizeof(int32_t) * (size_t)np, cudaMemcpyHostToDevice, s.stream));
             if (nwords > 0) {
@@ -1884,6 +1982,21 @@ try {
     return score_host(ctx, in, nprot, summaries, per_res, hits);
 } catch (...) {
     return api_caught(ctx, "plaac_score_packed");
+}
+
+int plaac_score_variants(plaac_ctx* ctx, const uint8_t* codes, const int64_t* offsets, int64_t nprot,
+                         const plaac_variants* variants, plaac_summary* summaries)
+try {
+    if (!ctx) return fail(nullptr, PLAAC_E_INVALID, "plaac_score_variants: NULL ctx");
+    if (!variants) return fail(ctx, PLAAC_E_INVALID, "plaac_score_variants: NULL variants");
+    HostInput in;
+    in.codes = codes;
+    in.offsets = offsets;
+    in.nref = nprot;
+    in.var = variants;
+    return score_host(ctx, in, variants->nvar, summaries, nullptr, nullptr);
+} catch (...) {
+    return api_caught(ctx, "plaac_score_variants");
 }
 
 }  // extern "C"

@@ -17,6 +17,13 @@
 //                   record-aligned pieces of --batch-mb, pieces round-robin over --gpus, rows formatted on all host
 //                   threads; summary table only.  The default for regular files of at least 1 MB; --host-reader forces
 //                   the reader of this program instead
+//   --variants FILE score sequence variants of the -i records instead of the records (plaac_score_variants): one line
+//                   per variant, "SEQid<TAB>spec", spec = WT or comma-separated substitutions <ref><pos><alt> with a
+//                   1-based position (D262V or D262V,P275S); SEQid is matched against record names as -p matches them.
+//                   One row per variant, named <name>:<SPEC>, in record order and within a record in file order
+//   --saturate      every single substitution of every -i record (wild type first, then positions in ascending order,
+//                   at each one the 20 residues A..Y other than the one there)
+#include <algorithm>
 #include <charconv>
 #include <cmath>
 #include <cstdint>
@@ -399,6 +406,8 @@ struct Options {
     bool compat_F = false;
     bool gpu_ingest = false, host_reader = false;
     bool rank = false, rank_core_only = false;
+    std::string variants_file;  // --variants
+    bool saturate = false;      // --saturate
 };
 
 struct Scorers {
@@ -442,18 +451,30 @@ int die(const Scorers& S, int rc, const char* what)
     return 2;
 }
 
+// Substitutions of a sequence variant (positions ascending): the string columns of its row are the wild type's cut with
+// these patched in, so a row costs no more than its printed residues.
+struct SubList {
+    const int32_t* pos = nullptr;
+    const uint8_t* code = nullptr;
+    int64_t n = 0;
+};
+
 // One row of the summary table (plaac.java:899-945) appended to `out`.
-void aa_sub_into(std::string& out, const uint8_t* aa, int m, int r1, int r2)
+void aa_sub_into(std::string& out, const uint8_t* aa, int m, int r1, int r2, const SubList& subs = SubList())
 {
     if (m <= 0) return;
     if (r1 < 0) r1 = 0;
     if (r2 < r1) r2 = r1;
     if (r1 >= m) r1 = m - 1;
     if (r2 >= m) r2 = m - 1;
+    const size_t o = out.size();
     for (int i = r1; i <= r2; i++) out.push_back(kAaNames[aa[i]]);
+    for (const int32_t* p = std::lower_bound(subs.pos, subs.pos + subs.n, r1); p < subs.pos + subs.n && *p <= r2; p++)
+        out[o + (size_t)(*p - r1)] = kAaNames[subs.code[p - subs.pos]];
 }
 
-void append_summary_row(const Options& o, std::string_view name, const plaac_summary& s, const uint8_t* aa, std::string& out)
+void append_summary_row(const Options& o, std::string_view name, const plaac_summary& s, const uint8_t* aa, std::string& out,
+                        const SubList& subs = SubList())
 {
     const int n = s.prot_len;
     if (n < 1) return;  // :762
@@ -468,15 +489,15 @@ void append_summary_row(const Options& o, std::string_view name, const plaac_sum
     F(inf2nan(s.core_score)), I(s.core_start + 1), I(s.core_end + 1), I(s.core_end - s.core_start + 1);
     F(s.prd_score), I(s.prd_start + 1), I(s.prd_end + 1), I(prdlen), I(n), F(s.hmm_all), F(s.hmm_vit);
     if (prdlen >= o.corelength) {  // :915-931
-        out.push_back('\t'), aa_sub_into(out, aa, n, s.core_start, s.core_end);
-        out.push_back('\t'), aa_sub_into(out, aa, n, s.prd_start, s.prd_start + 14);
-        out.push_back('\t'), aa_sub_into(out, aa, n, s.prd_end - 14, s.prd_end);
-        out.push_back('\t'), aa_sub_into(out, aa, n, s.prd_start, s.prd_end);
+        out.push_back('\t'), aa_sub_into(out, aa, n, s.core_start, s.core_end, subs);
+        out.push_back('\t'), aa_sub_into(out, aa, n, s.prd_start, s.prd_start + 14, subs);
+        out.push_back('\t'), aa_sub_into(out, aa, n, s.prd_end - 14, s.prd_end, subs);
+        out.push_back('\t'), aa_sub_into(out, aa, n, s.prd_start, s.prd_end, subs);
     } else
         out += "\t-\t-\t-\t-";
     I(s.fi_numaa), F(s.fi_meanhydro), F(s.fi_meancharge), F(s.fi_meancombo), I(s.fi_maxrun);
     F(inf2nan(s.papa_combo)), F(s.papa_prop), F(s.papa_fi), F(s.papa_llr), F(s.papa_llr2), I(s.papa_center + 1);
-    out.push_back('\t'), aa_sub_into(out, aa, n, s.papa_center - o.ww2 / 2, s.papa_center + o.ww2 / 2);
+    out.push_back('\t'), aa_sub_into(out, aa, n, s.papa_center - o.ww2 / 2, s.papa_center + o.ww2 / 2, subs);
     out.push_back('\n');
 }
 
@@ -870,6 +891,218 @@ void read_plot_list(const std::string& path, std::map<std::string, std::string>&
     }
 }
 
+// ---------------------------------------------------------------------------------------------- sequence variants
+// One line of a --variants file.
+struct VariantLine {
+    int line = 0;
+    std::string spec;                  // upper-cased, as printed after "<name>:"
+    std::vector<int32_t> pos;          // 0-based, ascending
+    std::vector<uint8_t> ref, alt;     // codes
+};
+
+struct VariantFile {
+    std::vector<VariantLine> lines;
+    std::map<std::string, std::vector<int>> by_id;  // SEQid -> indices into lines, in file order
+    std::map<std::string, bool> matched;
+};
+
+int letter_code(char c)
+{
+    const char u = (char)std::toupper((unsigned char)c);
+    const char* p = std::strchr(kAaNames, u);
+    return (u && p) ? (int)(p - kAaNames) : -1;
+}
+
+// Syntax only (needs no record and no device); false after printing the message.
+bool read_variant_file(const std::string& path, VariantFile& V)
+{
+    std::ifstream in(path);
+    if (!in.good()) {
+        std::fprintf(stderr, "plaac: cannot open variant file %s\n", path.c_str());
+        return false;
+    }
+    std::string line;
+    for (int ln = 1; std::getline(in, line); ln++) {
+        if (!line.empty() && line.back() == '\r') line.pop_back();
+        if (line.empty()) continue;
+        auto bad = [&](const std::string& why) {
+            std::fprintf(stderr, "plaac: %s line %d: %s\n", path.c_str(), ln, why.c_str());
+            return false;
+        };
+        const size_t tab = line.find('\t');
+        if (tab == std::string::npos || tab == 0) return bad("expected SEQid<TAB>spec");
+        VariantLine L;
+        L.line = ln;
+        L.spec = line.substr(tab + 1);
+        for (char& c : L.spec) c = (char)std::toupper((unsigned char)c);
+        if (L.spec != "WT") {
+            std::vector<std::pair<int32_t, std::pair<uint8_t, uint8_t>>> subs;
+            size_t a = 0;
+            while (a <= L.spec.size()) {
+                size_t b = L.spec.find(',', a);
+                if (b == std::string::npos) b = L.spec.size();
+                const std::string tok = L.spec.substr(a, b - a);
+                if (tok.size() < 3) return bad("substitution '" + tok + "' is not <ref><pos><alt>");
+                const int r = letter_code(tok.front()), t = letter_code(tok.back());
+                if (r < 0 || t < 0) return bad("unknown residue letter in '" + tok + "'");
+                const std::string num = tok.substr(1, tok.size() - 2);
+                long long p = 0;
+                const auto res = std::from_chars(num.data(), num.data() + num.size(), p);
+                if (res.ec != std::errc() || res.ptr != num.data() + num.size() || p < 1 || p > 0x7fffffff)
+                    return bad("substitution '" + tok + "' has no valid 1-based position");
+                subs.push_back({(int32_t)(p - 1), {(uint8_t)r, (uint8_t)t}});
+                a = b + 1;
+            }
+            std::sort(subs.begin(), subs.end(), [](const auto& x, const auto& y) { return x.first < y.first; });
+            for (size_t k = 0; k < subs.size(); k++) {
+                if (k > 0 && subs[k].first == subs[k - 1].first)
+                    return bad("position " + std::to_string(subs[k].first + 1) + " is substituted twice");
+                L.pos.push_back(subs[k].first);
+                L.ref.push_back(subs[k].second.first);
+                L.alt.push_back(subs[k].second.second);
+            }
+        }
+        const std::string id = line.substr(0, tab);
+        V.by_id[id].push_back((int)V.lines.size());
+        V.matched[id] = false;
+        V.lines.push_back(std::move(L));
+    }
+    return true;
+}
+
+// Variants of the current batch over its reference records, and the names of their rows.
+struct VariantBatch {
+    Batch ref;
+    std::vector<int32_t> protein;
+    std::vector<int64_t> first_sub{0};
+    std::vector<int32_t> pos;
+    std::vector<uint8_t> code;
+    std::vector<std::string> rows;
+    int64_t nres = 0;
+    void clear()
+    {
+        ref.clear();
+        protein.clear();
+        first_sub.assign(1, 0);
+        pos.clear();
+        code.clear();
+        rows.clear();
+        nres = 0;
+    }
+};
+
+int score_variant_batch(const Options& o, Scorers& S, VariantBatch& B)
+{
+    const int64_t nvar = (int64_t)B.protein.size();
+    if (nvar == 0) {
+        B.clear();
+        return 0;
+    }
+    std::vector<plaac_summary> sum((size_t)nvar);
+    const plaac_variants V = {nvar, B.protein.data(), B.first_sub.data(), B.pos.data(), B.code.data()};
+    const int rc = plaac_score_variants(S.ctx[0], B.ref.codes.data(), B.ref.offsets.data(), B.ref.nprot(), &V, sum.data());
+    if (rc != PLAAC_OK) return die(S, rc, "plaac_score_variants");
+    std::string out;
+    for (int64_t v = 0; v < nvar; v++) {
+        const int64_t f = B.first_sub[(size_t)v];
+        const SubList subs{B.pos.data() + f, B.code.data() + f, B.first_sub[(size_t)v + 1] - f};
+        append_summary_row(o, B.rows[(size_t)v], sum[(size_t)v], B.ref.codes.data() + B.ref.offsets[(size_t)B.protein[(size_t)v]], out, subs);
+        if (out.size() >= ((size_t)1 << 20)) {
+            std::fwrite(out.data(), 1, out.size(), stdout);
+            out.clear();
+        }
+    }
+    std::fwrite(out.data(), 1, out.size(), stdout);
+    B.clear();
+    return 0;
+}
+
+// --variants / --saturate: the -i records through this program's reader, their variants scored batch by batch.
+int score_variants_file(const Options& o, Scorers& S, VariantFile* VF)
+{
+    VariantBatch B;
+    FastaReader fr(o.inputfile);
+    std::string seq, name;
+    std::vector<uint8_t> aa;
+    while (fr.hasmore()) {
+        name = fr.name();
+        fr.next(seq);
+        if (seq.empty()) continue;
+        strip_stop(seq);
+        if (seq.empty()) continue;
+        aa.resize(seq.size());
+        plaac_encode_host(seq.data(), (int64_t)seq.size(), aa.data());
+        const int64_t len = (int64_t)seq.size();
+        std::vector<int> mine;
+        if (VF) {
+            for (const std::string& id : {name, ">" + name}) {
+                auto it = VF->by_id.find(id);
+                if (it == VF->by_id.end()) continue;
+                mine.insert(mine.end(), it->second.begin(), it->second.end());
+                VF->matched[id] = true;
+            }
+            if (mine.empty()) continue;
+            std::sort(mine.begin(), mine.end());
+            for (int k : mine) {  // every line of this record is checked before any of its variants is scored
+                const VariantLine& L = VF->lines[(size_t)k];
+                for (size_t j = 0; j < L.pos.size(); j++) {
+                    if (L.pos[j] >= len) {
+                        std::fprintf(stderr, "plaac: %s line %d: position %d is beyond the end of %s (%lld residues)\n",
+                                     o.variants_file.c_str(), L.line, L.pos[j] + 1, name.c_str(), (long long)len);
+                        return 2;
+                    }
+                    if (aa[(size_t)L.pos[j]] != L.ref[j]) {
+                        std::fprintf(stderr, "plaac: %s line %d: %s has %c at position %d, not %c\n", o.variants_file.c_str(),
+                                     L.line, name.c_str(), kAaNames[aa[(size_t)L.pos[j]]], L.pos[j] + 1, kAaNames[L.ref[j]]);
+                        return 2;
+                    }
+                }
+            }
+        }
+        int32_t p = -1;  // this record's index in B.ref, once one of its variants is in the batch
+        auto add = [&](const std::string& spec, const int32_t* ps, const uint8_t* cs, size_t n) -> int {
+            if (p < 0) {
+                B.ref.add(name, "", seq);
+                p = (int32_t)B.ref.nprot() - 1;
+            }
+            B.protein.push_back(p);
+            B.pos.insert(B.pos.end(), ps, ps + n);
+            B.code.insert(B.code.end(), cs, cs + n);
+            B.first_sub.push_back((int64_t)B.pos.size());
+            B.rows.push_back(name + ":" + spec);
+            B.nres += len;
+            if (B.nres >= o.batch_res || (int64_t)B.protein.size() >= (4 << 20)) {
+                p = -1;
+                return score_variant_batch(o, S, B);
+            }
+            return 0;
+        };
+        int rc = 0;
+        if (VF) {
+            for (int k : mine) {
+                const VariantLine& L = VF->lines[(size_t)k];
+                if ((rc = add(L.spec, L.pos.data(), L.alt.data(), L.pos.size()))) return rc;
+            }
+        } else {
+            if ((rc = add("WT", nullptr, nullptr, 0))) return rc;
+            for (int32_t i = 0; i < (int32_t)len; i++)
+                for (uint8_t c = 1; c <= 20; c++) {
+                    if (c == aa[(size_t)i]) continue;
+                    const std::string spec = kAaNames[aa[(size_t)i]] + std::to_string(i + 1) + kAaNames[c];
+                    if ((rc = add(spec, &i, &c, 1))) return rc;
+                }
+        }
+    }
+    if (VF)
+        for (const auto& m : VF->matched)
+            if (!m.second) {
+                std::fprintf(stderr, "plaac: %s line %d: %s is the name of no record of %s\n", o.variants_file.c_str(),
+                             VF->lines[(size_t)VF->by_id.at(m.first).front()].line, m.first.c_str(), o.inputfile.c_str());
+                return 2;
+            }
+    return score_variant_batch(o, S, B);
+}
+
 void usage()
 {
     std::puts("------------------------------------------------------------");
@@ -889,6 +1122,8 @@ void usage()
     std::puts("  -s               skip the run-time parameter block");
     std::puts("  -p list.txt|all  per-residue table for the listed proteins (one name per line) or for all");
     std::puts("  --gpus N, --device D, --batch-mb M, --rank, --rank-core, --gpu-ingest, --host-reader   (this host only)");
+    std::puts("  --variants FILE  score the variants listed in FILE (SEQid<TAB>WT or D262V,P275S) instead of the records");
+    std::puts("  --saturate       score every single substitution of every record");
     std::puts("  --compat-F       -F reads the -B file, as plaac.jar does (plaac.java:388); without it -F reads its own file,");
     std::puts("                   so the parameter block and every score differ from the jar's for the same command line");
 }
@@ -924,6 +1159,10 @@ int main(int argc, char** argv)
             o.gpu_ingest = true;
         else if (a == "--host-reader")
             o.host_reader = true;
+        else if (a == "--variants")
+            o.variants_file = val("--variants");
+        else if (a == "--saturate")
+            o.saturate = true;
         else if (a == "--format-check") {
             // test hook: lines "decimals value" on stdin -> the Java-formatted value on stdout
             int d;
@@ -961,6 +1200,23 @@ int main(int argc, char** argv)
         i++;
     }
     o.ww3 = o.ww2;  // :355
+
+    const bool variants = o.saturate || !o.variants_file.empty();
+    VariantFile vfile;
+    if (variants) {
+        const char* clash = o.saturate && !o.variants_file.empty() ? "--variants"
+                            : !o.plotlist.empty()                  ? "-p"
+                            : o.rank                               ? "--rank / --rank-core"
+                            : o.gpu_ingest                         ? "--gpu-ingest"
+                            : o.gpus > 1                           ? "--gpus > 1"
+                                                                   : nullptr;
+        if (clash) {
+            std::fprintf(stderr, "plaac: %s cannot be combined with %s\n", o.saturate ? "--saturate" : "--variants", clash);
+            return 2;
+        }
+        if (!o.variants_file.empty() && !read_variant_file(o.variants_file, vfile)) return 2;
+        o.host_reader = true;  // the work is the quadratic scoring, not the reading
+    }
 
     // The file-to-table fast path (GPU ingest) is the default for regular input files of at least 1 MB in summary mode;
     // --host-reader forces the reader of this program, --gpu-ingest the GPU one.
@@ -1111,6 +1367,13 @@ int main(int argc, char** argv)
 
     if (make_params()) return 2;
     print_preamble();
+    if (variants) {
+        print_table_head();
+        if ((rc = open_devices())) return rc;
+        rc = score_variants_file(o, S, o.saturate ? nullptr : &vfile);
+        std::fflush(stdout);
+        return rc;
+    }
     Batch B;
     std::string seq, name;
     if (o.plotlist.empty()) {
