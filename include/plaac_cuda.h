@@ -224,6 +224,38 @@ typedef struct plaac_variants {
 int plaac_score_variants(plaac_ctx *ctx, const uint8_t *codes, const int64_t *offsets, int64_t nprot,
                          const plaac_variants *variants, plaac_summary *summaries);
 
+/* Effect columns of plaac_score_variant_effects: bit k (0..12) = the k-th double of plaac_summary in declaration order,
+ * bit 13 = CORE change. */
+#define PLAAC_EFFECT_LLR           (1 << 0)
+#define PLAAC_EFFECT_CORE_SCORE    (1 << 1)
+#define PLAAC_EFFECT_PRD_SCORE     (1 << 2)
+#define PLAAC_EFFECT_HMM_ALL       (1 << 3)
+#define PLAAC_EFFECT_HMM_VIT       (1 << 4)
+#define PLAAC_EFFECT_FI_MEANHYDRO  (1 << 5)
+#define PLAAC_EFFECT_FI_MEANCHARGE (1 << 6)
+#define PLAAC_EFFECT_FI_MEANCOMBO  (1 << 7)
+#define PLAAC_EFFECT_PAPA_COMBO    (1 << 8)
+#define PLAAC_EFFECT_PAPA_PROP     (1 << 9)
+#define PLAAC_EFFECT_PAPA_FI       (1 << 10)
+#define PLAAC_EFFECT_PAPA_LLR      (1 << 11)
+#define PLAAC_EFFECT_PAPA_LLR2     (1 << 12)
+#define PLAAC_EFFECT_CORE_CHANGE   (1 << 13)
+
+/* The effect of each variant against its wild type, in place of whole records (DESIGN.md section 11).  Arguments as
+ * plaac_score_variants; columns is a non-zero mask of PLAAC_EFFECT_* bits.
+ *   effects  HOST array (pinned or pageable) of nvar x popcount(columns) doubles, row-major: one row per variant in
+ *            variant order, columns in ascending bit order.  Bits 0-12: variant.field - wild.field, one IEEE double
+ *            subtraction and nothing else (NaN on either side gives NaN, -Inf - -Inf gives NaN, a PAPA centre that
+ *            appears gives +Inf).  Bit 13: has_core(variant) - has_core(wild) as a double (+1 gained, -1 lost, 0
+ *            unchanged), has_core meaning core_score is not NaN.
+ *   wild     NULL, or nprot HOST records, each byte-identical to what plaac_score(codes, offsets, nprot) returns.
+ * The variants' records and the wild-type records stay on the device; only the effects are copied back.  Errors, their
+ * messages, the nvar == 0 case and the long-path rule are those of plaac_score_variants.  In addition PLAAC_E_INVALID
+ * for columns == 0, a bit above 13, or a NULL effects with nvar > 0.  Reference bytes > 21 are scored as X: the effects
+ * are written and the call then returns PLAAC_E_INVALID, as plaac_score does. */
+int plaac_score_variant_effects(plaac_ctx *ctx, const uint8_t *codes, const int64_t *offsets, int64_t nprot,
+                                const plaac_variants *variants, int32_t columns, double *effects, plaac_summary *wild);
+
 /* ---- multi-GPU (SURVEY.md section 8e): proteins are independent, so the batch is cut into contiguous,
  * residue-balanced shards, one per ctx (each ctx on its own GPU), scored concurrently by one host thread per
  * ctx, each writing its records / per-residue rows straight into the caller's arrays at the input position.

@@ -84,6 +84,11 @@ class Variants(C.Structure):
 
 assert C.sizeof(Variants) == 40
 
+# Effect columns of plaac_score_variant_effects in bit order (PLAAC_EFFECT_*): the doubles of the record, then the
+# CORE change (+1 gained, -1 lost, 0 unchanged).
+EFFECT_COLUMNS = tuple(n for n, t in Summary._fields_ if t is C.c_double) + ("core_change",)
+assert len(EFFECT_COLUMNS) == 14
+
 _lib = None
 
 
@@ -159,6 +164,8 @@ def lib():
         L.plaac_score_hits.restype = C.c_int
         L.plaac_score_variants.restype = C.c_int
         L.plaac_score_variants.argtypes = [vp, vp, vp, i64, C.POINTER(Variants), vp]
+        L.plaac_score_variant_effects.restype = C.c_int
+        L.plaac_score_variant_effects.argtypes = [vp, vp, vp, i64, C.POINTER(Variants), i32, vp, vp]
         L.plaac_score_hits.argtypes = [vp, vp, vp, i64, C.POINTER(Hits)]
         L.plaac_bench_synth_lengths.restype = C.c_int
         L.plaac_bench_synth_lengths.argtypes = [vp, C.c_uint64, i64, i64, dbl, dbl, i32, i32, vp]
@@ -416,6 +423,44 @@ class Scorer:
                                                C.byref(v), out.ctypes.data))
         return out
 
+    def variant_effects(self, codes: np.ndarray, offsets: np.ndarray, protein: np.ndarray, first_sub: np.ndarray,
+                        pos: np.ndarray, code: np.ndarray, columns=("core_score", "llr"), wild: bool = False,
+                        out: np.ndarray | None = None):
+        """plaac_score_variant_effects: the variants of score_variants(), but per variant only the selected columns of its
+        record minus those of its wild type's (the record score() gives for reference protein protein[v]); 'core_change'
+        is +1 if the variant gains a CORE, -1 if it loses it, 0 otherwise.  columns: names of EFFECT_COLUMNS (the double
+        fields of SUMMARY_DTYPE and 'core_change').  Returns a structured array with one f8 field per selected column, in
+        the order of EFFECT_COLUMNS whatever the order given; with wild=True, (effects, the reference's records).
+        out: optional array of that dtype (e.g. a PinnedBuffer's) of len(protein) rows."""
+        if isinstance(columns, str):
+            columns = (columns,)
+        unknown = [c for c in columns if c not in EFFECT_COLUMNS]
+        if unknown or not len(columns):
+            raise ValueError(f"effect columns must be a non-empty subset of {EFFECT_COLUMNS}, got {list(columns)}")
+        mask = 0
+        for c in columns:
+            mask |= 1 << EFFECT_COLUMNS.index(c)
+        dtype = effects_dtype(mask)
+        codes = np.ascontiguousarray(codes, dtype=np.uint8)
+        offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+        protein = np.ascontiguousarray(protein, dtype=np.int32)
+        first_sub = np.ascontiguousarray(first_sub, dtype=np.int64)
+        pos = np.ascontiguousarray(pos, dtype=np.int32)
+        code = np.ascontiguousarray(code, dtype=np.uint8)
+        nvar = len(protein)
+        if len(first_sub) != nvar + 1:
+            raise ValueError(f"first_sub has {len(first_sub)} entries, expected nvar + 1 = {nvar + 1}")
+        if out is None:
+            out = np.zeros(nvar, dtype=dtype)
+        assert out.dtype == dtype and out.flags.c_contiguous and len(out) == nvar
+        wt = np.zeros(len(offsets) - 1, dtype=SUMMARY_DTYPE) if wild else None
+        v = Variants(nvar=nvar, protein=protein.ctypes.data, first_sub=first_sub.ctypes.data, pos=pos.ctypes.data,
+                     code=code.ctypes.data)
+        self._check(lib().plaac_score_variant_effects(self._h, codes.ctypes.data, offsets.ctypes.data, len(offsets) - 1,
+                                                      C.byref(v), mask, out.ctypes.data,
+                                                      wt.ctypes.data if wild else None))
+        return (out, wt) if wild else out
+
     def score_ptr(self, codes_ptr: int, offsets_ptr: int, nprot: int, summaries_ptr: int):
         """Raw host pointers (e.g. pinned torch tensors)."""
         self._check(lib().plaac_score(self._h, codes_ptr, offsets_ptr, nprot, summaries_ptr, None))
@@ -536,6 +581,37 @@ def saturation(codes: np.ndarray, offsets: np.ndarray, proteins=None):
     first_sub = np.zeros(len(protein) + 1, dtype=np.int64)
     np.cumsum(nsub, out=first_sub[1:])
     return protein, first_sub, np.ascontiguousarray(pos, dtype=np.int32), np.ascontiguousarray(code, dtype=np.uint8)
+
+
+def effects_dtype(columns: int) -> np.dtype:
+    """The row of plaac_score_variant_effects for a PLAAC_EFFECT_* mask: one f8 field per set bit, in bit order."""
+    return np.dtype([(n, "<f8") for k, n in enumerate(EFFECT_COLUMNS) if columns >> k & 1])
+
+
+def saturation_map(effects_column: np.ndarray, codes: np.ndarray, offsets: np.ndarray, proteins=None):
+    """One effect column of a scan built by saturation(codes, offsets, proteins) (e.g. variant_effects(...)['llr']) as
+    the scan's heat maps: per protein an (n, 20) array, row i = position i, columns A C D E F G H I K L M N P Q R S T V W
+    Y (SATURATION_CODES), with NaN in the cell of the residue already there.  The wild-type row of each protein is left
+    out."""
+    codes = np.asarray(codes, dtype=np.uint8)
+    offsets = np.asarray(offsets, dtype=np.int64)
+    if proteins is None:
+        proteins = np.arange(len(offsets) - 1)
+    col = np.asarray(effects_column, dtype=np.float64)
+    maps, at = [], 0
+    for p in np.asarray(proteins, dtype=np.int64):
+        ref = codes[offsets[p]:offsets[p + 1]]
+        keep = SATURATION_CODES[None, :] != ref[:, None]
+        nsub = int(keep.sum())
+        if at + 1 + nsub > len(col):
+            raise ValueError(f"{len(col)} effects are fewer than the scan of these proteins has variants")
+        m = np.full((len(ref), 20), np.nan)
+        m[keep] = col[at + 1:at + 1 + nsub]  # (row-major: positions ascending, codes ascending, as saturation() lists them)
+        maps.append(m)
+        at += 1 + nsub
+    if at != len(col):
+        raise ValueError(f"{len(col)} effects, but the scan of these proteins has {at} variants")
+    return maps
 
 
 def shard_plan(offsets: np.ndarray, nshards: int) -> np.ndarray:

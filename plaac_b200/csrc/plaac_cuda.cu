@@ -47,6 +47,7 @@ struct Slot {
     DevBuf codes, offsets, summaries;  // staging for the host-buffer API
     DevBuf words, lengths;             // ... of its packed form (plaac_score_packed)
     DevBuf v_prot, v_first, v_pos, v_code;  // the chunk's slice of a variant list (plaac_score_variants)
+    DevBuf v_effects;                       // the chunk's effects (plaac_score_variant_effects)
     DevBuf hit_flag, hit_pos;          // compact ranked output (plaac_hits)
     DevBuf res_u8, res_f64;            // per-residue staging for the host-buffer API
     DevBuf res_b0, res_b1, res_a0, res_a1, res_mapw, res_lpseq;  // per-residue scratch (bucketed layout)
@@ -64,7 +65,7 @@ struct Slot {
     size_t h_stage_codes_cap = 0;
     void* h_stage_sum = nullptr;
     size_t h_stage_sum_cap = 0;
-    plaac_summary* out_dst = nullptr;  // where the staged records of the chunk in flight go once it has finished
+    void* out_dst = nullptr;  // where the staged records (or effects) of the chunk in flight go once it has finished
     size_t out_bytes = 0;
     cudaEvent_t ev_fork = nullptr, ev_j1 = nullptr, ev_j2 = nullptr, ev_j3 = nullptr, ev_j4 = nullptr, ev_j5 = nullptr;
     int64_t* h_total = nullptr;        // pinned
@@ -89,6 +90,7 @@ struct plaac_ctx {
     DevBuf all_summaries;      // records of a whole host-buffer call, kept on the device for the compact ranked output
     DevBuf union_rec, union_idx, union_order, union_out_idx;  // plaac_score_multi_packed: the shards' hit rows merged on this GPU
     DevBuf var_ref, var_ref_off;  // reference batch of plaac_score_variants, uploaded once per call
+    DevBuf var_wild;              // its records (plaac_score_variant_effects), uploaded once per call
     // pageable <-> device copies of the FASTA calls: two pinned staging buffers, filled / emptied by a multi-threaded memcpy
     void* stage_buf[2] = {nullptr, nullptr};
     cudaEvent_t stage_ev[2] = {nullptr, nullptr};
@@ -398,7 +400,7 @@ int slot_init(plaac_ctx* ctx, Slot& s)
 void slot_free(Slot& s)
 {
     for (DevBuf* b : {&s.gen_f64, &s.scan_tmp, &s.hist, &s.cursor, &s.order, &s.nchunks, &s.chunk_base, &s.stream_buf, &s.tbw, &s.slot_bucket, &s.errflag,
-                      &s.core_list, &s.core_count, &s.codes, &s.offsets, &s.summaries, &s.words, &s.lengths, &s.v_prot, &s.v_first, &s.v_pos, &s.v_code, &s.hit_flag, &s.hit_pos, &s.res_u8, &s.res_f64, &s.res_b0,
+                      &s.core_list, &s.core_count, &s.codes, &s.offsets, &s.summaries, &s.words, &s.lengths, &s.v_prot, &s.v_first, &s.v_pos, &s.v_code, &s.v_effects, &s.hit_flag, &s.hit_pos, &s.res_u8, &s.res_f64, &s.res_b0,
                       &s.res_b1, &s.res_a0, &s.res_a1, &s.res_mapw, &s.res_lpseq, &s.ing_agg, &s.ing_cnt, &s.ing_base,
                       &s.ing_misc, &s.ing_text, &s.ing_codes, &s.ing_offsets, &s.ing_npos, &s.ing_nlen, &s.ing_flags,
                       &s.ing_hist, &s.rk_keys[0], &s.rk_keys[1], &s.rk_vals[0], &s.rk_vals[1], &s.rk_hist, &s.rk_offs,
@@ -1245,7 +1247,7 @@ void plaac_destroy(plaac_ctx* ctx)
     cudaSetDevice(ctx->device);
     for (int i = 0; i < kSlots; i++) slot_free(ctx->slot[i]);
     release(ctx->all_summaries);
-    for (DevBuf* b : {&ctx->union_rec, &ctx->union_idx, &ctx->union_order, &ctx->union_out_idx, &ctx->var_ref, &ctx->var_ref_off}) release(*b);
+    for (DevBuf* b : {&ctx->union_rec, &ctx->union_idx, &ctx->union_order, &ctx->union_out_idx, &ctx->var_ref, &ctx->var_ref_off, &ctx->var_wild}) release(*b);
     for (int b = 0; b < 2; b++) {
         if (ctx->stage_buf[b]) cudaFreeHost(ctx->stage_buf[b]);
         if (ctx->stage_ev[b]) cudaEventDestroy(ctx->stage_ev[b]);
@@ -1632,8 +1634,16 @@ int finish_hits(plaac_ctx* ctx, int64_t nprot, plaac_hits* hits, bool on_device 
     return PLAAC_OK;
 }
 
+// The effect output of a variant call (plaac_score_variant_effects): per variant, the selected columns of its record
+// minus those of its wild type's.
+struct EffectOut {
+    uint32_t columns = 0;        // PLAAC_EFFECT_* mask, checked by the caller
+    double* effects = nullptr;   // nvar x popcount(columns)
+    plaac_summary* wild = nullptr;  // NULL or the reference's nref records
+};
+
 int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary* summaries, const plaac_residue_out* per_res,
-               plaac_hits* hits, bool hits_on_device = false)
+               plaac_hits* hits, bool hits_on_device = false, const EffectOut* eff = nullptr)
 {
     if (nprot < 0) return fail(ctx, PLAAC_E_INVALID, "negative nprot");
     if (hits) {
@@ -1658,13 +1668,38 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
         if (!in.offsets) return fail(ctx, PLAAC_E_INVALID, "NULL offsets");
         if (!in.codes && in.offsets[nprot] != in.offsets[0]) return fail(ctx, PLAAC_E_INVALID, "NULL codes");
     }
-    if (!summaries && !per_res && !hits) return fail(ctx, PLAAC_E_INVALID, "no output requested");
+    if (!summaries && !per_res && !hits && !eff) return fail(ctx, PLAAC_E_INVALID, "no output requested");
     CU(ctx, cudaSetDevice(ctx->device));
-    const bool want_rec = summaries || hits;  // the device computes records
+    const bool want_rec = summaries || hits || eff;  // the device computes records
     int rc = PLAAC_OK;
     if (hits && (rc = ensure(ctx, ctx->all_summaries, sizeof(plaac_summary) * (size_t)nprot))) return rc;
     int64_t var_total = 0;
     if (var && (rc = variants_prepare(ctx, in, var_total))) return rc;
+    // Effects: the wild-type records are those of a plain call on the reference (so `wild` equals plaac_score's by
+    // construction), uploaded into a device table that k_variant_effect reads.  Reference bytes > 21 make that call
+    // return PLAAC_E_INVALID after writing its records; the variants are then scored all the same and the error is
+    // returned at the end, as plaac_score returns it after the batch.
+    const int ek = eff ? __builtin_popcount(eff->columns) : 0;
+    int rc_wild = PLAAC_OK;
+    std::string err_wild;
+    if (eff) {
+        std::vector<plaac_summary> wild_host;
+        plaac_summary* wild = eff->wild;
+        if (!wild) {
+            wild_host.resize((size_t)in.nref);
+            wild = wild_host.data();
+        }
+        HostInput ref;
+        ref.codes = in.codes;
+        ref.offsets = in.offsets;
+        rc_wild = score_host(ctx, ref, in.nref, wild, nullptr, nullptr);
+        if (rc_wild != PLAAC_OK && rc_wild != PLAAC_E_INVALID) return rc_wild;
+        err_wild = ctx->err;
+        if ((rc = ensure(ctx, ctx->var_wild, sizeof(plaac_summary) * (size_t)in.nref))) return rc;
+        cudaStream_t st = ctx->slot[0].stream;
+        if ((rc = h2d_any(ctx, ctx->var_wild.p, wild, sizeof(plaac_summary) * (size_t)in.nref, st))) return rc;
+        CU(ctx, cudaStreamSynchronize(st));
+    }
 
     // Chunking: bounded device footprint; kSlots sets of buffers so the next chunks' H2D overlap this chunk's kernels and
     // D2H.  Chunk sizes ramp up from max/8 and down again towards the end: the first chunk's copy and the last chunk's
@@ -1687,7 +1722,10 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
     // and kernels of the other slots.
     const void* in_main = packed ? (const void*)in.words : (const void*)(in.codes + first_off);
     const bool stage_in = !var && total_res > 0 && !host_is_pinned(in_main);
-    const bool stage_sum = summaries && !host_is_pinned(summaries);
+    // (the host rows of the call: records, or effects)
+    const void* out_rows = eff ? (const void*)eff->effects : (const void*)summaries;
+    const size_t row_bytes = eff ? sizeof(double) * (size_t)ek : sizeof(plaac_summary);
+    const bool stage_sum = out_rows && !host_is_pinned(out_rows);
     auto drain = [&](int i) -> int {
         if (!pending[i]) return PLAAC_OK;
         pending[i] = false;
@@ -1795,10 +1833,11 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
         plaac_summary* d_sum = nullptr;
         if (hits)
             d_sum = (plaac_summary*)ctx->all_summaries.p + start;
-        else if (summaries) {
+        else if (summaries || eff) {
             if ((rc = ensure(ctx, s.summaries, sizeof(plaac_summary) * np))) break;
             d_sum = (plaac_summary*)s.summaries.p;
         }
+        if (eff && (rc = ensure(ctx, s.v_effects, row_bytes * (size_t)np))) break;
         plaac_residue_out dres;
         if (per_res) {
             if ((rc = ensure(ctx, s.res_u8, (size_t)2 * (nres + 16)))) break;
@@ -1828,7 +1867,7 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
             par_memcpy(s.h_stage_codes, src_main, main_bytes);
             src_main = s.h_stage_codes;
         }
-        if (stage_sum && (rc = ensure_host(ctx, s.h_stage_sum, s.h_stage_sum_cap, sizeof(plaac_summary) * (size_t)np))) break;
+        if (stage_sum && (rc = ensure_host(ctx, s.h_stage_sum, s.h_stage_sum_cap, row_bytes * (size_t)np))) break;
         const uint8_t* d_codes = (const uint8_t*)s.codes.p;
         int64_t off_base = first_off + pos;  // offsets[] of the chunk are relative to this residue index
         if (var) {
@@ -1882,10 +1921,17 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
         } else if (summaries) {
             CUB(cudaMemcpyAsync(stage_sum ? (plaac_summary*)s.h_stage_sum : summaries + start, s.summaries.p,
                                 sizeof(plaac_summary) * np, cudaMemcpyDeviceToHost, s.stream));
+        } else if (eff) {
+            // the records stay on the device; only the chunk's np x ek effects cross the link
+            k_variant_effect<<<(unsigned)((np * ek + 255) / 256), 256, 0, s.stream>>>(
+                d_sum, (const plaac_summary*)ctx->var_wild.p, (const int32_t*)s.v_prot.p, np, eff->columns, (double*)s.v_effects.p);
+            ctx->stats.kernel_launches += 1;
+            CUB(cudaMemcpyAsync(stage_sum ? s.h_stage_sum : (void*)(eff->effects + start * ek), s.v_effects.p, row_bytes * (size_t)np,
+                                cudaMemcpyDeviceToHost, s.stream));
         }
-        if (summaries && stage_sum) {
-            s.out_dst = summaries + start;
-            s.out_bytes = sizeof(plaac_summary) * (size_t)np;
+        if (out_rows && stage_sum) {
+            s.out_dst = (char*)out_rows + row_bytes * (size_t)start;
+            s.out_bytes = row_bytes * (size_t)np;
         }
         if (per_res && nres > 0) {
             const int64_t o = pos - pos0;
@@ -1926,6 +1972,10 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
         }
         cudaGetLastError();
         ctx->err = keep;
+    }
+    if (rc == PLAAC_OK && rc_wild != PLAAC_OK) {
+        rc = rc_wild;
+        ctx->err = err_wild;
     }
     if (hits && (rc == PLAAC_OK || (rc == PLAAC_E_INVALID && start >= nprot))) {
         // (invalid residue codes are reported after the batch, with every record computed: the compact output too)
@@ -1997,6 +2047,30 @@ try {
     return score_host(ctx, in, variants->nvar, summaries, nullptr, nullptr);
 } catch (...) {
     return api_caught(ctx, "plaac_score_variants");
+}
+
+int plaac_score_variant_effects(plaac_ctx* ctx, const uint8_t* codes, const int64_t* offsets, int64_t nprot,
+                                const plaac_variants* variants, int32_t columns, double* effects, plaac_summary* wild)
+try {
+    if (!ctx) return fail(nullptr, PLAAC_E_INVALID, "plaac_score_variant_effects: NULL ctx");
+    if (!variants) return fail(ctx, PLAAC_E_INVALID, "plaac_score_variant_effects: NULL variants");
+    if (columns <= 0 || columns >= (PLAAC_EFFECT_CORE_CHANGE << 1))
+        return fail(ctx, PLAAC_E_INVALID, "plaac_score_variant_effects: columns 0x%x is not a non-empty set of PLAAC_EFFECT_* bits",
+                    (unsigned)columns);
+    if (variants->nvar > 0 && !effects) return fail(ctx, PLAAC_E_INVALID, "plaac_score_variant_effects: NULL effects with nvar = %lld",
+                                                    (long long)variants->nvar);
+    HostInput in;
+    in.codes = codes;
+    in.offsets = offsets;
+    in.nref = nprot;
+    in.var = variants;
+    EffectOut eff;
+    eff.columns = (uint32_t)columns;
+    eff.effects = effects;
+    eff.wild = wild;
+    return score_host(ctx, in, variants->nvar, nullptr, nullptr, nullptr, false, &eff);
+} catch (...) {
+    return api_caught(ctx, "plaac_score_variant_effects");
 }
 
 }  // extern "C"

@@ -1,10 +1,13 @@
 // Sequence variants built on the device (plaac_score_variants): the reference batch is uploaded once per call, and each
 // chunk of the variant list is expanded from it into the slot's code buffer that k_pack reads, so only the substitution
 // list crosses the host link.  Per chunk, on the slot's stream:
-//   k_variant_lengths -> launch_scan (offsets) -> k_variant_expand -> k_variant_apply -> run_batch.
+//   k_variant_lengths -> launch_scan (offsets) -> k_variant_expand -> k_variant_apply -> run_batch
+//   [-> k_variant_effect for plaac_score_variant_effects].
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+
+#include "lean.cuh"  // rec_has_core
 
 namespace plaac {
 
@@ -113,6 +116,26 @@ k_variant_apply(const int64_t* __restrict__ first_sub, int64_t fs0, int64_t nvar
     if (j >= nsub) return;
     const int64_t v = last_not_above(first_sub, 0, nvar - 1, fs0 + j);
     codes[off[v] + pos[j]] = code[j];
+}
+
+// plaac_score_variant_effects: out[v * k + c] = effect of variant v in the c-th set bit of `columns` (k of them), against
+// the wild-type record of its reference protein (wild[protein[v]]).  One thread per output element, so the row-major
+// stores coalesce; the record reads are 160-byte-strided gathers.  Bits 0..12 index the doubles of plaac_summary from
+// llr on; bit 13 is the CORE change.  Runs after run_batch in stream order.
+constexpr int kEffectCoreChange = 13;
+
+__global__ void __launch_bounds__(256)
+k_variant_effect(const plaac_summary* __restrict__ rec, const plaac_summary* __restrict__ wild,
+                 const int32_t* __restrict__ protein, int64_t nvar, uint32_t columns, double* __restrict__ out)
+{
+    const int k = __popc(columns);
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= nvar * k) return;
+    const int64_t v = e / k;
+    const int f = (int)__fns(columns, 0, (int)(e - v * k) + 1);  // position of the (c+1)-th set bit
+    const plaac_summary& a = rec[v];
+    const plaac_summary& b = wild[protein[v]];
+    out[e] = f == kEffectCoreChange ? (double)rec_has_core(a) - (double)rec_has_core(b) : __dsub_rn((&a.llr)[f], (&b.llr)[f]);
 }
 
 }  // namespace plaac

@@ -23,6 +23,11 @@
 //                   One row per variant, named <name>:<SPEC>, in record order and within a record in file order
 //   --saturate      every single substitution of every -i record (wild type first, then positions in ascending order,
 //                   at each one the 20 residues A..Y other than the one there)
+//   --effects COLS  with --variants or --saturate: print per variant only the change of the listed summary columns
+//                   against the wild type (plaac_score_variant_effects) instead of its row.  COLS is a comma-separated
+//                   list of LLR COREscore PRDscore HMMall HMMvit FImeanhydro FImeancharge FImeancombo PAPAcombo PAPAprop
+//                   PAPAfi PAPAllr PAPAllr2 (printed as d<NAME>, variant minus wild type) and COREchange (1 gained,
+//                   -1 lost, 0 unchanged)
 #include <algorithm>
 #include <charconv>
 #include <cmath>
@@ -408,7 +413,43 @@ struct Options {
     bool rank = false, rank_core_only = false;
     std::string variants_file;  // --variants
     bool saturate = false;      // --saturate
+    std::string effects;        // --effects, as given
+    bool effects_set = false;
+    int32_t effects_mask = 0;   // PLAAC_EFFECT_* bits of --effects
 };
+
+// --effects names, bit k = PLAAC_EFFECT_* bit k (the doubles of plaac_summary in declaration order, then COREchange)
+const char* const kEffectNames[] = {"LLR",          "COREscore",   "PRDscore",  "HMMall",   "HMMvit",
+                                    "FImeanhydro",  "FImeancharge", "FImeancombo", "PAPAcombo", "PAPAprop",
+                                    "PAPAfi",       "PAPAllr",     "PAPAllr2",  "COREchange"};
+constexpr int kEffectCoreChange = 13;
+
+// Comma-separated --effects names -> mask; 0 after printing the message.
+int32_t parse_effects(const std::string& list)
+{
+    int32_t mask = 0;
+    size_t a = 0;
+    while (a <= list.size()) {
+        size_t b = list.find(',', a);
+        if (b == std::string::npos) b = list.size();
+        const std::string name = list.substr(a, b - a);
+        int k = 0;
+        while (k <= kEffectCoreChange && name != kEffectNames[k]) k++;
+        if (k > kEffectCoreChange) {
+            if (name.empty())
+                std::fprintf(stderr, "plaac: --effects: empty column name in '%s'\n", list.c_str());
+            else
+                std::fprintf(stderr, "plaac: --effects: unknown column '%s'\n", name.c_str());
+            std::fprintf(stderr, "plaac: --effects takes a comma-separated list of");
+            for (const char* n : kEffectNames) std::fprintf(stderr, " %s", n);
+            std::fprintf(stderr, "\n");
+            return 0;
+        }
+        mask |= 1 << k;
+        a = b + 1;
+    }
+    return mask;
+}
 
 struct Scorers {
     std::vector<plaac_ctx*> ctx;
@@ -991,6 +1032,39 @@ struct VariantBatch {
     }
 };
 
+// --effects: one row per variant, its name and the changes of the selected columns.
+int score_effect_batch(const Options& o, Scorers& S, VariantBatch& B)
+{
+    const int64_t nvar = (int64_t)B.protein.size();
+    const int k = __builtin_popcount((unsigned)o.effects_mask);
+    std::vector<double> eff((size_t)nvar * (size_t)k);
+    const plaac_variants V = {nvar, B.protein.data(), B.first_sub.data(), B.pos.data(), B.code.data()};
+    const int rc = plaac_score_variant_effects(S.ctx[0], B.ref.codes.data(), B.ref.offsets.data(), B.ref.nprot(), &V,
+                                               o.effects_mask, eff.data(), nullptr);
+    if (rc != PLAAC_OK) return die(S, rc, "plaac_score_variant_effects");
+    const bool last_is_core = (o.effects_mask >> kEffectCoreChange) & 1;  // (the highest bit: the last column)
+    std::string out;
+    for (int64_t v = 0; v < nvar; v++) {
+        out += B.rows[(size_t)v];
+        const double* e = eff.data() + (size_t)v * (size_t)k;
+        for (int c = 0; c < k; c++) {
+            out.push_back('\t');
+            if (last_is_core && c == k - 1)
+                put_int(out, (long)e[c]);
+            else
+                put_fixed(out, e[c], 3);
+        }
+        out.push_back('\n');
+        if (out.size() >= ((size_t)1 << 20)) {
+            std::fwrite(out.data(), 1, out.size(), stdout);
+            out.clear();
+        }
+    }
+    std::fwrite(out.data(), 1, out.size(), stdout);
+    B.clear();
+    return 0;
+}
+
 int score_variant_batch(const Options& o, Scorers& S, VariantBatch& B)
 {
     const int64_t nvar = (int64_t)B.protein.size();
@@ -998,6 +1072,7 @@ int score_variant_batch(const Options& o, Scorers& S, VariantBatch& B)
         B.clear();
         return 0;
     }
+    if (o.effects_mask) return score_effect_batch(o, S, B);
     std::vector<plaac_summary> sum((size_t)nvar);
     const plaac_variants V = {nvar, B.protein.data(), B.first_sub.data(), B.pos.data(), B.code.data()};
     const int rc = plaac_score_variants(S.ctx[0], B.ref.codes.data(), B.ref.offsets.data(), B.ref.nprot(), &V, sum.data());
@@ -1124,6 +1199,10 @@ void usage()
     std::puts("  --gpus N, --device D, --batch-mb M, --rank, --rank-core, --gpu-ingest, --host-reader   (this host only)");
     std::puts("  --variants FILE  score the variants listed in FILE (SEQid<TAB>WT or D262V,P275S) instead of the records");
     std::puts("  --saturate       score every single substitution of every record");
+    std::puts("  --effects COLS   with --variants or --saturate: print only each variant's change against the wild type in");
+    std::puts("                   the listed columns (comma-separated: LLR COREscore PRDscore HMMall HMMvit FImeanhydro");
+    std::puts("                   FImeancharge FImeancombo PAPAcombo PAPAprop PAPAfi PAPAllr PAPAllr2, printed as d<NAME>;");
+    std::puts("                   COREchange: 1 CORE gained, -1 lost, 0 unchanged)");
     std::puts("  --compat-F       -F reads the -B file, as plaac.jar does (plaac.java:388); without it -F reads its own file,");
     std::puts("                   so the parameter block and every score differ from the jar's for the same command line");
 }
@@ -1163,6 +1242,8 @@ int main(int argc, char** argv)
             o.variants_file = val("--variants");
         else if (a == "--saturate")
             o.saturate = true;
+        else if (a == "--effects")
+            o.effects = val("--effects"), o.effects_set = true;
         else if (a == "--format-check") {
             // test hook: lines "decimals value" on stdin -> the Java-formatted value on stdout
             int d;
@@ -1214,8 +1295,12 @@ int main(int argc, char** argv)
             std::fprintf(stderr, "plaac: %s cannot be combined with %s\n", o.saturate ? "--saturate" : "--variants", clash);
             return 2;
         }
+        if (o.effects_set && !(o.effects_mask = parse_effects(o.effects))) return 2;
         if (!o.variants_file.empty() && !read_variant_file(o.variants_file, vfile)) return 2;
         o.host_reader = true;  // the work is the quadratic scoring, not the reading
+    } else if (o.effects_set) {
+        std::fprintf(stderr, "plaac: --effects needs --variants FILE or --saturate\n");
+        return 2;
     }
 
     // The file-to-table fast path (GPU ingest) is the default for regular input files of at least 1 MB in summary mode;
@@ -1368,7 +1453,15 @@ int main(int argc, char** argv)
     if (make_params()) return 2;
     print_preamble();
     if (variants) {
-        print_table_head();
+        if (o.effects_mask) {
+            std::string head = "SEQid";
+            for (int k = 0; k <= kEffectCoreChange; k++)
+                if ((o.effects_mask >> k) & 1) head += std::string("\t") + (k == kEffectCoreChange ? "" : "d") + kEffectNames[k];
+            std::puts(head.c_str());
+            std::fflush(stdout);
+        } else {
+            print_table_head();
+        }
         if ((rc = open_devices())) return rc;
         rc = score_variants_file(o, S, o.saturate ? nullptr : &vfile);
         std::fflush(stdout);

@@ -156,16 +156,8 @@ def run_workload(name, codes, offsets, var, sample_res):
     return r
 
 
-def main():
-    ap = argparse.ArgumentParser()
-    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "variants_bench.json"))
-    ap.add_argument("--sample-res", type=float, default=4e8)
-    a = ap.parse_args()
-    if plaac_b200.lib().plaac_device_count() <= 0:
-        sys.exit("variants_bench: no CUDA device")
-    info = {"card": card(), "results": []}
-    print("card:", info["card"], flush=True)
-
+def workloads():
+    """The three workloads of the module docstring: (name, reference codes, reference offsets, variant arrays)."""
     codes, offs = synth.long_proteins(seed=2001, lengths=(34000,))
     wl = [("a: saturation of one 34 000-residue protein", codes, offs, plaac_b200.saturation(codes, offs))]
     codes, offs = synth.proteome(1000, seed=2002, median=290.0, sigma=0.62)
@@ -190,8 +182,20 @@ def main():
     code = rng.integers(1, 21, len(pos)).astype(np.uint8)
     wl.append(("c: 200 000 random single and double substitutions over a yeast-sized reference", codes, offs,
                (protein, first_sub, pos, code)))
+    return wl
 
-    for name, c, o, var in wl:
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "variants_bench.json"))
+    ap.add_argument("--sample-res", type=float, default=4e8)
+    a = ap.parse_args()
+    if plaac_b200.lib().plaac_device_count() <= 0:
+        sys.exit("variants_bench: no CUDA device")
+    info = {"card": card(), "results": []}
+    print("card:", info["card"], flush=True)
+
+    for name, c, o, var in workloads():
         r = run_workload(name, c, o, var, a.sample_res)
         info["results"].append(r)
         v, s = r["variant_call"], r["sample"]
