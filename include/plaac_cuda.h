@@ -256,6 +256,33 @@ int plaac_score_variants(plaac_ctx *ctx, const uint8_t *codes, const int64_t *of
 int plaac_score_variant_effects(plaac_ctx *ctx, const uint8_t *codes, const int64_t *offsets, int64_t nprot,
                                 const plaac_variants *variants, int32_t columns, double *effects, plaac_summary *wild);
 
+/* ---- prion-like segments of the Viterbi parse (DESIGN.md section 12) ----------------------------------------------
+ * A segment of protein i is a maximal run of residues whose Viterbi state is 1 (PrD-like): a maximal run of 1s of the
+ * VIT column of per-residue mode.  start and end are 0-based, end inclusive (as prd_start / prd_end); score is
+ * 0.0 + llr[aa[start]] + ... + llr[aa[end]] summed in residue order (the PRDscore rule, plaac.java:861-873), codes > 21
+ * counting as X.  The segment that holds a protein's CORE therefore equals (prd_start, prd_end, prd_score) bit for bit,
+ * and the longest segment's length is vit_maxrun. */
+typedef struct plaac_segments {
+    int64_t capacity;  /* in: entries start / end / score can hold */
+    int64_t *first;    /* out: nprot + 1; the segments of protein i are [first[i], first[i+1]), complete even when
+                          count > capacity */
+    int32_t *start;    /* out: 0-based */
+    int32_t *end;      /* out: 0-based, inclusive */
+    double *score;     /* out: the PRDscore rule over the segment */
+    int64_t count;     /* out: segments in the batch; the first min(count, capacity) are stored, in input order */
+} plaac_segments;
+
+/* Summary mode with the segment list of every protein.  codes / offsets / nprot as plaac_score; HOST buffers (pinned or
+ * pageable) everywhere; blocks until done.  summaries: NULL (records are not copied back) or nprot records,
+ * byte-identical to plaac_score's.  The segments are extracted on the device from the parse the summary kernels leave
+ * behind and do not depend on the chunking, the long-path setting or the kernel variant.  Call again with
+ * capacity = count when count > capacity.
+ * PLAAC_E_INVALID for a negative capacity, a NULL first with nprot > 0, or a NULL start / end / score with
+ * capacity > 0.  Reference bytes > 21 are scored as X: everything is written and the call then returns
+ * PLAAC_E_INVALID, as plaac_score does.  nprot == 0: first[0] = 0, count = 0, PLAAC_OK. */
+int plaac_score_segments(plaac_ctx *ctx, const uint8_t *codes, const int64_t *offsets, int64_t nprot,
+                         plaac_summary *summaries, plaac_segments *segments);
+
 /* ---- multi-GPU (SURVEY.md section 8e): proteins are independent, so the batch is cut into contiguous,
  * residue-balanced shards, one per ctx (each ctx on its own GPU), scored concurrently by one host thread per
  * ctx, each writing its records / per-residue rows straight into the caller's arrays at the input position.

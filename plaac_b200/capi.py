@@ -84,6 +84,14 @@ class Variants(C.Structure):
 
 assert C.sizeof(Variants) == 40
 
+
+class Segments(C.Structure):
+    _fields_ = [("capacity", C.c_int64), ("first", C.c_void_p), ("start", C.c_void_p), ("end", C.c_void_p),
+                ("score", C.c_void_p), ("count", C.c_int64)]
+
+
+assert C.sizeof(Segments) == 48
+
 # Effect columns of plaac_score_variant_effects in bit order (PLAAC_EFFECT_*): the doubles of the record, then the
 # CORE change (+1 gained, -1 lost, 0 unchanged).
 EFFECT_COLUMNS = tuple(n for n, t in Summary._fields_ if t is C.c_double) + ("core_change",)
@@ -167,6 +175,8 @@ def lib():
         L.plaac_score_variant_effects.restype = C.c_int
         L.plaac_score_variant_effects.argtypes = [vp, vp, vp, i64, C.POINTER(Variants), i32, vp, vp]
         L.plaac_score_hits.argtypes = [vp, vp, vp, i64, C.POINTER(Hits)]
+        L.plaac_score_segments.restype = C.c_int
+        L.plaac_score_segments.argtypes = [vp, vp, vp, i64, vp, C.POINTER(Segments)]
         L.plaac_bench_synth_lengths.restype = C.c_int
         L.plaac_bench_synth_lengths.argtypes = [vp, C.c_uint64, i64, i64, dbl, dbl, i32, i32, vp]
         L.plaac_bench_synth_residues.restype = C.c_int
@@ -460,6 +470,33 @@ class Scorer:
                                                       C.byref(v), mask, out.ctypes.data,
                                                       wt.ctypes.data if wild else None))
         return (out, wt) if wild else out
+
+    def score_segments(self, codes: np.ndarray, offsets: np.ndarray, summaries: bool = True, capacity: int | None = None):
+        """plaac_score_segments: summary mode plus every prion-like segment of each protein's Viterbi parse (maximal runs
+        of PrD-state residues).  Returns (records or None, {"first", "start", "end", "score"}): the segments of protein i
+        are [first[i], first[i+1]), 0-based with end inclusive, score the PRDscore sum over the segment.  capacity: entries
+        to make room for (default nprot); if the batch has more segments, the batch is scored a second time with room
+        for all of them."""
+        codes = np.ascontiguousarray(codes, dtype=np.uint8)
+        offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+        nprot = len(offsets) - 1
+        cap = nprot if capacity is None else int(capacity)
+        while True:
+            out = np.zeros(nprot, dtype=SUMMARY_DTYPE) if summaries else None
+            first = np.zeros(nprot + 1, dtype=np.int64)
+            start = np.zeros(max(cap, 0), dtype=np.int32)
+            end = np.zeros(max(cap, 0), dtype=np.int32)
+            score = np.zeros(max(cap, 0), dtype=np.float64)
+            sg = Segments(capacity=cap, first=first.ctypes.data, start=start.ctypes.data if cap > 0 else None,
+                          end=end.ctypes.data if cap > 0 else None, score=score.ctypes.data if cap > 0 else None, count=0)
+            self._check(lib().plaac_score_segments(self._h, codes.ctypes.data, offsets.ctypes.data if nprot >= 0 else None,
+                                                   nprot, out.ctypes.data if out is not None and nprot else None,
+                                                   C.byref(sg)))
+            if sg.count <= cap:
+                break
+            cap = int(sg.count)
+        n = int(sg.count)
+        return out, {"first": first, "start": start[:n], "end": end[:n], "score": score[:n]}
 
     def score_ptr(self, codes_ptr: int, offsets_ptr: int, nprot: int, summaries_ptr: int):
         """Raw host pointers (e.g. pinned torch tensors)."""

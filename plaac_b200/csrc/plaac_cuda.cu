@@ -28,6 +28,7 @@
 #include "lean.cuh"
 #include "generic_windows.cuh"
 #include "variants.cuh"
+#include "segments.cuh"
 
 using namespace plaac;
 
@@ -48,6 +49,7 @@ struct Slot {
     DevBuf words, lengths;             // ... of its packed form (plaac_score_packed)
     DevBuf v_prot, v_first, v_pos, v_code;  // the chunk's slice of a variant list (plaac_score_variants)
     DevBuf v_effects;                       // the chunk's effects (plaac_score_variant_effects)
+    DevBuf sg_cnt, sg_first, sg_ent;        // the chunk's segments (plaac_score_segments): counts, their scan, entries
     DevBuf hit_flag, hit_pos;          // compact ranked output (plaac_hits)
     DevBuf res_u8, res_f64;            // per-residue staging for the host-buffer API
     DevBuf res_b0, res_b1, res_a0, res_a1, res_mapw, res_lpseq;  // per-residue scratch (bucketed layout)
@@ -68,6 +70,14 @@ struct Slot {
     void* out_dst = nullptr;  // where the staged records (or effects) of the chunk in flight go once it has finished
     size_t out_bytes = 0;
     cudaEvent_t ev_fork = nullptr, ev_j1 = nullptr, ev_j2 = nullptr, ev_j3 = nullptr, ev_j4 = nullptr, ev_j5 = nullptr;
+    // segments of the chunk in flight (plaac_score_segments): pinned copies of its first[] and of its stored entries,
+    // and what a rerun of the bounds / score kernels needs if the entries overflowed seg_cap
+    void* h_sg_first = nullptr;
+    size_t h_sg_first_cap = 0;
+    void* h_sg_ent = nullptr;
+    size_t h_sg_ent_cap = 0;
+    SegArgs seg_args;
+    int64_t seg_np = -1, seg_cap = 0, seg_p0 = 0;  // proteins of the chunk (-1: no segments pending), capacity, first protein
     int64_t* h_total = nullptr;        // pinned
     int* h_err = nullptr;              // pinned
     cudaEvent_t ev_a = nullptr, ev_b = nullptr, ev_c = nullptr, ev_d = nullptr;
@@ -400,7 +410,7 @@ int slot_init(plaac_ctx* ctx, Slot& s)
 void slot_free(Slot& s)
 {
     for (DevBuf* b : {&s.gen_f64, &s.scan_tmp, &s.hist, &s.cursor, &s.order, &s.nchunks, &s.chunk_base, &s.stream_buf, &s.tbw, &s.slot_bucket, &s.errflag,
-                      &s.core_list, &s.core_count, &s.codes, &s.offsets, &s.summaries, &s.words, &s.lengths, &s.v_prot, &s.v_first, &s.v_pos, &s.v_code, &s.v_effects, &s.hit_flag, &s.hit_pos, &s.res_u8, &s.res_f64, &s.res_b0,
+                      &s.core_list, &s.core_count, &s.codes, &s.offsets, &s.summaries, &s.words, &s.lengths, &s.v_prot, &s.v_first, &s.v_pos, &s.v_code, &s.v_effects, &s.sg_cnt, &s.sg_first, &s.sg_ent, &s.hit_flag, &s.hit_pos, &s.res_u8, &s.res_f64, &s.res_b0,
                       &s.res_b1, &s.res_a0, &s.res_a1, &s.res_mapw, &s.res_lpseq, &s.ing_agg, &s.ing_cnt, &s.ing_base,
                       &s.ing_misc, &s.ing_text, &s.ing_codes, &s.ing_offsets, &s.ing_npos, &s.ing_nlen, &s.ing_flags,
                       &s.ing_hist, &s.rk_keys[0], &s.rk_keys[1], &s.rk_vals[0], &s.rk_vals[1], &s.rk_hist, &s.rk_offs,
@@ -409,6 +419,8 @@ void slot_free(Slot& s)
     if (s.h_long) cudaFreeHost(s.h_long);
     if (s.h_stage_codes) cudaFreeHost(s.h_stage_codes);
     if (s.h_stage_sum) cudaFreeHost(s.h_stage_sum);
+    if (s.h_sg_first) cudaFreeHost(s.h_sg_first);
+    if (s.h_sg_ent) cudaFreeHost(s.h_sg_ent);
     s.h_stage_codes = s.h_stage_sum = nullptr;
     s.h_stage_codes_cap = s.h_stage_sum_cap = 0;
     if (s.h_total) cudaFreeHost(s.h_total);
@@ -517,10 +529,41 @@ int launch_scan(plaac_ctx* ctx, Slot& s, const int32_t* in, int64_t* out, int64_
     return PLAAC_OK;
 }
 
+// The segment kernels of a chunk (segments.cuh) on the slot's stream: with counts, k_seg_count[_long] and their scan
+// into a.first first; then the bounds of the first a.cap segments and their scores.
+int launch_segments(plaac_ctx* ctx, Slot& s, const SegArgs& a, int64_t np, bool counts)
+{
+    cudaStream_t st = s.stream;
+    const unsigned gp = (unsigned)((np + 255) / 256);
+    if (counts) {
+        k_seg_count<<<gp, 256, 0, st>>>(a);
+        ctx->stats.kernel_launches += 1;
+        if (a.nlong > 0) {
+            k_seg_count_long<<<(unsigned)a.nlong, kSegLongThreads, 0, st>>>(a);
+            ctx->stats.kernel_launches += 1;
+        }
+        int rc = launch_scan(ctx, s, a.count, (int64_t*)a.first, np, st);
+        if (rc) return rc;
+    }
+    if (a.cap > 0) {
+        k_seg_bounds<<<gp, 256, 0, st>>>(a);
+        ctx->stats.kernel_launches += 1;
+        if (a.nlong > 0) {
+            k_seg_bounds_long<<<(unsigned)a.nlong, kSegLongThreads, 0, st>>>(a);
+            ctx->stats.kernel_launches += 1;
+        }
+        const unsigned gs = (unsigned)std::min<int64_t>((a.cap + 127) / 128, (int64_t)ctx->sm_count * 32);
+        k_seg_score<<<gs, 128, 0, st>>>(a, np);
+        ctx->stats.kernel_launches += 1;
+    }
+    CU(ctx, cudaGetLastError());
+    return PLAAC_OK;
+}
+
 int run_batch(plaac_ctx* ctx, Slot& s, const uint8_t* d_codes, const int64_t* d_offsets, int64_t off_base,
               int64_t nprot, int64_t ntotal, plaac_summary* d_summaries, const plaac_residue_out* d_res,
               int64_t res_base, int64_t slots_bound = -1, int64_t nlong_known = -1, int64_t long_scratch_known = -1,
-              int64_t long_thr_known = -1, int64_t nbig_known = -1)
+              int64_t long_thr_known = -1, int64_t nbig_known = -1, int64_t seg_cap = -1)
 {
     if (nprot == 0) return PLAAC_OK;
     if (nprot > 0x7fffffff) return fail(ctx, PLAAC_E_INVALID, "more than 2^31-1 proteins in one device batch");
@@ -917,6 +960,33 @@ int run_batch(plaac_ctx* ctx, Slot& s, const uint8_t* d_codes, const int64_t* d_
                     CU(ctx, cudaMemcpyAsync(dst[k] + (off_base - res_base), src[k], sizeof(double) * (size_t)ntotal,
                                             cudaMemcpyDeviceToDevice, st));
         }
+    }
+    if (seg_cap >= 0 && d_summaries) {
+        // segments (plaac_score_segments): both parses are final here -- the CORE search ran on st, and st has joined
+        // the long-path streams
+        if ((rc = ensure(ctx, s.sg_cnt, sizeof(int32_t) * (size_t)nprot))) return rc;
+        if ((rc = ensure(ctx, s.sg_first, sizeof(int64_t) * (size_t)(nprot + 1)))) return rc;
+        if ((rc = ensure(ctx, s.sg_ent, (3 * sizeof(int32_t) + sizeof(double)) * (size_t)std::max<int64_t>(seg_cap, 1)))) return rc;
+        SegArgs a;
+        a.bv = bv;
+        a.codes = d_codes;
+        a.tabs = ctx->d_tabs;
+        a.long_list = long_launched ? (const int32_t*)s.lg_list.p : nullptr;
+        a.long_off = long_launched ? (const int64_t*)s.lg_off.p : nullptr;
+        a.long_vit = long_launched ? (const uint32_t*)s.lg_vit.p : nullptr;
+        a.nlong = long_launched ? nlong : 0;
+        a.count = (int32_t*)s.sg_cnt.p;
+        a.first = (const int64_t*)s.sg_first.p;
+        a.cap = seg_cap;
+        double* ent = (double*)s.sg_ent.p;
+        a.score = ent;
+        a.prot = (int32_t*)(ent + seg_cap);
+        a.start = a.prot + seg_cap;
+        a.end = a.start + seg_cap;
+        s.seg_args = a;
+        s.seg_np = nprot;
+        s.seg_cap = seg_cap;
+        if ((rc = launch_segments(ctx, s, a, nprot, true))) return rc;
     }
     CU(ctx, cudaEventRecord(s.ev_d, st));
     CU(ctx, cudaGetLastError());
@@ -1643,7 +1713,7 @@ struct EffectOut {
 };
 
 int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary* summaries, const plaac_residue_out* per_res,
-               plaac_hits* hits, bool hits_on_device = false, const EffectOut* eff = nullptr)
+               plaac_hits* hits, bool hits_on_device = false, const EffectOut* eff = nullptr, plaac_segments* seg = nullptr)
 {
     if (nprot < 0) return fail(ctx, PLAAC_E_INVALID, "negative nprot");
     if (hits) {
@@ -1668,9 +1738,9 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
         if (!in.offsets) return fail(ctx, PLAAC_E_INVALID, "NULL offsets");
         if (!in.codes && in.offsets[nprot] != in.offsets[0]) return fail(ctx, PLAAC_E_INVALID, "NULL codes");
     }
-    if (!summaries && !per_res && !hits && !eff) return fail(ctx, PLAAC_E_INVALID, "no output requested");
+    if (!summaries && !per_res && !hits && !eff && !seg) return fail(ctx, PLAAC_E_INVALID, "no output requested");
     CU(ctx, cudaSetDevice(ctx->device));
-    const bool want_rec = summaries || hits || eff;  // the device computes records
+    const bool want_rec = summaries || hits || eff || seg;  // the device computes records
     int rc = PLAAC_OK;
     if (hits && (rc = ensure(ctx, ctx->all_summaries, sizeof(plaac_summary) * (size_t)nprot))) return rc;
     int64_t var_total = 0;
@@ -1726,10 +1796,57 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
     const void* out_rows = eff ? (const void*)eff->effects : (const void*)summaries;
     const size_t row_bytes = eff ? sizeof(double) * (size_t)ek : sizeof(plaac_summary);
     const bool stage_sum = out_rows && !host_is_pinned(out_rows);
+    // Segments: drained in chunk order, so seg_base is the number of segments of the proteins before the chunk.  A chunk
+    // whose segments overflowed the slot's entries (and are wanted) reruns its bounds and score kernels with room for all
+    // of them: the parse, codes and offsets are still in the slot.
+    int64_t seg_base = 0;
+    auto seg_drain = [&](Slot& s) -> int {
+        const int64_t np = s.seg_np;
+        s.seg_np = -1;
+        const int64_t* hf = (const int64_t*)s.h_sg_first;
+        const int64_t total = hf[np];
+        for (int64_t i = 0; i < np; i++) seg->first[s.seg_p0 + i] = seg_base + hf[i];
+        const int64_t want = std::min(total, std::max<int64_t>(seg->capacity - seg_base, 0));
+        if (want > s.seg_cap) {
+            int rc2;
+            if ((rc2 = ensure(ctx, s.sg_ent, (3 * sizeof(int32_t) + sizeof(double)) * (size_t)total))) return rc2;
+            SegArgs a = s.seg_args;
+            double* ent = (double*)s.sg_ent.p;
+            a.cap = total;
+            a.score = ent;
+            a.prot = (int32_t*)(ent + total);
+            a.start = a.prot + total;
+            a.end = a.start + total;
+            if ((rc2 = launch_segments(ctx, s, a, np, false))) return rc2;
+            if ((rc2 = ensure_host(ctx, s.h_sg_ent, s.h_sg_ent_cap, 16 * (size_t)total))) return rc2;
+            CU(ctx, cudaMemcpyAsync(s.h_sg_ent, a.score, sizeof(double) * (size_t)total, cudaMemcpyDeviceToHost, s.stream));
+            CU(ctx, cudaMemcpyAsync((double*)s.h_sg_ent + total, a.start, 2 * sizeof(int32_t) * (size_t)total, cudaMemcpyDeviceToHost, s.stream));
+            CU(ctx, cudaStreamSynchronize(s.stream));
+            s.seg_cap = total;
+        }
+        const double* hs = (const double*)s.h_sg_ent;
+        const int32_t* hb = (const int32_t*)(hs + s.seg_cap);
+        if (want > 0) {
+            memcpy(seg->score + seg_base, hs, sizeof(double) * (size_t)want);
+            memcpy(seg->start + seg_base, hb, sizeof(int32_t) * (size_t)want);
+            memcpy(seg->end + seg_base, hb + s.seg_cap, sizeof(int32_t) * (size_t)want);
+        }
+        seg_base += total;
+        return PLAAC_OK;
+    };
     auto drain = [&](int i) -> int {
         if (!pending[i]) return PLAAC_OK;
         pending[i] = false;
-        return finish_slot(ctx, ctx->slot[i]);
+        Slot& s = ctx->slot[i];
+        int rcf = finish_slot(ctx, s);
+        // (input bytes > 21: the chunk was scored in full, its segments are written like its records)
+        if (seg && s.seg_np >= 0 && (rcf == PLAAC_OK || rcf == PLAAC_E_INVALID)) {
+            const std::string keep = ctx->err;
+            const int rcs = seg_drain(s);
+            if (rcs != PLAAC_OK) return rcs;
+            ctx->err = keep;
+        }
+        return rcf;
     };
     // Inside the chunk loop a CUDA error may not return at once: copies into the caller's buffers may be in flight on
     // other slots, and the header promises "blocks until done".  Errors break out to the drain loop below.
@@ -1833,7 +1950,7 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
         plaac_summary* d_sum = nullptr;
         if (hits)
             d_sum = (plaac_summary*)ctx->all_summaries.p + start;
-        else if (summaries || eff) {
+        else if (summaries || eff || seg) {
             if ((rc = ensure(ctx, s.summaries, sizeof(plaac_summary) * np))) break;
             d_sum = (plaac_summary*)s.summaries.p;
         }
@@ -1912,9 +2029,23 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
             if (nres > 0) CUB(cudaMemcpyAsync(s.codes.p, src_main, (size_t)nres, cudaMemcpyHostToDevice, s.stream));
             CUB(cudaMemcpyAsync(s.offsets.p, in.offsets + start, sizeof(int64_t) * (np + 1), cudaMemcpyHostToDevice, s.stream));
         }
+        // segment entries the slot keeps per chunk: several times the density of prion-like runs in proteomes (about
+        // one per 10 000 residues); a denser chunk reruns its bounds and score kernels at drain
+        const int64_t seg_cap = seg ? nres / 2048 + 1024 : -1;
+        s.seg_np = -1;
         rc = run_batch(ctx, s, d_codes, (const int64_t*)s.offsets.p, off_base, np, nres, want_rec ? d_sum : nullptr,
-                       per_res ? &dres : nullptr, off_base, slots_bound, nlp, lp_scratch, long_thr, nbigp);
+                       per_res ? &dres : nullptr, off_base, slots_bound, nlp, lp_scratch, long_thr, nbigp, seg_cap);
         if (rc) break;
+        if (seg) {
+            s.seg_p0 = start;
+            if ((rc = ensure_host(ctx, s.h_sg_first, s.h_sg_first_cap, sizeof(int64_t) * (size_t)(np + 1)))) break;
+            if ((rc = ensure_host(ctx, s.h_sg_ent, s.h_sg_ent_cap, 16 * (size_t)seg_cap))) break;
+            const SegArgs& a = s.seg_args;
+            CUB(cudaMemcpyAsync(s.h_sg_first, a.first, sizeof(int64_t) * (size_t)(np + 1), cudaMemcpyDeviceToHost, s.stream));
+            CUB(cudaMemcpyAsync(s.h_sg_ent, a.score, sizeof(double) * (size_t)seg_cap, cudaMemcpyDeviceToHost, s.stream));
+            CUB(cudaMemcpyAsync((double*)s.h_sg_ent + seg_cap, a.start, 2 * sizeof(int32_t) * (size_t)seg_cap,
+                                cudaMemcpyDeviceToHost, s.stream));
+        }
         if (summaries && hits) {
             CUB(cudaMemcpyAsync(stage_sum ? (plaac_summary*)s.h_stage_sum : summaries + start, d_sum, sizeof(plaac_summary) * np,
                                 cudaMemcpyDeviceToHost, s.stream));
@@ -1972,6 +2103,10 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
         }
         cudaGetLastError();
         ctx->err = keep;
+    }
+    if (seg) {
+        seg->first[start] = seg_base;  // (start == nprot unless the call failed part-way)
+        seg->count = seg_base;
     }
     if (rc == PLAAC_OK && rc_wild != PLAAC_OK) {
         rc = rc_wild;
@@ -2071,6 +2206,32 @@ try {
     return score_host(ctx, in, variants->nvar, nullptr, nullptr, nullptr, false, &eff);
 } catch (...) {
     return api_caught(ctx, "plaac_score_variant_effects");
+}
+
+int plaac_score_segments(plaac_ctx* ctx, const uint8_t* codes, const int64_t* offsets, int64_t nprot,
+                         plaac_summary* summaries, plaac_segments* segments)
+try {
+    if (!ctx) return fail(nullptr, PLAAC_E_INVALID, "plaac_score_segments: NULL ctx");
+    if (!segments) return fail(ctx, PLAAC_E_INVALID, "plaac_score_segments: NULL segments");
+    segments->count = 0;
+    if (nprot < 0) return fail(ctx, PLAAC_E_INVALID, "negative nprot");
+    if (segments->capacity < 0)
+        return fail(ctx, PLAAC_E_INVALID, "plaac_score_segments: negative capacity %lld", (long long)segments->capacity);
+    if (nprot > 0 && !segments->first) return fail(ctx, PLAAC_E_INVALID, "plaac_score_segments: NULL first with nprot = %lld", (long long)nprot);
+    if (segments->capacity > 0 && (!segments->start || !segments->end || !segments->score))
+        return fail(ctx, PLAAC_E_INVALID, "plaac_score_segments: NULL start, end or score with capacity = %lld",
+                    (long long)segments->capacity);
+    if (nprot > 0 && !offsets) return fail(ctx, PLAAC_E_INVALID, "NULL offsets");
+    if (nprot == 0) {
+        if (segments->first) segments->first[0] = 0;
+        return PLAAC_OK;
+    }
+    HostInput in;
+    in.codes = codes;
+    in.offsets = offsets;
+    return score_host(ctx, in, nprot, summaries, nullptr, nullptr, false, nullptr, segments);
+} catch (...) {
+    return api_caught(ctx, "plaac_score_segments");
 }
 
 }  // extern "C"

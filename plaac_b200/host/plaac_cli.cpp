@@ -28,6 +28,10 @@
 //                   list of LLR COREscore PRDscore HMMall HMMvit FImeanhydro FImeancharge FImeancombo PAPAcombo PAPAprop
 //                   PAPAfi PAPAllr PAPAllr2 (printed as d<NAME>, variant minus wild type) and COREchange (1 gained,
 //                   -1 lost, 0 unchanged)
+//   --segments FILE also write every prion-like segment of each record's Viterbi parse (each maximal run of PrD-state
+//                   residues; plaac_score_segments) to FILE as a table: SEQid SEGstart SEGend SEGlen SEGscore PRD, 1-based
+//                   positions, SEGscore the PRDscore sum over the segment, PRD 1 for the segment that is the row's PrD.
+//                   One line per segment, in record order (also with --rank); the summary table is unchanged
 #include <algorithm>
 #include <charconv>
 #include <cmath>
@@ -416,6 +420,8 @@ struct Options {
     std::string effects;        // --effects, as given
     bool effects_set = false;
     int32_t effects_mask = 0;   // PLAAC_EFFECT_* bits of --effects
+    std::string segments_file;  // --segments
+    FILE* seg_out = nullptr;    // ... open
 };
 
 // --effects names, bit k = PLAAC_EFFECT_* bit k (the doubles of plaac_summary in declaration order, then COREchange)
@@ -549,13 +555,52 @@ void print_summary_row(const Options& o, const std::string& name, const plaac_su
     std::fwrite(line.data(), 1, line.size(), stdout);
 }
 
+// --segments: the records of the batch and the segments of their Viterbi parses; the segment table is written here.
+int score_segment_batch(const Options& o, Scorers& S, Batch& B, std::vector<plaac_summary>& sum)
+{
+    const int64_t np = B.nprot();
+    std::vector<int64_t> first((size_t)np + 1);
+    std::vector<int32_t> st, en;
+    std::vector<double> sc;
+    plaac_segments G = {};
+    for (int64_t cap = np;;) {  // (a second pass only for a batch with more segments than records)
+        st.resize((size_t)std::max<int64_t>(cap, 1)), en.resize(st.size()), sc.resize(st.size());
+        G = {cap, first.data(), st.data(), en.data(), sc.data(), 0};
+        const int rc = plaac_score_segments(S.ctx[0], B.codes.data(), B.offsets.data(), np, sum.data(), &G);
+        if (rc != PLAAC_OK) return die(S, rc, "plaac_score_segments");
+        if (G.count <= cap) break;
+        cap = G.count;
+    }
+    std::string out;
+    for (int64_t i = 0; i < np; i++) {
+        const plaac_summary& r = sum[(size_t)i];
+        for (int64_t k = first[(size_t)i]; k < first[(size_t)i + 1]; k++) {
+            out.append(B.names[(size_t)i]);
+            auto I = [&](long v) { out.push_back('\t'), put_int(out, v); };
+            I(st[(size_t)k] + 1), I(en[(size_t)k] + 1), I(en[(size_t)k] - st[(size_t)k] + 1);
+            out.push_back('\t'), put_fixed(out, sc[(size_t)k], 3);
+            I(st[(size_t)k] == r.prd_start && en[(size_t)k] == r.prd_end ? 1 : 0);
+            out.push_back('\n');
+        }
+    }
+    if (std::fwrite(out.data(), 1, out.size(), o.seg_out) != out.size() || std::fflush(o.seg_out) != 0) {
+        std::fprintf(stderr, "plaac: cannot write %s\n", o.segments_file.c_str());
+        return 2;
+    }
+    return 0;
+}
+
 int score_summary_batch(const Options& o, Scorers& S, Batch& B)
 {
     if (B.nprot() == 0) return 0;
     std::vector<plaac_summary> sum((size_t)B.nprot());
-    const int rc = plaac_score_multi(S.ctx.data(), (int)S.ctx.size(), B.codes.data(), B.offsets.data(), B.nprot(),
-                                     sum.data(), nullptr);
-    if (rc != PLAAC_OK) return die(S, rc, "plaac_score");
+    if (o.seg_out) {
+        if (const int rs = score_segment_batch(o, S, B, sum)) return rs;
+    } else {
+        const int rc = plaac_score_multi(S.ctx.data(), (int)S.ctx.size(), B.codes.data(), B.offsets.data(), B.nprot(),
+                                         sum.data(), nullptr);
+        if (rc != PLAAC_OK) return die(S, rc, "plaac_score");
+    }
     std::string line;
     if (o.rank) {
         std::vector<int32_t> order((size_t)B.nprot());
@@ -1203,6 +1248,8 @@ void usage()
     std::puts("                   the listed columns (comma-separated: LLR COREscore PRDscore HMMall HMMvit FImeanhydro");
     std::puts("                   FImeancharge FImeancombo PAPAcombo PAPAprop PAPAfi PAPAllr PAPAllr2, printed as d<NAME>;");
     std::puts("                   COREchange: 1 CORE gained, -1 lost, 0 unchanged)");
+    std::puts("  --segments FILE  also write every prion-like segment (maximal run of PrD-state residues of the Viterbi");
+    std::puts("                   parse) of every record to FILE: SEQid SEGstart SEGend SEGlen SEGscore PRD");
     std::puts("  --compat-F       -F reads the -B file, as plaac.jar does (plaac.java:388); without it -F reads its own file,");
     std::puts("                   so the parameter block and every score differ from the jar's for the same command line");
 }
@@ -1244,6 +1291,8 @@ int main(int argc, char** argv)
             o.saturate = true;
         else if (a == "--effects")
             o.effects = val("--effects"), o.effects_set = true;
+        else if (a == "--segments")
+            o.segments_file = val("--segments");
         else if (a == "--format-check") {
             // test hook: lines "decimals value" on stdin -> the Java-formatted value on stdout
             int d;
@@ -1282,6 +1331,19 @@ int main(int argc, char** argv)
     }
     o.ww3 = o.ww2;  // :355
 
+    if (!o.segments_file.empty()) {
+        const char* clash = !o.plotlist.empty()        ? "-p"
+                            : !o.variants_file.empty() ? "--variants"
+                            : o.saturate               ? "--saturate"
+                            : o.gpu_ingest             ? "--gpu-ingest"
+                            : o.gpus > 1               ? "--gpus > 1"
+                                                       : nullptr;
+        if (clash) {
+            std::fprintf(stderr, "plaac: --segments cannot be combined with %s\n", clash);
+            return 2;
+        }
+        o.host_reader = true;  // segments come with the records of plaac_score_segments, not the GPU reader's
+    }
     const bool variants = o.saturate || !o.variants_file.empty();
     VariantFile vfile;
     if (variants) {
@@ -1469,6 +1531,16 @@ int main(int argc, char** argv)
     }
     Batch B;
     std::string seq, name;
+    std::unique_ptr<FILE, int (*)(FILE*)> seg_file(nullptr, std::fclose);
+    if (!o.segments_file.empty()) {
+        seg_file.reset(std::fopen(o.segments_file.c_str(), "w"));
+        if (!seg_file) {
+            std::fprintf(stderr, "plaac: cannot open %s for writing\n", o.segments_file.c_str());
+            return 2;
+        }
+        o.seg_out = seg_file.get();
+        std::fputs("SEQid\tSEGstart\tSEGend\tSEGlen\tSEGscore\tPRD\n", o.seg_out);
+    }
     if (o.plotlist.empty()) {
         print_table_head();
         if ((rc = open_devices())) return rc;
