@@ -28,6 +28,8 @@ struct DeviceTables {
     // sliding-window sums of the summary kernels are then exact, i.e. independent of the order and of where a running
     // sum was (re)started; hyd stays exact for the sequential mean and the per-residue tracks
     double hydw[kTabN];
+    // hydw[e] ~ hydi[e] / q when the host proved the integer form of the FoldIndex tests exact (plan_int_fold), else 0
+    int32_t hydi[kTabN];
     double lut[PLAAC_LUT_LEN + 3];
 };
 

@@ -10,6 +10,7 @@
 #include <cstring>
 #include <memory>
 #include <new>
+#include <numeric>
 #include <string>
 #include <thread>
 #include <vector>
@@ -35,6 +36,13 @@ using namespace plaac;
 namespace {
 
 thread_local std::string g_last_error = "";
+
+// Integer form of the v3 kernel's FoldIndex / PAPA sign tests (kV3IntFold, plan_int_fold): hydw[c] ~ h[c] / q and
+// M * (cc0 * X + cc1 * C + cc2 * taps) = a * (sum of h) + b * C + c * taps
+struct IntFold {
+    int32_t h[PLAAC_NAA];
+    int32_t a, b, c;
+};
 
 struct DevBuf {
     void* p = nullptr;
@@ -111,7 +119,8 @@ struct plaac_ctx {
     size_t v2_smem_bytes = 0;
     int v3_nwr = 0, v3_opt = 0, v3_mix = 0, v3_nt = 768;  // v3 kernel (same preconditions as v2): warps per role, option bits, role placement
     size_t v3_smem_bytes = 0;
-    int v2_always_in = 0;      // forward recurrence provably keeps |a-b| < 40 (no LUT range test needed)
+    IntFold ifold = {};        // valid when v3_opt has kV3IntFold
+    int v2_always_in = 0;     // forward recurrence provably keeps |a-b| < 40 (no LUT range test needed)
     ResidueV2Plan res_plan;
     int variant = 0;           // 0 auto, 1 = v1 (reference-order anchor), 2 = v2
     std::string v2_why;
@@ -214,6 +223,8 @@ int next_pow2(int x)
     return p;
 }
 
+bool plan_int_fold(const plaac_params& P, int w, IntFold& f);
+
 int setup_scalars(plaac_ctx* ctx)
 {
     const plaac_params& P = ctx->params;
@@ -300,6 +311,8 @@ int setup_scalars(plaac_ctx* ctx)
             if (const char* e = getenv("PLAAC_V3_OPT")) opt = atoi(e);
             // the packed Q/N window needs counts that fit a byte and the jar's Q/N code set
             if (P.mw_window > 100 || k.qn_mask != ((1u << 12) | (1u << 14))) opt &= ~kV3SwarMw;
+            // ... and the integer FoldIndex tests a proof that they give the FP64 signs for these tables and windows
+            if (!plan_int_fold(P, k.w, ctx->ifold)) opt &= ~kV3IntFold;
             int nt = 768;
             if (const char* e = getenv("PLAAC_V3_NT")) nt = atoi(e);
             nwr = std::min(nwr, nt / 64);
@@ -354,7 +367,14 @@ double sum_grid(const double* tab, int w)
     return std::ldexp(1.0, k);
 }
 
-void fill_tables(const plaac_params& P, DeviceTables& T, int w)
+// hydropathy on the exact-sum grid gridh = sum_grid(P.hydro2, w) (DeviceTables::hydw)
+double hyd_on_grid(const plaac_params& P, int c, double gridh)
+{
+    return gridh > 0 ? std::nearbyint(P.hydro2[c] / gridh) * gridh : P.hydro2[c];
+}
+
+// ifold: the integer hydropathy table of kV3IntFold, or null
+void fill_tables(const plaac_params& P, DeviceTables& T, int w, const IntFold* ifold)
 {
     memset(&T, 0, sizeof(T));
     const double grid = sum_grid(P.papa_lod, w);
@@ -370,12 +390,101 @@ void fill_tables(const plaac_params& P, DeviceTables& T, int w)
         T.lebg[e] = P.le0[c];
         T.llr[e] = P.llr[c];
         T.hyd[e] = P.hydro2[c];
-        T.hydw[e] = gridh > 0 ? std::nearbyint(P.hydro2[c] / gridh) * gridh : P.hydro2[c];
+        T.hydw[e] = hyd_on_grid(P, c, gridh);
+        if (ifold) T.hydi[e] = ifold->h[c];
         double pl = P.papa_lod[c];
         if (grid > 0) pl = std::nearbyint(pl / grid) * grid;
         T.pap[e] = (e & kPapaMaskBit) ? 0.0 : pl;
     }
     for (int i = 0; i < PLAAC_LUT_LEN; i++) T.lut[i] = P.loglut[i];
+}
+
+// Smallest d in [1, maxd] with x*d within 1e-9 of an integer n (the tolerance only picks the candidate; plan_int_fold's
+// error bound decides), or 0.
+int64_t small_denominator(double x, int64_t maxd, int64_t& n)
+{
+    if (!(std::fabs(x) < 1e6)) return 0;
+    for (int64_t d = 1; d <= maxd; d++) {
+        const double y = x * (double)d;
+        if (std::fabs(y - std::nearbyint(y)) <= 1e-9) {
+            n = (int64_t)std::nearbyint(y);
+            return d;
+        }
+    }
+    return 0;
+}
+
+// Can the v3 kernel's role B test the signs of fi = (cc0 * X + cc1 * C) + cc2 * taps (X = a hydropathy window sum on the
+// hydw grid, C = |charge sum|; the FoldIndex run test over 2w+1 taps, the PAPA gate over (2w+1)^2) in exact int32?
+//   * the grid must be in use: only then is X exactly the sum of hydw, independent of order;
+//   * hydw[c] ~ h[c] / q and cc_i ~ n_i / d_i with small q, d_i, so that for M = lcm(q d0, d1, d2) the rational value
+//     of fi is V / M, V = a * sum(h) + b * C + c * taps an integer (PLAAC: q = 90, M = 18000, V = 557 S - 18000 C - 20718 taps);
+//   * every V over the (2w+1)^2 taps of the PAPA gate lies in int32 (the kernel wraps, only the final value counts);
+//   * the FP64 value v2 computes differs from V / M by at most E (representation errors of the tables and coefficients,
+//     five roundings), and E < 1 / (2M): where V != 0, |V / M| >= 1/M and the FP64 value has V's sign.
+// A bucket where a deciding test has V == 0 is scored again with the FP64 sums (role_b3).
+bool plan_int_fold(const plaac_params& P, int w, IntFold& f)
+{
+    const double gridh = sum_grid(P.hydro2, w);
+    if (!(gridh > 0)) return false;
+    double hw[PLAAC_NAA];
+    double hmax = 0;
+    for (int c = 0; c < PLAAC_NAA; c++) {
+        hw[c] = hyd_on_grid(P, c, gridh);
+        hmax = std::max(hmax, std::fabs(hw[c]));
+    }
+    int q = 0;
+    for (int qq = 1; qq <= 1000 && q == 0; qq++) {
+        bool ok = true;
+        for (int c = 0; c < PLAAC_NAA && ok; c++) ok = std::fabs(hw[c] * qq - std::nearbyint(hw[c] * qq)) <= 1e-9;
+        if (ok) q = qq;
+    }
+    if (q == 0) return false;
+    int64_t num[3], den[3];
+    for (int i = 0; i < 3; i++)
+        if ((den[i] = small_denominator(P.fi_cc[i], 10000, num[i])) == 0) return false;
+    const int64_t d0 = q * den[0];
+    int64_t M = d0 / std::gcd(d0, den[1]) * den[1];
+    M = M / std::gcd(M, den[2]) * den[2];
+    if (M >= ((int64_t)1 << 31)) return false;
+    const double coef[3] = {(double)(num[0] * (M / d0)), (double)(num[1] * (M / den[1])), (double)(num[2] * (M / den[2]))};
+    // value range over every window: sum(h) in W*[min(0, hmin), max(0, hmax)] (padding counts 0), C in [0, W], taps in [1, W]
+    const double full = 2.0 * w + 1.0, W = full * full;
+    double hlo = 0, hhi = 0;
+    for (int c = 0; c < PLAAC_NAA; c++) {
+        f.h[c] = (int32_t)std::nearbyint(hw[c] * q);
+        hlo = std::min(hlo, (double)f.h[c]);
+        hhi = std::max(hhi, (double)f.h[c]);
+    }
+    const double lim = 2147483647.0;
+    const double vlo = std::min(coef[0] * hlo * W, coef[0] * hhi * W) + std::min(0.0, coef[1] * W) + std::min(coef[2], coef[2] * W);
+    const double vhi = std::max(coef[0] * hlo * W, coef[0] * hhi * W) + std::max(0.0, coef[1] * W) + std::max(coef[2], coef[2] * W);
+    if (!(vlo > -lim && vhi < lim && std::max(-hlo, hhi) * W < lim)) return false;
+    // error bound at W taps (the larger test); every value below is an upper bound, with one ulp for its own rounding
+    constexpr double u = 1.0 / 4503599627370496.0;  // 2^-52
+    double eh = 0;  // max |hw[c] - h[c]/q|
+    for (int c = 0; c < PLAAC_NAA; c++) eh = std::max(eh, (std::fabs(hw[c] * q - f.h[c]) + u * std::fabs(hw[c] * q)) / q);
+    double dc[3];  // |cc_i - n_i/d_i|
+    for (int i = 0; i < 3; i++) {
+        const double y = P.fi_cc[i] * (double)den[i];
+        dc[i] = (std::fabs(y - (double)num[i]) + u * std::fabs(y)) / (double)den[i];
+    }
+    const double cc0 = std::fabs(P.fi_cc[0]), cc1 = std::fabs(P.fi_cc[1]), cc2 = std::fabs(P.fi_cc[2]);
+    const double mag = (cc0 * hmax + cc1 + cc2) * W;  // bound on every intermediate of the FP64 expression
+    const double E = (dc[0] * hmax + cc0 * eh + dc[1] + dc[2]) * W + 5.0 * u * mag;
+    if (!(E * (double)M < 0.5)) return false;
+    // the kernel does not look for zeros of its unclipped FoldIndex test (2w+1 residues, |charge sum| C <= 2w+1): no
+    // sum of hydi over 2w+1 residues may give V == 0 there
+    for (int64_t C = 0; C <= 2 * w + 1; C++) {
+        const int64_t rest = -((int64_t)coef[1] * C + (int64_t)coef[2] * (2 * w + 1));
+        if (coef[0] == 0 ? rest == 0 : (rest % (int64_t)coef[0] == 0 && rest / (int64_t)coef[0] >= hlo * full &&
+                                        rest / (int64_t)coef[0] <= hhi * full))
+            return false;
+    }
+    f.a = (int32_t)coef[0];
+    f.b = (int32_t)coef[1];
+    f.c = (int32_t)coef[2];
+    return true;
 }
 
 int slot_init(plaac_ctx* ctx, Slot& s)
@@ -819,6 +928,11 @@ int run_batch(plaac_ctx* ctx, Slot& s, const uint8_t* d_codes, const int64_t* d_
             g.ks_cc2w = ctx->ks.cc2 * g.ks_wfull;
             g.ks_cc2full = ctx->ks.cc2 * (double)full;
             g.mix_roles = ctx->v3_mix;
+            g.fi_a = ctx->ifold.a;
+            g.fi_b = ctx->ifold.b;
+            g.fi_c = ctx->ifold.c;
+            g.fi_cfull = ctx->ifold.c * full;
+            g.fi_cw = ctx->ifold.c * full * full;
         }
         const int64_t nitems = 2 * nbuckets, wpc = 2 * g.nwr;
         const unsigned grid = (unsigned)std::min<int64_t>((nitems + wpc - 1) / wpc, ctx->sm_count);  // 1 CTA per SM
@@ -1255,7 +1369,7 @@ try {
     }
     {
         std::unique_ptr<DeviceTables> h(new DeviceTables());
-        fill_tables(ctx->params, *h, ctx->ks.w);
+        fill_tables(ctx->params, *h, ctx->ks.w, (ctx->v3_opt & kV3IntFold) ? &ctx->ifold : nullptr);
         cudaError_t e = cudaMalloc((void**)&ctx->d_tabs, sizeof(DeviceTables));
         if (e == cudaSuccess) e = cudaMemcpy(ctx->d_tabs, h.get(), sizeof(DeviceTables), cudaMemcpyHostToDevice);
         if (e != cudaSuccess) {

@@ -6,7 +6,10 @@
 //     flags, the window count after each residue and the "new maximum?" test for a whole word cost ~20 instructions
 //     instead of ~12 per residue; only a lane that does see a new maximum walks its four residues one by one;
 //   * traceback bits are collected per word in a nibble with predicated ORs and shifted into the bit planes once per word;
-//   * role B gets (2w+1)^2, cc2 * (2w+1)^2 and cc2 * (2w+1) as doubles from the host instead of re-converting them.
+//   * role B gets (2w+1)^2, cc2 * (2w+1)^2 and cc2 * (2w+1) as doubles from the host instead of re-converting them;
+//   * kV3IntFold: role B's hydropathy window sums and the FoldIndex / PAPA sign tests built on them run on the integer
+//     pipes (3 IADD3 for the sums, 2 IMAD + ISETP per test, 32-bit table loads) instead of 18 FP64 instructions per
+//     residue, where the host proved that the integer sign is v2's FP64 sign (plan_int_fold, plaac_cuda.cu).
 //
 // OPT is a compile-time bit set so that single steps can be measured against each other (PLAAC_V3_OPT).  Measured and
 // dropped (round 2, profiles/r02_v3_variants.json): a merged {le0, le1, llr} table entry (32-byte stride: two of the
@@ -24,8 +27,23 @@ namespace plaac {
 constexpr int kV3SwarMw = 1;    // SWAR Q/N window in role A's fast path (needs mw_window <= 100 and the Q/N code set {12, 14})
 constexpr int kV3NibbleTb = 2;  // traceback bits per word in a nibble
 constexpr int kV3Segments = 8;  // segmented word loop (measured slower; kept for the record)
+constexpr int kV3IntFold = 16;  // role B's hydropathy sums and FoldIndex / PAPA sign tests in exact int32 (plan_int_fold)
 
-// (shared-memory layout: v2's, kOff* / kV2FixedBytes / kV2AlignSlack)
+// (shared-memory layout: v2's, kOff* / kV2FixedBytes / kV2AlignSlack; under kV3IntFold the kOffHydB slots hold
+// DeviceTables::hydi in their low word instead of hydw)
+
+__device__ __forceinline__ int lds_s32(uint32_t addr)
+{
+    int v;
+    asm("ld.shared.s32 %0, [%1];" : "=r"(v) : "r"(addr));
+    return v;
+}
+
+// a*x + b*y + c in wrapping 32-bit arithmetic: the host proved that the true value of every test lies in int32
+__device__ __forceinline__ int fold_int(int a, int x, int b, int y, int c)
+{
+    return (int)((uint32_t)a * (uint32_t)x + (uint32_t)b * (uint32_t)y + (uint32_t)c);
+}
 
 // ------------------------------------------------------------------------------------------------ role A
 template <int OPT>
@@ -329,8 +347,11 @@ __device__ __forceinline__ void role_a3(const V2Args& g, uint32_t sbase, uint32_
 }
 
 // ------------------------------------------------------------------------------------------------ role B
-template <int OPT>
-__device__ __forceinline__ void role_b3(const V2Args& g, uint32_t sbase, uint32_t* ring, int lane, int64_t b)
+// Returns true, with no record written, when the integer form of a FoldIndex test or PAPA gate that decides something
+// is exactly 0 for a lane of the bucket (IFOLD only): the FP64 sign is then rounding, and the caller scores the bucket
+// again with the FP64 sums (GH: hydw read from global memory, the shared slots holding hydi).
+template <int OPT, bool GH = false>
+__device__ __forceinline__ bool role_b3(const V2Args& g, uint32_t sbase, uint32_t* ring, int lane, int64_t b)
 {
     const KScalars& ks = g.ks;
     const BatchView& bv = g.bv;
@@ -353,6 +374,7 @@ __device__ __forceinline__ void role_b3(const V2Args& g, uint32_t sbase, uint32_
     const int a2o = off2 >> 2, s2o = 8 * (4 - (off2 & 3));
     const int full = 2 * w + 1;
     const int Wfull = full * full;
+    constexpr bool IFOLD = (OPT & kV3IntFold) != 0;
 
     const uint32_t hb = sbase + kOffHydB + (uint32_t)(lane & 15) * 8u;
 
@@ -365,8 +387,11 @@ __device__ __forceinline__ void role_b3(const V2Args& g, uint32_t sbase, uint32_
     double sh = 0;
     int csum = 0;
     double SLh = 0, SGh = 0, Th = 0, Dp = 0, Tp = 0;
+    int SLi = 0, SGi = 0, Ti = 0;  // IFOLD: the same window sums in units of 1/q (DeviceTables::hydi)
     int SLc = 0, SGc = 0, Tac = 0;
     double Tb = 0, Wb = 1, vfib = 0;
+    int Tacb = 0;      // IFOLD: Tac at the PAPA centre (vfib is rebuilt from it after the loop)
+    bool amb = false;  // IFOLD: an integer test that decides something was exactly 0
     int pcen = -1;
     int halfw = ks.h_fi;
     if (halfw > n / 2) halfw = n / 2;
@@ -374,6 +399,7 @@ __device__ __forceinline__ void role_b3(const V2Args& g, uint32_t sbase, uint32_
     const int edge_hi = n - 1 - w;   // windows centred beyond this are clipped on the right
     int fi_run = 0, fi_numaa = 0, fi_maxrun = 0;  // fi_run: length of the open run of fi < 0 (snaps included)
     uint32_t lo1 = kPadW, lo2 = kPadW;
+    const double* hydw = g.tabs->hydw;
     // (host-computed: (double)(2w+1)^2, cc2 * that, cc2 * (2w+1); the compiler otherwise rematerialises the conversion
     // inside the loop to save registers)
     const double WfullD = g.ks_wfull, cc2W = g.ks_cc2w, cc2full = g.ks_cc2full;
@@ -391,9 +417,10 @@ __device__ __forceinline__ void role_b3(const V2Args& g, uint32_t sbase, uint32_
         const uint32_t k0 = (i == 0 ? (w0 << 7) : (w0 >> (8 * i - 7))) & (63u << 7);
         const uint32_t k1 = (i == 0 ? (w1 << 7) : (w1 >> (8 * i - 7))) & (63u << 7);
         const uint32_t k2 = (i == 0 ? (w2 << 7) : (w2 >> (8 * i - 7))) & (63u << 7);
-        const double hy0 = lds_f64(hb | k0), pa0 = lds_f64_off<kOffPapB>(hb | k0);
-        const double hy1 = lds_f64(hb | k1), pa1 = lds_f64_off<kOffPapB>(hb | k1);
-        const double hy2 = lds_f64(hb | k2), pa2 = lds_f64_off<kOffPapB>(hb | k2);
+        // (under IFOLD the FP64 hydropathy loads and conversions below are dead and compiled out)
+        const double hy0 = IFOLD ? 0.0 : GH ? hydw[k0 >> 7] : lds_f64(hb | k0), pa0 = lds_f64_off<kOffPapB>(hb | k0);
+        const double hy1 = IFOLD ? 0.0 : GH ? hydw[k1 >> 7] : lds_f64(hb | k1), pa1 = lds_f64_off<kOffPapB>(hb | k1);
+        const double hy2 = IFOLD ? 0.0 : GH ? hydw[k2 >> 7] : lds_f64(hb | k2), pa2 = lds_f64_off<kOffPapB>(hb | k2);
         const int ch0 = (int)(w0 << (24 - 8 * i)) >> 30;
         const int ch1 = (int)(w1 << (24 - 8 * i)) >> 30;
         const int ch2 = (int)(w2 << (24 - 8 * i)) >> 30;
@@ -405,27 +432,39 @@ __device__ __forceinline__ void role_b3(const V2Args& g, uint32_t sbase, uint32_
         const double aSLd = u2d((uint32_t)aSL);
         if (FAST || t < n) sh = sh + lds_f64_off<kOffHydX>(hb | k0);  // mean() :1584, sequential, exact table values
         // window sums of the zero-padded sequence: lead centre p = t-w, lag centre p-(2w+1)
-        SLh = (SLh + hy0) - hy1;
-        SGh = (SGh + hy1) - hy2;
-        Th = (Th + SLh) - SGh;
+        if (IFOLD) {
+            const int h0 = lds_s32(hb | k0), h1 = lds_s32(hb | k1), h2 = lds_s32(hb | k2);
+            SLi += h0 - h1;
+            SGi += h1 - h2;
+            Ti += SLi - SGi;
+        } else {
+            SLh = (SLh + hy0) - hy1;
+            SGh = (SGh + hy1) - hy2;
+            Th = (Th + SLh) - SGh;
+        }
         Dp = Dp + ((pa0 + pa2) - (pa1 + pa1));  // exact: PAPA log-odds live on a 2^-k grid
         Tp = Tp + Dp;
         const double TacD = u2d((uint32_t)Tac);
         const int p = t - w;
+        // IFOLD: a nonzero integer form has the FP64 sign (plan_int_fold); a zero one sets amb
         // FoldIndex run scan :5010-5059 over i in [halfw, n-halfw):
         // sign of fi[p] = cc0*hydro + cc1*|charge| + cc2, scaled by the tap count (> 0)
         if (FAST) {
-            const double fis = (cc0 * SLh + cc1 * aSLd) + cc2full;
-            const bool neg = fis < 0;
+            // (IFOLD: the host proved that the unclipped integer test is never 0)
+            const double fis = IFOLD ? 0.0 : (cc0 * SLh + cc1 * aSLd) + cc2full;
+            const bool neg = IFOLD ? fold_int(g.fi_a, SLi, g.fi_b, aSL, g.fi_cfull) < 0 : fis < 0;
             const int closed = (!neg && fi_run >= 5) ? fi_run : 0;
             fi_numaa += closed;
             fi_maxrun = max(fi_maxrun, closed);
             fi_run = neg ? fi_run + 1 : 0;
         } else if (p >= halfw && p < fi_hi) {
             double c2 = cc2full;
-            if (p < w || p > edge_hi) c2 = ks.cc2 * u2d((uint32_t)(full - max(0, w - p) - max(0, p - edge_hi)));
-            const double fis = (cc0 * SLh + cc1 * aSLd) + c2;
-            const bool neg = fis < 0;
+            const int taps = full - max(0, w - p) - max(0, p - edge_hi);
+            if (p < w || p > edge_hi) c2 = ks.cc2 * u2d((uint32_t)taps);
+            const double fis = IFOLD ? 0.0 : (cc0 * SLh + cc1 * aSLd) + c2;
+            const int v = IFOLD ? fold_int(g.fi_a, SLi, g.fi_b, aSL, g.fi_c * taps) : 0;
+            if (IFOLD && v == 0) amb = true;
+            const bool neg = IFOLD ? v < 0 : fis < 0;
             const bool last = (p == fi_hi - 1);
             // a run that starts at the first scanned position is snapped back to residue 0,
             // one that reaches the last scanned position is snapped forward to residue n-1
@@ -441,27 +480,38 @@ __device__ __forceinline__ void role_b3(const V2Args& g, uint32_t sbase, uint32_
         }
         // PAPA centre k = p - w: first strict maximum of Tp/W among centres with fix2 < 0 (:4941-4948)
         // Tp/Wd > Tb/Wb  <=>  Tp*Wb > Tb*Wd (both positive); products of grid units and small ints
+        // (IFOLD: vfib is not carried; the gate's value at the centre is rebuilt after the loop from Tacb)
         if (FAST) {
-            const double vfi = (cc0 * Th + cc1 * TacD) + cc2W;
-            if ((pcen < 0 || Tp * Wb > Tb * WfullD) && vfi < 0) {
+            const double vfi = IFOLD ? 0.0 : (cc0 * Th + cc1 * TacD) + cc2W;
+            const int v = IFOLD ? fold_int(g.fi_a, Ti, g.fi_b, Tac, g.fi_cw) : 0;
+            const bool better = pcen < 0 || Tp * Wb > Tb * WfullD;
+            if (IFOLD && better && v == 0) amb = true;
+            if (better && (IFOLD ? v < 0 : vfi < 0)) {
                 Tb = Tp;
                 Wb = WfullD;
                 vfib = vfi;
+                Tacb = Tac;
                 pcen = t - 2 * w;
             }
         } else {
             const int k = p - w;
             if (k >= w && k <= edge_hi) {
+                int Wi = Wfull;
                 double Wd = WfullD;
                 if (k < 2 * w || k > edge_hi - w) {
                     const int ml = 2 * w - k, mr = k - (edge_hi - w);
-                    Wd = u2d((uint32_t)(Wfull - (ml > 0 ? (ml * (ml + 1)) >> 1 : 0) - (mr > 0 ? (mr * (mr + 1)) >> 1 : 0)));
+                    Wi = Wfull - (ml > 0 ? (ml * (ml + 1)) >> 1 : 0) - (mr > 0 ? (mr * (mr + 1)) >> 1 : 0);
+                    Wd = u2d((uint32_t)Wi);
                 }
-                const double vfi = (cc0 * Th + cc1 * TacD) + ks.cc2 * Wd;
-                if ((pcen < 0 || Tp * Wb > Tb * Wd) && vfi < 0) {
+                const double vfi = IFOLD ? 0.0 : (cc0 * Th + cc1 * TacD) + ks.cc2 * Wd;
+                const int v = IFOLD ? fold_int(g.fi_a, Ti, g.fi_b, Tac, g.fi_c * Wi) : 0;
+                const bool better = pcen < 0 || Tp * Wb > Tb * Wd;
+                if (IFOLD && better && v == 0) amb = true;
+                if (better && (IFOLD ? v < 0 : vfi < 0)) {
                     Tb = Tp;
                     Wb = Wd;
                     vfib = vfi;
+                    Tacb = Tac;
                     pcen = k;
                 }
             }
@@ -513,13 +563,14 @@ __device__ __forceinline__ void role_b3(const V2Args& g, uint32_t sbase, uint32_
         }
     }
 
-    if (prot < 0) return;
+    if (IFOLD && __any_sync(0xffffffffu, amb)) return true;
+    if (prot < 0) return false;
     plaac_summary* r = g.out + prot;
     if (n < 1) {
         r->fi_numaa = r->fi_maxrun = r->papa_center = 0;
         r->fi_meanhydro = r->fi_meancharge = r->fi_meancombo = 0;
         r->papa_combo = r->papa_prop = r->papa_fi = r->papa_llr = r->papa_llr2 = 0;
-        return;
+        return false;
     }
     const double mh = (1.0 * sh) / (double)n;
     const double mc = (1.0 * (double)csum) / (double)n;
@@ -533,7 +584,7 @@ __device__ __forceinline__ void role_b3(const V2Args& g, uint32_t sbase, uint32_
         const double prop = Tb / Wb;
         r->papa_combo = prop;
         r->papa_prop = prop;
-        r->papa_fi = vfib / Wb;
+        if (!IFOLD) r->papa_fi = vfib / Wb;
         // PAPAllr = plaacllr[pcen]: 2w+1 taps in reference order (:2604-2620; pcen is interior).
         // PAPAllr2 = plaacllrx2[pcen] = sum_q (2w+1-|q-pcen|) llr[q] / W over the zero-padded sequence.
         // The 4w+1 residues around the centre are re-staged into the lane's ring column (whole 16-byte slots,
@@ -556,7 +607,7 @@ __device__ __forceinline__ void role_b3(const V2Args& g, uint32_t sbase, uint32_
                 }
             }
         }
-        double sc = 0.0, den = 0.0, t2 = 0.0;
+        double sc = 0.0, den = 0.0, t2 = 0.0, th = 0.0;
         for (int q = q0; q <= q1; q++) {
             const int rel = q - (j0 << 4);
             const uint32_t e = (ring[(rel >> 2) * 32] >> ((rel & 3) * 8)) & 63u;
@@ -567,13 +618,18 @@ __device__ __forceinline__ void role_b3(const V2Args& g, uint32_t sbase, uint32_
                 sc = sc + 1.0 * x;
             }
             t2 = t2 + x * (double)(full - dist);
+            // IFOLD: v2's Th at the centre; the products and sums on the hydw grid are exact, so any order gives its bits
+            if (IFOLD) th = th + hydw[e] * (double)(full - dist);
         }
+        // the PAPA gate's FP64 value at the centre; cc2 * Wb is the product v2 added (the host's cc2W: the same)
+        if (IFOLD) r->papa_fi = ((cc0 * th + cc1 * u2d((uint32_t)Tacb)) + ks.cc2 * Wb) / Wb;
         r->papa_llr = sc / den;
         r->papa_llr2 = t2 / Wb;
     } else {
         r->papa_combo = -INFINITY;
         r->papa_prop = r->papa_fi = r->papa_llr = r->papa_llr2 = nan("");
     }
+    return false;
 }
 
 template <int OPT, int NT>
@@ -602,7 +658,10 @@ __global__ void __launch_bounds__(NT, 1) k_score_summary_v3(V2Args g)
         double* hx = reinterpret_cast<double*>(sm + kOffHydX);
         for (int i = tid; i < kTabN * 16; i += blockDim.x) {
             hx[i] = T->hyd[i >> 4];
-            hy[i] = T->hydw[i >> 4];
+            if (OPT & kV3IntFold)
+                reinterpret_cast<int2*>(hy)[i] = make_int2(T->hydi[i >> 4], 0);
+            else
+                hy[i] = T->hydw[i >> 4];
             pa[i] = T->pap[i >> 4];
             lb[i] = T->llr[i >> 4];
         }
@@ -631,7 +690,10 @@ __global__ void __launch_bounds__(NT, 1) k_score_summary_v3(V2Args g)
             for (int i = 0; i < g.ring_words; i++) ring[i * 32] = kPadW;
             // (g.mix_roles bits 8/9: timing experiments that skip role B / role A; the records are then incomplete)
             if (role) {
-                if (!(g.mix_roles & 256)) role_b3<OPT>(g, sbase, ring, lane, item);
+                if (!(g.mix_roles & 256) && role_b3<OPT>(g, sbase, ring, lane, item)) {
+                    for (int i = 0; i < g.ring_words; i++) ring[i * 32] = kPadW;
+                    role_b3<OPT & ~kV3IntFold, true>(g, sbase, ring, lane, item);
+                }
             } else {
                 if (!(g.mix_roles & 512)) role_a3<OPT>(g, sbase, ring, lane, item);
             }
@@ -643,7 +705,7 @@ __global__ void __launch_bounds__(NT, 1) k_score_summary_v3(V2Args g)
 }
 
 // The instantiations that exist (PLAAC_V3_OPT picks one for experiments).
-constexpr int kV3DefaultOpt = kV3SwarMw;
+constexpr int kV3DefaultOpt = kV3SwarMw | kV3IntFold;
 using V3Kernel = void (*)(V2Args);
 // nt: threads per CTA the kernel is compiled for (768: 80 registers per thread)
 inline V3Kernel v3_kernel(int opt, int nt)
@@ -651,6 +713,8 @@ inline V3Kernel v3_kernel(int opt, int nt)
     if (nt == 768) switch (opt) {
         case 0: return k_score_summary_v3<0, 768>;
         case 1: return k_score_summary_v3<1, 768>;
+        case 16: return k_score_summary_v3<16, 768>;
+        case 17: return k_score_summary_v3<17, 768>;
         case 3: return k_score_summary_v3<3, 768>;
         case 8: return k_score_summary_v3<8, 768>;
     }
