@@ -283,6 +283,46 @@ typedef struct plaac_segments {
 int plaac_score_segments(plaac_ctx *ctx, const uint8_t *codes, const int64_t *offsets, int64_t nprot,
                          plaac_summary *summaries, plaac_segments *segments);
 
+/* ---- shuffled replicates: a composition-preserving null per protein (DESIGN.md section 13) -----------------------
+ * Replicate r of reference protein i (length n) is rep[t] = ref[pi(t)], pi a bijection of [0, n) that is a pure function
+ * of (seed, i, r, n): a 6-round cycle-walking Feistel network on [0, 2^b), 2^b the smallest power of two >= n, defined
+ * in DESIGN.md section 13; the identity for n <= 1.  Bytes > 21 move like any other byte. */
+
+/* Writes replicate `replicate` of `protein` (the protein's index in its batch, which selects the permutation) into
+ * out[0 .. n): out[t] = codes[pi(t)], codes the protein's n residues.  Host only, no ctx or GPU needed.
+ * PLAAC_E_INVALID for n < 0 or n >= 2^31, a negative protein or replicate, or NULL codes / out with n > 0. */
+int plaac_shuffle_host(const uint8_t *codes, int64_t n, uint64_t seed, int64_t protein, int64_t replicate, uint8_t *out);
+
+/* Column bit of plaac_null: replicates that have a CORE (the other bits are the PLAAC_EFFECT_* bits 0..12). */
+#define PLAAC_NULL_HAS_CORE (1 << 13)
+
+typedef struct plaac_null {
+    int64_t replicates;      /* in: K >= 0 shuffles per selected protein */
+    uint64_t seed;           /* in */
+    int32_t columns;         /* in: non-zero mask of PLAAC_EFFECT_* bits 0..12, plus PLAAC_NULL_HAS_CORE */
+    int32_t reserved;        /* in: must be 0 */
+    int64_t nsel;            /* in: -1 = every protein of the batch, else the length of `proteins` */
+    const int32_t *proteins; /* in: nsel reference indices (may repeat), or NULL when nsel == -1 */
+    int64_t *counts;         /* out: nsel x popcount(columns), row-major, columns in ascending bit order */
+    double *values;          /* out: NULL, or nsel x K x popcount(columns): the replicates' column values,
+                                row j*K + r = replicate r of selected protein j */
+} plaac_null;
+
+/* Scores K shuffles of each selected protein, built on the device, and counts per protein and column the replicates that
+ * reach the observed score.  codes / offsets / nprot: the reference batch, as plaac_score takes it.  For a double
+ * column f a replicate counts when key(rep.f) >= key(obs.f), key(x) = isnan(x) ? -Inf : x (a missing CORE or PAPA ranks
+ * lowest); PLAAC_NULL_HAS_CORE counts the replicates with a CORE (its value is 0 or 1).  The empirical p-value of a
+ * column is (1 + count) / (1 + K).  observed: NULL or nsel records, observed[j] byte-identical to plaac_score's record
+ * of protein proteins[j].  HOST buffers (pinned or pageable) everywhere; blocks until done.  Counts and values do not
+ * depend on the chunking, the long-path setting, the kernel variant or the selection; chunks use the automatic long-path
+ * threshold, as plaac_score_variants.
+ * PLAAC_E_INVALID, with the offending index in plaac_last_error: replicates < 0, nsel < -1, reserved != 0, columns == 0
+ * or a bit above 13, a selected index outside [0, nprot), NULL proteins with nsel >= 0, NULL counts with nsel != 0.
+ * K == 0: counts are 0 and observed is written.  nprot == 0 or nsel == 0: PLAAC_OK, nothing written.  Reference bytes
+ * > 21 are scored as X: everything is written and the call then returns PLAAC_E_INVALID, as plaac_score does. */
+int plaac_score_shuffles(plaac_ctx *ctx, const uint8_t *codes, const int64_t *offsets, int64_t nprot,
+                         plaac_null *null_spec, plaac_summary *observed);
+
 /* ---- multi-GPU (SURVEY.md section 8e): proteins are independent, so the batch is cut into contiguous,
  * residue-balanced shards, one per ctx (each ctx on its own GPU), scored concurrently by one host thread per
  * ctx, each writing its records / per-residue rows straight into the caller's arrays at the input position.

@@ -97,6 +97,18 @@ assert C.sizeof(Segments) == 48
 EFFECT_COLUMNS = tuple(n for n, t in Summary._fields_ if t is C.c_double) + ("core_change",)
 assert len(EFFECT_COLUMNS) == 14
 
+
+class Null(C.Structure):
+    _fields_ = [("replicates", C.c_int64), ("seed", C.c_uint64), ("columns", C.c_int32), ("reserved", C.c_int32),
+                ("nsel", C.c_int64), ("proteins", C.c_void_p), ("counts", C.c_void_p), ("values", C.c_void_p)]
+
+
+assert C.sizeof(Null) == 56
+
+# Columns of plaac_score_shuffles in bit order: the doubles of the record (bits 0..12, as EFFECT_COLUMNS), then the
+# replicates that have a CORE (PLAAC_NULL_HAS_CORE).
+NULL_COLUMNS = EFFECT_COLUMNS[:13] + ("has_core",)
+
 _lib = None
 
 
@@ -177,6 +189,10 @@ def lib():
         L.plaac_score_hits.argtypes = [vp, vp, vp, i64, C.POINTER(Hits)]
         L.plaac_score_segments.restype = C.c_int
         L.plaac_score_segments.argtypes = [vp, vp, vp, i64, vp, C.POINTER(Segments)]
+        L.plaac_score_shuffles.restype = C.c_int
+        L.plaac_score_shuffles.argtypes = [vp, vp, vp, i64, C.POINTER(Null), vp]
+        L.plaac_shuffle_host.restype = C.c_int
+        L.plaac_shuffle_host.argtypes = [vp, i64, C.c_uint64, i64, i64, vp]
         L.plaac_bench_synth_lengths.restype = C.c_int
         L.plaac_bench_synth_lengths.argtypes = [vp, C.c_uint64, i64, i64, dbl, dbl, i32, i32, vp]
         L.plaac_bench_synth_residues.restype = C.c_int
@@ -498,6 +514,43 @@ class Scorer:
         n = int(sg.count)
         return out, {"first": first, "start": start[:n], "end": end[:n], "score": score[:n]}
 
+    def shuffle_null(self, codes: np.ndarray, offsets: np.ndarray, replicates: int, seed: int = 0,
+                     columns=("core_score", "llr", "hmm_all"), proteins=None, values: bool = False, observed: bool = False):
+        """plaac_score_shuffles: scores `replicates` (K) composition-preserving shuffles of each selected protein (all of
+        them, or the reference indices in `proteins`, which may repeat), built on the GPU, and counts per protein the
+        replicates that reach its observed score.  A replicate counts for a double column when its value, NaN taken as
+        -Inf, is >= the observed one; 'has_core' counts the replicates with a CORE.  The empirical p-value of a column is
+        (1 + count) / (1 + K).  columns: names of NULL_COLUMNS.  Returns a structured array of one int64 field per
+        selected column, in the order of NULL_COLUMNS whatever the order given, one row per selected protein; with
+        values=True also the replicates' values as an (nsel, K) structured array of f8 fields (has_core: 0 or 1); with
+        observed=True also the selected proteins' records (those of score()).  Replicate r of protein i is
+        shuffle(codes, offsets, i, r, seed)."""
+        if isinstance(columns, str):
+            columns = (columns,)
+        unknown = [c for c in columns if c not in NULL_COLUMNS]
+        if unknown or not len(columns):
+            raise ValueError(f"null columns must be a non-empty subset of {NULL_COLUMNS}, got {list(columns)}")
+        mask = 0
+        for c in columns:
+            mask |= 1 << NULL_COLUMNS.index(c)
+        names = [n for k, n in enumerate(NULL_COLUMNS) if mask >> k & 1]
+        codes = np.ascontiguousarray(codes, dtype=np.uint8)
+        offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+        nprot = len(offsets) - 1
+        K = int(replicates)
+        sel = None if proteins is None else np.ascontiguousarray(proteins, dtype=np.int32)
+        nsel = nprot if sel is None else len(sel)
+        counts = np.zeros(nsel, dtype=[(n, "<i8") for n in names])
+        vals = np.zeros((nsel, max(K, 0)), dtype=[(n, "<f8") for n in names]) if values else None
+        obs = np.zeros(nsel, dtype=SUMMARY_DTYPE) if observed else None
+        nl = Null(replicates=K, seed=int(seed) & (2**64 - 1), columns=mask, reserved=0, nsel=-1 if sel is None else nsel,
+                  proteins=sel.ctypes.data if sel is not None else None, counts=counts.ctypes.data,
+                  values=vals.ctypes.data if values else None)
+        self._check(lib().plaac_score_shuffles(self._h, codes.ctypes.data, offsets.ctypes.data, nprot, C.byref(nl),
+                                               obs.ctypes.data if observed else None))
+        ret = [counts] + ([vals] if values else []) + ([obs] if observed else [])
+        return ret[0] if len(ret) == 1 else tuple(ret)
+
     def score_ptr(self, codes_ptr: int, offsets_ptr: int, nprot: int, summaries_ptr: int):
         """Raw host pointers (e.g. pinned torch tensors)."""
         self._check(lib().plaac_score(self._h, codes_ptr, offsets_ptr, nprot, summaries_ptr, None))
@@ -618,6 +671,20 @@ def saturation(codes: np.ndarray, offsets: np.ndarray, proteins=None):
     first_sub = np.zeros(len(protein) + 1, dtype=np.int64)
     np.cumsum(nsub, out=first_sub[1:])
     return protein, first_sub, np.ascontiguousarray(pos, dtype=np.int32), np.ascontiguousarray(code, dtype=np.uint8)
+
+
+def shuffle(codes: np.ndarray, offsets: np.ndarray, protein: int, replicate: int, seed: int = 0) -> np.ndarray:
+    """plaac_shuffle_host: replicate `replicate` of protein `protein` of the batch (codes, offsets), exactly as
+    Scorer.shuffle_null builds it on the GPU: a permutation of the protein's residues.  No GPU needed."""
+    codes = np.ascontiguousarray(codes, dtype=np.uint8)
+    a, b = int(offsets[protein]), int(offsets[protein + 1])
+    src = np.ascontiguousarray(codes[a:b])
+    out = np.empty(b - a, dtype=np.uint8)
+    rc = lib().plaac_shuffle_host(src.ctypes.data, b - a, int(seed) & (2**64 - 1), int(protein), int(replicate),
+                                  out.ctypes.data)
+    if rc != 0:
+        raise PlaacError(rc, lib().plaac_last_error(None).decode())
+    return out
 
 
 def effects_dtype(columns: int) -> np.dtype:

@@ -30,6 +30,7 @@
 #include "generic_windows.cuh"
 #include "variants.cuh"
 #include "segments.cuh"
+#include "shuffle.cuh"
 
 using namespace plaac;
 
@@ -56,7 +57,8 @@ struct Slot {
     DevBuf codes, offsets, summaries;  // staging for the host-buffer API
     DevBuf words, lengths;             // ... of its packed form (plaac_score_packed)
     DevBuf v_prot, v_first, v_pos, v_code;  // the chunk's slice of a variant list (plaac_score_variants)
-    DevBuf v_effects;                       // the chunk's effects (plaac_score_variant_effects)
+    DevBuf v_effects;                       // the chunk's effects (plaac_score_variant_effects) or null values
+    DevBuf sh_rep;                          // the chunk's replicates (plaac_score_shuffles): ShuffleRep each
     DevBuf sg_cnt, sg_first, sg_ent;        // the chunk's segments (plaac_score_segments): counts, their scan, entries
     DevBuf hit_flag, hit_pos;          // compact ranked output (plaac_hits)
     DevBuf res_u8, res_f64;            // per-residue staging for the host-buffer API
@@ -108,7 +110,9 @@ struct plaac_ctx {
     DevBuf all_summaries;      // records of a whole host-buffer call, kept on the device for the compact ranked output
     DevBuf union_rec, union_idx, union_order, union_out_idx;  // plaac_score_multi_packed: the shards' hit rows merged on this GPU
     DevBuf var_ref, var_ref_off;  // reference batch of plaac_score_variants, uploaded once per call
-    DevBuf var_wild;              // its records (plaac_score_variant_effects), uploaded once per call
+    DevBuf var_wild;              // its records (plaac_score_variant_effects), or the observed records of the selection
+                                  // (plaac_score_shuffles), uploaded once per call
+    DevBuf null_counts;           // plaac_score_shuffles: nsel x k counts, summed over the chunks
     // pageable <-> device copies of the FASTA calls: two pinned staging buffers, filled / emptied by a multi-threaded memcpy
     void* stage_buf[2] = {nullptr, nullptr};
     cudaEvent_t stage_ev[2] = {nullptr, nullptr};
@@ -519,7 +523,7 @@ int slot_init(plaac_ctx* ctx, Slot& s)
 void slot_free(Slot& s)
 {
     for (DevBuf* b : {&s.gen_f64, &s.scan_tmp, &s.hist, &s.cursor, &s.order, &s.nchunks, &s.chunk_base, &s.stream_buf, &s.tbw, &s.slot_bucket, &s.errflag,
-                      &s.core_list, &s.core_count, &s.codes, &s.offsets, &s.summaries, &s.words, &s.lengths, &s.v_prot, &s.v_first, &s.v_pos, &s.v_code, &s.v_effects, &s.sg_cnt, &s.sg_first, &s.sg_ent, &s.hit_flag, &s.hit_pos, &s.res_u8, &s.res_f64, &s.res_b0,
+                      &s.core_list, &s.core_count, &s.codes, &s.offsets, &s.summaries, &s.words, &s.lengths, &s.v_prot, &s.v_first, &s.v_pos, &s.v_code, &s.v_effects, &s.sh_rep, &s.sg_cnt, &s.sg_first, &s.sg_ent, &s.hit_flag, &s.hit_pos, &s.res_u8, &s.res_f64, &s.res_b0,
                       &s.res_b1, &s.res_a0, &s.res_a1, &s.res_mapw, &s.res_lpseq, &s.ing_agg, &s.ing_cnt, &s.ing_base,
                       &s.ing_misc, &s.ing_text, &s.ing_codes, &s.ing_offsets, &s.ing_npos, &s.ing_nlen, &s.ing_flags,
                       &s.ing_hist, &s.rk_keys[0], &s.rk_keys[1], &s.rk_vals[0], &s.rk_vals[1], &s.rk_hist, &s.rk_offs,
@@ -1431,7 +1435,7 @@ void plaac_destroy(plaac_ctx* ctx)
     cudaSetDevice(ctx->device);
     for (int i = 0; i < kSlots; i++) slot_free(ctx->slot[i]);
     release(ctx->all_summaries);
-    for (DevBuf* b : {&ctx->union_rec, &ctx->union_idx, &ctx->union_order, &ctx->union_out_idx, &ctx->var_ref, &ctx->var_ref_off, &ctx->var_wild}) release(*b);
+    for (DevBuf* b : {&ctx->union_rec, &ctx->union_idx, &ctx->union_order, &ctx->union_out_idx, &ctx->var_ref, &ctx->var_ref_off, &ctx->var_wild, &ctx->null_counts}) release(*b);
     for (int b = 0; b < 2; b++) {
         if (ctx->stage_buf[b]) cudaFreeHost(ctx->stage_buf[b]);
         if (ctx->stage_ev[b]) cudaEventDestroy(ctx->stage_ev[b]);
@@ -1681,7 +1685,8 @@ try {
 namespace {
 
 // What the host-buffer calls are given: one-byte codes + int64 offsets (plaac_score), radix-22 words + int32
-// lengths (plaac_score_packed), or a variant list over a reference batch of one-byte codes (plaac_score_variants).
+// lengths (plaac_score_packed), a variant list over a reference batch of one-byte codes (plaac_score_variants), or
+// shuffled replicates of that batch's proteins (plaac_score_shuffles).
 struct HostInput {
     const uint8_t* codes = nullptr;
     const int64_t* offsets = nullptr;
@@ -1692,23 +1697,38 @@ struct HostInput {
                        // larger batch starts in the middle of a word)
     const plaac_variants* var = nullptr;  // variant input: codes / offsets hold the nref proteins of the reference
     int64_t nref = 0;
+    // shuffle input (over the reference, as var): replicate q = j * K + r is shuffle r of protein sel[j] (j for a NULL
+    // sel), j < nsel; its output form is the per-protein tally of k_shuffle_tally into ctx->null_counts (and the rows of
+    // nul->values), against the observed records in ctx->var_wild
+    const plaac_null* nul = nullptr;  // nsel >= 0, proteins NULL for every protein; checked by plaac_score_shuffles
     bool packed() const { return words != nullptr || lengths != nullptr; }
 };
 
-// Variant input: checks the reference, uploads it into the ctx buffers (once per call) and returns the total residue
-// count of the variants.  Protein indices and first_sub are checked here, the substitutions during the chunk walk.
+// Variant or shuffle input: checks the reference, uploads it into the ctx buffers (once per call) and returns the total
+// residue count of the variants or replicates.  Protein indices and first_sub are checked here, the substitutions
+// during the chunk walk; a shuffle's selection is checked by plaac_score_shuffles.
 int variants_prepare(plaac_ctx* ctx, const HostInput& in, int64_t& total)
 {
-    const plaac_variants& V = *in.var;
     if (in.nref < 0) return fail(ctx, PLAAC_E_INVALID, "negative reference protein count");
-    if (!V.protein || !V.first_sub || !V.pos || !V.code) return fail(ctx, PLAAC_E_INVALID, "NULL variant array with nvar = %lld", (long long)V.nvar);
+    if (in.var) {
+        const plaac_variants& V = *in.var;
+        if (!V.protein || !V.first_sub || !V.pos || !V.code) return fail(ctx, PLAAC_E_INVALID, "NULL variant array with nvar = %lld", (long long)V.nvar);
+    }
     if (!in.offsets) return fail(ctx, PLAAC_E_INVALID, "NULL reference offsets");
     for (int64_t i = 0; i < in.nref; i++)
         if (in.offsets[i + 1] < in.offsets[i]) return fail(ctx, PLAAC_E_INVALID, "reference offsets not monotone at protein %lld", (long long)i);
     const int64_t ref_base = in.offsets[0], ref_n = in.offsets[in.nref] - ref_base;
     if (ref_n > 0 && !in.codes) return fail(ctx, PLAAC_E_INVALID, "NULL reference codes");
-    if (V.first_sub[0] != 0) return fail(ctx, PLAAC_E_INVALID, "variant 0: first_sub[0] is %lld, not 0", (long long)V.first_sub[0]);
     total = 0;
+    if (in.nul) {
+        const plaac_null& N = *in.nul;
+        for (int64_t j = 0; j < N.nsel; j++) {
+            const int64_t i = N.proteins ? N.proteins[j] : j;
+            total += (in.offsets[i + 1] - in.offsets[i]) * N.replicates;
+        }
+    }
+    const plaac_variants& V = in.var ? *in.var : plaac_variants{};
+    if (in.var && V.first_sub[0] != 0) return fail(ctx, PLAAC_E_INVALID, "variant 0: first_sub[0] is %lld, not 0", (long long)V.first_sub[0]);
     for (int64_t v = 0; v < V.nvar; v++) {
         const int32_t p = V.protein[v];
         if (p < 0 || p >= in.nref)
@@ -1843,7 +1863,8 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
     }
     const bool packed = in.packed();
     const plaac_variants* var = in.var;
-    if (var) {
+    const plaac_null* nul = in.nul;
+    if (var || nul) {
         if (per_res || hits) return fail(ctx, PLAAC_E_INVALID, "variants are scored in summary mode only");
     } else if (packed) {
         if (!in.lengths) return fail(ctx, PLAAC_E_INVALID, "NULL lengths");
@@ -1852,18 +1873,19 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
         if (!in.offsets) return fail(ctx, PLAAC_E_INVALID, "NULL offsets");
         if (!in.codes && in.offsets[nprot] != in.offsets[0]) return fail(ctx, PLAAC_E_INVALID, "NULL codes");
     }
-    if (!summaries && !per_res && !hits && !eff && !seg) return fail(ctx, PLAAC_E_INVALID, "no output requested");
+    if (!summaries && !per_res && !hits && !eff && !seg && !nul) return fail(ctx, PLAAC_E_INVALID, "no output requested");
     CU(ctx, cudaSetDevice(ctx->device));
-    const bool want_rec = summaries || hits || eff || seg;  // the device computes records
+    const bool want_rec = summaries || hits || eff || seg || nul;  // the device computes records
     int rc = PLAAC_OK;
     if (hits && (rc = ensure(ctx, ctx->all_summaries, sizeof(plaac_summary) * (size_t)nprot))) return rc;
     int64_t var_total = 0;
-    if (var && (rc = variants_prepare(ctx, in, var_total))) return rc;
+    if ((var || nul) && (rc = variants_prepare(ctx, in, var_total))) return rc;
     // Effects: the wild-type records are those of a plain call on the reference (so `wild` equals plaac_score's by
     // construction), uploaded into a device table that k_variant_effect reads.  Reference bytes > 21 make that call
     // return PLAAC_E_INVALID after writing its records; the variants are then scored all the same and the error is
     // returned at the end, as plaac_score returns it after the batch.
-    const int ek = eff ? __builtin_popcount(eff->columns) : 0;
+    const int ek = eff ? __builtin_popcount(eff->columns) : nul ? __builtin_popcount((uint32_t)nul->columns) : 0;
+    const int64_t K = nul ? nul->replicates : 1;
     int rc_wild = PLAAC_OK;
     std::string err_wild;
     if (eff) {
@@ -1891,8 +1913,8 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
     // (different half-widths of the windows: 64 bytes of track scratch per residue, so summary mode chunks like per-residue mode)
     const int64_t max_res_full = (per_res || ctx->generic_windows) ? std::min(ctx->chunk_res_pr, ctx->chunk_res) : ctx->chunk_res;
     const int64_t min_res = std::max<int64_t>(max_res_full / 8, 1 << 20);
-    const int64_t first_off = packed || var ? 0 : in.offsets[0];
-    const int64_t total_res = var ? var_total : packed ? in.nres : in.offsets[nprot] - first_off;
+    const int64_t first_off = packed || var || nul ? 0 : in.offsets[0];
+    const int64_t total_res = var || nul ? var_total : packed ? in.nres : in.offsets[nprot] - first_off;
     int64_t ramp = min_res;
     const int64_t max_prot = ctx->chunk_prot;
     int64_t start = 0;
@@ -1905,10 +1927,10 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
     // through pinned staging buffers of the slot, filled / emptied by a multi-threaded memcpy that overlaps the copies
     // and kernels of the other slots.
     const void* in_main = packed ? (const void*)in.words : (const void*)(in.codes + first_off);
-    const bool stage_in = !var && total_res > 0 && !host_is_pinned(in_main);
-    // (the host rows of the call: records, or effects)
-    const void* out_rows = eff ? (const void*)eff->effects : (const void*)summaries;
-    const size_t row_bytes = eff ? sizeof(double) * (size_t)ek : sizeof(plaac_summary);
+    const bool stage_in = !var && !nul && total_res > 0 && !host_is_pinned(in_main);
+    // (the host rows of the call: records, effects or null values)
+    const void* out_rows = nul ? (const void*)nul->values : eff ? (const void*)eff->effects : (const void*)summaries;
+    const size_t row_bytes = eff || nul ? sizeof(double) * (size_t)ek : sizeof(plaac_summary);
     const bool stage_sum = out_rows && !host_is_pinned(out_rows);
     // Segments: drained in chunk order, so seg_base is the number of segments of the proteins before the chunk.  A chunk
     // whose segments overflowed the slot's entries (and are wanted) reruns its bounds and score kernels with room for all
@@ -1978,12 +2000,23 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
         int64_t long_min = long_allowed ? effective_long_min(ctx) : 0;
         // (variants: always the automatic threshold -- at a fixed one, a saturation scan of a 10 000-residue protein would
         // send 190 000 equal-length variants to the latency path instead of the bucketed kernel)
-        const bool long_auto = long_allowed && (ctx->long_min < 0 || var) && ctx->v2_nwr > 0 && ctx->variant != 1;
+        const bool long_auto = long_allowed && (ctx->long_min < 0 || var || nul) && ctx->v2_nwr > 0 && ctx->variant != 1;
         unsigned long long bins[3 * kLongBins];
         if (long_auto) memset(bins, 0, sizeof(bins));
         while (end < nprot && end - start < max_prot) {
-            const int64_t len = var ? in.offsets[var->protein[end] + 1] - in.offsets[var->protein[end]]
-                                    : packed ? (int64_t)in.lengths[end] : in.offsets[end + 1] - in.offsets[end];
+            // (shuffles: a run of cnt replicates of one protein, so the walk is O(nsel + chunks), not O(nsel * K))
+            int64_t cnt = 1;
+            int64_t len;
+            if (nul) {
+                const int64_t j = end / K, i = nul->proteins ? nul->proteins[j] : j;
+                len = in.offsets[i + 1] - in.offsets[i];
+                cnt = std::min((j + 1) * K - end, max_prot - (end - start));
+                if (len > 0) cnt = std::min(cnt, std::max<int64_t>((max_res - nres) / len, end == start));
+                if (cnt == 0) break;
+            } else {
+                len = var ? in.offsets[var->protein[end] + 1] - in.offsets[var->protein[end]]
+                          : packed ? (int64_t)in.lengths[end] : in.offsets[end + 1] - in.offsets[end];
+            }
             if (len < 0) {
                 rc = fail(ctx, PLAAC_E_INVALID, packed ? "negative length at protein %lld" : "offsets not monotone at protein %lld",
                           (long long)end);
@@ -1998,20 +2031,20 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
             if (long_auto && len >= 1024) {
                 // decided after the walk (choose_long_threshold)
                 const int b = long_bin(len);
-                bins[b]++;
-                bins[kLongBins + b] += (unsigned long long)long_scratch_need(len);
+                bins[b] += cnt;
+                bins[kLongBins + b] += (unsigned long long)long_scratch_need(len) * cnt;
                 bins[2 * kLongBins + b] = std::max<unsigned long long>(bins[2 * kLongBins + b], (unsigned long long)len);
             } else if (long_min > 0 && len >= long_min) {
                 // scored by the long-sequence path; the bucketed stream sees an empty protein
-                nlp++;
-                nbigp += len >= kLpBigMin;
-                lp_scratch += long_scratch_need(len);
+                nlp += cnt;
+                nbigp += (len >= kLpBigMin) * cnt;
+                lp_scratch += long_scratch_need(len) * cnt;
             } else {
                 lmax = std::max(lmax, len);
-                nlong += len >= kHistBins;
+                nlong += (len >= kHistBins) * cnt;
             }
-            nres += len;
-            end++;
+            nres += len * cnt;
+            end += cnt;
         }
         if (rc != PLAAC_OK) break;
         if (packed && (pos - pos0) + nres > in.nres) {
@@ -2053,7 +2086,13 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
         }
         if ((rc = ensure(ctx, s.offsets, sizeof(int64_t) * (np + 1)))) break;
         if (packed && (rc = ensure(ctx, s.words, sizeof(uint32_t) * (size_t)(nwords + 4)))) break;
-        if ((packed || var) && (rc = ensure(ctx, s.lengths, sizeof(int32_t) * (size_t)np))) break;
+        if ((packed || var || nul) && (rc = ensure(ctx, s.lengths, sizeof(int32_t) * (size_t)np))) break;
+        // shuffles: the chunk's replicates are those of selected proteins [j0, j1]
+        const int64_t j0 = nul ? start / K : 0, j1 = nul ? (end - 1) / K : -1;
+        if (nul) {
+            if ((rc = ensure(ctx, s.sh_rep, sizeof(ShuffleRep) * (size_t)np))) break;
+            if (nul->proteins && (rc = ensure(ctx, s.v_prot, sizeof(int32_t) * (size_t)(j1 - j0 + 1)))) break;
+        }
         const int64_t fs0 = var ? var->first_sub[start] : 0, nsub = var ? var->first_sub[end] - fs0 : 0;
         if (var) {
             if ((rc = ensure(ctx, s.v_prot, sizeof(int32_t) * (size_t)np))) break;
@@ -2064,11 +2103,11 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
         plaac_summary* d_sum = nullptr;
         if (hits)
             d_sum = (plaac_summary*)ctx->all_summaries.p + start;
-        else if (summaries || eff || seg) {
+        else if (summaries || eff || seg || nul) {
             if ((rc = ensure(ctx, s.summaries, sizeof(plaac_summary) * np))) break;
             d_sum = (plaac_summary*)s.summaries.p;
         }
-        if (eff && (rc = ensure(ctx, s.v_effects, row_bytes * (size_t)np))) break;
+        if ((eff || (nul && nul->values)) && (rc = ensure(ctx, s.v_effects, row_bytes * (size_t)np))) break;
         plaac_residue_out dres;
         if (per_res) {
             if ((rc = ensure(ctx, s.res_u8, (size_t)2 * (nres + 16)))) break;
@@ -2126,6 +2165,22 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
                 ctx->stats.kernel_launches += 1;
             }
             off_base = 0;
+        } else if (nul) {
+            const int32_t* d_sel = nullptr;
+            if (nul->proteins) {
+                CUB(cudaMemcpyAsync(s.v_prot.p, nul->proteins + j0, sizeof(int32_t) * (size_t)(j1 - j0 + 1), cudaMemcpyHostToDevice, s.stream));
+                d_sel = (const int32_t*)s.v_prot.p;
+            }
+            k_shuffle_prep<<<(unsigned)((np + 255) / 256), 256, 0, s.stream>>>(d_sel, j0, start, K, np, (const int64_t*)ctx->var_ref_off.p,
+                                                                               nul->seed, (int32_t*)s.lengths.p, (ShuffleRep*)s.sh_rep.p);
+            ctx->stats.kernel_launches += 1;
+            if ((rc = launch_scan(ctx, s, (const int32_t*)s.lengths.p, (int64_t*)s.offsets.p, np, s.stream))) break;
+            if (nres > 0) {
+                k_shuffle_expand<<<(unsigned)((nres + kExpandTile - 1) / kExpandTile), kExpandThreads, 0, s.stream>>>(
+                    (const uint8_t*)ctx->var_ref.p, (const ShuffleRep*)s.sh_rep.p, (const int64_t*)s.offsets.p, np, nres, (uint8_t*)s.codes.p);
+                ctx->stats.kernel_launches += 1;
+            }
+            off_base = 0;
         } else if (packed) {
             if (main_bytes > 0) CUB(cudaMemcpyAsync(s.words.p, src_main, main_bytes, cudaMemcpyHostToDevice, s.stream));
             CUB(cudaMemcpyAsync(s.lengths.p, in.lengths + start, sizeof(int32_t) * (size_t)np, cudaMemcpyHostToDevice, s.stream));
@@ -2173,6 +2228,16 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
             ctx->stats.kernel_launches += 1;
             CUB(cudaMemcpyAsync(stage_sum ? s.h_stage_sum : (void*)(eff->effects + start * ek), s.v_effects.p, row_bytes * (size_t)np,
                                 cudaMemcpyDeviceToHost, s.stream));
+        } else if (nul) {
+            // the records stay on the device: the counts are summed there, and only the values rows (if any) cross the link
+            double* d_val = nul->values ? (double*)s.v_effects.p : nullptr;
+            k_shuffle_tally<<<(unsigned)((np * ek + 255) / 256), 256, 0, s.stream>>>(
+                d_sum, (const plaac_summary*)ctx->var_wild.p, start, K, np, (uint32_t)nul->columns,
+                (unsigned long long*)ctx->null_counts.p, d_val);
+            ctx->stats.kernel_launches += 1;
+            if (d_val)
+                CUB(cudaMemcpyAsync(stage_sum ? s.h_stage_sum : (void*)(nul->values + start * ek), d_val, row_bytes * (size_t)np,
+                                    cudaMemcpyDeviceToHost, s.stream));
         }
         if (out_rows && stage_sum) {
             s.out_dst = (char*)out_rows + row_bytes * (size_t)start;
@@ -2346,6 +2411,111 @@ try {
     return score_host(ctx, in, nprot, summaries, nullptr, nullptr, false, nullptr, segments);
 } catch (...) {
     return api_caught(ctx, "plaac_score_segments");
+}
+
+int plaac_shuffle_host(const uint8_t* codes, int64_t n, uint64_t seed, int64_t protein, int64_t replicate, uint8_t* out)
+try {
+    if (n < 0 || n > 0x7fffffffLL) return fail(nullptr, PLAAC_E_INVALID, "plaac_shuffle_host: length %lld outside [0, 2^31)", (long long)n);
+    if (protein < 0 || replicate < 0)
+        return fail(nullptr, PLAAC_E_INVALID, "plaac_shuffle_host: negative protein %lld or replicate %lld", (long long)protein,
+                    (long long)replicate);
+    if (n > 0 && (!codes || !out)) return fail(nullptr, PLAAC_E_INVALID, "plaac_shuffle_host: NULL codes or out");
+    const ShuffleKey k = shuffle_key(seed, protein, replicate, n);
+    for (int64_t t = 0; t < n; t++) out[t] = codes[shuffle_index(k, (uint32_t)t)];
+    return PLAAC_OK;
+} catch (...) {
+    return api_caught(nullptr, "plaac_shuffle_host");
+}
+
+int plaac_score_shuffles(plaac_ctx* ctx, const uint8_t* codes, const int64_t* offsets, int64_t nprot, plaac_null* null_spec,
+                         plaac_summary* observed)
+try {
+    if (!ctx) return fail(nullptr, PLAAC_E_INVALID, "plaac_score_shuffles: NULL ctx");
+    if (!null_spec) return fail(ctx, PLAAC_E_INVALID, "plaac_score_shuffles: NULL null_spec");
+    const plaac_null& N = *null_spec;
+    const int64_t K = N.replicates;
+    if (K < 0) return fail(ctx, PLAAC_E_INVALID, "plaac_score_shuffles: replicates %lld is negative", (long long)K);
+    if (N.nsel < -1) return fail(ctx, PLAAC_E_INVALID, "plaac_score_shuffles: nsel %lld is below -1", (long long)N.nsel);
+    if (N.reserved != 0) return fail(ctx, PLAAC_E_INVALID, "plaac_score_shuffles: reserved is %d, not 0", (int)N.reserved);
+    if (N.columns <= 0 || N.columns >= (PLAAC_NULL_HAS_CORE << 1))
+        return fail(ctx, PLAAC_E_INVALID, "plaac_score_shuffles: columns 0x%x is not a non-empty set of bits 0..13", (unsigned)N.columns);
+    if (nprot < 0) return fail(ctx, PLAAC_E_INVALID, "negative nprot");
+    if (N.nsel >= 0 && !N.proteins) return fail(ctx, PLAAC_E_INVALID, "plaac_score_shuffles: NULL proteins with nsel = %lld", (long long)N.nsel);
+    const int64_t nsel = N.nsel < 0 ? nprot : N.nsel;
+    if (nsel != 0 && !N.counts) return fail(ctx, PLAAC_E_INVALID, "plaac_score_shuffles: NULL counts with nsel = %lld", (long long)N.nsel);
+    const int32_t* sel = N.nsel < 0 ? nullptr : N.proteins;
+    for (int64_t j = 0; sel && j < nsel; j++)
+        if (sel[j] < 0 || sel[j] >= nprot)
+            return fail(ctx, PLAAC_E_INVALID, "plaac_score_shuffles: selected protein %lld: index %d outside [0, %lld)", (long long)j,
+                        (int)sel[j], (long long)nprot);
+    if (nsel == 0) return PLAAC_OK;
+    if (nsel > 0x7fffffffLL) return fail(ctx, PLAAC_E_INVALID, "plaac_score_shuffles: more than 2^31-1 selected proteins");
+    if (K > INT64_MAX / nsel) return fail(ctx, PLAAC_E_INVALID, "plaac_score_shuffles: nsel x replicates overflows");
+
+    // The observed records: the selection through the variant input form with no substitution, whose records equal
+    // plaac_score's.  Reference bytes > 21 make it return PLAAC_E_INVALID after writing them; the replicates are then
+    // scored all the same and the error is returned at the end, as plaac_score returns it after the batch.
+    std::vector<int32_t> all;
+    if (!sel) {
+        all.resize((size_t)nsel);
+        for (int64_t j = 0; j < nsel; j++) all[(size_t)j] = (int32_t)j;
+    }
+    std::vector<int64_t> no_sub((size_t)nsel + 1, 0);
+    const int32_t no_pos = 0;
+    const uint8_t no_code = 0;
+    plaac_variants V = {nsel, sel ? sel : all.data(), no_sub.data(), &no_pos, &no_code};
+    std::vector<plaac_summary> obs_host;
+    plaac_summary* obs = observed;
+    if (!obs) {
+        obs_host.resize((size_t)nsel);
+        obs = obs_host.data();
+    }
+    HostInput vin;
+    vin.codes = codes;
+    vin.offsets = offsets;
+    vin.nref = nprot;
+    vin.var = &V;
+    const int rc_obs = score_host(ctx, vin, nsel, obs, nullptr, nullptr);
+    if (rc_obs != PLAAC_OK && rc_obs != PLAAC_E_INVALID) return rc_obs;
+    const std::string err_obs = ctx->err;
+
+    // the tables k_shuffle_tally reads and sums into; every slot's stream starts after this synchronisation
+    const int k = __builtin_popcount((uint32_t)N.columns);
+    const size_t count_bytes = sizeof(int64_t) * (size_t)nsel * (size_t)k;
+    int rc;
+    if ((rc = ensure(ctx, ctx->var_wild, sizeof(plaac_summary) * (size_t)nsel))) return rc;
+    if ((rc = ensure(ctx, ctx->null_counts, count_bytes))) return rc;
+    cudaStream_t st = ctx->slot[0].stream;
+    if ((rc = h2d_any(ctx, ctx->var_wild.p, obs, sizeof(plaac_summary) * (size_t)nsel, st))) return rc;
+    CU(ctx, cudaMemsetAsync(ctx->null_counts.p, 0, count_bytes, st));
+    CU(ctx, cudaStreamSynchronize(st));
+
+    rc = PLAAC_OK;
+    if (K > 0) {
+        plaac_null R = N;
+        R.nsel = nsel;
+        R.proteins = sel;
+        HostInput in;
+        in.codes = codes;
+        in.offsets = offsets;
+        in.nref = nprot;
+        in.nul = &R;
+        rc = score_host(ctx, in, nsel * K, nullptr, nullptr, nullptr);
+        if (rc != PLAAC_OK && rc != PLAAC_E_INVALID) return rc;
+    }
+    // (bytes > 21: the replicates were scored in full, so the counts are complete)
+    const std::string keep = ctx->err;
+    int rcc;
+    if ((rcc = d2h_any(ctx, N.counts, ctx->null_counts.p, count_bytes, st))) return rcc;
+    CU(ctx, cudaStreamSynchronize(st));
+    ctx->err = keep;
+    if (rc == PLAAC_OK && rc_obs != PLAAC_OK) {
+        rc = rc_obs;
+        ctx->err = err_obs;
+    }
+    return rc;
+} catch (...) {
+    return api_caught(ctx, "plaac_score_shuffles");
 }
 
 }  // extern "C"

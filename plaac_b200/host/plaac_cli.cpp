@@ -32,6 +32,14 @@
 //                   residues; plaac_score_segments) to FILE as a table: SEQid SEGstart SEGend SEGlen SEGscore PRD, 1-based
 //                   positions, SEGscore the PRDscore sum over the segment, PRD 1 for the segment that is the row's PrD.
 //                   One line per segment, in record order (also with --rank); the summary table is unchanged
+//   --null FILE --replicates K [--seed S] [--null-columns COLS]
+//                   also score K composition-preserving shuffles of every record on the GPU (plaac_score_shuffles) and
+//                   write to FILE one line per printed record, in record order: SEQid NULLreps, then n<NAME> p<NAME> per
+//                   column, n the shuffles whose value (NaN lowest) reaches the record's and p = (1+n)/(1+K) (%.6g).
+//                   COLS: the names of --effects with hasCORE (shuffles with a CORE, no p column) for COREchange;
+//                   default COREscore,LLR,HMMall.  A record's shuffles are those of its index in its batch (--batch-mb),
+//                   so the file depends on --seed and, for inputs beyond one batch, on --batch-mb; the summary table is
+//                   unchanged
 #include <algorithm>
 #include <charconv>
 #include <cmath>
@@ -422,6 +430,13 @@ struct Options {
     int32_t effects_mask = 0;   // PLAAC_EFFECT_* bits of --effects
     std::string segments_file;  // --segments
     FILE* seg_out = nullptr;    // ... open
+    std::string null_file;      // --null
+    FILE* null_out = nullptr;   // ... open
+    int64_t replicates = 0;     // --replicates
+    uint64_t seed = 0;          // --seed
+    std::string null_columns = "COREscore,LLR,HMMall";  // --null-columns, as given
+    bool replicates_set = false, seed_set = false, null_columns_set = false;
+    int32_t null_mask = 0;      // plaac_null.columns of --null-columns
 };
 
 // --effects names, bit k = PLAAC_EFFECT_* bit k (the doubles of plaac_summary in declaration order, then COREchange)
@@ -429,9 +444,13 @@ const char* const kEffectNames[] = {"LLR",          "COREscore",   "PRDscore",  
                                     "FImeanhydro",  "FImeancharge", "FImeancombo", "PAPAcombo", "PAPAprop",
                                     "PAPAfi",       "PAPAllr",     "PAPAllr2",  "COREchange"};
 constexpr int kEffectCoreChange = 13;
+// --null-columns names: those of --effects, with hasCORE (replicates with a CORE) for bit 13
+const char* const kNullNames[] = {"LLR",          "COREscore",   "PRDscore",  "HMMall",   "HMMvit",
+                                  "FImeanhydro",  "FImeancharge", "FImeancombo", "PAPAcombo", "PAPAprop",
+                                  "PAPAfi",       "PAPAllr",     "PAPAllr2",  "hasCORE"};
 
-// Comma-separated --effects names -> mask; 0 after printing the message.
-int32_t parse_effects(const std::string& list)
+// Comma-separated column names of option `opt` (--effects or --null-columns) -> mask; 0 after printing the message.
+int32_t parse_columns(const std::string& list, const char* opt, const char* const (&names)[14])
 {
     int32_t mask = 0;
     size_t a = 0;
@@ -440,14 +459,14 @@ int32_t parse_effects(const std::string& list)
         if (b == std::string::npos) b = list.size();
         const std::string name = list.substr(a, b - a);
         int k = 0;
-        while (k <= kEffectCoreChange && name != kEffectNames[k]) k++;
+        while (k <= kEffectCoreChange && name != names[k]) k++;
         if (k > kEffectCoreChange) {
             if (name.empty())
-                std::fprintf(stderr, "plaac: --effects: empty column name in '%s'\n", list.c_str());
+                std::fprintf(stderr, "plaac: %s: empty column name in '%s'\n", opt, list.c_str());
             else
-                std::fprintf(stderr, "plaac: --effects: unknown column '%s'\n", name.c_str());
-            std::fprintf(stderr, "plaac: --effects takes a comma-separated list of");
-            for (const char* n : kEffectNames) std::fprintf(stderr, " %s", n);
+                std::fprintf(stderr, "plaac: %s: unknown column '%s'\n", opt, name.c_str());
+            std::fprintf(stderr, "plaac: %s takes a comma-separated list of", opt);
+            for (int j = 0; j <= kEffectCoreChange; j++) std::fprintf(stderr, " %s", names[j]);
             std::fprintf(stderr, "\n");
             return 0;
         }
@@ -590,12 +609,55 @@ int score_segment_batch(const Options& o, Scorers& S, Batch& B, std::vector<plaa
     return 0;
 }
 
+// --null: the records of the batch (plaac_score_shuffles' observed records) and, per printed record in record order,
+// the counts of its shuffles that reach it and the p-values (1 + n) / (1 + K); the table is written here.
+int score_null_batch(const Options& o, Scorers& S, Batch& B, std::vector<plaac_summary>& sum)
+{
+    const int64_t np = B.nprot();
+    const int k = __builtin_popcount((unsigned)o.null_mask);
+    std::vector<int64_t> counts((size_t)np * (size_t)k);
+    plaac_null N = {};
+    N.replicates = o.replicates;
+    N.seed = o.seed;
+    N.columns = o.null_mask;
+    N.nsel = -1;
+    N.counts = counts.data();
+    const int rc = plaac_score_shuffles(S.ctx[0], B.codes.data(), B.offsets.data(), np, &N, sum.data());
+    if (rc != PLAAC_OK) return die(S, rc, "plaac_score_shuffles");
+    std::string out;
+    char buf[64];
+    for (int64_t i = 0; i < np; i++) {
+        const plaac_summary& r = sum[(size_t)i];
+        if (r.prot_len < 1 || (o.rank_core_only && !(r.core_score == r.core_score))) continue;  // (rows not printed)
+        out.append(B.names[(size_t)i]);
+        out.push_back('\t'), put_int(out, (long)o.replicates);
+        int c = 0;
+        for (int b = 0; b <= kEffectCoreChange; b++) {
+            if (!((o.null_mask >> b) & 1)) continue;
+            const int64_t n = counts[(size_t)i * (size_t)k + (size_t)c++];
+            out.push_back('\t'), put_int(out, (long)n);
+            if (b != kEffectCoreChange) {
+                std::snprintf(buf, sizeof(buf), "\t%.6g", (double)(1 + n) / (double)(1 + o.replicates));
+                out += buf;
+            }
+        }
+        out.push_back('\n');
+    }
+    if (std::fwrite(out.data(), 1, out.size(), o.null_out) != out.size() || std::fflush(o.null_out) != 0) {
+        std::fprintf(stderr, "plaac: cannot write %s\n", o.null_file.c_str());
+        return 2;
+    }
+    return 0;
+}
+
 int score_summary_batch(const Options& o, Scorers& S, Batch& B)
 {
     if (B.nprot() == 0) return 0;
     std::vector<plaac_summary> sum((size_t)B.nprot());
     if (o.seg_out) {
         if (const int rs = score_segment_batch(o, S, B, sum)) return rs;
+    } else if (o.null_out) {
+        if (const int rs = score_null_batch(o, S, B, sum)) return rs;
     } else {
         const int rc = plaac_score_multi(S.ctx.data(), (int)S.ctx.size(), B.codes.data(), B.offsets.data(), B.nprot(),
                                          sum.data(), nullptr);
@@ -1250,6 +1312,11 @@ void usage()
     std::puts("                   COREchange: 1 CORE gained, -1 lost, 0 unchanged)");
     std::puts("  --segments FILE  also write every prion-like segment (maximal run of PrD-state residues of the Viterbi");
     std::puts("                   parse) of every record to FILE: SEQid SEGstart SEGend SEGlen SEGscore PRD");
+    std::puts("  --null FILE --replicates K [--seed S] [--null-columns COLS]");
+    std::puts("                   also score K composition-preserving shuffles of every record and write to FILE, per record,");
+    std::puts("                   SEQid NULLreps and n<NAME> p<NAME> per column: the shuffles that reach the record's score");
+    std::puts("                   (NaN lowest) and the empirical p-value (1+n)/(1+K).  COLS as --effects, with hasCORE (the");
+    std::puts("                   shuffles with a CORE, no p) in place of COREchange; default COREscore,LLR,HMMall");
     std::puts("  --compat-F       -F reads the -B file, as plaac.jar does (plaac.java:388); without it -F reads its own file,");
     std::puts("                   so the parameter block and every score differ from the jar's for the same command line");
 }
@@ -1293,6 +1360,14 @@ int main(int argc, char** argv)
             o.effects = val("--effects"), o.effects_set = true;
         else if (a == "--segments")
             o.segments_file = val("--segments");
+        else if (a == "--null")
+            o.null_file = val("--null");
+        else if (a == "--replicates")
+            o.replicates = std::atoll(val("--replicates")), o.replicates_set = true;
+        else if (a == "--seed")
+            o.seed = std::strtoull(val("--seed"), nullptr, 10), o.seed_set = true;
+        else if (a == "--null-columns")
+            o.null_columns = val("--null-columns"), o.null_columns_set = true;
         else if (a == "--format-check") {
             // test hook: lines "decimals value" on stdin -> the Java-formatted value on stdout
             int d;
@@ -1344,6 +1419,29 @@ int main(int argc, char** argv)
         }
         o.host_reader = true;  // segments come with the records of plaac_score_segments, not the GPU reader's
     }
+    if (!o.null_file.empty()) {
+        const char* clash = !o.plotlist.empty()        ? "-p"
+                            : !o.variants_file.empty() ? "--variants"
+                            : o.saturate               ? "--saturate"
+                            : !o.segments_file.empty() ? "--segments"
+                            : o.gpu_ingest             ? "--gpu-ingest"
+                            : o.gpus > 1               ? "--gpus > 1"
+                                                       : nullptr;
+        if (clash) {
+            std::fprintf(stderr, "plaac: --null cannot be combined with %s\n", clash);
+            return 2;
+        }
+        if (o.replicates < 1) {
+            std::fprintf(stderr, "plaac: --null needs --replicates K with K >= 1\n");
+            return 2;
+        }
+        if (!(o.null_mask = parse_columns(o.null_columns, "--null-columns", kNullNames))) return 2;
+        o.host_reader = true;  // the shuffles come with the records of plaac_score_shuffles, not the GPU reader's
+    } else if (o.replicates_set || o.seed_set || o.null_columns_set) {
+        std::fprintf(stderr, "plaac: %s needs --null FILE\n",
+                     o.replicates_set ? "--replicates" : o.seed_set ? "--seed" : "--null-columns");
+        return 2;
+    }
     const bool variants = o.saturate || !o.variants_file.empty();
     VariantFile vfile;
     if (variants) {
@@ -1357,7 +1455,7 @@ int main(int argc, char** argv)
             std::fprintf(stderr, "plaac: %s cannot be combined with %s\n", o.saturate ? "--saturate" : "--variants", clash);
             return 2;
         }
-        if (o.effects_set && !(o.effects_mask = parse_effects(o.effects))) return 2;
+        if (o.effects_set && !(o.effects_mask = parse_columns(o.effects, "--effects", kEffectNames))) return 2;
         if (!o.variants_file.empty() && !read_variant_file(o.variants_file, vfile)) return 2;
         o.host_reader = true;  // the work is the quadratic scoring, not the reading
     } else if (o.effects_set) {
@@ -1540,6 +1638,21 @@ int main(int argc, char** argv)
         }
         o.seg_out = seg_file.get();
         std::fputs("SEQid\tSEGstart\tSEGend\tSEGlen\tSEGscore\tPRD\n", o.seg_out);
+    }
+    std::unique_ptr<FILE, int (*)(FILE*)> null_file(nullptr, std::fclose);
+    if (!o.null_file.empty()) {
+        null_file.reset(std::fopen(o.null_file.c_str(), "w"));
+        if (!null_file) {
+            std::fprintf(stderr, "plaac: cannot open %s for writing\n", o.null_file.c_str());
+            return 2;
+        }
+        o.null_out = null_file.get();
+        std::string head = "SEQid\tNULLreps";
+        for (int b = 0; b <= kEffectCoreChange; b++)
+            if ((o.null_mask >> b) & 1)
+                head += std::string("\tn") + kNullNames[b] + (b == kEffectCoreChange ? "" : std::string("\tp") + kNullNames[b]);
+        head += "\n";
+        std::fputs(head.c_str(), o.null_out);
     }
     if (o.plotlist.empty()) {
         print_table_head();
