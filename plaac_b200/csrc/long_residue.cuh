@@ -36,6 +36,7 @@ namespace cg = cooperative_groups;
 
 constexpr int kLpThreads = 512;   // chunk lanes per CTA
 constexpr int kLpMinChunk = 32;
+constexpr int kLpWarm2 = 64;      // warm-up residues of pass 2, which starts from pass 1's d (within a few ulps of the jar's)
 constexpr int kLpBigCluster = 8;  // CTAs per protein of at least kLpBigMin residues
 constexpr int kLpBigMin = 32768;  // (an edge of k_long_levels' length bins: the host counts the classes from them)
 // Boundary scratch: five planes (gA, gB, gV0, gV1, bytes) of bnd_plane doubles; a protein's row starts at scratch_off / 32
@@ -59,7 +60,6 @@ struct LongPostArgs {
     int64_t bnd_plane;
     double* lpseq;               // per listed protein
     int warm;                    // warm-up residues of pass 1 (rounded up to whole chunks): d coalesces from a generic start
-    int warm2;                   // ... of pass 2, which starts from pass 1's d (within a few ulps of the jar's)
     int cluster;                 // CTAs per protein of this launch; the launch handles proteins of its size class only
     int64_t big_min;             // class boundary: n >= big_min belongs to the kLpBigCluster launch
     unsigned long long* redone;  // statistics: chunks redone sequentially although they had frames
@@ -71,7 +71,6 @@ struct LongPostArgs {
     uint8_t* vbytes;             // Viterbi parse, one byte per residue at scratch_off + t, when out.vit is NULL
     uint8_t* tb;                 // 4 traceback bits per residue, indexed scratch_off + t
     unsigned long long vit_tie_mask;  // binades in which a Viterbi constant is an exact rounding tie (plaac_create)
-    long long* dbg_clocks;       // optional: phase time stamps of the first CTA (PLAAC_LONG_CLOCKS)
     int* errflag;                // invalid residue codes (> 21) are scored as X and reported, as by k_pack
 };
 
@@ -182,11 +181,6 @@ __device__ __forceinline__ LpMP lp_mp_mul(const LpMP& a, const LpMP& b)
     return r;
 }
 
-#define LP_STAMP(i)                                                                     \
-    do {                                                                               \
-        if (g.dbg_clocks && threadIdx.x == 0 && blockIdx.x == 0) g.dbg_clocks[i] = clock64(); \
-    } while (0)
-
 __global__ void __launch_bounds__(kLpThreads, 1) k_long_post(LongPostArgs g)
 {
     cg::cluster_group cluster = cg::this_cluster();
@@ -237,7 +231,6 @@ __global__ void __launch_bounds__(kLpThreads, 1) k_long_post(LongPostArgs g)
     const uint32_t lut = smem_u32(&sm.lut2[0]);
     uint32_t sbase;
     asm volatile("mov.u32 %0, %1;" : "=r"(sbase) : "r"(smem_u32(lp_smem)));
-    LP_STAMP(0);
     // invalid input (> 21) is scored as X, as everywhere else (reported by k_pack)
     auto LE = [&](int t) -> double2 {
         const uint32_t c = src[t];
@@ -247,7 +240,7 @@ __global__ void __launch_bounds__(kLpThreads, 1) k_long_post(LongPostArgs g)
     const int kg = rank * kLpThreads + tid;  // this lane's chunk
     const bool live = kg < K;
     const int cs = kg * C, ce = min(n, cs + C);
-    const int m2 = min(m, (max(1, g.warm2) + C - 1) / C);
+    const int m2 = min(m, (kLpWarm2 + C - 1) / C);
     // forward: state initialised AT residue fi (true init when fi == 0), first step at fi + 1; pass 2 starts AT fi2 >= fi
     const int fi = (kg - m <= 0) ? 0 : (kg - m) * C - 1;
     const int fi2 = (kg - m2 <= 0) ? 0 : (kg - m2) * C - 1;
@@ -396,7 +389,6 @@ __global__ void __launch_bounds__(kLpThreads, 1) k_long_post(LongPostArgs g)
     }
     lp_cluster_sync(cluster);
 
-    LP_STAMP(2);
     // ================= pass 2: the jar's own binade, two frames one ulp apart =================
     if (live) {
         // ---- forward (frames start AT fi2 with pass 1's d and the approximate absolute x0 there)
@@ -492,7 +484,6 @@ __global__ void __launch_bounds__(kLpThreads, 1) k_long_post(LongPostArgs g)
         sm.mode[0][tid] = sm.mode[1][tid] = 1;
     }
     lp_cluster_sync(cluster);
-    LP_STAMP(3);
     // link to the chunk before this one in walking order (the neighbour lane, or the neighbour CTA's edge lane over DSMEM)
     {
 #pragma unroll
@@ -509,7 +500,6 @@ __global__ void __launch_bounds__(kLpThreads, 1) k_long_post(LongPostArgs g)
     }
     lp_cluster_sync(cluster);
 
-    LP_STAMP(4);
     // ================= carry: exact state at every chunk boundary, in chunk order, relayed over the cluster =================
     // One lane per chain (forward, backward, Viterbi) on three different warps.  The values of the next chunk are loaded
     // while the current one is added: the dependent chain of the common case is one fp64 addition per chunk.
@@ -519,7 +509,6 @@ __global__ void __launch_bounds__(kLpThreads, 1) k_long_post(LongPostArgs g)
             // exact Viterbi scores in chunk order (first strict maximum as in :3090-3099), choice bits per chunk
             const int k_lo = rank * kLpThreads, k_hi = min(K, k_lo + kLpThreads);
             double Sx0 = *reinterpret_cast<volatile double*>(&sm.vcarry[0]), Sx1 = *reinterpret_cast<volatile double*>(&sm.vcarry[1]);
-            const long long tw0 = clock64();
             const uint32_t aM = sbase + LP_OFF(vMi), aX = sbase + LP_OFF(vcross), aCh = sbase + LP_OFF(vchoice);
             int k = k_lo;
             if (k == 0) {  // the first chunk is the true chain of pass 1
@@ -566,12 +555,6 @@ __global__ void __launch_bounds__(kLpThreads, 1) k_long_post(LongPostArgs g)
                     lp_sts_u8(aCh + (uint32_t)l, (uint32_t)(ch0 | (ch1 << 1)));
                 }
             }
-            if (g.dbg_clocks) {
-                atomicAdd((unsigned long long*)&g.dbg_clocks[8], (unsigned long long)(clock64() - tw0));
-                int nc = 0;
-                for (int k = k_lo; k < k_hi; k++) nc += sm.vcross[k - k_lo];
-                atomicAdd((unsigned long long*)&g.dbg_clocks[11], (unsigned long long)nc << 32);
-            }
             if (rank + 1 < R) {
                 LpShared* o = cluster.map_shared_rank(&sm, rank + 1);
                 *reinterpret_cast<volatile double*>(&o->vcarry[0]) = Sx0;
@@ -592,8 +575,7 @@ __global__ void __launch_bounds__(kLpThreads, 1) k_long_post(LongPostArgs g)
             double x0 = *reinterpret_cast<volatile double*>(&sm.carry[dir][0]);   // (unused by the first walker)
             double x1 = *reinterpret_cast<volatile double*>(&sm.carry[dir][1]);
             bool acc = !first && *reinterpret_cast<volatile int*>(&sm.carry_acc[dir]) != 0;  // the chunk before was accepted with its frames
-            int nredo = 0, nfast = 0, nseq = 0;
-            const long long tw0 = clock64();
+            int nredo = 0;
             const uint32_t aL = sbase + LP_OFF(link) + (uint32_t)dir * kLpThreads;
             const uint32_t aI = sbase + LP_OFF(g_inc) + (uint32_t)dir * 2u * kLpThreads * 8u;  // [dir][0][.]
             const uint32_t aD = sbase + LP_OFF(g_dex) + (uint32_t)dir * 2u * kLpThreads * 8u;
@@ -615,7 +597,6 @@ __global__ void __launch_bounds__(kLpThreads, 1) k_long_post(LongPostArgs g)
                 if (lk && acc) {
                     x0 = x0 + inc;
                     x1 = x0 + dexo;
-                    nfast++;
                     continue;
                 }
                 const int md = sm.mode[dir][l];
@@ -651,14 +632,8 @@ __global__ void __launch_bounds__(kLpThreads, 1) k_long_post(LongPostArgs g)
                         for (int t = e - 1; t >= s; t--) lp_bwd_step(x0, x1, LE(t + 1), ks, lut);
                     }
                     nredo += md == 0 ? 1 : 0;
-                    nseq++;
                     acc = false;
                 }
-            }
-            if (g.dbg_clocks) {
-                atomicAdd((unsigned long long*)&g.dbg_clocks[9 + dir], (unsigned long long)(clock64() - tw0));
-                atomicAdd((unsigned long long*)&g.dbg_clocks[11], (unsigned long long)nfast);
-                atomicAdd((unsigned long long*)&g.dbg_clocks[12 + dir], (unsigned long long)nseq);
             }
             if (nredo) atomicAdd(&sm.redone, nredo);
             // hand the exact state to the neighbour
@@ -682,7 +657,6 @@ __global__ void __launch_bounds__(kLpThreads, 1) k_long_post(LongPostArgs g)
         lp_cluster_sync(cluster);
     }
 
-    LP_STAMP(5);
     // ================= pass 3: every chunk from its exact boundary state =================
     if (live && post) {
         {
@@ -792,7 +766,6 @@ __global__ void __launch_bounds__(kLpThreads, 1) k_long_post(LongPostArgs g)
     __threadfence();
     lp_cluster_sync(cluster);
 
-    LP_STAMP(6);
     // ================= pass 4: posteriors and MAP bytes, coalesced =================
     if (post) {
         const double lpseq = g.lpseq[pslot];
@@ -809,7 +782,6 @@ __global__ void __launch_bounds__(kLpThreads, 1) k_long_post(LongPostArgs g)
         }
         if (bad && g.errflag) atomicOr(g.errflag, 1);
     }
-    LP_STAMP(7);
 }
 
 }  // namespace plaac

@@ -119,10 +119,9 @@ struct plaac_ctx {
     bool stage_pending[2] = {false, false};
     int nwarps = 0, ring_words = 0;
     size_t smem_bytes = 0;
-    int v2_nwr = 0;            // warps per role of the v2 kernel (0 = v2 unavailable for these params)
-    size_t v2_smem_bytes = 0;
-    int v3_nwr = 0, v3_opt = 0, v3_mix = 0, v3_nt = 768;  // v3 kernel (same preconditions as v2): warps per role, option bits, role placement
-    size_t v3_smem_bytes = 0;
+    int v2_nwr = 0;            // warps per role of the v2 and v3 kernels (0 = both unavailable for these params)
+    size_t v2_smem_bytes = 0;  // ... and their shared memory (the same layout)
+    int v3_opt = 0;            // option bits of the v3 kernel (summary_kernel_v3.cuh)
     IntFold ifold = {};        // valid when v3_opt has kV3IntFold
     int v2_always_in = 0;     // forward recurrence provably keeps |a-b| < 40 (no LUT range test needed)
     ResidueV2Plan res_plan;
@@ -137,6 +136,7 @@ struct plaac_ctx {
     int64_t long_min = 8192;
     int long_warm = 256;       // forward warm-up of that path
     unsigned long long long_tie[4] = {0, 0, 0, 0};  // binades with an exact rounding tie among the table constants
+    int64_t lp_big_min = kLpBigMin;  // proteins of at least this many residues take k_long_post's cluster launch
     std::string err;
     int last_slot = 0;
 };
@@ -298,36 +298,19 @@ int setup_scalars(plaac_ctx* ctx)
     else {
         const size_t fixed2 = (size_t)kV2FixedBytes + kV2AlignSlack;
         if (fixed2 + 2 * per_warp <= limit) {
-            int nwr = (int)std::min<size_t>(kV2MaxThreads / 64, (limit - fixed2) / (2 * per_warp));
-            if (const char* e = getenv("PLAAC_V2_WARP_PAIRS")) nwr = std::max(1, std::min(nwr, atoi(e)));  // experiments
+            const int nwr = (int)std::min<size_t>(kV2MaxThreads / 64, (limit - fixed2) / (2 * per_warp));
             ctx->v2_nwr = nwr;
             ctx->v2_smem_bytes = fixed2 + per_warp * 2 * nwr;
         } else
             ctx->v2_why = "ring does not fit beside the v2 tables";
-        // v3: same design, fewer issue slots per residue (summary_kernel_v3.cuh); on unless PLAAC_SUMMARY_KERNEL=2
-        ctx->v3_nwr = 0;
-        const size_t fixed3 = (size_t)kV2FixedBytes + kV2AlignSlack;
-        const char* ek = getenv("PLAAC_SUMMARY_KERNEL");
-        if (ctx->v2_nwr > 0 && fixed3 + 2 * per_warp <= limit && !(ek && atoi(ek) == 2)) {
-            int nwr = (int)std::min<size_t>(kV2MaxThreads / 64, (limit - fixed3) / (2 * per_warp));
-            if (const char* e = getenv("PLAAC_V2_WARP_PAIRS")) nwr = std::max(1, std::min(nwr, atoi(e)));
+        // v3: same design, warps and shared-memory layout, fewer issue slots per residue (summary_kernel_v3.cuh)
+        if (ctx->v2_nwr > 0) {
             int opt = kV3DefaultOpt;
-            if (const char* e = getenv("PLAAC_V3_OPT")) opt = atoi(e);
             // the packed Q/N window needs counts that fit a byte and the jar's Q/N code set
             if (P.mw_window > 100 || k.qn_mask != ((1u << 12) | (1u << 14))) opt &= ~kV3SwarMw;
             // ... and the integer FoldIndex tests a proof that they give the FP64 signs for these tables and windows
             if (!plan_int_fold(P, k.w, ctx->ifold)) opt &= ~kV3IntFold;
-            int nt = 768;
-            if (const char* e = getenv("PLAAC_V3_NT")) nt = atoi(e);
-            nwr = std::min(nwr, nt / 64);
-            if (v3_kernel(opt, nt)) {
-                ctx->v3_nt = nt;
-                ctx->v3_nwr = nwr;
-                ctx->v3_opt = opt;
-                ctx->v3_smem_bytes = fixed3 + per_warp * 2 * nwr;
-                // both roles on every scheduler partition: measured 1 % faster than one role per partition (round 2)
-                ctx->v3_mix = getenv("PLAAC_V3_MIX") ? atoi(getenv("PLAAC_V3_MIX")) : 1;
-            }
+            ctx->v3_opt = opt;
         }
         // Range of d = a0 - a1 in the forward recurrence: alpha0/alpha1 is a Moebius image of the previous
         // ratio, so for t >= 1  d in [lt10 - lt11 + min(le0-le1), lt00 - lt01 + max(le0-le1)], and the two
@@ -515,8 +498,8 @@ int slot_init(plaac_ctx* ctx, Slot& s)
     int rc = ensure(ctx, s.errflag, sizeof(int));
     if (rc) return rc;
     CU(ctx, cudaMemsetAsync(s.errflag.p, 0, sizeof(int), s.stream));
-    if ((rc = ensure(ctx, s.lg_cnt, 32 + 16 * 8))) return rc;
-    CU(ctx, cudaMemsetAsync(s.lg_cnt.p, 0, 32 + 16 * 8, s.stream));
+    if ((rc = ensure(ctx, s.lg_cnt, 32))) return rc;
+    CU(ctx, cudaMemsetAsync(s.lg_cnt.p, 0, 32, s.stream));
     return PLAAC_OK;
 }
 
@@ -576,7 +559,7 @@ int64_t effective_long_min(const plaac_ctx* ctx)
 // the bookkeeping below assumes k_res_tracks).
 bool long_res_ok(const plaac_ctx* ctx)
 {
-    return ctx->res_plan.ok && ctx->v2_nwr > 0 && ctx->variant != 1 && !getenv("PLAAC_NO_LONG_RES");
+    return ctx->res_plan.ok && ctx->v2_nwr > 0 && ctx->variant != 1;
 }
 
 // Automatic threshold (long_min == -1).  The long-sequence path is a LATENCY device: whole CTAs per protein are far less
@@ -711,7 +694,7 @@ int run_batch(plaac_ctx* ctx, Slot& s, const uint8_t* d_codes, const int64_t* d_
         if ((rc = ensure(ctx, s.lg_list, sizeof(int32_t) * (size_t)cap))) return rc;
         if ((rc = ensure(ctx, s.lg_off, sizeof(int64_t) * (size_t)cap))) return rc;
         // [0] count, [1] scratch cursor, [2] count of >= kLpBigMin residues, [3] redone chunks (cumulative)
-        if ((rc = ensure(ctx, s.lg_cnt, 32 + 16 * 8))) return rc;
+        if ((rc = ensure(ctx, s.lg_cnt, 32))) return rc;
         CU(ctx, cudaMemsetAsync(s.lg_cnt.p, 0, 24, st));
         k_long_select<<<(unsigned)((nprot + 255) / 256), 256, 0, st>>>(d_offsets, nprot, long_min, (int32_t*)s.lg_list.p,
                                                                       (int64_t*)s.lg_off.p, (unsigned long long*)s.lg_cnt.p,
@@ -767,11 +750,8 @@ int run_batch(plaac_ctx* ctx, Slot& s, const uint8_t* d_codes, const int64_t* d_
     // one block per 8 buckets, no grid-stride: buckets come in descending length, so handing them out as blocks retire is
     // longest-first list scheduling.  A resident grid with a stride gave the warps that own the first (longest) buckets
     // twice the average work (measured at 4 M proteins, time outside the scoring kernel: 1.28 ms with 5 CTAs per SM,
-    // 1.17 with 8, 1.03 with 32).  PLAAC_PACK_CTAS caps the grid at that many blocks per SM.
-    static const int pack_ctas_env = [] { const char* e = getenv("PLAAC_PACK_CTAS"); return e ? atoi(e) : 0; }();
-    int64_t pack_blocks64 = (nbuckets + 7) / 8;
-    if (pack_ctas_env > 0) pack_blocks64 = std::min<int64_t>(pack_blocks64, (int64_t)ctx->sm_count * pack_ctas_env);
-    const unsigned pack_blocks = (unsigned)std::min<int64_t>(pack_blocks64, 0x7fffffff);
+    // 1.17 with 8, 1.03 with 32).
+    const unsigned pack_blocks = (unsigned)std::min<int64_t>((nbuckets + 7) / 8, 0x7fffffff);
     {
         auto pack = k_pack<false, false>;
         if (pack_is_std(ctx->ks.charge_plus, ctx->ks.charge_minus)) pack = ctx->ks.adjust_prolines ? k_pack<true, true> : k_pack<true, false>;
@@ -813,10 +793,6 @@ int run_batch(plaac_ctx* ctx, Slot& s, const uint8_t* d_codes, const int64_t* d_
         if ((rc = ensure(ctx, s.lg_ext_win, (size_t)long_scratch + 256))) return rc;
         if ((rc = ensure(ctx, s.lg_tb, (size_t)long_scratch + 256))) return rc;
         if ((rc = ensure(ctx, s.lg_vit, (size_t)long_scratch / 8 + 256))) return rc;
-        // PLAAC_LONG_TIES (testing): "1" treats every binade as a tie binade (everything redone sequentially), "0"
-        // ignores the masks (shows what they are for)
-        const char* ties_env = getenv("PLAAC_LONG_TIES");
-        auto tie_mask = [&](int i) { return !ties_env ? ctx->long_tie[i] : (ties_env[0] == '0' ? 0ull : ~0ull >> 1); };
         LongArgs la;
         la.codes = d_codes;
         la.offsets = d_offsets;
@@ -830,7 +806,7 @@ int run_batch(plaac_ctx* ctx, Slot& s, const uint8_t* d_codes, const int64_t* d_
         la.ext_win = (uint8_t*)s.lg_ext_win.p;
         la.vit = (uint32_t*)s.lg_vit.p;
         la.errflag = (int*)s.errflag.p;
-        for (int i = 0; i < 3; i++) la.tie_mask[i] = tie_mask(1 + i);
+        for (int i = 0; i < 3; i++) la.tie_mask[i] = ctx->long_tie[1 + i];
         CU(ctx, cudaEventRecord(s.ev_fork, st));
         CU(ctx, cudaStreamWaitEvent(long_st, s.ev_fork, 0));
         const bool run_score = d_summaries != nullptr;
@@ -872,17 +848,15 @@ int run_batch(plaac_ctx* ctx, Slot& s, const uint8_t* d_codes, const int64_t* d_
         pa.bnd_plane = bnd_plane;
         pa.lpseq = d_res ? (double*)s.lp_lpseq.p : nullptr;
         pa.warm = std::max(1, std::abs(ctx->long_warm));
-        pa.warm2 = getenv("PLAAC_LP_WARM2") ? atoi(getenv("PLAAC_LP_WARM2")) : 64;
-        pa.big_min = getenv("PLAAC_LP_BIG_MIN") ? atoll(getenv("PLAAC_LP_BIG_MIN")) : (int64_t)kLpBigMin;
+        pa.big_min = ctx->lp_big_min;
         pa.redone = (unsigned long long*)((char*)s.lg_cnt.p + 24);
         pa.want_post = d_res ? 1 : 0;
         pa.want_vit = (run_score || d_res->vit) ? 1 : 0;
         pa.hmm_out = run_score ? (double*)s.lg_hmm.p : nullptr;
         pa.vbytes = (run_score && !(d_res && d_res->vit)) ? (uint8_t*)s.lg_vb.p : nullptr;
         pa.tb = (uint8_t*)s.lg_tb.p;
-        pa.vit_tie_mask = tie_mask(0);
+        pa.vit_tie_mask = ctx->long_tie[0];
         pa.errflag = la.errflag;
-        pa.dbg_clocks = (getenv("PLAAC_LONG_CLOCKS") && !run_score) ? (long long*)((char*)s.lg_cnt.p + 32) : nullptr;
         CU(ctx, cudaStreamWaitEvent(s.aux5, s.ev_fork, 0));
         if (pa.big_min != kLpBigMin) nbig = -1;  // (testing: the class counts are those of the default boundary)
         for (int cls = 0; cls < 2; cls++) {
@@ -924,14 +898,12 @@ int run_batch(plaac_ctx* ctx, Slot& s, const uint8_t* d_codes, const int64_t* d_
         g.core_count = (int32_t*)s.core_count.p;
         g.always_in = ctx->v2_always_in;
         g.work_counter = (unsigned long long*)((char*)s.core_count.p + 8);
-        const bool use_v3 = ctx->v3_nwr > 0 && ctx->variant != 2;
+        const bool use_v3 = ctx->variant != 2;
         if (use_v3) {
             const int full = 2 * ctx->ks.w + 1;
-            g.nwr = ctx->v3_nwr;
             g.ks_wfull = (double)(full * full);
             g.ks_cc2w = ctx->ks.cc2 * g.ks_wfull;
             g.ks_cc2full = ctx->ks.cc2 * (double)full;
-            g.mix_roles = ctx->v3_mix;
             g.fi_a = ctx->ifold.a;
             g.fi_b = ctx->ifold.b;
             g.fi_c = ctx->ifold.c;
@@ -941,7 +913,7 @@ int run_batch(plaac_ctx* ctx, Slot& s, const uint8_t* d_codes, const int64_t* d_
         const int64_t nitems = 2 * nbuckets, wpc = 2 * g.nwr;
         const unsigned grid = (unsigned)std::min<int64_t>((nitems + wpc - 1) / wpc, ctx->sm_count);  // 1 CTA per SM
         if (use_v3)
-            v3_kernel(ctx->v3_opt, ctx->v3_nt)<<<grid, g.nwr * 64, ctx->v3_smem_bytes, st>>>(g);
+            v3_kernel(ctx->v3_opt)<<<grid, g.nwr * 64, ctx->v2_smem_bytes, st>>>(g);
         else
             k_score_summary_v2<<<grid, g.nwr * 64, ctx->v2_smem_bytes, st>>>(g);
         // masked stretches can be jumped exactly when the masking constant is a negative integer (it is -1e6)
@@ -1145,8 +1117,7 @@ int ensure_host(plaac_ctx* ctx, void*& p, size_t& cap, size_t bytes)
 void par_memcpy(void* dst, const void* src, size_t n)
 {
     constexpr size_t kMinPerThread = (size_t)8 << 20;
-    unsigned hw = std::thread::hardware_concurrency();
-    if (const char* e = getenv("PLAAC_STAGE_THREADS")) hw = (unsigned)std::max(1, atoi(e));
+    const unsigned hw = std::thread::hardware_concurrency();
     const size_t nt = std::min<size_t>(std::min<size_t>(hw ? hw : 1, 8), std::max<size_t>(1, n / kMinPerThread));
     if (nt <= 1) {
         memcpy(dst, src, n);
@@ -1391,7 +1362,7 @@ try {
                                                       {(const void*)k_len_hist, kHistSmemBytes},
                                                       {(const void*)k_scatter, kHistSmemBytes}};
         std::vector<std::pair<const void*, size_t>> all(std::begin(fns), std::end(fns));
-        if (ctx->v3_nwr > 0) all.push_back({(const void*)v3_kernel(ctx->v3_opt, ctx->v3_nt), ctx->v3_smem_bytes});
+        if (ctx->v2_nwr > 0) all.push_back({(const void*)v3_kernel(ctx->v3_opt), ctx->v2_smem_bytes});
         for (const auto& f : all) {
             const cudaError_t e = raise_dynamic_smem_limit(f.first, optin, f.second);
             if (e != cudaSuccess) {
@@ -1411,6 +1382,13 @@ try {
         ctx->long_tie[2] = tie_binades(P.le[0], PLAAC_NAA);
         ctx->long_tie[3] = tie_binades(P.hydro2, PLAAC_NAA);
     }
+    // Two test hooks, and the library's only environment reads.  Each chooses which exact path of the long-sequence path
+    // computes a value, so neither can change a result; they let tests reach paths that ordinary inputs reach only at
+    // great cost.  PLAAC_LONG_TIES=1 marks every binade as a tie binade (every chunk is redone sequentially);
+    // PLAAC_LP_BIG_MIN moves the boundary of k_long_post's cluster size class.
+    if (const char* e = getenv("PLAAC_LONG_TIES"); e && strcmp(e, "1") == 0)
+        for (unsigned long long& m : ctx->long_tie) m = ~0ull >> 1;
+    if (const char* e = getenv("PLAAC_LP_BIG_MIN")) ctx->lp_big_min = atoll(e);
     ctx->res_plan = residue_v2_plan(ctx->ks);
     rc = residue_v2_setup(ctx->res_plan, (int)prop.sharedMemPerBlockOptin);
     if (rc == PLAAC_OK) rc = residue_setup(ctx->ks, ctx->ring_words);
@@ -1513,7 +1491,6 @@ try {
     if (variant < 0 || variant > 3) return fail(ctx, PLAAC_E_INVALID, "variant must be 0, 1, 2 or 3");
     if (variant >= 2 && ctx->v2_nwr <= 0)
         return fail(ctx, PLAAC_E_UNSUPPORTED, "v2/v3 kernel unavailable for these parameters: %s", ctx->v2_why.c_str());
-    if (variant == 3 && ctx->v3_nwr <= 0) return fail(ctx, PLAAC_E_UNSUPPORTED, "v3 kernel switched off (PLAAC_SUMMARY_KERNEL=2)");
     ctx->variant = variant;
     return PLAAC_OK;
 } catch (...) {
@@ -1529,14 +1506,6 @@ try {
         if (ctx->slot[i].lg_cnt.p && cudaSetDevice(ctx->device) == cudaSuccess &&
             cudaMemcpy(&v, (char*)ctx->slot[i].lg_cnt.p + 24, sizeof(v), cudaMemcpyDeviceToHost) == cudaSuccess)
             ctx->stats.long_redone_chunks += (int64_t)v;
-    }
-    if (getenv("PLAAC_LONG_CLOCKS") && ctx->slot[0].lg_cnt.p) {
-        long long ck[16];
-        if (cudaMemcpy(ck, (char*)ctx->slot[0].lg_cnt.p + 32, sizeof(ck), cudaMemcpyDeviceToHost) == cudaSuccess) {
-            std::fprintf(stderr, "long-path clocks (cycles since kernel start):");
-            for (int i = 1; i <= 13; i++) std::fprintf(stderr, " %lld", ck[i] ? (i >= 8 && getenv("PLAAC_LONG_CLOCKS")[0] == '2' ? ck[i] : ck[i] - ck[0]) : 0LL);
-            std::fprintf(stderr, "\n");
-        }
     }
     *out = ctx->stats;
     return PLAAC_OK;

@@ -738,7 +738,6 @@ inline int launch_residue_v2(const ResidueV2Plan& P, const ResArgs& ra, const Tr
     int w_hmm = kResHmmThreads / 32, w_vit = kResThreads / 32;
     while (w_hmm > 1 && (nb + w_hmm - 1) / w_hmm < (int64_t)sm_count) w_hmm >>= 1;
     while (w_vit > 1 && (nb + w_vit - 1) / w_vit < (int64_t)sm_count) w_vit >>= 1;
-    if (getenv("PLAAC_RES_WIDE_CTAS")) w_hmm = kResHmmThreads / 32, w_vit = kResThreads / 32;  // (the round-1 shape, for comparison)
     const unsigned g_vit = (unsigned)std::min<int64_t>((nb + w_vit - 1) / w_vit, (int64_t)sm_count * 8);
     const unsigned g_hmm = (unsigned)std::min<int64_t>((nb + w_hmm - 1) / w_hmm, (int64_t)sm_count * 2);
     const unsigned g_trk = (unsigned)std::min<int64_t>((ta.nprot + kTrackWarps - 1) / kTrackWarps, (int64_t)sm_count * 8);
@@ -746,7 +745,7 @@ inline int launch_residue_v2(const ResidueV2Plan& P, const ResArgs& ra, const Tr
     const unsigned g_post = (unsigned)std::min<int64_t>((ra.bv.nslots + kResPostThreads / 32 - 1) / (kResPostThreads / 32) + 1, (int64_t)sm_count * 12);
     // The tracks join last on large batches: nothing behind them reads what they write, and the posterior / byte passes
     // then run beside their tail (200 k proteins: 5.53 -> 5.17 ms; a yeast-sized set loses 2 % to the extra sharing).
-    const bool late = getenv("PLAAC_RES_LATE_JOIN") ? getenv("PLAAC_RES_LATE_JOIN")[0] != '0' : nb >= 1024;
+    const bool late = nb >= 1024;
     k_res_bwd<<<g_hmm, w_hmm * 32, P.bwd_smem, s1>>>(ra);
     k_res_fwd<<<g_hmm, w_hmm * 32, P.fwd_smem, s2>>>(ra);
     k_res_vit<<<g_vit, w_vit * 32, 0, st>>>(ra);

@@ -111,9 +111,8 @@ struct V2Args {
     int32_t* core_count;
     int always_in;        // 1: |a-b| < 40 is guaranteed inside the forward recurrence (bound checked on the host)
     unsigned long long* work_counter;  // zeroed before the launch
-    // v3 only: host-computed (double)(2w+1)^2, cc2 * that, cc2 * (2w+1); role placement
+    // v3 only: host-computed (double)(2w+1)^2, cc2 * that, cc2 * (2w+1)
     double ks_wfull, ks_cc2w, ks_cc2full;
-    int mix_roles;
     // v3 with kV3IntFold: the FoldIndex / PAPA tests as fi_a * (sum of hydi) + fi_b * |charge| + fi_c * taps, and fi_c
     // times the unclipped tap counts 2w+1 and (2w+1)^2
     int fi_a, fi_b, fi_c, fi_cfull, fi_cw;

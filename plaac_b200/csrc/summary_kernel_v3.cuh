@@ -5,17 +5,17 @@
 //   * the Q/N window of the MW column (plaac.java:764-771) is counted four residues at a time in packed bytes (SWAR):
 //     flags, the window count after each residue and the "new maximum?" test for a whole word cost ~20 instructions
 //     instead of ~12 per residue; only a lane that does see a new maximum walks its four residues one by one;
-//   * traceback bits are collected per word in a nibble with predicated ORs and shifted into the bit planes once per word;
 //   * role B gets (2w+1)^2, cc2 * (2w+1)^2 and cc2 * (2w+1) as doubles from the host instead of re-converting them;
 //   * kV3IntFold: role B's hydropathy window sums and the FoldIndex / PAPA sign tests built on them run on the integer
 //     pipes (3 IADD3 for the sums, 2 IMAD + ISETP per test, 32-bit table loads) instead of 18 FP64 instructions per
 //     residue, where the host proved that the integer sign is v2's FP64 sign (plan_int_fold, plaac_cuda.cu).
 //
-// OPT is a compile-time bit set so that single steps can be measured against each other (PLAAC_V3_OPT).  Measured and
-// dropped (round 2, profiles/r02_v3_variants.json): a merged {le0, le1, llr} table entry (32-byte stride: two of the
-// eight lanes of a quarter warp always share a bank group, +10 %), the charge window sums on the FP64 pipe from a table
-// (three more shared-memory loads per residue, +3 %), a segmented word loop (a second copy of the generic body pushes
-// the executed code past the 32 KB instruction cache, +5 %).
+// OPT is a compile-time bit set; setup_scalars (plaac_cuda.cu) clears each bit whose precondition the parameters do not
+// meet.  Measured and dropped (round 2, profiles/r02_kernel_experiments.md): a merged {le0, le1, llr} table entry
+// (32-byte stride: two of the eight lanes of a quarter warp always share a bank group, +10 %), the charge window sums on
+// the FP64 pipe from a table (three more shared-memory loads per residue, +3 %), a segmented word loop (a second copy of
+// the generic body pushes the executed code past the 32 KB instruction cache, +5 %), traceback bits collected per word
+// in a nibble (no gain).
 #pragma once
 #include <type_traits>
 
@@ -25,8 +25,6 @@
 namespace plaac {
 
 constexpr int kV3SwarMw = 1;    // SWAR Q/N window in role A's fast path (needs mw_window <= 100 and the Q/N code set {12, 14})
-constexpr int kV3NibbleTb = 2;  // traceback bits per word in a nibble
-constexpr int kV3Segments = 8;  // segmented word loop (measured slower; kept for the record)
 constexpr int kV3IntFold = 16;  // role B's hydropathy sums and FoldIndex / PAPA sign tests in exact int32 (plan_int_fold)
 
 // (shared-memory layout: v2's, kOff* / kV2FixedBytes / kV2AlignSlack; under kV3IntFold the kOffHydB slots hold
@@ -94,7 +92,7 @@ __device__ __forceinline__ void role_a3(const V2Args& g, uint32_t sbase, uint32_
     const int wv_c1 = (c - 1) >> 2, wv_m1 = (mw - 1) >> 2;  // words holding the first complete LLR / MW window
 
     // one residue step; FAST: every lane has 0 < t < n-1 and t is not the first complete window of either search
-    auto step = [&](auto fast_tag, auto in_tag, int t, int i, uint32_t w0, uint32_t wc, uint32_t wm, uint32_t& nib0, uint32_t& nib1) {
+    auto step = [&](auto fast_tag, auto in_tag, int t, int i, uint32_t w0, uint32_t wc, uint32_t wm) {
         constexpr bool FAST = decltype(fast_tag)::value;
         constexpr bool AIN = decltype(in_tag)::value;
         // code bits 4:0 of byte i moved to address bits 11:7
@@ -147,18 +145,8 @@ __device__ __forceinline__ void role_a3(const V2Args& g, uint32_t sbase, uint32_
                 }
             }
         }
-        if (OPT & kV3NibbleTb) {
-            if (i == 0) {
-                nib0 = tb0 ? 1u : 0u;
-                nib1 = tb1 ? 1u : 0u;
-            } else {
-                if (tb0) nib0 |= 1u << i;
-                if (tb1) nib1 |= 1u << i;
-            }
-        } else {
-            acc0 = __funnelshift_r(acc0, tb0 ? 1u : 0u, 1);  // after 16 steps the bit of residue 16j+i sits at 16+i
-            acc1 = __funnelshift_r(acc1, tb1 ? 1u : 0u, 1);
-        }
+        acc0 = __funnelshift_r(acc0, tb0 ? 1u : 0u, 1);  // after 16 steps the bit of residue 16j+i sits at 16+i
+        acc1 = __funnelshift_r(acc1, tb1 ? 1u : 0u, 1);
     };
 
     // one word = 4 residues: ring traffic, the three byte streams, 4 steps, traceback word every fourth word
@@ -181,7 +169,6 @@ __device__ __forceinline__ void role_a3(const V2Args& g, uint32_t sbase, uint32_
         lo_c = hi_c;
         lo_m = hi_m;
         const int tbase = wv * 4;
-        uint32_t nib0 = 0, nib1 = 0;
         if (FASTW) {
             if (OPT & kV3SwarMw) {
                 // Q/N window four residues at a time.  A byte is Q or N iff (code & 0x1d) == 0x0c (codes 14, 12;
@@ -210,19 +197,15 @@ __device__ __forceinline__ void role_a3(const V2Args& g, uint32_t sbase, uint32_
             }
             if (g.always_in) {
 #pragma unroll
-                for (int i = 0; i < 4; i++) step(std::true_type{}, std::true_type{}, tbase + i, i, w0, wc, wm, nib0, nib1);
+                for (int i = 0; i < 4; i++) step(std::true_type{}, std::true_type{}, tbase + i, i, w0, wc, wm);
             } else {
 #pragma unroll
-                for (int i = 0; i < 4; i++) step(std::true_type{}, std::false_type{}, tbase + i, i, w0, wc, wm, nib0, nib1);
+                for (int i = 0; i < 4; i++) step(std::true_type{}, std::false_type{}, tbase + i, i, w0, wc, wm);
             }
         } else {
 #pragma unroll
-            for (int i = 0; i < 4; i++) step(std::false_type{}, std::false_type{}, tbase + i, i, w0, wc, wm, nib0, nib1);
+            for (int i = 0; i < 4; i++) step(std::false_type{}, std::false_type{}, tbase + i, i, w0, wc, wm);
             if (OPT & kV3SwarMw) mwb1 = (uint32_t)(min(mw_best, 127) + 1) * 0x01010101u;
-        }
-        if (OPT & kV3NibbleTb) {
-            acc0 = __funnelshift_r(acc0, nib0, 4);  // after 4 words the bit of residue 16j+i sits at 16+i
-            acc1 = __funnelshift_r(acc1, nib1, 4);
         }
         if ((wv & 3) == 3) {
             // low half: predecessor-of-state-0 bits of the slot's 16 residues, high half: predecessor-of-state-1 bits
@@ -233,29 +216,12 @@ __device__ __forceinline__ void role_a3(const V2Args& g, uint32_t sbase, uint32_
     // fast words: wv != 0, not the word of the first complete LLR / MW window, and tbase + 3 < nmin - 1 (t = nmin-1 stays
     // generic so the "whole protein is one MW window" case, n < mw, is seen there)
     const int fast_end = nmin >= 5 ? (nmin - 1) >> 2 : 0;  // words wv < fast_end have 4*wv + 3 < nmin - 1
-    if (OPT & kV3Segments) {
-        int wv = 0;
 #pragma unroll 1
-        while (wv < nwords) {
-            if (wv == 0 || wv == wv_c1 || wv == wv_m1 || wv >= fast_end) {
-                word(std::false_type{}, wv);
-                wv++;
-                continue;
-            }
-            int stop = min(fast_end, nwords);
-            if (wv < wv_c1) stop = min(stop, wv_c1);
-            if (wv < wv_m1) stop = min(stop, wv_m1);
-#pragma unroll 1
-            for (; wv < stop; wv++) word(std::true_type{}, wv);
-        }
-    } else {
-#pragma unroll 1
-        for (int wv = 0; wv < nwords; wv++) {
-            if (wv != 0 && wv != wv_c1 && wv != wv_m1 && wv < fast_end)
-                word(std::true_type{}, wv);
-            else
-                word(std::false_type{}, wv);
-        }
+    for (int wv = 0; wv < nwords; wv++) {
+        if (wv != 0 && wv != wv_c1 && wv != wv_m1 && wv < fast_end)
+            word(std::true_type{}, wv);
+        else
+            word(std::false_type{}, wv);
     }
 
     if (prot < 0) return;
@@ -545,22 +511,12 @@ __device__ __forceinline__ bool role_b3(const V2Args& g, uint32_t sbase, uint32_
     // p = n-1-halfw, out of the fast path)
     const int fast_end = nmin >= 5 ? (nmin - 1) >> 2 : 0;
     const int fast_begin = (fast_lo + 3) >> 2;
-    if (OPT & kV3Segments) {
-        int wv = 0;
 #pragma unroll 1
-        for (; wv < min(fast_begin, nwords); wv++) word(std::false_type{}, wv);
-#pragma unroll 1
-        for (; wv < min(fast_end, nwords); wv++) word(std::true_type{}, wv);
-#pragma unroll 1
-        for (; wv < nwords; wv++) word(std::false_type{}, wv);
-    } else {
-#pragma unroll 1
-        for (int wv = 0; wv < nwords; wv++) {
-            if (wv >= fast_begin && wv < fast_end)
-                word(std::true_type{}, wv);
-            else
-                word(std::false_type{}, wv);
-        }
+    for (int wv = 0; wv < nwords; wv++) {
+        if (wv >= fast_begin && wv < fast_end)
+            word(std::true_type{}, wv);
+        else
+            word(std::false_type{}, wv);
     }
 
     if (IFOLD && __any_sync(0xffffffffu, amb)) return true;
@@ -632,8 +588,9 @@ __device__ __forceinline__ bool role_b3(const V2Args& g, uint32_t sbase, uint32_
     return false;
 }
 
-template <int OPT, int NT>
-__global__ void __launch_bounds__(NT, 1) k_score_summary_v3(V2Args g)
+// 768 threads (kV2MaxThreads): 80 registers per thread
+template <int OPT>
+__global__ void __launch_bounds__(kV2MaxThreads, 1) k_score_summary_v3(V2Args g)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const uint32_t raw = smem_u32(smem_raw);
@@ -671,11 +628,11 @@ __global__ void __launch_bounds__(NT, 1) k_score_summary_v3(V2Args g)
     constexpr uint32_t kPadW = 0x01010101u * kPad;
     __syncthreads();
 
-    // Persistent warps, one role per warp while that role has buckets left (see k_score_summary_v2).  g.mix_roles:
-    // 0 = one role per scheduler partition (even warps A, odd warps B), 1 = both roles on every partition.
+    // Persistent warps, one role per warp while that role has buckets left (see k_score_summary_v2), both roles on every
+    // scheduler partition (measured 1 % faster than one role per partition, round 2): warps 2k and 2k+1 take different
+    // roles, and the roles alternate along every partition (wid & 3).
     const int64_t nb = g.bv.nbuckets;
-    // mixed: warps 2k and 2k+1 still take different roles, and the roles alternate along every partition (wid & 3)
-    int role = (g.mix_roles & 1) ? (((wid >> 2) ^ wid) & 1) : (wid & 1);
+    int role = ((wid >> 2) ^ wid) & 1;
     const int64_t per_role = (int64_t)(blockDim.x >> 6);
     const int slot_in_role = wid >> 1;
     int64_t item = (int64_t)blockIdx.x * per_role + slot_in_role;
@@ -688,14 +645,13 @@ __global__ void __launch_bounds__(NT, 1) k_score_summary_v3(V2Args g)
             role ^= 1;
         } else {
             for (int i = 0; i < g.ring_words; i++) ring[i * 32] = kPadW;
-            // (g.mix_roles bits 8/9: timing experiments that skip role B / role A; the records are then incomplete)
             if (role) {
-                if (!(g.mix_roles & 256) && role_b3<OPT>(g, sbase, ring, lane, item)) {
+                if (role_b3<OPT>(g, sbase, ring, lane, item)) {
                     for (int i = 0; i < g.ring_words; i++) ring[i * 32] = kPadW;
                     role_b3<OPT & ~kV3IntFold, true>(g, sbase, ring, lane, item);
                 }
             } else {
-                if (!(g.mix_roles & 512)) role_a3<OPT>(g, sbase, ring, lane, item);
+                role_a3<OPT>(g, sbase, ring, lane, item);
             }
         }
         unsigned long long nx = 0;
@@ -704,19 +660,16 @@ __global__ void __launch_bounds__(NT, 1) k_score_summary_v3(V2Args g)
     }
 }
 
-// The instantiations that exist (PLAAC_V3_OPT picks one for experiments).
+// Every subset of the default bits has an instantiation: setup_scalars clears bits per parameter set.
 constexpr int kV3DefaultOpt = kV3SwarMw | kV3IntFold;
 using V3Kernel = void (*)(V2Args);
-// nt: threads per CTA the kernel is compiled for (768: 80 registers per thread)
-inline V3Kernel v3_kernel(int opt, int nt)
+inline V3Kernel v3_kernel(int opt)
 {
-    if (nt == 768) switch (opt) {
-        case 0: return k_score_summary_v3<0, 768>;
-        case 1: return k_score_summary_v3<1, 768>;
-        case 16: return k_score_summary_v3<16, 768>;
-        case 17: return k_score_summary_v3<17, 768>;
-        case 3: return k_score_summary_v3<3, 768>;
-        case 8: return k_score_summary_v3<8, 768>;
+    switch (opt) {
+        case 0: return k_score_summary_v3<0>;
+        case kV3SwarMw: return k_score_summary_v3<kV3SwarMw>;
+        case kV3IntFold: return k_score_summary_v3<kV3IntFold>;
+        case kV3SwarMw | kV3IntFold: return k_score_summary_v3<kV3SwarMw | kV3IntFold>;
     }
     return nullptr;
 }

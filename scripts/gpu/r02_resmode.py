@@ -56,8 +56,10 @@ for n in (9000, 35000, 100000):
     res = {}
     for tag, thr, env in (("long_path", 1024, {}), ("long_path_one_cta", 1024, {"PLAAC_LP_BIG_MIN": "10000000"}), ("cluster8", 1024, {"PLAAC_LP_BIG_MIN": "1024"}), ("single_lane_walk", 0, {})):
         for k, v in env.items(): os.environ[k] = v
+        sc = plaac_b200.Scorer()  # (PLAAC_LP_BIG_MIN is read when a Scorer is created)
         sc.set_long_path(thr)
         res[tag + "_ms"] = timeit(codes, offsets, 1, n, ptrs)
+        sc.close()
         for k in env: del os.environ[k]
     print(n, res, flush=True)
     out["n%d" % n] = res

@@ -16,7 +16,9 @@ for f in ("core_start", "core_end", "vit_maxrun", "llr_start", "mw_score", "fi_n
     assert (got_s[f] == ref_s[f]).all(), f
 assert np.abs(got_s["hmm_all"] - ref_s["hmm_all"]).max() < 1e-9 and np.abs(got_s["hmm_vit"] - ref_s["hmm_vit"]).max() < 1e-9
 for big in (None, "1024"):
-    if big: os.environ["PLAAC_LP_BIG_MIN"] = big
+    if big:
+        os.environ["PLAAC_LP_BIG_MIN"] = big  # (read when a Scorer is created)
+        sc = plaac_b200.Scorer(); sc.set_long_path(1024)
     summ, res = sc.score(codes, offs, per_residue=True)
     dev = torch.device("cuda", 0)
     dc = torch.from_numpy(np.concatenate([codes, np.zeros(64, np.uint8)])).to(dev); do = torch.from_numpy(offs).to(dev)

@@ -5,6 +5,7 @@ import numpy as np, torch
 import plaac_b200
 from tests import synth
 which = sys.argv[1]
+if which == "big": os.environ["PLAAC_LP_BIG_MIN"] = "1024"  # (read when the Scorer is created)
 lc, lo = synth.long_proteins(seed=1009, lengths=(1300, 5000, 2049, 9000))
 sc = plaac_b200.Scorer(); sc.set_long_path(1024)
 if which == "summary":
@@ -17,6 +18,5 @@ else:
     u8 = torch.zeros(2 * n, dtype=torch.uint8, device=dev); f64 = torch.zeros(10 * n, dtype=torch.float64, device=dev)
     ptrs = {"vit": u8.data_ptr(), "map": u8.data_ptr() + n}
     for k, nm in enumerate(plaac_b200.RESIDUE_F64): ptrs[nm] = f64.data_ptr() + 8 * k * n
-    if which == "big": os.environ["PLAAC_LP_BIG_MIN"] = "1024"
     sc.score_device(dc.data_ptr(), do.data_ptr(), 4, n, 0, residue_ptrs=ptrs, sync=True)
     print("per-residue ok", which, sc.stats().long_proteins)

@@ -516,7 +516,7 @@ def _residue_equal_bits(a, b, what):
         assert same.all(), (what, k, int((~same).sum()), a[k][~same][:3], b[k][~same][:3])
 
 
-def test_per_residue_long_path_is_the_sequential_walk_bit_for_bit(monkeypatch):
+def test_per_residue_long_path_matches_the_sequential_walk_bit_for_bit(monkeypatch):
     """Long proteins in per-residue mode (long_residue.cuh: one thread-block cluster per protein, binade-frame forward
     and backward recurrences with an exact carry over the chunk boundaries) against (i) the oracle and (ii) the bucketed
     kernels' single-lane walk of the same proteins: the same bits in every column, in both cluster size classes, with
@@ -533,12 +533,11 @@ def test_per_residue_long_path_is_the_sequential_walk_bit_for_bit(monkeypatch):
     ref = orc.residue_batch(P, codes, offs, nthreads=NT)
     ref_s = orc.score_batch(P, codes, offs, nthreads=NT)
 
-    monkeypatch.setenv("PLAAC_NO_LONG_RES", "1")
     sc = plaac_b200.Scorer()
-    sc.set_long_path(1024)
+    sc.set_long_path(0)
     _, walk = sc.score(codes, offs, per_residue=True)
     assert sc.stats().long_proteins == 0
-    monkeypatch.delenv("PLAAC_NO_LONG_RES")
+    sc.close()
     _check_residue(walk, ref, "sequential walk")
 
     import torch
@@ -552,7 +551,7 @@ def test_per_residue_long_path_is_the_sequential_walk_bit_for_bit(monkeypatch):
     for k, nm in enumerate(plaac_b200.RESIDUE_F64):
         ptrs[nm] = f64.data_ptr() + 8 * k * ntot
 
-    def device_call(what):
+    def device_call(sc, what):
         # per-residue arrays only (no records): the Viterbi parse of the long proteins then comes from k_long_post
         u8.zero_()
         f64.zero_()
@@ -564,30 +563,32 @@ def test_per_residue_long_path_is_the_sequential_walk_bit_for_bit(monkeypatch):
         _residue_equal_bits(dev_got, walk, "device-resident, no records: " + what)
 
     for warm, big_min, ties in ((256, None, None), (3, None, None), (64, "1024", None), (256, "200000", None), (256, None, "1")):
+        # (the test hooks are read when the Scorer is created)
         if big_min:
             monkeypatch.setenv("PLAAC_LP_BIG_MIN", big_min)
         if ties:
             monkeypatch.setenv("PLAAC_LONG_TIES", ties)   # every binade a tie binade: every Viterbi chunk redone sequentially
+        sc = plaac_b200.Scorer()
         what = f"warm={warm} big_min={big_min} ties={ties}"
         sc.set_long_path(1024, warm)
-        n0 = sc.stats().long_proteins
         summ, got = sc.score(codes, offs, per_residue=True)
-        assert sc.stats().long_proteins - n0 == int((lens >= 1024).sum())
+        assert sc.stats().long_proteins == int((lens >= 1024).sum())
         _check_residue(got, ref, "long per-residue " + what)
         _residue_equal_bits(got, walk, "long path vs walk " + what)
         _check(summ, ref_s, "records beside the long per-residue path", P, codes, offs, max_ties=2)
-        device_call(what)
+        device_call(sc, what)
+        sc.close()
         if big_min:
             monkeypatch.delenv("PLAAC_LP_BIG_MIN")
         if ties:
             monkeypatch.delenv("PLAAC_LONG_TIES")
     # automatic threshold
+    sc = plaac_b200.Scorer()
     sc.set_long_path(-1, 256)
-    n0 = sc.stats().long_proteins
     _, got = sc.score(codes, offs, per_residue=True)
-    assert sc.stats().long_proteins > n0
+    assert sc.stats().long_proteins > 0
     _residue_equal_bits(got, walk, "automatic threshold")
-    device_call("automatic threshold")
+    device_call(sc, "automatic threshold")
     sc.close()
 
 
@@ -693,7 +694,7 @@ def test_long_path_with_exact_tie_constants():
     """Table constants that are exact round-half-even ties in the binades a long protein walks through (bits below
     the ulp exactly 1000...0): there a sum's rounding depends on its parity, the shift argument of the long-sequence
     path does not hold, and plaac_create must route those binades to the sequential redo (tie_binades).  The oracle
-    does the same arithmetic sequentially.  (With PLAAC_LONG_TIES=0, which ignores the masks, this test fails.)"""
+    does the same arithmetic sequentially.  (With the masks ignored, this test fails.)"""
     rng = np.random.default_rng(99)
     bg = synth.BG_SCER / synth.BG_SCER.sum()
     prd = synth.PRD_28 / synth.PRD_28.sum()
@@ -729,3 +730,41 @@ def test_long_path_with_exact_tie_constants():
         sc.close()
         assert st.long_proteins == (2 if min_len else 0)
         _check(got, ref, f"tie constants, long_min={min_len}")
+
+
+# Settings that once came from the environment and changed what a caller got back (a skipped role of the v3 kernel,
+# ignored tie masks, another kernel or path): a variable left in a user's shell must not reach the results.
+RETIRED_ENV = {"PLAAC_V3_MIX": "256", "PLAAC_SUMMARY_KERNEL": "2", "PLAAC_V3_OPT": "8", "PLAAC_V3_NT": "512",
+               "PLAAC_LONG_TIES": "0", "PLAAC_NO_LONG_RES": "1"}
+
+
+def test_retired_environment_variables_change_nothing(monkeypatch):
+    """Records and per-residue arrays of a proteome with long proteins on the long-sequence path: a Scorer created with
+    each retired variable set, and with all of them, gives the bytes of one created without them."""
+    sc_, so = synth.proteome(2000, seed=31, median=300.0)
+    lc, lo = synth.long_proteins(seed=1011, lengths=(1100, 2500, 9000))
+    codes = np.concatenate([sc_, lc])
+    offs = np.concatenate([so, lo[1:] + so[-1]])
+
+    def run():
+        sc = plaac_b200.Scorer()
+        sc.set_long_path(1024)
+        only = sc.score(codes, offs)
+        summ, res = sc.score(codes, offs, per_residue=True)
+        nlong = sc.stats().long_proteins
+        sc.close()
+        return only, summ, res, nlong
+
+    want = run()
+    assert want[3] == 2 * int((np.diff(offs) >= 1024).sum())
+    for env in [{k: v} for k, v in RETIRED_ENV.items()] + [RETIRED_ENV]:
+        for k, v in env.items():
+            monkeypatch.setenv(k, v)
+        got = run()
+        for k in env:
+            monkeypatch.delenv(k)
+        what = ", ".join(f"{k}={v}" for k, v in env.items())
+        assert got[0].tobytes() == want[0].tobytes(), what
+        assert got[1].tobytes() == want[1].tobytes(), what
+        _residue_equal_bits(got[2], want[2], what)
+        assert got[3] == want[3], what

@@ -128,10 +128,10 @@ def test_cuda_per_residue_against_the_jar(which, monkeypatch):
     which = which.replace("_cluster", "")
     enc, kw, prots = jarvec.scenario(which)
     codes, offs = plaac_b200.pack([c for _, c in enc])
+    if cluster:
+        monkeypatch.setenv("PLAAC_LP_BIG_MIN", "1024")  # (read when the Scorer is created)
     sc = plaac_b200.Scorer(plaac_b200.default_params(**kw))
     if which == "long_residue":
-        if cluster:
-            monkeypatch.setenv("PLAAC_LP_BIG_MIN", "1024")
         sc.set_long_path(1024)
     _, res = sc.score(codes, offs, per_residue=True)
     if which == "long_residue":
