@@ -323,6 +323,27 @@ typedef struct plaac_null {
 int plaac_score_shuffles(plaac_ctx *ctx, const uint8_t *codes, const int64_t *offsets, int64_t nprot,
                          plaac_null *null_spec, plaac_summary *observed);
 
+/* Sequential shuffle null (Besag and Clifford, Biometrika 78:301, 1991; DESIGN.md section 14): as plaac_score_shuffles,
+ * but each (selected protein, column) stops once h = stop_hits of its replicates have reached the observed score, after
+ * at most K_max = null_spec->replicates replicates.  With hit(r) the counting rule of plaac_score_shuffles applied to
+ * replicate r of the protein:
+ *   L     = the smallest L in [1, K_max] with hit(0) + ... + hit(L-1) == h; K_max if there is none;
+ *   count = hit(0) + ... + hit(L-1): h if the column stopped, below h otherwise.
+ * Both are pure functions of (seed, reference index, columns, h, K_max): they do not depend on the selection's order or
+ * repeats, the chunking, the long-path setting, the kernel variant or the round schedule.  With h > K_max nothing stops:
+ * count equals plaac_score_shuffles' count for K = K_max, and L = K_max.  The p-value is h / L when count == h, and
+ * (count + 1) / (K_max + 1) otherwise.  A protein is scored in rounds while any of its columns is below h, so a protein
+ * with true p-value p costs about min(h / p, K_max) replicates.
+ * null_spec: replicates = K_max; seed, columns, nsel, proteins as plaac_score_shuffles; reserved must be 0; counts
+ * receives count (nsel x popcount(columns), row-major, columns in ascending bit order); values must be NULL.  scored
+ * receives L in the same layout.  observed: NULL or nsel records, byte-identical to plaac_score's.  HOST buffers (pinned
+ * or pageable); blocks until done.
+ * PLAAC_E_INVALID as plaac_score_shuffles, and for stop_hits < 1, a non-NULL values, a NULL scored with nsel != 0.
+ * K_max == 0: counts and scored are 0 and observed is written.  nsel == 0: PLAAC_OK, nothing written.  Reference bytes
+ * > 21 are scored as X: everything is written and the call then returns PLAAC_E_INVALID. */
+int plaac_score_shuffles_seq(plaac_ctx *ctx, const uint8_t *codes, const int64_t *offsets, int64_t nprot,
+                             const plaac_null *null_spec, int64_t stop_hits, int64_t *scored, plaac_summary *observed);
+
 /* ---- multi-GPU (SURVEY.md section 8e): proteins are independent, so the batch is cut into contiguous,
  * residue-balanced shards, one per ctx (each ctx on its own GPU), scored concurrently by one host thread per
  * ctx, each writing its records / per-residue rows straight into the caller's arrays at the input position.

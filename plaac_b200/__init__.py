@@ -9,4 +9,5 @@ from .capi import (  # noqa: F401
     RESIDUE_F64, RESIDUE_U8, MultiScorer, shard_plan, PinnedBuffer, host_register, host_unregister,
     pack_words, pack_append, pack_chars, unpack_words, Hits, HITS_CORE, HITS_TOPK, PACK_PER_WORD, Variants, Segments, saturation,
     EFFECT_COLUMNS, effects_dtype, saturation_map, NULL_COLUMNS, Null, shuffle,
+    seq_pvalues,
 )

@@ -191,6 +191,8 @@ def lib():
         L.plaac_score_segments.argtypes = [vp, vp, vp, i64, vp, C.POINTER(Segments)]
         L.plaac_score_shuffles.restype = C.c_int
         L.plaac_score_shuffles.argtypes = [vp, vp, vp, i64, C.POINTER(Null), vp]
+        L.plaac_score_shuffles_seq.restype = C.c_int
+        L.plaac_score_shuffles_seq.argtypes = [vp, vp, vp, i64, C.POINTER(Null), i64, vp, vp]
         L.plaac_shuffle_host.restype = C.c_int
         L.plaac_shuffle_host.argtypes = [vp, i64, C.c_uint64, i64, i64, vp]
         L.plaac_bench_synth_lengths.restype = C.c_int
@@ -525,15 +527,7 @@ class Scorer:
         values=True also the replicates' values as an (nsel, K) structured array of f8 fields (has_core: 0 or 1); with
         observed=True also the selected proteins' records (those of score()).  Replicate r of protein i is
         shuffle(codes, offsets, i, r, seed)."""
-        if isinstance(columns, str):
-            columns = (columns,)
-        unknown = [c for c in columns if c not in NULL_COLUMNS]
-        if unknown or not len(columns):
-            raise ValueError(f"null columns must be a non-empty subset of {NULL_COLUMNS}, got {list(columns)}")
-        mask = 0
-        for c in columns:
-            mask |= 1 << NULL_COLUMNS.index(c)
-        names = [n for k, n in enumerate(NULL_COLUMNS) if mask >> k & 1]
+        mask, names = _null_mask(columns)
         codes = np.ascontiguousarray(codes, dtype=np.uint8)
         offsets = np.ascontiguousarray(offsets, dtype=np.int64)
         nprot = len(offsets) - 1
@@ -550,6 +544,34 @@ class Scorer:
                                                obs.ctypes.data if observed else None))
         ret = [counts] + ([vals] if values else []) + ([obs] if observed else [])
         return ret[0] if len(ret) == 1 else tuple(ret)
+
+    def shuffle_null_seq(self, codes: np.ndarray, offsets: np.ndarray, max_replicates: int, stop_hits: int = 10, seed: int = 0,
+                         columns=("core_score", "llr", "hmm_all"), proteins=None, observed: bool = False):
+        """plaac_score_shuffles_seq: the sequential null of Besag and Clifford.  The replicates of shuffle_null are scored
+        in order, and a protein's column stops once `stop_hits` (h) of them have reached the observed score, after at
+        most `max_replicates` (K_max).  Returns (counts, scored): structured int64 arrays with one field per selected
+        column in NULL_COLUMNS order, one row per selected protein; counts is h for a column that stopped and below h
+        otherwise, scored is the number of replicates that count covers (K_max if the column did not stop).  With
+        observed=True also the selected proteins' records (those of score()).  seq_pvalues turns them into p-values."""
+        mask, names = _null_mask(columns)
+        h, K = int(stop_hits), int(max_replicates)
+        if h < 1:
+            raise ValueError(f"stop_hits must be >= 1, got {h}")
+        if K < 0:
+            raise ValueError(f"max_replicates must be >= 0, got {K}")
+        codes = np.ascontiguousarray(codes, dtype=np.uint8)
+        offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+        nprot = len(offsets) - 1
+        sel = None if proteins is None else np.ascontiguousarray(proteins, dtype=np.int32)
+        nsel = nprot if sel is None else len(sel)
+        counts = np.zeros(nsel, dtype=[(n, "<i8") for n in names])
+        scored = np.zeros(nsel, dtype=counts.dtype)
+        obs = np.zeros(nsel, dtype=SUMMARY_DTYPE) if observed else None
+        nl = Null(replicates=K, seed=int(seed) & (2**64 - 1), columns=mask, reserved=0, nsel=-1 if sel is None else nsel,
+                  proteins=sel.ctypes.data if sel is not None else None, counts=counts.ctypes.data, values=None)
+        self._check(lib().plaac_score_shuffles_seq(self._h, codes.ctypes.data, offsets.ctypes.data, nprot, C.byref(nl), h,
+                                                   scored.ctypes.data, obs.ctypes.data if observed else None))
+        return (counts, scored, obs) if observed else (counts, scored)
 
     def score_ptr(self, codes_ptr: int, offsets_ptr: int, nprot: int, summaries_ptr: int):
         """Raw host pointers (e.g. pinned torch tensors)."""
@@ -684,6 +706,32 @@ def shuffle(codes: np.ndarray, offsets: np.ndarray, protein: int, replicate: int
                                   out.ctypes.data)
     if rc != 0:
         raise PlaacError(rc, lib().plaac_last_error(None).decode())
+    return out
+
+
+def _null_mask(columns):
+    """Column names of the shuffle nulls -> (PLAAC_EFFECT_* / PLAAC_NULL_HAS_CORE mask, the names in bit order)."""
+    if isinstance(columns, str):
+        columns = (columns,)
+    unknown = [c for c in columns if c not in NULL_COLUMNS]
+    if unknown or not len(columns):
+        raise ValueError(f"null columns must be a non-empty subset of {NULL_COLUMNS}, got {list(columns)}")
+    mask = 0
+    for c in columns:
+        mask |= 1 << NULL_COLUMNS.index(c)
+    return mask, [n for k, n in enumerate(NULL_COLUMNS) if mask >> k & 1]
+
+
+def seq_pvalues(counts: np.ndarray, scored: np.ndarray, stop_hits: int, max_replicates: int) -> np.ndarray:
+    """The p-values of Scorer.shuffle_null_seq's (counts, scored): h / L where a column stopped (count == h), else
+    (count + 1) / (K_max + 1).  One float64 field per double column; has_core is left out, as the CLI leaves out its p."""
+    h, K = int(stop_hits), int(max_replicates)
+    names = [n for n in counts.dtype.names if n != "has_core"]
+    out = np.zeros(len(counts), dtype=[(n, "<f8") for n in names])
+    for n in names:
+        c, L = counts[n].astype(np.float64), scored[n].astype(np.float64)
+        stopped = counts[n] == h
+        out[n] = np.where(stopped, h / np.where(stopped, L, 1.0), (c + 1.0) / (K + 1.0))
     return out
 
 

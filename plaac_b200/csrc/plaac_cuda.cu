@@ -31,6 +31,7 @@
 #include "variants.cuh"
 #include "segments.cuh"
 #include "shuffle.cuh"
+#include "shuffle_seq.cuh"
 
 using namespace plaac;
 
@@ -113,6 +114,9 @@ struct plaac_ctx {
     DevBuf var_wild;              // its records (plaac_score_variant_effects), or the observed records of the selection
                                   // (plaac_score_shuffles), uploaded once per call
     DevBuf null_counts;           // plaac_score_shuffles: nsel x k counts, summed over the chunks
+    // plaac_score_shuffles_seq: nsel x k replicates scored (null_counts holds the hits), the round's hit flags, the
+    // active flags of its list and their scan, and the list itself (two buffers, [0] = length, then the entries)
+    DevBuf seq_scored, seq_flags, seq_live, seq_pos, seq_act[2];
     // pageable <-> device copies of the FASTA calls: two pinned staging buffers, filled / emptied by a multi-threaded memcpy
     void* stage_buf[2] = {nullptr, nullptr};
     cudaEvent_t stage_ev[2] = {nullptr, nullptr};
@@ -1413,7 +1417,8 @@ void plaac_destroy(plaac_ctx* ctx)
     cudaSetDevice(ctx->device);
     for (int i = 0; i < kSlots; i++) slot_free(ctx->slot[i]);
     release(ctx->all_summaries);
-    for (DevBuf* b : {&ctx->union_rec, &ctx->union_idx, &ctx->union_order, &ctx->union_out_idx, &ctx->var_ref, &ctx->var_ref_off, &ctx->var_wild, &ctx->null_counts}) release(*b);
+    for (DevBuf* b : {&ctx->union_rec, &ctx->union_idx, &ctx->union_order, &ctx->union_out_idx, &ctx->var_ref, &ctx->var_ref_off, &ctx->var_wild, &ctx->null_counts,
+                      &ctx->seq_scored, &ctx->seq_flags, &ctx->seq_live, &ctx->seq_pos, &ctx->seq_act[0], &ctx->seq_act[1]}) release(*b);
     for (int b = 0; b < 2; b++) {
         if (ctx->stage_buf[b]) cudaFreeHost(ctx->stage_buf[b]);
         if (ctx->stage_ev[b]) cudaEventDestroy(ctx->stage_ev[b]);
@@ -1653,6 +1658,14 @@ try {
 
 namespace {
 
+// Where k_shuffle_flags of a round of plaac_score_shuffles_seq (a slice of its list) writes: act = the slice of the
+// device list (selection indices), flags = wpr words per (entry, column) row.
+struct SeqRound {
+    const int32_t* act;
+    uint32_t* flags;
+    int64_t wpr;
+};
+
 // What the host-buffer calls are given: one-byte codes + int64 offsets (plaac_score), radix-22 words + int32
 // lengths (plaac_score_packed), a variant list over a reference batch of one-byte codes (plaac_score_variants), or
 // shuffled replicates of that batch's proteins (plaac_score_shuffles).
@@ -1670,6 +1683,10 @@ struct HostInput {
     // sel), j < nsel; its output form is the per-protein tally of k_shuffle_tally into ctx->null_counts (and the rows of
     // nul->values), against the observed records in ctx->var_wild
     const plaac_null* nul = nullptr;  // nsel >= 0, proteins NULL for every protein; checked by plaac_score_shuffles
+    // ... in a round of plaac_score_shuffles_seq: the replicates are r0 + [0, K) of each protein, the output form is the
+    // round's hit flags (k_shuffle_flags), and the reference is already on the device
+    int64_t r0 = 0;
+    const SeqRound* seq = nullptr;
     bool packed() const { return words != nullptr || lengths != nullptr; }
 };
 
@@ -1707,6 +1724,7 @@ int variants_prepare(plaac_ctx* ctx, const HostInput& in, int64_t& total)
                         (long long)V.first_sub[v + 1], (long long)V.first_sub[v]);
         total += in.offsets[p + 1] - in.offsets[p];
     }
+    if (in.seq) return PLAAC_OK;  // (a round of plaac_score_shuffles_seq: uploaded with its observed records)
     int rc;
     if ((rc = ensure(ctx, ctx->var_ref, (size_t)ref_n + 64))) return rc;
     if ((rc = ensure(ctx, ctx->var_ref_off, sizeof(int64_t) * (size_t)(in.nref + 1)))) return rc;
@@ -2140,7 +2158,7 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
                 CUB(cudaMemcpyAsync(s.v_prot.p, nul->proteins + j0, sizeof(int32_t) * (size_t)(j1 - j0 + 1), cudaMemcpyHostToDevice, s.stream));
                 d_sel = (const int32_t*)s.v_prot.p;
             }
-            k_shuffle_prep<<<(unsigned)((np + 255) / 256), 256, 0, s.stream>>>(d_sel, j0, start, K, np, (const int64_t*)ctx->var_ref_off.p,
+            k_shuffle_prep<<<(unsigned)((np + 255) / 256), 256, 0, s.stream>>>(d_sel, j0, start, K, in.r0, np, (const int64_t*)ctx->var_ref_off.p,
                                                                                nul->seed, (int32_t*)s.lengths.p, (ShuffleRep*)s.sh_rep.p);
             ctx->stats.kernel_launches += 1;
             if ((rc = launch_scan(ctx, s, (const int32_t*)s.lengths.p, (int64_t*)s.offsets.p, np, s.stream))) break;
@@ -2197,6 +2215,12 @@ int score_host(plaac_ctx* ctx, const HostInput& in, int64_t nprot, plaac_summary
             ctx->stats.kernel_launches += 1;
             CUB(cudaMemcpyAsync(stage_sum ? s.h_stage_sum : (void*)(eff->effects + start * ek), s.v_effects.p, row_bytes * (size_t)np,
                                 cudaMemcpyDeviceToHost, s.stream));
+        } else if (in.seq) {
+            // (a round of plaac_score_shuffles_seq: the hits become flags, decided on by k_shuffle_stop after the round)
+            k_shuffle_flags<<<(unsigned)((np * ek + 255) / 256), 256, 0, s.stream>>>(
+                d_sum, (const plaac_summary*)ctx->var_wild.p, in.seq->act, start, K, np, (uint32_t)nul->columns, in.seq->wpr,
+                in.seq->flags);
+            ctx->stats.kernel_launches += 1;
         } else if (nul) {
             // the records stay on the device: the counts are summed there, and only the values rows (if any) cross the link
             double* d_val = nul->values ? (double*)s.v_effects.p : nullptr;
@@ -2396,34 +2420,43 @@ try {
     return api_caught(nullptr, "plaac_shuffle_host");
 }
 
-int plaac_score_shuffles(plaac_ctx* ctx, const uint8_t* codes, const int64_t* offsets, int64_t nprot, plaac_null* null_spec,
-                         plaac_summary* observed)
-try {
-    if (!ctx) return fail(nullptr, PLAAC_E_INVALID, "plaac_score_shuffles: NULL ctx");
-    if (!null_spec) return fail(ctx, PLAAC_E_INVALID, "plaac_score_shuffles: NULL null_spec");
-    const plaac_null& N = *null_spec;
+}  // extern "C"
+
+namespace {
+
+// The checks plaac_score_shuffles and plaac_score_shuffles_seq share (fn names the call in the messages).  nsel = the
+// number of selected proteins (0: nothing to do), sel = the selection, NULL for every protein of the batch.
+int null_check(plaac_ctx* ctx, const char* fn, int64_t nprot, const plaac_null& N, int64_t& nsel, const int32_t*& sel)
+{
     const int64_t K = N.replicates;
-    if (K < 0) return fail(ctx, PLAAC_E_INVALID, "plaac_score_shuffles: replicates %lld is negative", (long long)K);
-    if (N.nsel < -1) return fail(ctx, PLAAC_E_INVALID, "plaac_score_shuffles: nsel %lld is below -1", (long long)N.nsel);
-    if (N.reserved != 0) return fail(ctx, PLAAC_E_INVALID, "plaac_score_shuffles: reserved is %d, not 0", (int)N.reserved);
+    if (K < 0) return fail(ctx, PLAAC_E_INVALID, "%s: replicates %lld is negative", fn, (long long)K);
+    if (N.nsel < -1) return fail(ctx, PLAAC_E_INVALID, "%s: nsel %lld is below -1", fn, (long long)N.nsel);
+    if (N.reserved != 0) return fail(ctx, PLAAC_E_INVALID, "%s: reserved is %d, not 0", fn, (int)N.reserved);
     if (N.columns <= 0 || N.columns >= (PLAAC_NULL_HAS_CORE << 1))
-        return fail(ctx, PLAAC_E_INVALID, "plaac_score_shuffles: columns 0x%x is not a non-empty set of bits 0..13", (unsigned)N.columns);
+        return fail(ctx, PLAAC_E_INVALID, "%s: columns 0x%x is not a non-empty set of bits 0..13", fn, (unsigned)N.columns);
     if (nprot < 0) return fail(ctx, PLAAC_E_INVALID, "negative nprot");
-    if (N.nsel >= 0 && !N.proteins) return fail(ctx, PLAAC_E_INVALID, "plaac_score_shuffles: NULL proteins with nsel = %lld", (long long)N.nsel);
-    const int64_t nsel = N.nsel < 0 ? nprot : N.nsel;
-    if (nsel != 0 && !N.counts) return fail(ctx, PLAAC_E_INVALID, "plaac_score_shuffles: NULL counts with nsel = %lld", (long long)N.nsel);
-    const int32_t* sel = N.nsel < 0 ? nullptr : N.proteins;
+    if (N.nsel >= 0 && !N.proteins) return fail(ctx, PLAAC_E_INVALID, "%s: NULL proteins with nsel = %lld", fn, (long long)N.nsel);
+    nsel = N.nsel < 0 ? nprot : N.nsel;
+    if (nsel != 0 && !N.counts) return fail(ctx, PLAAC_E_INVALID, "%s: NULL counts with nsel = %lld", fn, (long long)N.nsel);
+    sel = N.nsel < 0 ? nullptr : N.proteins;
     for (int64_t j = 0; sel && j < nsel; j++)
         if (sel[j] < 0 || sel[j] >= nprot)
-            return fail(ctx, PLAAC_E_INVALID, "plaac_score_shuffles: selected protein %lld: index %d outside [0, %lld)", (long long)j,
+            return fail(ctx, PLAAC_E_INVALID, "%s: selected protein %lld: index %d outside [0, %lld)", fn, (long long)j,
                         (int)sel[j], (long long)nprot);
     if (nsel == 0) return PLAAC_OK;
-    if (nsel > 0x7fffffffLL) return fail(ctx, PLAAC_E_INVALID, "plaac_score_shuffles: more than 2^31-1 selected proteins");
-    if (K > INT64_MAX / nsel) return fail(ctx, PLAAC_E_INVALID, "plaac_score_shuffles: nsel x replicates overflows");
+    if (nsel > 0x7fffffffLL) return fail(ctx, PLAAC_E_INVALID, "%s: more than 2^31-1 selected proteins", fn);
+    if (K > INT64_MAX / nsel) return fail(ctx, PLAAC_E_INVALID, "%s: nsel x replicates overflows", fn);
+    return PLAAC_OK;
+}
 
-    // The observed records: the selection through the variant input form with no substitution, whose records equal
-    // plaac_score's.  Reference bytes > 21 make it return PLAAC_E_INVALID after writing them; the replicates are then
-    // scored all the same and the error is returned at the end, as plaac_score returns it after the batch.
+// The observed records: the selection through the variant input form with no substitution, whose records equal
+// plaac_score's.  Reference bytes > 21 make it return PLAAC_E_INVALID after writing them (rc_obs, err_obs); the
+// replicates are then scored all the same and the error is returned at the end, as plaac_score returns it after the
+// batch.  Then the tables the tallies read and sum into: the records in ctx->var_wild, nsel x k zero counts in
+// ctx->null_counts.  Every slot's stream starts after this function's synchronisation.
+int null_observed(plaac_ctx* ctx, const uint8_t* codes, const int64_t* offsets, int64_t nprot, int64_t nsel, const int32_t* sel,
+                  int k, plaac_summary* observed, int& rc_obs, std::string& err_obs)
+{
     std::vector<int32_t> all;
     if (!sel) {
         all.resize((size_t)nsel);
@@ -2444,12 +2477,10 @@ try {
     vin.offsets = offsets;
     vin.nref = nprot;
     vin.var = &V;
-    const int rc_obs = score_host(ctx, vin, nsel, obs, nullptr, nullptr);
+    rc_obs = score_host(ctx, vin, nsel, obs, nullptr, nullptr);
     if (rc_obs != PLAAC_OK && rc_obs != PLAAC_E_INVALID) return rc_obs;
-    const std::string err_obs = ctx->err;
+    err_obs = ctx->err;
 
-    // the tables k_shuffle_tally reads and sums into; every slot's stream starts after this synchronisation
-    const int k = __builtin_popcount((uint32_t)N.columns);
     const size_t count_bytes = sizeof(int64_t) * (size_t)nsel * (size_t)k;
     int rc;
     if ((rc = ensure(ctx, ctx->var_wild, sizeof(plaac_summary) * (size_t)nsel))) return rc;
@@ -2458,8 +2489,135 @@ try {
     if ((rc = h2d_any(ctx, ctx->var_wild.p, obs, sizeof(plaac_summary) * (size_t)nsel, st))) return rc;
     CU(ctx, cudaMemsetAsync(ctx->null_counts.p, 0, count_bytes, st));
     CU(ctx, cudaStreamSynchronize(st));
+    return PLAAC_OK;
+}
 
-    rc = PLAAC_OK;
+// The rounds of plaac_score_shuffles_seq (DESIGN.md section 14), after null_observed.  At the end ctx->null_counts holds
+// count and ctx->seq_scored L per (selection index, column).  Round g scores replicates [R_{g-1}, R_g) of the proteins
+// still active, R_0 = 0.  Its span W = R_g - R_{g-1} doubles (W = max(64, 4h) for the first round, R_{g-1} after it),
+// but is at least wmin = ceil(chunk_res / res), res the residues of one replicate of every active protein, so that a round
+// holds at least one chunk bound of work: a round's pipeline pays the latency of its first copy, its last chunk and its
+// longest protein once, whatever its size.  A remainder K - R_g below wmin joins the round.  W is capped at the flag
+// budget of one protein (wcap) and at K.  The hit flags take nact x k x W bits; where that exceeds the budget, the round
+// runs as sub-rounds, each a slice of the same list over the round's whole span.  rc_rep, err_rep: PLAAC_E_INVALID and its message if a round reported reference
+// bytes > 21 (it was scored in full).
+int seq_rounds(plaac_ctx* ctx, const uint8_t* codes, const int64_t* offsets, int64_t nprot, const plaac_null& N, int64_t nsel,
+               const int32_t* sel, int k, int64_t h, int& rc_rep, std::string& err_rep)
+{
+    const int64_t K = N.replicates;
+    Slot& s0 = ctx->slot[0];
+    cudaStream_t st = s0.stream;
+    // flag budget: one bit per residue of a chunk's bound (plaac_set_chunk), so a test can make it small; at least one
+    // word per column, and no round longer than the budget holds for one protein
+    const int64_t budget = std::max<int64_t>(ctx->chunk_res / 32, k);  // words
+    const int64_t wcap = budget / k * 32;
+    int rc;
+    if ((rc = ensure(ctx, ctx->seq_scored, sizeof(int64_t) * (size_t)nsel * (size_t)k))) return rc;
+    if ((rc = ensure(ctx, ctx->seq_live, sizeof(int32_t) * (size_t)nsel))) return rc;
+    if ((rc = ensure(ctx, ctx->seq_pos, sizeof(int64_t) * (size_t)(nsel + 1)))) return rc;
+    for (DevBuf& b : ctx->seq_act)
+        if ((rc = ensure(ctx, b, sizeof(int32_t) * (size_t)(nsel + 1)))) return rc;
+    // the round's list: its length, then selection indices (host act, device seq_act[cur]), and their reference indices
+    std::vector<int32_t> act((size_t)nsel + 1), ref((size_t)nsel);
+    act[0] = (int32_t)nsel;
+    for (int64_t j = 0; j < nsel; j++) act[(size_t)j + 1] = (int32_t)j;
+    if ((rc = h2d_any(ctx, ctx->seq_act[0].p, act.data(), sizeof(int32_t) * (size_t)(nsel + 1), st))) return rc;
+    CU(ctx, cudaMemsetAsync(ctx->seq_scored.p, 0, sizeof(int64_t) * (size_t)nsel * (size_t)k, st));
+    // the flags are zero between rounds (each sub-round clears what it set); a call that failed half-way may have left
+    // some set
+    if (ctx->seq_flags.cap > 0) CU(ctx, cudaMemsetAsync(ctx->seq_flags.p, 0, ctx->seq_flags.cap, st));
+    CU(ctx, cudaStreamSynchronize(st));
+
+    int cur = 0;
+    int64_t nact = nsel, r0 = 0;
+    while (nact > 0 && r0 < K) {
+        int64_t res = 0;
+        for (int64_t a = 0; a < nact; a++) {
+            const int32_t j = act[(size_t)a + 1];
+            ref[(size_t)a] = sel ? sel[j] : j;
+            res += offsets[ref[(size_t)a] + 1] - offsets[ref[(size_t)a]];
+        }
+        const int64_t wmin = (ctx->chunk_res + std::max<int64_t>(res, 1) - 1) / std::max<int64_t>(res, 1);
+        int64_t W = std::min(K - r0, std::max(r0 > 0 ? r0 : h > K / 4 ? K : std::max<int64_t>(64, 4 * h), wmin));
+        if (K - r0 - W < wmin) W = K - r0;
+        W = std::min(W, wcap);
+        const int64_t r1 = r0 + W, wpr = (W + 31) / 32;
+        const int64_t per = std::max<int64_t>(1, budget / (k * wpr));  // entries per sub-round
+        const int32_t* d_act = (const int32_t*)ctx->seq_act[cur].p + 1;
+        int32_t* d_live = (int32_t*)ctx->seq_live.p;
+        CU(ctx, cudaMemsetAsync(d_live, 0, sizeof(int32_t) * (size_t)nact, st));
+        for (int64_t a0 = 0; a0 < nact; a0 += per) {
+            const int64_t n = std::min(per, nact - a0);
+            const size_t fbytes = sizeof(uint32_t) * (size_t)(n * k * wpr);
+            const size_t cap0 = ctx->seq_flags.cap;
+            if ((rc = ensure(ctx, ctx->seq_flags, fbytes))) return rc;
+            if (ctx->seq_flags.cap != cap0) {
+                CU(ctx, cudaMemsetAsync(ctx->seq_flags.p, 0, ctx->seq_flags.cap, st));
+                CU(ctx, cudaStreamSynchronize(st));
+            }
+            const SeqRound sr = {d_act + a0, (uint32_t*)ctx->seq_flags.p, wpr};
+            plaac_null R = N;
+            R.replicates = W;
+            R.nsel = n;
+            R.proteins = ref.data() + a0;
+            R.counts = nullptr;
+            R.values = nullptr;
+            HostInput in;
+            in.codes = codes;
+            in.offsets = offsets;
+            in.nref = nprot;
+            in.nul = &R;
+            in.r0 = r0;
+            in.seq = &sr;
+            rc = score_host(ctx, in, n * W, nullptr, nullptr, nullptr);  // (returns with every slot synchronised)
+            if (rc == PLAAC_E_INVALID && rc_rep == PLAAC_OK) {
+                rc_rep = rc;
+                err_rep = ctx->err;
+            } else if (rc != PLAAC_OK && rc != PLAAC_E_INVALID) {
+                return rc;
+            }
+            k_shuffle_stop<<<(unsigned)((n * k + 7) / 8), 256, 0, st>>>(sr.flags, sr.act, n, k, wpr, h, r0, r1, K,
+                                                                       (int64_t*)ctx->null_counts.p, (int64_t*)ctx->seq_scored.p,
+                                                                       d_live + a0);
+            ctx->stats.kernel_launches += 1;
+            CU(ctx, cudaMemsetAsync(sr.flags, 0, fbytes, st));
+            // (the next sub-round's chunks run on the other slots' streams too)
+            if (a0 + n < nact) CU(ctx, cudaStreamSynchronize(st));
+        }
+        // the next round's list, compacted on the device, comes back with one small copy
+        int64_t* d_pos = (int64_t*)ctx->seq_pos.p;
+        if ((rc = launch_scan(ctx, s0, d_live, d_pos, nact, st))) return rc;
+        k_shuffle_compact<<<(unsigned)((nact + 255) / 256), 256, 0, st>>>(d_live, d_pos, d_act, nact, (int32_t*)ctx->seq_act[cur ^ 1].p);
+        ctx->stats.kernel_launches += 1;
+        CU(ctx, cudaMemcpyAsync(act.data(), ctx->seq_act[cur ^ 1].p, sizeof(int32_t) * (size_t)(nact + 1), cudaMemcpyDeviceToHost, st));
+        CU(ctx, cudaStreamSynchronize(st));
+        nact = act[0];
+        cur ^= 1;
+        r0 = r1;
+    }
+    return PLAAC_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int plaac_score_shuffles(plaac_ctx* ctx, const uint8_t* codes, const int64_t* offsets, int64_t nprot, plaac_null* null_spec,
+                         plaac_summary* observed)
+try {
+    if (!ctx) return fail(nullptr, PLAAC_E_INVALID, "plaac_score_shuffles: NULL ctx");
+    if (!null_spec) return fail(ctx, PLAAC_E_INVALID, "plaac_score_shuffles: NULL null_spec");
+    const plaac_null& N = *null_spec;
+    const int64_t K = N.replicates;
+    int64_t nsel = 0;
+    const int32_t* sel = nullptr;
+    int rc = null_check(ctx, "plaac_score_shuffles", nprot, N, nsel, sel);
+    if (rc != PLAAC_OK || nsel == 0) return rc;
+    const int k = __builtin_popcount((uint32_t)N.columns);
+    int rc_obs = PLAAC_OK;
+    std::string err_obs;
+    if ((rc = null_observed(ctx, codes, offsets, nprot, nsel, sel, k, observed, rc_obs, err_obs))) return rc;
+
     if (K > 0) {
         plaac_null R = N;
         R.nsel = nsel;
@@ -2475,7 +2633,8 @@ try {
     // (bytes > 21: the replicates were scored in full, so the counts are complete)
     const std::string keep = ctx->err;
     int rcc;
-    if ((rcc = d2h_any(ctx, N.counts, ctx->null_counts.p, count_bytes, st))) return rcc;
+    cudaStream_t st = ctx->slot[0].stream;
+    if ((rcc = d2h_any(ctx, N.counts, ctx->null_counts.p, sizeof(int64_t) * (size_t)nsel * (size_t)k, st))) return rcc;
     CU(ctx, cudaStreamSynchronize(st));
     ctx->err = keep;
     if (rc == PLAAC_OK && rc_obs != PLAAC_OK) {
@@ -2485,6 +2644,44 @@ try {
     return rc;
 } catch (...) {
     return api_caught(ctx, "plaac_score_shuffles");
+}
+
+int plaac_score_shuffles_seq(plaac_ctx* ctx, const uint8_t* codes, const int64_t* offsets, int64_t nprot,
+                             const plaac_null* null_spec, int64_t stop_hits, int64_t* scored, plaac_summary* observed)
+try {
+    const char* fn = "plaac_score_shuffles_seq";
+    if (!ctx) return fail(nullptr, PLAAC_E_INVALID, "%s: NULL ctx", fn);
+    if (!null_spec) return fail(ctx, PLAAC_E_INVALID, "%s: NULL null_spec", fn);
+    const plaac_null& N = *null_spec;
+    if (stop_hits < 1) return fail(ctx, PLAAC_E_INVALID, "%s: stop_hits %lld is below 1", fn, (long long)stop_hits);
+    if (N.values) return fail(ctx, PLAAC_E_INVALID, "%s: values must be NULL (the rows have unequal lengths)", fn);
+    int64_t nsel = 0;
+    const int32_t* sel = nullptr;
+    int rc = null_check(ctx, fn, nprot, N, nsel, sel);
+    if (rc != PLAAC_OK) return rc;
+    if (nsel != 0 && !scored) return fail(ctx, PLAAC_E_INVALID, "%s: NULL scored with nsel = %lld", fn, (long long)N.nsel);
+    if (nsel == 0) return PLAAC_OK;
+    const int k = __builtin_popcount((uint32_t)N.columns);
+    int rc_obs = PLAAC_OK;
+    std::string err_obs;
+    if ((rc = null_observed(ctx, codes, offsets, nprot, nsel, sel, k, observed, rc_obs, err_obs))) return rc;
+    int rc_rep = PLAAC_OK;
+    std::string err_rep;
+    if ((rc = seq_rounds(ctx, codes, offsets, nprot, N, nsel, sel, k, stop_hits, rc_rep, err_rep))) return rc;
+    const size_t bytes = sizeof(int64_t) * (size_t)nsel * (size_t)k;
+    cudaStream_t st = ctx->slot[0].stream;
+    if ((rc = d2h_any(ctx, N.counts, ctx->null_counts.p, bytes, st))) return rc;
+    if ((rc = d2h_any(ctx, scored, ctx->seq_scored.p, bytes, st))) return rc;
+    CU(ctx, cudaStreamSynchronize(st));
+    // (bytes > 21: the replicates were scored in full, so counts and scored are complete)
+    if (rc_rep != PLAAC_OK) {
+        ctx->err = err_rep;
+        return rc_rep;
+    }
+    if (rc_obs != PLAAC_OK) ctx->err = err_obs;
+    return rc_obs;
+} catch (...) {
+    return api_caught(ctx, "plaac_score_shuffles_seq");
 }
 
 }  // extern "C"

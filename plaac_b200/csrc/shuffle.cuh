@@ -20,14 +20,15 @@ struct ShuffleRep {
 };
 
 // One thread per replicate t of the chunk: its reference protein i (sel: the chunk's slice sel[j0 ..] of the selection,
-// NULL for every protein of the batch), length and permutation.
+// NULL for every protein of the batch), length and permutation.  q = j * K + (r - r0): a round of
+// plaac_score_shuffles_seq scores replicates [r0, r0 + K); plaac_score_shuffles passes r0 = 0.
 __global__ void __launch_bounds__(256)
-k_shuffle_prep(const int32_t* __restrict__ sel, int64_t j0, int64_t q0, int64_t K, int64_t np,
+k_shuffle_prep(const int32_t* __restrict__ sel, int64_t j0, int64_t q0, int64_t K, int64_t r0, int64_t np,
                const int64_t* __restrict__ ref_off, uint64_t seed, int32_t* __restrict__ len, ShuffleRep* __restrict__ rep)
 {
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= np) return;
-    const int64_t q = q0 + t, j = q / K, r = q - j * K;
+    const int64_t q = q0 + t, j = q / K, r = r0 + q - j * K;
     const int64_t i = sel ? (int64_t)sel[j - j0] : j;
     const int64_t b = ref_off[i], n = ref_off[i + 1] - b;
     len[t] = (int32_t)n;

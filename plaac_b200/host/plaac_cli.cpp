@@ -40,6 +40,12 @@
 //                   default COREscore,LLR,HMMall.  A record's shuffles are those of its index in its batch (--batch-mb),
 //                   so the file depends on --seed and, for inputs beyond one batch, on --batch-mb; the summary table is
 //                   unchanged
+//   --stop-hits H   with --null and --replicates K: the sequential null of Besag and Clifford
+//                   (plaac_score_shuffles_seq).  A record's column stops once H of its shuffles have reached it, after at
+//                   most K shuffles, so a protein far from significance costs about H shuffles instead of K.  The file
+//                   is then SEQid, followed by r<NAME> n<NAME> p<NAME> per column: r the shuffles scored for the column,
+//                   n the ones that reached the record (H if it stopped), p = H/r if it stopped and (1+n)/(1+K)
+//                   otherwise (%.6g); hasCORE gets r and n and no p
 #include <algorithm>
 #include <charconv>
 #include <cmath>
@@ -436,6 +442,8 @@ struct Options {
     uint64_t seed = 0;          // --seed
     std::string null_columns = "COREscore,LLR,HMMall";  // --null-columns, as given
     bool replicates_set = false, seed_set = false, null_columns_set = false;
+    const char* stop_hits_arg = nullptr;  // --stop-hits, as given
+    int64_t stop_hits = 0;                // ... parsed (0: the fixed null)
     int32_t null_mask = 0;      // plaac_null.columns of --null-columns
 };
 
@@ -616,28 +624,39 @@ int score_null_batch(const Options& o, Scorers& S, Batch& B, std::vector<plaac_s
     const int64_t np = B.nprot();
     const int k = __builtin_popcount((unsigned)o.null_mask);
     std::vector<int64_t> counts((size_t)np * (size_t)k);
+    std::vector<int64_t> scored(o.stop_hits > 0 ? counts.size() : 0);
     plaac_null N = {};
     N.replicates = o.replicates;
     N.seed = o.seed;
     N.columns = o.null_mask;
     N.nsel = -1;
     N.counts = counts.data();
-    const int rc = plaac_score_shuffles(S.ctx[0], B.codes.data(), B.offsets.data(), np, &N, sum.data());
-    if (rc != PLAAC_OK) return die(S, rc, "plaac_score_shuffles");
+    if (o.stop_hits > 0) {
+        const int rc = plaac_score_shuffles_seq(S.ctx[0], B.codes.data(), B.offsets.data(), np, &N, o.stop_hits, scored.data(),
+                                                sum.data());
+        if (rc != PLAAC_OK) return die(S, rc, "plaac_score_shuffles_seq");
+    } else {
+        const int rc = plaac_score_shuffles(S.ctx[0], B.codes.data(), B.offsets.data(), np, &N, sum.data());
+        if (rc != PLAAC_OK) return die(S, rc, "plaac_score_shuffles");
+    }
     std::string out;
     char buf[64];
     for (int64_t i = 0; i < np; i++) {
         const plaac_summary& r = sum[(size_t)i];
         if (r.prot_len < 1 || (o.rank_core_only && !(r.core_score == r.core_score))) continue;  // (rows not printed)
         out.append(B.names[(size_t)i]);
-        out.push_back('\t'), put_int(out, (long)o.replicates);
+        if (o.stop_hits == 0) out.push_back('\t'), put_int(out, (long)o.replicates);
         int c = 0;
         for (int b = 0; b <= kEffectCoreChange; b++) {
             if (!((o.null_mask >> b) & 1)) continue;
-            const int64_t n = counts[(size_t)i * (size_t)k + (size_t)c++];
+            const size_t at = (size_t)i * (size_t)k + (size_t)c++;
+            const int64_t n = counts[at];
+            if (o.stop_hits > 0) out.push_back('\t'), put_int(out, (long)scored[at]);
             out.push_back('\t'), put_int(out, (long)n);
             if (b != kEffectCoreChange) {
-                std::snprintf(buf, sizeof(buf), "\t%.6g", (double)(1 + n) / (double)(1 + o.replicates));
+                const double p = o.stop_hits > 0 && n == o.stop_hits ? (double)n / (double)scored[at]
+                                                                      : (double)(1 + n) / (double)(1 + o.replicates);
+                std::snprintf(buf, sizeof(buf), "\t%.6g", p);
                 out += buf;
             }
         }
@@ -1317,6 +1336,10 @@ void usage()
     std::puts("                   SEQid NULLreps and n<NAME> p<NAME> per column: the shuffles that reach the record's score");
     std::puts("                   (NaN lowest) and the empirical p-value (1+n)/(1+K).  COLS as --effects, with hasCORE (the");
     std::puts("                   shuffles with a CORE, no p) in place of COREchange; default COREscore,LLR,HMMall");
+    std::puts("  --stop-hits H    with --null: stop a record's column once H shuffles have reached it (at most K shuffles;");
+    std::puts("                   sequential p-values of Besag and Clifford).  FILE then holds SEQid and r<NAME> n<NAME>");
+    std::puts("                   p<NAME> per column: r shuffles scored, n = H if it stopped, p = H/r if it stopped, else");
+    std::puts("                   (1+n)/(1+K)");
     std::puts("  --compat-F       -F reads the -B file, as plaac.jar does (plaac.java:388); without it -F reads its own file,");
     std::puts("                   so the parameter block and every score differ from the jar's for the same command line");
 }
@@ -1368,6 +1391,8 @@ int main(int argc, char** argv)
             o.seed = std::strtoull(val("--seed"), nullptr, 10), o.seed_set = true;
         else if (a == "--null-columns")
             o.null_columns = val("--null-columns"), o.null_columns_set = true;
+        else if (a == "--stop-hits")
+            o.stop_hits_arg = val("--stop-hits");
         else if (a == "--format-check") {
             // test hook: lines "decimals value" on stdin -> the Java-formatted value on stdout
             int d;
@@ -1436,10 +1461,22 @@ int main(int argc, char** argv)
             return 2;
         }
         if (!(o.null_mask = parse_columns(o.null_columns, "--null-columns", kNullNames))) return 2;
+        if (o.stop_hits_arg) {
+            const char* e = o.stop_hits_arg + std::strlen(o.stop_hits_arg);
+            const auto [end, ec] = std::from_chars(o.stop_hits_arg, e, o.stop_hits);
+            if (ec != std::errc() || end != e || end == o.stop_hits_arg) {
+                std::fprintf(stderr, "plaac: --stop-hits needs an integer H, got '%s'\n", o.stop_hits_arg);
+                return 2;
+            }
+            if (o.stop_hits < 1) {
+                std::fprintf(stderr, "plaac: --stop-hits needs H >= 1, got %lld\n", (long long)o.stop_hits);
+                return 2;
+            }
+        }
         o.host_reader = true;  // the shuffles come with the records of plaac_score_shuffles, not the GPU reader's
-    } else if (o.replicates_set || o.seed_set || o.null_columns_set) {
+    } else if (o.replicates_set || o.seed_set || o.null_columns_set || o.stop_hits_arg) {
         std::fprintf(stderr, "plaac: %s needs --null FILE\n",
-                     o.replicates_set ? "--replicates" : o.seed_set ? "--seed" : "--null-columns");
+                     o.replicates_set ? "--replicates" : o.seed_set ? "--seed" : o.null_columns_set ? "--null-columns" : "--stop-hits");
         return 2;
     }
     const bool variants = o.saturate || !o.variants_file.empty();
@@ -1647,10 +1684,11 @@ int main(int argc, char** argv)
             return 2;
         }
         o.null_out = null_file.get();
-        std::string head = "SEQid\tNULLreps";
+        std::string head = o.stop_hits > 0 ? "SEQid" : "SEQid\tNULLreps";
         for (int b = 0; b <= kEffectCoreChange; b++)
             if ((o.null_mask >> b) & 1)
-                head += std::string("\tn") + kNullNames[b] + (b == kEffectCoreChange ? "" : std::string("\tp") + kNullNames[b]);
+                head += (o.stop_hits > 0 ? std::string("\tr") + kNullNames[b] : std::string()) + "\tn" + kNullNames[b] +
+                        (b == kEffectCoreChange ? "" : std::string("\tp") + kNullNames[b]);
         head += "\n";
         std::fputs(head.c_str(), o.null_out);
     }
