@@ -365,6 +365,25 @@ int plaac_score_multi(plaac_ctx *const *ctxs, int nctx, const uint8_t *codes, co
 int plaac_score_multi_packed(plaac_ctx *const *ctxs, int nctx, const uint32_t *words, const int32_t *lengths, int64_t nprot,
                              int64_t nres, plaac_summary *summaries, const plaac_residue_out *per_res, plaac_hits *hits);
 
+/* Shuffle nulls on nctx contexts (DESIGN.md section 15): the replicate axis is split, not the proteins.  Every ctx
+ * scores every selected protein, ctx k the replicates [floor(K k / nctx), floor(K (k+1) / nctx)) of each (of each
+ * round's span, for the sequential call, whose rounds run in lockstep on all ctxs).  counts, values, scored and
+ * observed are byte-identical to plaac_score_shuffles / plaac_score_shuffles_seq on ctxs[0], for every nctx, whichever
+ * devices the ctxs are on (several may share one) and whatever each ctx's chunk and long-path settings are; so are
+ * they under each ctx's kernel variant, but for the PAPA columns (bits 8..12), whose bytes kernel variant 1 computes in
+ * reference order (plaac_set_kernel_variant).  All ctxs must have been created with the same plaac_params.  nctx == 1
+ * calls the single function.  Every ctx computes the observed records of the whole selection (only ctxs[0] writes them
+ * to `observed`).
+ * Errors: PLAAC_E_INVALID for nctx < 1, a NULL ctxs or a NULL ctxs[k] (text in plaac_last_error(NULL)), and as the
+ * single call, before any device work, with this call's name and the text on ctxs[0].  Reference bytes > 21: everything
+ * is written, then PLAAC_E_INVALID with the text on ctxs[0].  A CUDA error returns the first non-zero code in ctx order,
+ * its text on that ctx.  Every host thread is joined before the call returns. */
+int plaac_score_shuffles_multi(plaac_ctx *const *ctxs, int nctx, const uint8_t *codes, const int64_t *offsets,
+                               int64_t nprot, plaac_null *null_spec, plaac_summary *observed);
+int plaac_score_shuffles_seq_multi(plaac_ctx *const *ctxs, int nctx, const uint8_t *codes, const int64_t *offsets,
+                                   int64_t nprot, const plaac_null *null_spec, int64_t stop_hits, int64_t *scored,
+                                   plaac_summary *observed);
+
 /* ---- GPU FASTA ingest and background counts (SURVEY.md section 8f, rows N2/N3) --------------------------------
  * Replaces fastareader (plaac.java:4302-4375) + string2aa (:1764-1769) + the terminal '*' strip (:758) for a whole
  * file image, and computeaafreq/isvalidprotein (:1655-1739) for the background counts.  Reader semantics are the

@@ -193,6 +193,10 @@ def lib():
         L.plaac_score_shuffles.argtypes = [vp, vp, vp, i64, C.POINTER(Null), vp]
         L.plaac_score_shuffles_seq.restype = C.c_int
         L.plaac_score_shuffles_seq.argtypes = [vp, vp, vp, i64, C.POINTER(Null), i64, vp, vp]
+        L.plaac_score_shuffles_multi.restype = C.c_int
+        L.plaac_score_shuffles_multi.argtypes = [C.POINTER(vp), C.c_int, vp, vp, i64, C.POINTER(Null), vp]
+        L.plaac_score_shuffles_seq_multi.restype = C.c_int
+        L.plaac_score_shuffles_seq_multi.argtypes = [C.POINTER(vp), C.c_int, vp, vp, i64, C.POINTER(Null), i64, vp, vp]
         L.plaac_shuffle_host.restype = C.c_int
         L.plaac_shuffle_host.argtypes = [vp, i64, C.c_uint64, i64, i64, vp]
         L.plaac_bench_synth_lengths.restype = C.c_int
@@ -527,23 +531,9 @@ class Scorer:
         values=True also the replicates' values as an (nsel, K) structured array of f8 fields (has_core: 0 or 1); with
         observed=True also the selected proteins' records (those of score()).  Replicate r of protein i is
         shuffle(codes, offsets, i, r, seed)."""
-        mask, names = _null_mask(columns)
-        codes = np.ascontiguousarray(codes, dtype=np.uint8)
-        offsets = np.ascontiguousarray(offsets, dtype=np.int64)
-        nprot = len(offsets) - 1
-        K = int(replicates)
-        sel = None if proteins is None else np.ascontiguousarray(proteins, dtype=np.int32)
-        nsel = nprot if sel is None else len(sel)
-        counts = np.zeros(nsel, dtype=[(n, "<i8") for n in names])
-        vals = np.zeros((nsel, max(K, 0)), dtype=[(n, "<f8") for n in names]) if values else None
-        obs = np.zeros(nsel, dtype=SUMMARY_DTYPE) if observed else None
-        nl = Null(replicates=K, seed=int(seed) & (2**64 - 1), columns=mask, reserved=0, nsel=-1 if sel is None else nsel,
-                  proteins=sel.ctypes.data if sel is not None else None, counts=counts.ctypes.data,
-                  values=vals.ctypes.data if values else None)
-        self._check(lib().plaac_score_shuffles(self._h, codes.ctypes.data, offsets.ctypes.data, nprot, C.byref(nl),
-                                               obs.ctypes.data if observed else None))
-        ret = [counts] + ([vals] if values else []) + ([obs] if observed else [])
-        return ret[0] if len(ret) == 1 else tuple(ret)
+        a = _NullArgs(codes, offsets, replicates, seed, columns, proteins, observed, values=values)
+        self._check(lib().plaac_score_shuffles(self._h, *a.head(), a.obs_ptr))
+        return a.fixed_result()
 
     def shuffle_null_seq(self, codes: np.ndarray, offsets: np.ndarray, max_replicates: int, stop_hits: int = 10, seed: int = 0,
                          columns=("core_score", "llr", "hmm_all"), proteins=None, observed: bool = False):
@@ -553,25 +543,9 @@ class Scorer:
         column in NULL_COLUMNS order, one row per selected protein; counts is h for a column that stopped and below h
         otherwise, scored is the number of replicates that count covers (K_max if the column did not stop).  With
         observed=True also the selected proteins' records (those of score()).  seq_pvalues turns them into p-values."""
-        mask, names = _null_mask(columns)
-        h, K = int(stop_hits), int(max_replicates)
-        if h < 1:
-            raise ValueError(f"stop_hits must be >= 1, got {h}")
-        if K < 0:
-            raise ValueError(f"max_replicates must be >= 0, got {K}")
-        codes = np.ascontiguousarray(codes, dtype=np.uint8)
-        offsets = np.ascontiguousarray(offsets, dtype=np.int64)
-        nprot = len(offsets) - 1
-        sel = None if proteins is None else np.ascontiguousarray(proteins, dtype=np.int32)
-        nsel = nprot if sel is None else len(sel)
-        counts = np.zeros(nsel, dtype=[(n, "<i8") for n in names])
-        scored = np.zeros(nsel, dtype=counts.dtype)
-        obs = np.zeros(nsel, dtype=SUMMARY_DTYPE) if observed else None
-        nl = Null(replicates=K, seed=int(seed) & (2**64 - 1), columns=mask, reserved=0, nsel=-1 if sel is None else nsel,
-                  proteins=sel.ctypes.data if sel is not None else None, counts=counts.ctypes.data, values=None)
-        self._check(lib().plaac_score_shuffles_seq(self._h, codes.ctypes.data, offsets.ctypes.data, nprot, C.byref(nl), h,
-                                                   scored.ctypes.data, obs.ctypes.data if observed else None))
-        return (counts, scored, obs) if observed else (counts, scored)
+        a = _NullArgs(codes, offsets, max_replicates, seed, columns, proteins, observed, stop_hits=stop_hits)
+        self._check(lib().plaac_score_shuffles_seq(self._h, *a.head(), a.h, a.scored.ctypes.data, a.obs_ptr))
+        return a.seq_result()
 
     def score_ptr(self, codes_ptr: int, offsets_ptr: int, nprot: int, summaries_ptr: int):
         """Raw host pointers (e.g. pinned torch tensors)."""
@@ -722,6 +696,45 @@ def _null_mask(columns):
     return mask, [n for k, n in enumerate(NULL_COLUMNS) if mask >> k & 1]
 
 
+class _NullArgs:
+    """The argument handling Scorer's and MultiScorer's shuffle nulls share: the checks (ValueError before any call),
+    the Null spec and the output arrays."""
+
+    def __init__(self, codes, offsets, replicates, seed, columns, proteins, observed, values=False, stop_hits=None):
+        mask, names = _null_mask(columns)
+        K = int(replicates)
+        if stop_hits is not None:
+            self.h = int(stop_hits)
+            if self.h < 1:
+                raise ValueError(f"stop_hits must be >= 1, got {self.h}")
+            if K < 0:
+                raise ValueError(f"max_replicates must be >= 0, got {K}")
+        self.codes = np.ascontiguousarray(codes, dtype=np.uint8)
+        self.offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+        self.nprot = len(self.offsets) - 1
+        self.sel = None if proteins is None else np.ascontiguousarray(proteins, dtype=np.int32)
+        nsel = self.nprot if self.sel is None else len(self.sel)
+        self.counts = np.zeros(nsel, dtype=[(n, "<i8") for n in names])
+        self.scored = np.zeros(nsel, dtype=self.counts.dtype) if stop_hits is not None else None
+        self.vals = np.zeros((nsel, max(K, 0)), dtype=[(n, "<f8") for n in names]) if values else None
+        self.obs = np.zeros(nsel, dtype=SUMMARY_DTYPE) if observed else None
+        self.obs_ptr = self.obs.ctypes.data if observed else None
+        self.null = Null(replicates=K, seed=int(seed) & (2**64 - 1), columns=mask, reserved=0,
+                         nsel=-1 if self.sel is None else nsel, proteins=self.sel.ctypes.data if self.sel is not None else None,
+                         counts=self.counts.ctypes.data, values=self.vals.ctypes.data if values else None)
+
+    def head(self):
+        """The arguments after the ctx(s): codes, offsets, nprot, null_spec."""
+        return self.codes.ctypes.data, self.offsets.ctypes.data, self.nprot, C.byref(self.null)
+
+    def fixed_result(self):
+        ret = [self.counts] + ([self.vals] if self.vals is not None else []) + ([self.obs] if self.obs is not None else [])
+        return ret[0] if len(ret) == 1 else tuple(ret)
+
+    def seq_result(self):
+        return (self.counts, self.scored, self.obs) if self.obs is not None else (self.counts, self.scored)
+
+
 def seq_pvalues(counts: np.ndarray, scored: np.ndarray, stop_hits: int, max_replicates: int) -> np.ndarray:
     """The p-values of Scorer.shuffle_null_seq's (counts, scored): h / L where a column stopped (count == h), else
     (count + 1) / (K_max + 1).  One float64 field per double column; has_core is left out, as the CLI leaves out its p."""
@@ -777,7 +790,8 @@ def shard_plan(offsets: np.ndarray, nshards: int) -> np.ndarray:
 
 
 class MultiScorer:
-    """One ctx per GPU of this box, driven from one process through plaac_score_multi (one host thread per GPU)."""
+    """One ctx per GPU of this box, driven from one process through plaac_score_multi and the multi-GPU shuffle nulls
+    (one host thread per GPU)."""
 
     def __init__(self, params: Params | None = None, devices=None):
         n = lib().plaac_device_count()
@@ -792,6 +806,15 @@ class MultiScorer:
             s.close()
         self.scorers = []
 
+    def _handles(self):
+        return (C.c_void_p * len(self.scorers))(*[s._h for s in self.scorers]), len(self.scorers)
+
+    def _check(self, rc):
+        """An error's text from every scorer (the call puts it on the ctx it happened on), else the global one."""
+        if rc != 0:
+            msgs = [lib().plaac_last_error(s._h).decode() for s in self.scorers]
+            raise PlaacError(rc, "; ".join(m for m in msgs if m) or lib().plaac_last_error(None).decode())
+
     def score(self, codes: np.ndarray, offsets: np.ndarray, per_residue: bool = False):
         codes = np.ascontiguousarray(codes, dtype=np.uint8)
         offsets = np.ascontiguousarray(offsets, dtype=np.int64)
@@ -803,12 +826,8 @@ class MultiScorer:
             res = {n: np.zeros(ntot, dtype=np.uint8) for n in RESIDUE_U8}
             res.update({n: np.zeros(ntot, dtype=np.float64) for n in RESIDUE_F64})
             ro = C.byref(ResidueOut(**{n: a.ctypes.data for n, a in res.items()}))
-        handles = (C.c_void_p * len(self.scorers))(*[s._h for s in self.scorers])
-        rc = lib().plaac_score_multi(handles, len(self.scorers), codes.ctypes.data, offsets.ctypes.data, nprot,
-                                     out.ctypes.data, ro)
-        if rc != 0:
-            msgs = [lib().plaac_last_error(s._h).decode() for s in self.scorers]
-            raise PlaacError(rc, "; ".join(m for m in msgs if m) or lib().plaac_last_error(None).decode())
+        self._check(lib().plaac_score_multi(*self._handles(), codes.ctypes.data, offsets.ctypes.data, nprot,
+                                            out.ctypes.data, ro))
         return (out, res) if per_residue else out
 
     def score_packed(self, words: np.ndarray, lengths: np.ndarray, per_residue: bool = False, hits: str | None = None,
@@ -827,15 +846,27 @@ class MultiScorer:
         h = rec = idx = None
         if hits is not None:
             h, rec, idx = self.scorers[0]._hits(HITS_CORE if hits == "core" else HITS_TOPK, nprot if capacity is None else capacity)
-        handles = (C.c_void_p * len(self.scorers))(*[s._h for s in self.scorers])
-        rc = lib().plaac_score_multi_packed(handles, len(self.scorers), words.ctypes.data, lengths.ctypes.data, nprot, nres,
-                                            out.ctypes.data, ro, C.byref(h) if h is not None else None)
-        if rc != 0:
-            msgs = [lib().plaac_last_error(s._h).decode() for s in self.scorers]
-            raise PlaacError(rc, "; ".join(m for m in msgs if m) or lib().plaac_last_error(None).decode())
+        self._check(lib().plaac_score_multi_packed(*self._handles(), words.ctypes.data, lengths.ctypes.data, nprot, nres,
+                                                   out.ctypes.data, ro, C.byref(h) if h is not None else None))
         ret = [out]
         if per_residue:
             ret.append(res)
         if h is not None:
             ret.append({"records": rec[:h.count], "index": idx[:h.count], "n_core": int(h.n_core)})
         return ret[0] if len(ret) == 1 else tuple(ret)
+
+    def shuffle_null(self, codes: np.ndarray, offsets: np.ndarray, replicates: int, seed: int = 0,
+                     columns=("core_score", "llr", "hmm_all"), proteins=None, values: bool = False, observed: bool = False):
+        """plaac_score_shuffles_multi: Scorer.shuffle_null on every GPU, each scoring a range of every protein's
+        replicates.  Same arguments, same results, byte for byte."""
+        a = _NullArgs(codes, offsets, replicates, seed, columns, proteins, observed, values=values)
+        self._check(lib().plaac_score_shuffles_multi(*self._handles(), *a.head(), a.obs_ptr))
+        return a.fixed_result()
+
+    def shuffle_null_seq(self, codes: np.ndarray, offsets: np.ndarray, max_replicates: int, stop_hits: int = 10, seed: int = 0,
+                         columns=("core_score", "llr", "hmm_all"), proteins=None, observed: bool = False):
+        """plaac_score_shuffles_seq_multi: Scorer.shuffle_null_seq with every round's replicates split over the GPUs.
+        Same arguments, same results, byte for byte."""
+        a = _NullArgs(codes, offsets, max_replicates, seed, columns, proteins, observed, stop_hits=stop_hits)
+        self._check(lib().plaac_score_shuffles_seq_multi(*self._handles(), *a.head(), a.h, a.scored.ctypes.data, a.obs_ptr))
+        return a.seq_result()

@@ -9,6 +9,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <memory>
+#include <mutex>
 #include <new>
 #include <numeric>
 #include <string>
@@ -2449,6 +2450,20 @@ int null_check(plaac_ctx* ctx, const char* fn, int64_t nprot, const plaac_null& 
     return PLAAC_OK;
 }
 
+// The checks of plaac_score_shuffles_seq and its multi-GPU form: null_check and the sequential call's own.
+int seq_check(plaac_ctx* ctx, const char* fn, int64_t nprot, const plaac_null* null_spec, int64_t stop_hits,
+              const int64_t* scored, int64_t& nsel, const int32_t*& sel)
+{
+    if (!null_spec) return fail(ctx, PLAAC_E_INVALID, "%s: NULL null_spec", fn);
+    const plaac_null& N = *null_spec;
+    if (stop_hits < 1) return fail(ctx, PLAAC_E_INVALID, "%s: stop_hits %lld is below 1", fn, (long long)stop_hits);
+    if (N.values) return fail(ctx, PLAAC_E_INVALID, "%s: values must be NULL (the rows have unequal lengths)", fn);
+    int rc = null_check(ctx, fn, nprot, N, nsel, sel);
+    if (rc != PLAAC_OK) return rc;
+    if (nsel != 0 && !scored) return fail(ctx, PLAAC_E_INVALID, "%s: NULL scored with nsel = %lld", fn, (long long)N.nsel);
+    return PLAAC_OK;
+}
+
 // The observed records: the selection through the variant input form with no substitution, whose records equal
 // plaac_score's.  Reference bytes > 21 make it return PLAAC_E_INVALID after writing them (rc_obs, err_obs); the
 // replicates are then scored all the same and the error is returned at the end, as plaac_score returns it after the
@@ -2492,24 +2507,38 @@ int null_observed(plaac_ctx* ctx, const uint8_t* codes, const int64_t* offsets, 
     return PLAAC_OK;
 }
 
+// The flag budget of a sequential null on ctx, in words: one bit per residue of a chunk's bound (plaac_set_chunk), so a
+// test can make it small, and at least one word per column.
+int64_t seq_budget(const plaac_ctx* ctx, int k) { return std::max<int64_t>(ctx->chunk_res / 32, k); }
+
+// The span W = R_g - R_{g-1} of the round of a sequential null that starts at r0 = R_{g-1} (DESIGN.md sections 14 and
+// 15).  W doubles (max(64, 4h) for the first round, or all of K when h > K / 4; r0 after it), but is at least wmin, so
+// that a round holds at least one chunk bound of work on each GPU: a round's pipeline pays the latency of its first copy,
+// its last chunk and its longest protein once, whatever its size.  A remainder K - R_g below wmin joins the round.  W is
+// capped at the flag budget of one protein (wcap) and at K.
+int64_t seq_span(int64_t K, int64_t r0, int64_t h, int64_t wmin, int64_t wcap)
+{
+    int64_t W = std::min(K - r0, std::max(r0 > 0 ? r0 : h > K / 4 ? K : std::max<int64_t>(64, 4 * h), wmin));
+    if (K - r0 - W < wmin) W = K - r0;
+    return std::min(W, wcap);
+}
+
+// ceil(chunk_res / res), res the residues of one replicate of every active protein
+int64_t seq_wmin(int64_t chunk_res, int64_t res) { return (chunk_res + std::max<int64_t>(res, 1) - 1) / std::max<int64_t>(res, 1); }
+
 // The rounds of plaac_score_shuffles_seq (DESIGN.md section 14), after null_observed.  At the end ctx->null_counts holds
 // count and ctx->seq_scored L per (selection index, column).  Round g scores replicates [R_{g-1}, R_g) of the proteins
-// still active, R_0 = 0.  Its span W = R_g - R_{g-1} doubles (W = max(64, 4h) for the first round, R_{g-1} after it),
-// but is at least wmin = ceil(chunk_res / res), res the residues of one replicate of every active protein, so that a round
-// holds at least one chunk bound of work: a round's pipeline pays the latency of its first copy, its last chunk and its
-// longest protein once, whatever its size.  A remainder K - R_g below wmin joins the round.  W is capped at the flag
-// budget of one protein (wcap) and at K.  The hit flags take nact x k x W bits; where that exceeds the budget, the round
-// runs as sub-rounds, each a slice of the same list over the round's whole span.  rc_rep, err_rep: PLAAC_E_INVALID and its message if a round reported reference
-// bytes > 21 (it was scored in full).
+// still active, R_0 = 0, its span from seq_span with wmin = seq_wmin(chunk_res, res).  The hit flags take nact x k x W
+// bits; where that exceeds the budget, the round runs as sub-rounds, each a slice of the same list over the round's whole
+// span.  rc_rep, err_rep: PLAAC_E_INVALID and its message if a round reported reference bytes > 21 (it was scored in
+// full).
 int seq_rounds(plaac_ctx* ctx, const uint8_t* codes, const int64_t* offsets, int64_t nprot, const plaac_null& N, int64_t nsel,
                const int32_t* sel, int k, int64_t h, int& rc_rep, std::string& err_rep)
 {
     const int64_t K = N.replicates;
     Slot& s0 = ctx->slot[0];
     cudaStream_t st = s0.stream;
-    // flag budget: one bit per residue of a chunk's bound (plaac_set_chunk), so a test can make it small; at least one
-    // word per column, and no round longer than the budget holds for one protein
-    const int64_t budget = std::max<int64_t>(ctx->chunk_res / 32, k);  // words
+    const int64_t budget = seq_budget(ctx, k);
     const int64_t wcap = budget / k * 32;
     int rc;
     if ((rc = ensure(ctx, ctx->seq_scored, sizeof(int64_t) * (size_t)nsel * (size_t)k))) return rc;
@@ -2537,10 +2566,7 @@ int seq_rounds(plaac_ctx* ctx, const uint8_t* codes, const int64_t* offsets, int
             ref[(size_t)a] = sel ? sel[j] : j;
             res += offsets[ref[(size_t)a] + 1] - offsets[ref[(size_t)a]];
         }
-        const int64_t wmin = (ctx->chunk_res + std::max<int64_t>(res, 1) - 1) / std::max<int64_t>(res, 1);
-        int64_t W = std::min(K - r0, std::max(r0 > 0 ? r0 : h > K / 4 ? K : std::max<int64_t>(64, 4 * h), wmin));
-        if (K - r0 - W < wmin) W = K - r0;
-        W = std::min(W, wcap);
+        const int64_t W = seq_span(K, r0, h, seq_wmin(ctx->chunk_res, res), wcap);
         const int64_t r1 = r0 + W, wpr = (W + 31) / 32;
         const int64_t per = std::max<int64_t>(1, budget / (k * wpr));  // entries per sub-round
         const int32_t* d_act = (const int32_t*)ctx->seq_act[cur].p + 1;
@@ -2651,16 +2677,11 @@ int plaac_score_shuffles_seq(plaac_ctx* ctx, const uint8_t* codes, const int64_t
 try {
     const char* fn = "plaac_score_shuffles_seq";
     if (!ctx) return fail(nullptr, PLAAC_E_INVALID, "%s: NULL ctx", fn);
-    if (!null_spec) return fail(ctx, PLAAC_E_INVALID, "%s: NULL null_spec", fn);
-    const plaac_null& N = *null_spec;
-    if (stop_hits < 1) return fail(ctx, PLAAC_E_INVALID, "%s: stop_hits %lld is below 1", fn, (long long)stop_hits);
-    if (N.values) return fail(ctx, PLAAC_E_INVALID, "%s: values must be NULL (the rows have unequal lengths)", fn);
     int64_t nsel = 0;
     const int32_t* sel = nullptr;
-    int rc = null_check(ctx, fn, nprot, N, nsel, sel);
-    if (rc != PLAAC_OK) return rc;
-    if (nsel != 0 && !scored) return fail(ctx, PLAAC_E_INVALID, "%s: NULL scored with nsel = %lld", fn, (long long)N.nsel);
-    if (nsel == 0) return PLAAC_OK;
+    int rc = seq_check(ctx, fn, nprot, null_spec, stop_hits, scored, nsel, sel);
+    if (rc != PLAAC_OK || nsel == 0) return rc;
+    const plaac_null& N = *null_spec;
     const int k = __builtin_popcount((uint32_t)N.columns);
     int rc_obs = PLAAC_OK;
     std::string err_obs;
@@ -2948,6 +2969,336 @@ try {
     return rc_shards;
 } catch (...) {
     return api_caught((ctxs && nctx > 0 ? ctxs[0] : nullptr), "plaac_score_multi_packed");
+}
+
+}  // extern "C"
+
+// The shuffle nulls on several ctxs (DESIGN.md section 15): every ctx scores every selected protein, each a range of
+// its replicates.
+namespace {
+
+// Start of ctx c's part of a span of W replicates cut into n parts: floor(W c / n).
+int64_t part_start(int64_t W, int c, int n) { return (int64_t)((__int128)W * c / n); }
+
+// One phase of a multi-ctx call: rcs[c] = f(c) for every ctx c, one host thread each (the calling thread where no thread
+// is to be had), all joined before it returns.  Returns the first non-zero code in ctx order.
+template <class F>
+int on_each_ctx(plaac_ctx* const* ctxs, int nctx, const char* fn, F f)
+{
+    std::vector<int> rcs((size_t)nctx, PLAAC_OK);
+    std::vector<std::thread> threads;
+    for (int c = 0; c < nctx; c++) {
+        auto run = [&, c]() {
+            try {
+                rcs[(size_t)c] = f(c);
+            } catch (...) {
+                rcs[(size_t)c] = api_caught(ctxs[c], fn);
+            }
+        };
+        try {
+            threads.emplace_back(run);
+        } catch (...) {
+            run();
+        }
+    }
+    for (auto& t : threads) t.join();
+    for (int c = 0; c < nctx; c++)
+        if (rcs[(size_t)c] != PLAAC_OK) return rcs[(size_t)c];
+    return PLAAC_OK;
+}
+
+// Reference bytes > 21 seen by any ctx (its observed records or its replicates were scored in full all the same): the
+// call returns PLAAC_E_INVALID at the end, with the text on ctxs[0], as the single call returns it.
+struct BadBytes {
+    std::mutex m;
+    int rc = PLAAC_OK;
+    std::string err;
+    void note(int r, const std::string& e)
+    {
+        if (r != PLAAC_E_INVALID) return;
+        std::lock_guard<std::mutex> g(m);
+        rc = r;
+        err = e;
+    }
+    int finish(plaac_ctx* c0)
+    {
+        if (rc != PLAAC_OK) c0->err = err;
+        return rc;
+    }
+};
+
+// Every ctx: null_observed over the whole selection (only ctxs[0] writes to the caller's observed).  Ctxs c >= 1 for
+// which skip(c) holds score nothing and need no reference.
+template <class Skip>
+int multi_observed(plaac_ctx* const* ctxs, int nctx, const char* fn, const uint8_t* codes, const int64_t* offsets, int64_t nprot,
+                   int64_t nsel, const int32_t* sel, int k, plaac_summary* observed, BadBytes& bad, Skip skip)
+{
+    return on_each_ctx(ctxs, nctx, fn, [&](int c) -> int {
+        if (c > 0 && skip(c)) return PLAAC_OK;
+        int rc_obs = PLAAC_OK;
+        std::string err_obs;
+        const int rc = null_observed(ctxs[c], codes, offsets, nprot, nsel, sel, k, c == 0 ? observed : nullptr, rc_obs, err_obs);
+        bad.note(rc_obs, err_obs);
+        return rc;
+    });
+}
+
+}  // namespace
+
+extern "C" {
+
+int plaac_score_shuffles_multi(plaac_ctx* const* ctxs, int nctx, const uint8_t* codes, const int64_t* offsets, int64_t nprot,
+                               plaac_null* null_spec, plaac_summary* observed)
+try {
+    const char* fn = "plaac_score_shuffles_multi";
+    if (!ctxs || nctx < 1) return fail(nullptr, PLAAC_E_INVALID, "%s: no contexts", fn);
+    for (int c = 0; c < nctx; c++)
+        if (!ctxs[c]) return fail(nullptr, PLAAC_E_INVALID, "%s: NULL ctx %d", fn, c);
+    if (nctx == 1) return plaac_score_shuffles(ctxs[0], codes, offsets, nprot, null_spec, observed);
+    plaac_ctx* c0 = ctxs[0];
+    if (!null_spec) return fail(c0, PLAAC_E_INVALID, "%s: NULL null_spec", fn);
+    const plaac_null& N = *null_spec;
+    const int64_t K = N.replicates;
+    int64_t nsel = 0;
+    const int32_t* sel = nullptr;
+    int rc = null_check(c0, fn, nprot, N, nsel, sel);
+    if (rc != PLAAC_OK || nsel == 0) return rc;
+    const int k = __builtin_popcount((uint32_t)N.columns);
+    const size_t ek = (size_t)k;
+    BadBytes bad;
+    auto r0 = [&](int c) { return part_start(K, c, nctx); };
+    if ((rc = multi_observed(ctxs, nctx, fn, codes, offsets, nprot, nsel, sel, k, observed, bad,
+                             [&](int c) { return r0(c + 1) == r0(c); })))
+        return rc;
+    // ctx c: replicates [r0(c), r0(c + 1)) of every selected protein, its counts and rows into host arrays of its own
+    std::vector<std::vector<int64_t>> counts((size_t)nctx);
+    rc = on_each_ctx(ctxs, nctx, fn, [&](int c) -> int {
+        plaac_ctx* ctx = ctxs[c];
+        const int64_t a = r0(c), W = r0(c + 1) - a;
+        if (W == 0) return PLAAC_OK;
+        std::vector<double> vals(N.values ? (size_t)nsel * (size_t)W * ek : 0);
+        plaac_null R = N;
+        R.replicates = W;
+        R.nsel = nsel;
+        R.proteins = sel;
+        R.values = N.values ? vals.data() : nullptr;
+        HostInput in;
+        in.codes = codes;
+        in.offsets = offsets;
+        in.nref = nprot;
+        in.nul = &R;
+        in.r0 = a;
+        int rc = score_host(ctx, in, nsel * W, nullptr, nullptr, nullptr);
+        if (rc != PLAAC_OK && rc != PLAAC_E_INVALID) return rc;
+        bad.note(rc, ctx->err);
+        std::vector<int64_t>& cnt = counts[(size_t)c];
+        cnt.resize((size_t)nsel * ek);
+        cudaStream_t st = ctx->slot[0].stream;
+        if ((rc = d2h_any(ctx, cnt.data(), ctx->null_counts.p, sizeof(int64_t) * cnt.size(), st))) return rc;
+        CU(ctx, cudaStreamSynchronize(st));
+        if (N.values)  // each protein's run of rows: j * K + a in the caller's array
+            for (int64_t j = 0; j < nsel; j++)
+                memcpy(N.values + ((size_t)j * (size_t)K + (size_t)a) * ek, vals.data() + (size_t)j * (size_t)W * ek,
+                       sizeof(double) * (size_t)W * ek);
+        return PLAAC_OK;
+    });
+    if (rc) return rc;
+    for (size_t i = 0; i < (size_t)nsel * ek; i++) {
+        int64_t sum = 0;
+        for (const auto& cnt : counts)
+            if (!cnt.empty()) sum += cnt[i];
+        N.counts[i] = sum;
+    }
+    return bad.finish(c0);
+} catch (...) {
+    return api_caught((ctxs && nctx > 0 ? ctxs[0] : nullptr), "plaac_score_shuffles_multi");
+}
+
+// The rounds of plaac_score_shuffles_seq in lockstep on every ctx (DESIGN.md section 15).  Round g's span [R_{g-1}, R_g)
+// is cut into one part per ctx; per slice of the active list (a sub-round, global over the ctxs): every ctx scores its
+// part into hit flags relative to the part's start and counts each row's hits there (k_shuffle_stop with h above any
+// count, over a zeroed table); the host walks each row's parts in ctx order from its count so far to the part where it
+// reaches h; the ctxs holding such rows find their replicates (k_shuffle_stop with the base counts, h for the other rows,
+// which it skips) and every ctx clears its flags.  count, L and the list live on the host.
+int plaac_score_shuffles_seq_multi(plaac_ctx* const* ctxs, int nctx, const uint8_t* codes, const int64_t* offsets, int64_t nprot,
+                                   const plaac_null* null_spec, int64_t stop_hits, int64_t* scored, plaac_summary* observed)
+try {
+    const char* fn = "plaac_score_shuffles_seq_multi";
+    if (!ctxs || nctx < 1) return fail(nullptr, PLAAC_E_INVALID, "%s: no contexts", fn);
+    for (int c = 0; c < nctx; c++)
+        if (!ctxs[c]) return fail(nullptr, PLAAC_E_INVALID, "%s: NULL ctx %d", fn, c);
+    if (nctx == 1) return plaac_score_shuffles_seq(ctxs[0], codes, offsets, nprot, null_spec, stop_hits, scored, observed);
+    plaac_ctx* c0 = ctxs[0];
+    int64_t nsel = 0;
+    const int32_t* sel = nullptr;
+    int rc = seq_check(c0, fn, nprot, null_spec, stop_hits, scored, nsel, sel);
+    if (rc != PLAAC_OK || nsel == 0) return rc;
+    const plaac_null& N = *null_spec;
+    const int64_t K = N.replicates, h = stop_hits;
+    const int k = __builtin_popcount((uint32_t)N.columns);
+    const size_t ek = (size_t)k;
+    BadBytes bad;
+    if ((rc = multi_observed(ctxs, nctx, fn, codes, offsets, nprot, nsel, sel, k, observed, bad, [](int) { return false; })))
+        return rc;
+    // per ctx: seq_act[0] = the round's list, seq_act[1] = 0, 1, 2, ... (the rows of a slice: k_shuffle_stop then counts
+    // and stops in tables of the slice's rows), null_counts = those tables, seq_scored and seq_live its other outputs
+    std::vector<int32_t> iota((size_t)nsel);
+    for (int64_t j = 0; j < nsel; j++) iota[(size_t)j] = (int32_t)j;
+    rc = on_each_ctx(ctxs, nctx, fn, [&](int c) -> int {
+        plaac_ctx* ctx = ctxs[c];
+        cudaStream_t st = ctx->slot[0].stream;
+        int rc;
+        CU(ctx, cudaSetDevice(ctx->device));
+        if ((rc = ensure(ctx, ctx->seq_scored, sizeof(int64_t) * (size_t)nsel * ek))) return rc;
+        if ((rc = ensure(ctx, ctx->seq_live, sizeof(int32_t) * (size_t)nsel))) return rc;
+        for (DevBuf& b : ctx->seq_act)
+            if ((rc = ensure(ctx, b, sizeof(int32_t) * (size_t)(nsel + 1)))) return rc;
+        if ((rc = h2d_any(ctx, ctx->seq_act[1].p, iota.data(), sizeof(int32_t) * (size_t)nsel, st))) return rc;
+        // (a call that failed half-way may have left flags set)
+        if (ctx->seq_flags.cap > 0) CU(ctx, cudaMemsetAsync(ctx->seq_flags.p, 0, ctx->seq_flags.cap, st));
+        CU(ctx, cudaStreamSynchronize(st));
+        return PLAAC_OK;
+    });
+    if (rc) return rc;
+
+    // the schedule of section 14 with each part holding at least its ctx's chunk bound, and the tightest flag budget
+    int64_t budget = INT64_MAX, chunk_res = 0;
+    for (int c = 0; c < nctx; c++) {
+        budget = std::min(budget, seq_budget(ctxs[c], k));
+        chunk_res = std::max(chunk_res, ctxs[c]->chunk_res);
+    }
+    const int64_t wcap = budget / k * 32;
+    std::vector<int64_t> count((size_t)nsel * ek, 0), L((size_t)nsel * ek, 0);
+    std::vector<int32_t> act((size_t)nsel), ref((size_t)nsel), live((size_t)nsel);
+    for (int64_t j = 0; j < nsel; j++) act[(size_t)j] = (int32_t)j;
+    std::vector<int64_t> pa((size_t)nctx + 1);
+    // per ctx, a row per (entry of the slice, column): its hits in the ctx's part, the base counts of step 3 and the L
+    // it found
+    std::vector<std::vector<int64_t>> hits((size_t)nctx), tab((size_t)nctx), at((size_t)nctx);
+    std::vector<char> stops((size_t)nctx);
+    int64_t nact = nsel, r0 = 0;
+    while (nact > 0 && r0 < K) {
+        int64_t res = 0;
+        for (int64_t a = 0; a < nact; a++) {
+            const int32_t j = act[(size_t)a];
+            ref[(size_t)a] = sel ? sel[j] : j;
+            res += offsets[ref[(size_t)a] + 1] - offsets[ref[(size_t)a]];
+        }
+        const int64_t W = seq_span(K, r0, h, nctx * seq_wmin(chunk_res, res), wcap), r1 = r0 + W;
+        int64_t wpr_max = 0;
+        for (int c = 0; c <= nctx; c++) pa[(size_t)c] = r0 + part_start(W, c, nctx);
+        for (int c = 0; c < nctx; c++) wpr_max = std::max(wpr_max, (pa[(size_t)c + 1] - pa[(size_t)c] + 31) / 32);
+        const int64_t per = std::max<int64_t>(1, budget / (k * wpr_max));  // entries per sub-round
+        std::fill(live.begin(), live.begin() + nact, 0);
+        for (int64_t a0 = 0; a0 < nact; a0 += per) {
+            const int64_t n = std::min(per, nact - a0), rows = n * k;
+            // 1. every ctx scores its part of the slice and counts each row's hits there
+            rc = on_each_ctx(ctxs, nctx, fn, [&](int c) -> int {
+                plaac_ctx* ctx = ctxs[c];
+                const int64_t p0 = pa[(size_t)c], p1 = pa[(size_t)c + 1], wpr = (p1 - p0 + 31) / 32;
+                hits[(size_t)c].assign((size_t)rows, 0);
+                if (p1 == p0) return PLAAC_OK;
+                cudaStream_t st = ctx->slot[0].stream;
+                int rc;
+                CU(ctx, cudaSetDevice(ctx->device));
+                if (a0 == 0) CU(ctx, cudaMemcpyAsync(ctx->seq_act[0].p, act.data(), sizeof(int32_t) * (size_t)nact, cudaMemcpyHostToDevice, st));
+                const size_t cap0 = ctx->seq_flags.cap;
+                if ((rc = ensure(ctx, ctx->seq_flags, sizeof(uint32_t) * (size_t)(rows * wpr)))) return rc;
+                if (ctx->seq_flags.cap != cap0) CU(ctx, cudaMemsetAsync(ctx->seq_flags.p, 0, ctx->seq_flags.cap, st));
+                CU(ctx, cudaStreamSynchronize(st));  // (the chunks run on the other slots' streams too)
+                const SeqRound sr = {(const int32_t*)ctx->seq_act[0].p + a0, (uint32_t*)ctx->seq_flags.p, wpr};
+                plaac_null R = N;
+                R.replicates = p1 - p0;
+                R.nsel = n;
+                R.proteins = ref.data() + a0;
+                R.counts = nullptr;
+                R.values = nullptr;
+                HostInput in;
+                in.codes = codes;
+                in.offsets = offsets;
+                in.nref = nprot;
+                in.nul = &R;
+                in.r0 = p0;
+                in.seq = &sr;
+                rc = score_host(ctx, in, n * (p1 - p0), nullptr, nullptr, nullptr);  // (returns with every slot synchronised)
+                if (rc != PLAAC_OK && rc != PLAAC_E_INVALID) return rc;
+                bad.note(rc, ctx->err);
+                int64_t* d_tab = (int64_t*)ctx->null_counts.p;
+                CU(ctx, cudaMemsetAsync(d_tab, 0, sizeof(int64_t) * (size_t)rows, st));
+                k_shuffle_stop<<<(unsigned)((rows + 7) / 8), 256, 0, st>>>(sr.flags, (const int32_t*)ctx->seq_act[1].p, n, k, wpr,
+                                                                           INT64_MAX, p0, p1, K, d_tab, (int64_t*)ctx->seq_scored.p,
+                                                                           (int32_t*)ctx->seq_live.p);
+                ctx->stats.kernel_launches += 1;
+                CU(ctx, cudaMemcpyAsync(hits[(size_t)c].data(), d_tab, sizeof(int64_t) * (size_t)rows, cudaMemcpyDeviceToHost, st));
+                CU(ctx, cudaStreamSynchronize(st));
+                return PLAAC_OK;
+            });
+            if (rc) return rc;
+            // 2. each row's parts in ctx order, from its count so far
+            std::fill(stops.begin(), stops.end(), 0);
+            for (int c = 0; c < nctx; c++) tab[(size_t)c].assign((size_t)rows, h);
+            for (int64_t row = 0; row < rows; row++) {
+                const int64_t a = a0 + row / k, s = (int64_t)act[(size_t)a] * k + row % k;
+                int64_t n_hit = count[(size_t)s];
+                if (n_hit >= h) continue;  // stopped in an earlier round
+                int c = 0;
+                for (; c < nctx; c++) {
+                    const int64_t x = hits[(size_t)c][(size_t)row];
+                    if (n_hit + x >= h) break;
+                    n_hit += x;
+                }
+                if (c < nctx) {
+                    tab[(size_t)c][(size_t)row] = n_hit;
+                    stops[(size_t)c] = 1;
+                    count[(size_t)s] = h;
+                } else {
+                    count[(size_t)s] = n_hit;
+                    L[(size_t)s] = r1;
+                    if (r1 < K) live[(size_t)a] = 1;
+                }
+            }
+            // 3. the ctxs holding stopping rows find their replicates; every ctx clears its flags
+            rc = on_each_ctx(ctxs, nctx, fn, [&](int c) -> int {
+                plaac_ctx* ctx = ctxs[c];
+                const int64_t p0 = pa[(size_t)c], p1 = pa[(size_t)c + 1], wpr = (p1 - p0 + 31) / 32;
+                if (p1 == p0) return PLAAC_OK;
+                cudaStream_t st = ctx->slot[0].stream;
+                CU(ctx, cudaSetDevice(ctx->device));
+                if (stops[(size_t)c]) {
+                    int64_t* d_tab = (int64_t*)ctx->null_counts.p;
+                    CU(ctx, cudaMemcpyAsync(d_tab, tab[(size_t)c].data(), sizeof(int64_t) * (size_t)rows, cudaMemcpyHostToDevice, st));
+                    k_shuffle_stop<<<(unsigned)((rows + 7) / 8), 256, 0, st>>>((const uint32_t*)ctx->seq_flags.p,
+                                                                               (const int32_t*)ctx->seq_act[1].p, n, k, wpr, h, p0, p1,
+                                                                               K, d_tab, (int64_t*)ctx->seq_scored.p,
+                                                                               (int32_t*)ctx->seq_live.p);
+                    ctx->stats.kernel_launches += 1;
+                    at[(size_t)c].resize((size_t)rows);
+                    CU(ctx, cudaMemcpyAsync(at[(size_t)c].data(), ctx->seq_scored.p, sizeof(int64_t) * (size_t)rows,
+                                            cudaMemcpyDeviceToHost, st));
+                }
+                CU(ctx, cudaMemsetAsync(ctx->seq_flags.p, 0, sizeof(uint32_t) * (size_t)(rows * wpr), st));
+                CU(ctx, cudaStreamSynchronize(st));
+                return PLAAC_OK;
+            });
+            if (rc) return rc;
+            for (int c = 0; c < nctx; c++)
+                if (stops[(size_t)c])
+                    for (int64_t row = 0; row < rows; row++)
+                        if (tab[(size_t)c][(size_t)row] < h)
+                            L[(size_t)act[(size_t)(a0 + row / k)] * ek + (size_t)(row % k)] = at[(size_t)c][(size_t)row];
+        }
+        // the next round's list: the entries with a column below h, in list order
+        int64_t m = 0;
+        for (int64_t a = 0; a < nact; a++)
+            if (live[(size_t)a]) act[(size_t)m++] = act[(size_t)a];
+        nact = m;
+        r0 = r1;
+    }
+    memcpy(N.counts, count.data(), sizeof(int64_t) * count.size());
+    memcpy(scored, L.data(), sizeof(int64_t) * L.size());
+    return bad.finish(c0);
+} catch (...) {
+    return api_caught((ctxs && nctx > 0 ? ctxs[0] : nullptr), "plaac_score_shuffles_seq_multi");
 }
 
 }  // extern "C"

@@ -3,6 +3,9 @@
 // that brings its hits to h.  Per chunk of a round, on the slot's stream, the shuffle input form of shuffle.cuh runs with
 // k_shuffle_flags in place of k_shuffle_tally; once per round (slice of the list), on one stream:
 //   k_shuffle_stop -> launch_scan (active flags) -> k_shuffle_compact.
+// On several ctxs (plaac_score_shuffles_seq_multi, DESIGN.md section 15) each ctx flags its part of the round's span, and
+// k_shuffle_stop runs twice per slice: with h above any count, to count each row's hits in the part, then from the host's
+// base counts, to find the replicate of the h-th hit in the part where a row reaches it.  The list stays on the host.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
